@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark of the HardNet hot path on B200 (contract: see the task brief / DESIGN.md section 5).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of HardNet.forward over this rank's shard of synthetic 32x32 patches
 (BASELINE.json configs[2], bulk extraction: 4,194,304 patches over 8 GPUs = 524,288 patches per GPU per step,
@@ -24,6 +24,7 @@ import threading
 import time
 from pathlib import Path
 
+import numpy as np
 import torch
 
 REPO = Path(__file__).resolve().parent
@@ -39,6 +40,7 @@ MATCH_FLOP_PER_PAIR = 256
 MATCH_N = 65536
 GEN_CHUNK = 65536
 REF_SAMPLE = 4096                 # patches per step of the CPU reference arm (bounded sample of the same workload)
+DUMP_MAX_ROWS = 65536             # --dump-outputs: 32 MiB of 128-d fp32 descriptors at most
 
 
 def parse_args():
@@ -50,7 +52,26 @@ def parse_args():
     ap.add_argument("--patches-per-gpu", type=int, default=PATCHES_PER_GPU)
     ap.add_argument("--no-extras", action="store_true", help="skip the matching / NAS / config-1 sub-records")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the descriptors of the last step (rank 0) as DIR/descriptors.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(directory, **arrays):
+    """Write each array as DIR/<name>.npy in float32. An array of more than DUMP_MAX_ROWS rows is sampled: the same seeded,
+    sorted row indices on every run, so the dumps of two builds of the project compare row for row."""
+    d = Path(directory)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in arrays.items():
+        n = t.shape[0]
+        if n > DUMP_MAX_ROWS:
+            rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ROWS].sort().values
+            t = t[rows.to(t.device)]
+            print(f"[bench] {name}: {DUMP_MAX_ROWS} of {n} rows (seeded sample)", file=sys.stderr)
+        np.save(d / f"{name}.npy", t.detach().float().cpu().numpy())
 
 
 def workload_config(args, world):
@@ -73,7 +94,7 @@ def workload_config(args, world):
 # ---------------------------------------------------------------------------------------------------------
 def reference_forward_fn():
     """-> (callable x -> descriptors, kind, description). The unmodified reference class when its sources are available
-    (/root/reference in the build container, the staged copy oracle/_ref on the GPU box), else the oracle port."""
+    (a checkout at ../reference, or the copy build() staged under oracle/_ref), else the oracle port."""
     from oracle import hardnet_oracle, ref_loader, synth
     root = ref_loader.root()
     if root is not None:
@@ -122,8 +143,10 @@ def run_reference(args):
         fwd(x)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        fwd(x)
+        y = fwd(x)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, descriptors=y)
     value = REF_SAMPLE * args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -374,6 +397,8 @@ def run_b200(args):
     dom_ms, dom_n = model.profile_read()
     model.profile_enable(0)
     value = world * P * args.steps / (ms_total / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, descriptors=out)
 
     peaks = load_peaks()
     dom_flops = 2.0 * stage_macs[dom] * P * args.steps      # algorithmic FLOPs of that stage over the region

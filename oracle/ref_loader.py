@@ -1,10 +1,12 @@
 """Import the UNMODIFIED reference code — TEST / BENCH INFRASTRUCTURE, never imported by the product package.
 
-The reference tree exists only in the build container (/root/reference). `stage()` (run by __graft_entry__.build() there)
-copies the handful of reference files this hot path consists of, byte for byte, into oracle/_ref/ — a git-ignored directory
-that travels to the GPU box with the snapshot like the built .so does, so that `bench.py --impl reference` can time the
-reference's own classes on the box's host cores (cpu_baseline.kind = "reference"). Nothing under oracle/_ref/ is ever
-committed, edited or read by hardnetnas_b200/.
+The reference is a checkout of the original project (iamwangyabin/hardnetNas), which this repository does not contain;
+by default it is looked for next to the repository, at ../reference. `stage()` (run by __graft_entry__.build()) copies the
+handful of reference files this hot path consists of, byte for byte, into oracle/_ref/ — a git-ignored directory that
+travels with the tree like the built .so does — so that `bench.py --impl reference` and the cpu_baseline records time the
+reference's own classes (cpu_baseline.kind = "reference"); without it they time the oracle port. Where the checkout is
+missing or unreadable, staging is skipped. `python oracle/ref_loader.py <checkout>` stages from another location. Nothing
+under oracle/_ref/ is ever committed, edited or read by hardnetnas_b200/.
 
 The import recipes work around the reference's import-time side effects (SURVEY.md section 8c): hardnet/HardNet.py parses
 argv, sets CUDA_VISIBLE_DEVICES and creates data/logs/ in the cwd; LookUpTable() reads a path relative to hardnetNAS/.
@@ -18,7 +20,7 @@ import tempfile
 from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
-SOURCE = Path("/root/reference")
+REFERENCE = HERE.parent.parent / "reference"
 STAGED = HERE / "_ref"
 
 # relative paths of the files the hot path consists of (SURVEY.md section 8a)
@@ -33,23 +35,35 @@ FILES = [
 ]
 
 
-def stage() -> Path | None:
-    """Copy the reference files into oracle/_ref/ (no-op where /root/reference does not exist)."""
-    if not SOURCE.exists():
-        return STAGED if STAGED.exists() else None
-    for rel in FILES:
-        dst = STAGED / rel
-        dst.parent.mkdir(parents=True, exist_ok=True)
-        shutil.copyfile(SOURCE / rel, dst)
-    return STAGED
+def _complete(tree: Path) -> bool:
+    """Every file of FILES is under `tree`. A tree the user may not read counts as absent (Path.exists() raises
+    PermissionError there instead of returning False)."""
+    try:
+        return all((tree / rel).is_file() for rel in FILES)
+    except OSError:
+        return False
+
+
+def stage(source: Path | None = None, dest: Path = STAGED) -> Path | None:
+    """Copy the reference files of the checkout `source` (default REFERENCE) into `dest`. Where the source is missing or
+    unreadable nothing is copied. Returns `dest` if it holds a complete copy afterwards, else None."""
+    source = REFERENCE if source is None else Path(source)
+    if _complete(source):
+        try:
+            for rel in FILES:
+                dst = dest / rel
+                dst.parent.mkdir(parents=True, exist_ok=True)
+                shutil.copyfile(source / rel, dst)
+        except OSError as exc:
+            print(f"[ref_loader] staging the reference from {source} failed: {exc}", file=sys.stderr)
+    return dest if _complete(dest) else None
 
 
 def root() -> Path | None:
-    """Where the reference can be imported from: the real tree if present, else the staged copy, else None."""
-    if all((SOURCE / rel).exists() for rel in FILES):
-        return SOURCE
-    if all((STAGED / rel).exists() for rel in FILES):
-        return STAGED
+    """Where the reference can be imported from: the checkout if present, else the staged copy, else None."""
+    for tree in (REFERENCE, STAGED):
+        if _complete(tree):
+            return tree
     return None
 
 
@@ -57,7 +71,7 @@ def load_hardnet(ref: Path | None = None):
     """(HardNet module, Losses module, EvalMetrics module) of hardnet/."""
     ref = ref or root()
     if ref is None:
-        raise FileNotFoundError("reference sources are neither at /root/reference nor staged under oracle/_ref")
+        raise FileNotFoundError(f"reference sources are neither at {REFERENCE} nor staged under oracle/_ref")
     saved_argv, saved_cwd = sys.argv, os.getcwd()
     saved_env = os.environ.get("CUDA_VISIBLE_DEVICES")
     tmp = tempfile.mkdtemp(prefix="hn_ref_")
@@ -84,7 +98,7 @@ def load_fdl(ref: Path | None = None):
     """(eval_utils, math_utils) of FDLNet-master/utils."""
     ref = ref or root()
     if ref is None:
-        raise FileNotFoundError("reference sources are neither at /root/reference nor staged under oracle/_ref")
+        raise FileNotFoundError(f"reference sources are neither at {REFERENCE} nor staged under oracle/_ref")
     for m in [k for k in sys.modules if k == "utils" or k.startswith("utils.")]:
         del sys.modules[m]
     sys.path.insert(0, str(ref / "FDLNet-master"))
@@ -99,7 +113,7 @@ def load_nas(ref: Path | None = None):
     """(PRIMITIVES, ConvBNRelu, Flatten, LookUpTable instance) of hardnetNAS/."""
     ref = ref or root()
     if ref is None:
-        raise FileNotFoundError("reference sources are neither at /root/reference nor staged under oracle/_ref")
+        raise FileNotFoundError(f"reference sources are neither at {REFERENCE} nor staged under oracle/_ref")
     nas = ref / "hardnetNAS"
     cwd = os.getcwd()
     os.chdir(nas)   # LookUpTable() reads ./supernet_functions/lookup_table.txt
@@ -117,4 +131,6 @@ def load_nas(ref: Path | None = None):
 
 
 if __name__ == "__main__":
-    print(stage())
+    if len(sys.argv) > 2:
+        raise SystemExit("usage: python oracle/ref_loader.py [checkout of the original hardnetNas project, default ../reference]")
+    print(stage(Path(sys.argv[1]) if len(sys.argv) == 2 else None))

@@ -32,7 +32,11 @@ def test_mirror_regenerates_reference_weights_and_state_dict_keys(golden_dir):
     g = np.load(golden_dir / "neimask.npz")
     model = _model()
     w, m, v = _wmv(model)
-    assert np.array_equal(synth.weights_fingerprint(w), g["weights_fingerprint"])
+    # orthogonal_ runs a LAPACK QR whose last bits depend on the host's CPU and thread count: bit for bit the mirror draws
+    # what the reference recipe draws on this host, and the golden (another host) it matches to float32 rounding
+    recipe = synth.hardnet_weights_from_seed(0, 3)[0]
+    assert len(w) == len(recipe) and all(torch.equal(a, b) for a, b in zip(w, recipe))
+    np.testing.assert_allclose(synth.weights_fingerprint(w), g["weights_fingerprint"], rtol=1e-5, atol=1e-6)
     assert np.array_equal(synth.weights_fingerprint(list(m) + list(v)), g["bn_fingerprint"])
     keys = set(model.state_dict().keys())
     assert "features.18.weight" in keys and "features.19.running_mean" in keys and not any(k.startswith("features.20") for k in keys)

@@ -1,5 +1,6 @@
 import os, sys, json, torch
-sys.path.insert(0,'/root/repo')
+from pathlib import Path
+sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 from tools.nas_resident_check import build, timing, parity
 for env in ({}, {"HN_NAS_DW_F32":"1"}):
     for arch in ("wang2","wang3","wang4"):
