@@ -86,10 +86,8 @@ struct FfBias {
   float v[32];
 };
 
-// The kernel body as a device function: `blk` of `nblk` CTAs work on patches blk, blk + nblk, ... (the stand-alone kernel passes
-// blockIdx.x / gridDim.x; the co-scheduled front + conv3/conv4 launch of front_c34.cuh gives this role a sub-range of the grid).
-// ready != nullptr (HardNet variant only): each of the eight conv2 epilogue warps stamps ready[patch * 8 + its index] = 1 once
-// its part of the patch is in global memory (release at gpu scope) - the consumer role of the same launch polls these flags.
+// The kernel body as a device function, shared by front_fused_kernel and front_fused_clip_kernel: CTA `blk` of `nblk` works on
+// patches blk, blk + nblk, ...
 // CLIP (HardNet variant, TIn = float): there is no patch tensor - `in` is unused and patch clip->n0 + i is cropped around its
 // keypoint from the image stack (the reference's clip_patch, FDLNet-master/utils/image_utils.py:11-158, arithmetic in clip.cuh) by
 // the stage-1 epilogue warps, which otherwise wait for the stage-1 MMAs most of the time: they fill the raw ring two patches
@@ -99,11 +97,11 @@ __device__ __forceinline__ void front_fused_body(const TIn* __restrict__ in, uin
                                                  const float* __restrict__ bias1, const uint4* __restrict__ w2img, const FfBias& bias2,
                                                  int do_norm, int num_patches, int act_bf16, float norm_eps, const CUtensorMap& tm_out,
                                                  const float* __restrict__ dw_w, const float* __restrict__ dw_b, int dw_relu, int fdw_planar,
-                                                 const int blk, const int nblk, int* __restrict__ ready,
                                                  const ClipSrc* __restrict__ clip = nullptr) {
   static_assert(FDW == 0 || PW2, "the fused depthwise stage sits behind the pointwise variant");
   static_assert(!CLIP || (sizeof(TIn) == 4 && !PW2), "the cropped patch is fp32 in the raw ring; HardNet variant only");
   constexpr int NACT1 = FDW ? 1 : 2;   // stage-1 activation buffers
+  const int blk = static_cast<int>(blockIdx.x), nblk = static_cast<int>(gridDim.x);
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_addr = smem_u32(smem_raw);
   const uint32_t base = (raw_addr + 1023u) & ~1023u;
@@ -667,13 +665,6 @@ __device__ __forceinline__ void front_fused_body(const TIn* __restrict__ in, uin
         __syncwarp();
         if (lane == 0) mbar_arrive(c2_empty(a));
       }
-      if constexpr (!PW2) {
-        if (ready != nullptr) {   // this warp's four tiles of the patch are stored: publish them to the consumer role
-          __threadfence();
-          __syncwarp();
-          if (lane == 0) asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(ready + static_cast<size_t>(patch) * 8 + (warp - 4)), "r"(1) : "memory");
-        }
-      }
       if constexpr (FDW != 0) {
         // ---- stride-2 depthwise conv / max-pool of the patch-resident tile by the same eight warps: a thread owns 8
         // channels x one output column x a strip of 4 output rows (4 planes x 16 columns x 4 strips = 256 items) ----
@@ -794,7 +785,7 @@ front_fused_kernel(const TIn* __restrict__ in, uint16_t* __restrict__ out /*[n][
                    const float* __restrict__ dw_w = nullptr /*FDW 3 | 5: [k * k][32] folded*/, const float* __restrict__ dw_b = nullptr /*[32]*/,
                    int dw_relu = 0, int fdw_planar = 0 /*FDW output channel-planar [n][4][16][16][8] (the tail kernel's bulk-copy layout)*/) {
   front_fused_body<TIn, PW2, FDW>(in, out, w1, bias1, w2img, bias2, do_norm, num_patches, act_bf16, norm_eps, tm_out, dw_w, dw_b, dw_relu,
-                                  fdw_planar, static_cast<int>(blockIdx.x), static_cast<int>(gridDim.x), nullptr);
+                                  fdw_planar);
 }
 
 // The HardNet front kernel fed by clip_patch on the fly (hn_forward_clip): same stages, patches cropped inside the kernel.
@@ -803,7 +794,7 @@ front_fused_clip_kernel(const __grid_constant__ ClipSrc clip, uint16_t* __restri
                         const float* __restrict__ bias1, const uint4* __restrict__ w2img, const __grid_constant__ FfBias bias2,
                         int num_patches, int act_bf16, float norm_eps, const __grid_constant__ CUtensorMap tm_out) {
   front_fused_body<float, false, 0, true>(nullptr, out, w1, bias1, w2img, bias2, 1, num_patches, act_bf16, norm_eps, tm_out, nullptr,
-                                          nullptr, 0, 0, static_cast<int>(blockIdx.x), static_cast<int>(gridDim.x), nullptr, &clip);
+                                          nullptr, 0, 0, &clip);
 }
 
 }  // namespace hn

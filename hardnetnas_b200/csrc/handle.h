@@ -7,7 +7,6 @@
 
 #include "../../include/hardnet_b200.h"
 #include "tc_conv.cuh"
-#include "tc_conv34.cuh"
 
 namespace hn {
 // internal value of `in_dtype` next to HN_F32 / HN_U8: the input pointer is a HOST ClipSrc (clip.cuh) and the patches are cropped
@@ -37,28 +36,19 @@ struct HnEnv {
   bool nas_front = true;      // HN_NAS_FRONT=0: stem and first pointwise conv as separate kernels
   bool nas_dw_smem = true;    // HN_NAS_DW_SMEM=0: register-strip depthwise / max-pool kernels
   bool nas_dw_sh8 = true;     // HN_NAS_DW_SH8=0: 4-row strips for every depthwise shape
-  int nas_front_chunk = 0;    // HN_NAS_FRONT_CHUNK: patches per front-kernel + first-reader sub-pass (0 = whole pass); keeps the
-                              // 64 KB/patch stem output inside L2
   bool nas_front_dw = true;   // HN_NAS_FRONT_DW=0: the stride-2 depthwise conv / max-pool behind the stem as its own kernel
   bool nas_dw_f32 = false;    // HN_NAS_DW_F32=1: fp32 depthwise arithmetic also for fp16 activations (default: packed half2)
-  bool nas_resident = false;  // HN_NAS_RESIDENT=1: runs of NAS ops as patch-resident segment kernels (nas_resident.cuh). Off by
-                              // default: measured slower than one kernel per op (DESIGN.md section 4, profiles/r2_nas_resident_*)
-  int nas_minb = 0;           // HN_NAS_MINB: CTAs per SM of the segment kernel (0 = choose)
-  int nas_cut_ratio = 4;      // HN_NAS_CUT_RATIO: start a new segment at a block boundary whose tensor is <= 1/ratio of the segment input
-  int nas_gmax = 8;           // HN_NAS_GMAX: cap on patches per group
   bool nas_tail = true;       // HN_NAS_TAIL=0: no warpgroup-per-patch tail kernel (nas_tail.cuh) behind the fused front stage
   bool nas_fold = true;       // HN_NAS_FOLD=0: the tail runs the packed ops one by one (no folding of linear 1x1 convs into their consumers)
   int nas_tail_cut = 2;       // HN_NAS_TAIL_CUT: start a new tail launch at a block boundary whose tensor is <= 1/cut of the launch's
                               // input (smaller maps -> smaller buffers -> more warpgroups per SM); 0 = one launch for the whole tail
   int nas_tail_minops = 4;    // HN_NAS_TAIL_MINOPS: ... and only if at least this many ops remain behind the cut
   int nas_tail_wg = 6;        // HN_NAS_TAIL_WG: cap on warpgroups (patches in flight) per CTA
-  char nas_split[128] = {0};  // HN_NAS_SPLIT="i,j,...": explicit op indices that start a new segment (overrides the heuristic)
 };
 
 struct hn_handle {
   HnEnv env;
   int chunk = 0;            // patches per conv-stack pass
-  int front_chunk = 0;      // patches per front-kernel + conv3 sub-pass (keeps the conv2 output L2 resident)
   long long head_rows = 0;  // capacity of the L6 output buffer (patches)
   int sm_count = 0;
   bool packed = false;
@@ -74,18 +64,11 @@ struct hn_handle {
   float bias2_host[32] = {0};   // conv2's folded BN shift on the host: passed to the fused front kernel by value
   float* head_partial = nullptr;  // split-K partial sums of the head GEMM at small batches ([#SM][128][128] fp32)
   float2* stats = nullptr;                                             // per-patch (mean, 1/std), chunk entries
-  hn::TcParams conv_params[5];
-  hn::TcParams pair_params[5];   // same layers for the CTA-pair kernels (tc_conv_pair.cuh)
-  unsigned pair_mask = 0;        // bit li: layer li runs on CTA pairs
+  hn::TcParams conv_params[5];   // 3x3 layers on the CTA-pair kernel (tc_conv_pair.cuh); [0] unused (conv2 is in the front kernel)
   hn::TcParams head_params;
-  int fuse34 = 0;                // HN_FUSE34: conv3 + conv4 in one kernel (tc_conv34.cuh): 0 = off, 1 / 2 = shifted-copies kernel,
-                                 // 3 = stacked-N kernel (default); the deeper layers then read / write the other ping-pong buffer
-  int fuse34_sched = 2;          // HN_FUSE34_SCHED (mode 3: bit 0 = fp16-pair shuffles, bit 1 = two TMA producer warps)
+  bool fuse34 = true;            // conv3 + conv4 in one kernel (tc_conv34.cuh); HN_FUSE34=0: two kernels, the reference of the
+                                 // fused one. The deeper layers then read / write the other ping-pong buffer (act_buf)
   hn::Conv34Params c34;
-  int cosched = 0;               // HN_COSCHED=1: front kernel and fused conv3 + conv4 kernel as the two roles of ONE launch (front_c34.cuh):
-                                 // the conv2 output is consumed out of L2 a few microseconds after it was written
-  int cosched_nf = 72;           // HN_COSCHED_NF: CTAs of the front role (even)
-  int* c34_ready = nullptr;      // [chunk][8] producer -> consumer flags of that launch (all zero between launches)
   // optional per-stage CUDA-event timing (stage 0 = L1, 1..5 = 3x3 convs, 6 = head)
   unsigned profile_mask = 0;
   std::vector<cudaEvent_t> ev[7];

@@ -1,7 +1,7 @@
 // HardNet.forward (hardnet/HardNet.py:312-315) behind the C ABI: weight packing (BatchNorm fold),
 // static TMA descriptors over handle-owned activation scratch, and the per-chunk launch sequence
-//   fused front (input_norm + conv1 + conv2, front_fused.cuh) -> conv3..conv6 (tcgen05 implicit GEMM over
-//   channel-planar activations) -> head GEMM + L2Norm.
+//   fused front (input_norm + conv1 + conv2, front_fused.cuh) -> fused conv3 + conv4 (tc_conv34.cuh) -> conv5, conv6
+//   (tcgen05 implicit GEMM over channel-planar activations, tc_conv_pair.cuh) -> head GEMM + L2Norm.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
@@ -17,7 +17,6 @@
 #include "tc_conv.cuh"
 #include "tc_conv_pair.cuh"
 #include "tc_conv34.cuh"
-#include "front_c34.cuh"
 
 namespace hn {
 
@@ -59,23 +58,6 @@ struct StageTimer {
   }
 };
 
-template <int CIN, int COUT, int HOUT, int STRIDE, int G, int STAGES, bool WRES, int MINB, bool ROWSHIFT, bool OUT_PARITY,
-          int TILES = 1, int KCB_ = 0>
-static int launch_conv_cfg(const TcParams& p, int sm_count, cudaStream_t stream) {
-  using C = ConvCfg<CIN, COUT, HOUT, STRIDE, G, STAGES, WRES, ROWSHIFT, TILES, KCB_>;
-  auto kern = conv3x3_kernel<CIN, COUT, HOUT, STRIDE, G, STAGES, WRES, MINB, ROWSHIFT, OUT_PARITY, TILES, KCB_>;
-  static DeviceOnce attr_once;  // per instantiation
-  if (attr_once.first_time()) {
-    HN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(C::SMEM)));
-  }
-  if (p.num_tiles <= 0) return HN_OK;
-  const int grid = std::min((p.num_tiles + TILES - 1) / TILES, sm_count * MINB);
-  kern<<<grid, kTcThreads, C::SMEM, stream>>>(p);
-  HN_CUDA(cudaGetLastError());
-  count_launch();
-  return HN_OK;
-}
-
 template <int CIN, int COUT, int HOUT, int STRIDE, int STAGES, bool ROWSHIFT, bool OUT_PARITY, int KCB_ = 0>
 static int launch_conv_pair_cfg(const TcParams& p, int sm_count, cudaStream_t stream) {
   using C = PairCfg<CIN, COUT, HOUT, STRIDE, STAGES, ROWSHIFT, KCB_>;
@@ -93,77 +75,31 @@ static int launch_conv_pair_cfg(const TcParams& p, int sm_count, cudaStream_t st
   return HN_OK;
 }
 
-// conv2 (li = 0) lives in the fused front kernel. OUT_PARITY: the consumer is a stride-2 conv and wants parity sub-planes.
-//                         CIN COUT HOUT STRIDE  G STAGES WRES  CTAs/SM ROWSHIFT OUT_PARITY
-#define HN_CONV_L3 launch_conv_cfg<32, 64, 16, 2, 1, 9, true, 2, false, false>
-#define HN_CONV_L4 launch_conv_cfg<64, 64, 16, 1, 1, 7, true, 1, true, true>
-//   conv5: weights streamed so that TILES = 2 doubles the activation bytes in flight per stage
-//   conv6: ROWSHIFT over two-patch tiles + TILES = 2: 132 KB / patch through the SM's L2 port instead of 288 KB
-#define HN_CONV_L5 launch_conv_cfg<64, 128, 8, 2, 1, 4, false, 1, false, false, 2>
-#define HN_CONV_L6 launch_conv_cfg<128, 128, 8, 1, 1, 4, false, 1, true, false, 2, 64>
-// CTA-pair (cta_group::2) variants: weights resident (half per CTA), M = 256 per MMA
-//                                   CIN COUT HOUT STRIDE STAGES ROWSHIFT OUT_PARITY KCB
-#define HN_PAIR_L3 launch_conv_pair_cfg<32, 64, 16, 2, 9, false, false>
-#define HN_PAIR_L4 launch_conv_pair_cfg<64, 64, 16, 1, 9, true, true>
-#define HN_PAIR_L5 launch_conv_pair_cfg<64, 128, 8, 2, 9, false, false>
-#define HN_PAIR_L6 launch_conv_pair_cfg<128, 128, 8, 1, 4, true, false>
-static const bool kRowShift[5] = {true, false, true, false, true};
-static const bool kPairRowShift[5] = {false, false, true, false, true};
-static const int kPairKcb[5] = {64, 64, 128, 128, 128};
-static const unsigned kDefaultPairMask = 0x1c;   // conv4, conv5, conv6 (conv3 is faster with two independent CTAs per SM)
-static const int kDefaultFuse34 = 3;
-static const int kDefaultCosched = 0;
-static const int kKcb[5] = {64, 64, 128, 128, 64};   // bytes of one pixel's channel chunk per k-block (ConvCfg::KCB)
-
-static int launch_conv_pair(int li, const TcParams& p, int sm_count, cudaStream_t s) {
-  switch (li) {
-    case 1: return HN_PAIR_L3(p, sm_count, s);
-    case 2: return HN_PAIR_L4(p, sm_count, s);
-    case 3: return HN_PAIR_L5(p, sm_count, s);
-    case 4: return HN_PAIR_L6(p, sm_count, s);
-  }
-  return HN_ERR_INVALID;
-}
+// conv2 (li = 0) lives in the fused front kernel. Every 3x3 layer runs on CTA pairs (cta_group::2): weights resident (half per
+// CTA), M = 256 per MMA. OUT_PARITY: the consumer is a stride-2 conv and wants parity sub-planes.
+static const bool kRowShift[5] = {false, false, true, false, true};
+static const int kKcb[5] = {64, 64, 128, 128, 128};   // bytes of one pixel's channel chunk per k-block (PairCfg::KCB)
 
 static int launch_conv(int li, const TcParams& p, int sm_count, cudaStream_t s) {
-  switch (li) {
-    case 1: return HN_CONV_L3(p, sm_count, s);
-    case 2: return HN_CONV_L4(p, sm_count, s);
-    case 3: return HN_CONV_L5(p, sm_count, s);
-    case 4: return HN_CONV_L6(p, sm_count, s);
+  switch (li) {   //                          CIN COUT HOUT STRIDE STAGES ROWSHIFT OUT_PARITY
+    case 1: return launch_conv_pair_cfg<32, 64, 16, 2, 9, false, false>(p, sm_count, s);
+    case 2: return launch_conv_pair_cfg<64, 64, 16, 1, 9, true, true>(p, sm_count, s);
+    case 3: return launch_conv_pair_cfg<64, 128, 8, 2, 9, false, false>(p, sm_count, s);
+    case 4: return launch_conv_pair_cfg<128, 128, 8, 1, 4, true, false>(p, sm_count, s);
   }
   return HN_ERR_INVALID;
 }
 
 // conv3 + conv4 in one kernel (tc_conv34.cuh): conv2 output in act[1] -> conv4 output in `out`.
-template <bool SIX, int SCHED>
-static int launch_conv34_cfg(const Conv34Params& p, int sm_count, cudaStream_t stream) {
-  using C = C34Cfg<SIX>;
-  auto kern = conv34_pair_kernel<SIX, SCHED>;
-  static DeviceOnce attr_once;  // per instantiation
+static int launch_conv34(const Conv34Params& p, int sm_count, cudaStream_t stream) {
+  static DeviceOnce attr_once;
   if (attr_once.first_time()) {
-    HN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(C::SMEM)));
+    HN_CUDA(cudaFuncSetAttribute(conv34_stack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(C34SCfg::SMEM)));
   }
   if (p.n_patches <= 0) return HN_OK;
   const int groups = (p.n_patches + 1) / 2;
   const int grid = 2 * std::min(groups, sm_count / 2);   // whole CTA pairs (__cluster_dims__(2, 1, 1))
-  kern<<<grid, kC34Threads, C::SMEM, stream>>>(p);
-  HN_CUDA(cudaGetLastError());
-  count_launch();
-  return HN_OK;
-}
-
-template <int SHFL16, int NPROD>
-static int launch_conv34_stack(const Conv34Params& p, int sm_count, cudaStream_t stream) {
-  auto kern = conv34_stack_kernel<SHFL16, NPROD>;
-  static DeviceOnce attr_once;  // per instantiation
-  if (attr_once.first_time()) {
-    HN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(C34SCfg::SMEM)));
-  }
-  if (p.n_patches <= 0) return HN_OK;
-  const int groups = (p.n_patches + 1) / 2;
-  const int grid = 2 * std::min(groups, sm_count / 2);   // whole CTA pairs (__cluster_dims__(2, 1, 1))
-  kern<<<grid, kC34SThreads, C34SCfg::SMEM, stream>>>(p);
+  conv34_stack_kernel<<<grid, kC34SThreads, C34SCfg::SMEM, stream>>>(p);
   HN_CUDA(cudaGetLastError());
   count_launch();
   return HN_OK;
@@ -174,8 +110,7 @@ static int build_conv34_params(hn_handle* h) {
   memset(&p, 0, sizeof(p));
   if (!h->fuse34) return HN_OK;
   const uint16_t* in = h->act[1];   // conv2 output: parity sub-planes [patch][4 planes][ypar][xpar][16][16][8]
-  const uint32_t rows = h->fuse34 >= 2 ? 9u : 8u;
-  const uint32_t box[4] = {16 * 8, rows, 1, 4};
+  const uint32_t box[4] = {16 * 8, 9, 1, 4};
   for (int ypar = 0; ypar < 2; ++ypar)
     for (int xpar = 0; xpar < 2; ++xpar) {
       const uint64_t dims[4] = {16 * 8, 16, static_cast<uint64_t>(h->chunk), 4};
@@ -203,48 +138,7 @@ static int run_conv34(hn_handle* h, int n, void* out, cudaStream_t s) {
   p.act_bf16 = h->act_bf16;
   p.out = out;
   StageTimer timer(h, 2, s);   // reported as the conv3 stage; the conv4 stage then has no launches of its own
-  if (h->fuse34 == 3) {   // HN_FUSE34_SCHED: bit 0 = fp16-pair shuffles, bit 1 = two TMA producer warps
-    switch (h->fuse34_sched & 3) {
-      case 0: return launch_conv34_stack<0, 1>(p, h->sm_count, s);
-      case 1: return launch_conv34_stack<1, 1>(p, h->sm_count, s);
-      case 2: return launch_conv34_stack<0, 2>(p, h->sm_count, s);
-      default: return launch_conv34_stack<1, 2>(p, h->sm_count, s);
-    }
-  }
-  if (h->fuse34 == 1) return launch_conv34_cfg<false, 0>(p, h->sm_count, s);
-  return launch_conv34_cfg<true, 6>(p, h->sm_count, s);
-}
-
-// Front kernel + fused conv3 + conv4 kernel as the two roles of one launch (front_c34.cuh): patches -> conv4 output in `out`.
-static int run_front_c34(hn_handle* h, const void* patches, int in_dtype, int n, void* out, cudaStream_t s) {
-  static DeviceOnce attr_once;
-  if (attr_once.first_time()) {
-    HN_CUDA(cudaFuncSetAttribute(front_c34_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kFrontC34Smem)));
-    HN_CUDA(cudaFuncSetAttribute(front_c34_kernel<uint8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kFrontC34Smem)));
-  }
-  FrontC34Params P;
-  P.in = patches;
-  P.conv2_out = h->act[1];
-  P.w1 = h->w1;
-  P.bias1 = h->bias;
-  P.w2img = reinterpret_cast<const uint4*>(h->w2img);
-  memcpy(P.bias2.v, h->bias2_host, sizeof(P.bias2.v));
-  P.norm_eps = h->norm_eps;
-  P.n_patches = n;
-  P.act_bf16 = h->act_bf16;
-  const int grid = h->sm_count & ~1;
-  P.nf = std::min(std::max(2, h->cosched_nf & ~1), grid - 2);
-  P.ready = h->c34_ready;
-  P.c34 = h->c34;
-  P.c34.n_patches = n;
-  P.c34.act_bf16 = h->act_bf16;
-  P.c34.out = out;
-  StageTimer timer(h, 1, s);   // reported as the front stage; the conv3 / conv4 stages then have no launches of their own
-  if (in_dtype == HN_F32) front_c34_kernel<float><<<grid, kFfThreads, kFrontC34Smem, s>>>(P);
-  else front_c34_kernel<uint8_t><<<grid, kFfThreads, kFrontC34Smem, s>>>(P);
-  HN_CUDA(cudaGetLastError());
-  count_launch();
-  return HN_OK;
+  return launch_conv34(p, h->sm_count, s);
 }
 
 // Stage 1 (input_norm + conv 1->32 + BN + ReLU) on the tensor core; do_norm = 0 gives the NAS stem.
@@ -388,8 +282,7 @@ int launch_head(const TcParams& p_in, int sm_count, cudaStream_t stream) {
   }
   p.k_splits = splits;
   const int items = p.num_tiles * splits;
-  static const bool two_tiles = [] { const char* e = getenv("HN_HEAD_TILES"); return e ? atoi(e) == 2 : true; }();   // read once
-  if (splits == 1 && two_tiles && p.num_tiles > sm_count) {
+  if (splits == 1 && p.num_tiles > sm_count) {
     // bulk batches: two row tiles per streamed weight block (the kernel is bound by the L2 -> SM traffic)
     gemm_l2norm_kernel<kHeadN, 2><<<std::min((p.num_tiles + 1) / 2, sm_count), kTcThreads, kHeadSmem, stream>>>(p);
     HN_CUDA(cudaGetLastError());
@@ -418,20 +311,25 @@ static uint16_t to16(float v, int bf16) {
   return *reinterpret_cast<uint16_t*>(&h);
 }
 
+// The ping-pong buffer that holds the output of `stage` (1 = stage 1, 2 = conv2 ... 5 = conv5; conv6 writes l6). The front
+// kernel writes act[1] and the stages alternate. With conv3 + conv4 fused the conv4 output lands in act[0] (the fused kernel
+// cannot write the buffer it reads), so conv4 and conv5 use the opposite buffers.
+static uint16_t* act_buf(const hn_handle* h, int stage) {
+  return h->act[((stage - 1) & 1) ^ ((h->fuse34 && stage >= 4) ? 1 : 0)];
+}
+
 // Static descriptors of one 3x3 layer over the handle's buffers; only the tile counts change per call.
-// kcb = bytes of one pixel's channel chunk per k-block; half_b: weight box of C_out / 2 rows (CTA-pair kernels).
-static int build_conv_params(hn_handle* h, int li, int kcb, bool rowshift, bool half_b, TcParams& p) {
+// kcb = bytes of one pixel's channel chunk per k-block; the weight box covers the C_out / 2 rows of one CTA of the pair.
+static int build_conv_params(hn_handle* h, int li, int kcb, bool rowshift, TcParams& p) {
   const ConvLayer& L = kConv[li];
   memset(&p, 0, sizeof(p));
   const int kc = kcb / 2;
-  // the front kernel writes act[1]; layers alternate. With conv3 + conv4 fused the conv4 output lands in act[0] (the fused
-  // kernel cannot write the buffer it reads), so conv5 / conv6 use the opposite buffers.
-  const uint16_t* in = h->act[(li & 1) ^ ((h->fuse34 && li >= 3) ? 1 : 0)];
+  const uint16_t* in = act_buf(h, li + 1);   // the output of the layer before (stage li + 1)
   const int pix_out = L.hout * L.hout;
   const int rows_per_tile = pix_out >= kTileM ? kTileM / L.hout : L.hout;
   const int patches_per_tile = pix_out >= kTileM ? 1 : kTileM / pix_out;
   // channel-planar input [patch][plane][y][x][8] seen as (x * 8, y, patch, plane); box = whole rows of NPL planes.
-  // ROWSHIFT layers order the box (x * 8, patch, y, plane) instead (see ConvCfg).
+  // ROWSHIFT layers order the box (x * 8, patch, y, plane) instead (see PairCfg).
   const uint64_t C = L.cin, W = L.hin, H = L.hin;
   if (L.stride == 1 && rowshift) {
     const uint32_t box[4] = {static_cast<uint32_t>(L.hout * 8), static_cast<uint32_t>(patches_per_tile),
@@ -461,7 +359,7 @@ static int build_conv_params(hn_handle* h, int li, int kcb, bool rowshift, bool 
     const uint64_t K = 9ull * L.cin;
     const uint64_t dims[2] = {K, static_cast<uint64_t>(L.cout)};
     const uint64_t str[1] = {K * 2};
-    const uint32_t wbox[2] = {static_cast<uint32_t>(kc), static_cast<uint32_t>(half_b ? L.cout / 2 : L.cout)};
+    const uint32_t wbox[2] = {static_cast<uint32_t>(kc), static_cast<uint32_t>(L.cout / 2)};
     HN_TRY(make_tmap_16bit(&p.tmB, h->wconv[li], 2, dims, str, wbox, kcb));
   }
   p.bias = h->bias + 128 * (li + 1);
@@ -470,8 +368,7 @@ static int build_conv_params(hn_handle* h, int li, int kcb, bool rowshift, bool 
 
 static int build_params(hn_handle* h) {
   for (int li = 1; li < 5; ++li) {   // conv2 (li = 0) is part of the fused front kernel
-    HN_TRY(build_conv_params(h, li, kKcb[li], kRowShift[li], false, h->conv_params[li]));
-    HN_TRY(build_conv_params(h, li, kPairKcb[li], kPairRowShift[li], true, h->pair_params[li]));
+    HN_TRY(build_conv_params(h, li, kKcb[li], kRowShift[li], h->conv_params[li]));
   }
   {
     TcParams& p = h->head_params;
@@ -491,18 +388,16 @@ static int build_params(hn_handle* h) {
   return HN_OK;
 }
 
-// Runs the conv stack up to `last_layer` for `n` patches (n <= chunk); the conv6 output lands in l6 + l6_row * 8192.
 static int run_one_conv(hn_handle* h, int li, int n, void* out, cudaStream_t s) {
   const ConvLayer& L = kConv[li];
-  const bool pair = (h->pair_mask >> li) & 1;
-  TcParams p = pair ? h->pair_params[li] : h->conv_params[li];
+  TcParams p = h->conv_params[li];
   const long long pix_out = static_cast<long long>(L.hout) * L.hout;
   p.total_rows = pix_out * n;
   p.num_tiles = static_cast<int>((p.total_rows + kTileM - 1) / kTileM);
   p.act_bf16 = h->act_bf16;
   p.out = out;
   StageTimer timer(h, li + 1, s);
-  return pair ? launch_conv_pair(li, p, h->sm_count, s) : launch_conv(li, p, h->sm_count, s);
+  return launch_conv(li, p, h->sm_count, s);
 }
 
 // The input `off` patches further on: a pointer into the patch tensor, or (kInClip) a copy of the host ClipSrc whose first
@@ -516,6 +411,7 @@ static const void* input_at(const void* patches, int in_dtype, long long off, Cl
   return static_cast<const char*>(patches) + static_cast<size_t>(off) * 1024 * (in_dtype == HN_F32 ? 4 : 1);
 }
 
+// Runs the conv stack up to `last_layer` for `n` patches (n <= chunk); the conv6 output lands in l6 + l6_row * 8192.
 static int run_conv_stack(hn_handle* h, const void* patches, int in_dtype, int n, long long l6_row, int last_layer,
                           cudaStream_t s) {
   if (last_layer < 2) {
@@ -524,34 +420,19 @@ static int run_conv_stack(hn_handle* h, const void* patches, int in_dtype, int n
       return HN_ERR_INVALID;
     }
     StageTimer timer(h, 0, s);  // stage 1 alone (activation dump only), NHWC
-    return launch_l1(patches, in_dtype, h->act[0], h->w1, h->bias, h->stats, n, h->act_bf16, h->sm_count, s, h->norm_eps);
+    return launch_l1(patches, in_dtype, act_buf(h, 1), h->w1, h->bias, h->stats, n, h->act_bf16, h->sm_count, s, h->norm_eps);
   }
-  // The 64 KB/patch conv2 output is the largest tensor of the stack. The front kernel and conv3 run in sub-passes of
-  // `front_chunk` patches over the SAME head of act[1], so it is produced and consumed inside the 126 MB L2 instead of
-  // making an HBM round trip; conv3 writes into the full-size act[0] and the deeper stages run once over the whole pass.
-  const int front = last_layer >= 3 ? std::min(h->front_chunk, n) : n;
-  const bool fuse = h->fuse34 != 0 && last_layer >= 4;   // a dump of conv3's own output runs the layer on its own
-  for (int off = 0; off < n; off += front) {
-    const int m = std::min(front, n - off);
-    ClipSrc clip_at;
-    const void* src = input_at(patches, in_dtype, off, &clip_at);
-    // both roles need enough patches to fill their share of the SMs; small batches keep the two launches (every SM on each stage)
-    if (fuse && h->fuse34 == 3 && h->cosched && m >= 32 * h->sm_count && in_dtype != kInClip) {
-      HN_TRY(run_front_c34(h, src, in_dtype, m, h->act[0] + static_cast<size_t>(off) * 16 * 16 * 64, s));
-      continue;
-    }
-    {
-      StageTimer timer(h, 1, s);  // stage 1 + conv2 (the stage-1 activation never reaches global memory)
-      HN_TRY(launch_front_fused(h, src, in_dtype, h->act[1], m, s));
-    }
-    if (fuse) HN_TRY(run_conv34(h, m, h->act[0] + static_cast<size_t>(off) * 16 * 16 * 64, s));
-    else if (last_layer >= 3) HN_TRY(run_one_conv(h, 1, m, h->act[0] + static_cast<size_t>(off) * 16 * 16 * 64, s));
+  {
+    StageTimer timer(h, 1, s);  // stage 1 + conv2 (the stage-1 activation never reaches global memory)
+    HN_TRY(launch_front_fused(h, patches, in_dtype, act_buf(h, 2), n, s));
   }
+  const bool fuse = h->fuse34 && last_layer >= 4;   // a dump of conv3's own output runs the layer on its own
+  if (fuse) HN_TRY(run_conv34(h, n, act_buf(h, 4), s));
+  else if (last_layer >= 3) HN_TRY(run_one_conv(h, 1, n, act_buf(h, 3), s));
   for (int li = fuse ? 3 : 2; li < 5 && li + 2 <= last_layer; ++li)
-    HN_TRY(run_one_conv(h, li, n, (li == 4) ? static_cast<void*>(h->l6 + l6_row * kHeadK) : static_cast<void*>(h->act[((li + 1) & 1) ^ (fuse ? 1 : 0)]), s));
+    HN_TRY(run_one_conv(h, li, n, (li == 4) ? static_cast<void*>(h->l6 + l6_row * kHeadK) : static_cast<void*>(act_buf(h, li + 2)), s));
   return HN_OK;
 }
-
 
 }  // namespace hn
 
@@ -585,35 +466,13 @@ extern "C" int hn_create(hn_handle** out, int chunk_patches, long long head_rows
     h->env.nas_dw_sh8 = flag("HN_NAS_DW_SH8", true);
     h->env.nas_dw_f32 = flag("HN_NAS_DW_F32", false);
     h->env.nas_front_dw = flag("HN_NAS_FRONT_DW", true);
-    h->env.nas_front_chunk = std::max(0, num("HN_NAS_FRONT_CHUNK", 0)) & ~1;
-    h->env.nas_resident = flag("HN_NAS_RESIDENT", false);
-    h->env.nas_minb = num("HN_NAS_MINB", 0);
-    h->env.nas_cut_ratio = std::max(1, num("HN_NAS_CUT_RATIO", 4));
-    h->env.nas_gmax = std::max(1, num("HN_NAS_GMAX", 8));
     h->env.nas_tail = flag("HN_NAS_TAIL", true);
     h->env.nas_fold = flag("HN_NAS_FOLD", true);
     h->env.nas_tail_cut = std::max(0, num("HN_NAS_TAIL_CUT", 2));
     h->env.nas_tail_minops = std::max(1, num("HN_NAS_TAIL_MINOPS", 4));
     h->env.nas_tail_wg = std::min(6, std::max(1, num("HN_NAS_TAIL_WG", 6)));
-    if (const char* e = getenv("HN_NAS_SPLIT")) snprintf(h->env.nas_split, sizeof(h->env.nas_split), "%s", e);
-  }
-  {
-    const char* e = getenv("HN_FRONT_CHUNK");   // patches per front-kernel + conv3 sub-pass
-    h->front_chunk = e ? std::max(2, atoi(e)) : chunk_patches;
-  }
-  {
-    // conv3 + conv4 in one kernel (tc_conv34.cuh): 0 = off, 1 = three x-shifted copies of the activation, a load per tap,
-    // 2 = the same with a load per (row parity, kx), 3 = conv4's kx taps stacked on N (default)
-    const char* e = getenv("HN_FUSE34");
-    h->fuse34 = e ? std::min(3, std::max(0, atoi(e))) : kDefaultFuse34;
-    h->cosched = getenv("HN_COSCHED") ? atoi(getenv("HN_COSCHED")) : kDefaultCosched;
-    h->cosched_nf = getenv("HN_COSCHED_NF") ? atoi(getenv("HN_COSCHED_NF")) : 72;
-    const char* e2 = getenv("HN_FUSE34_SCHED");   // mode 3: bit 0 = fp16-pair shuffles, bit 1 = two TMA producer warps
-    h->fuse34_sched = e2 ? atoi(e2) : 2;
-  }
-  {
-    const char* e = getenv("HN_PAIR_MASK");   // bit li: run 3x3 layer li (1 = conv3 .. 4 = conv6) on CTA pairs
-    h->pair_mask = e ? static_cast<unsigned>(strtoul(e, nullptr, 0)) : kDefaultPairMask;
+    // HN_FUSE34=0: conv3 and conv4 as two kernels (the reference the fused kernel is tested against)
+    h->fuse34 = flag("HN_FUSE34", true);
   }
   const size_t act_elems = static_cast<size_t>(chunk_patches) * 32 * 32 * 32;
   auto fail = [&](int code) { hn_destroy(h); return code; };
@@ -639,8 +498,6 @@ extern "C" int hn_create(hn_handle** out, int chunk_patches, long long head_rows
   HN_CUDA_H(cudaMalloc(&h->w2img, kFfW2));
   HN_CUDA_H(cudaMalloc(&h->bias, 7 * 128 * sizeof(float)));
   HN_CUDA_H(cudaMalloc(&h->stats, static_cast<size_t>(chunk_patches) * sizeof(float2)));
-  HN_CUDA_H(cudaMalloc(&h->c34_ready, static_cast<size_t>(chunk_patches) * 8 * sizeof(int)));
-  HN_CUDA_H(cudaMemset(h->c34_ready, 0, static_cast<size_t>(chunk_patches) * 8 * sizeof(int)));
   // split-K partials of the head at small batches: tiles x splits <= #SM work items of 128 x 128 fp32 each
   HN_CUDA_H(cudaMalloc(&h->head_partial, static_cast<size_t>(h->sm_count) * kTileM * kHeadN * sizeof(float)));
 #undef HN_CUDA_H
@@ -661,7 +518,6 @@ extern "C" int hn_destroy(hn_handle* h) {
   cudaFree(h->w2img);
   cudaFree(h->bias);
   cudaFree(h->stats);
-  cudaFree(h->c34_ready);
   cudaFree(h->head_partial);
   for (auto& v : h->ev)
     for (cudaEvent_t e : v) cudaEventDestroy(e);
@@ -744,10 +600,8 @@ extern "C" int hn_pack_hardnet(hn_handle* h, const float* const w[7], const floa
   memcpy(h->bias2_host, bias.data() + 128, sizeof(h->bias2_host));
   memcpy(h->c34.bias3, bias.data() + 128 * 2, sizeof(h->c34.bias3));
   memcpy(h->c34.bias4, bias.data() + 128 * 3, sizeof(h->c34.bias4));
-  for (int li = 0; li < 5; ++li) {   // by-value copies for the conv kernels' epilogues
+  for (int li = 0; li < 5; ++li)   // by-value copies for the conv kernels' epilogues
     memcpy(h->conv_params[li].bias_v, bias.data() + 128 * (li + 1), sizeof(h->conv_params[li].bias_v));
-    memcpy(h->pair_params[li].bias_v, bias.data() + 128 * (li + 1), sizeof(h->pair_params[li].bias_v));
-  }
   // ... and every copy (small pageable H2D copies return once staged, before their DMA lands) must be complete before a
   // forward on another stream can read the new weights.
   HN_CUDA(cudaDeviceSynchronize());
@@ -839,7 +693,7 @@ extern "C" int hn_forward_dump(hn_handle* h, const void* patches, int in_dtype, 
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   HN_TRY(run_conv_stack(h, patches, in_dtype, static_cast<int>(B), 0, layer, s));
   static const size_t per_patch[7] = {0, 32 * 32 * 32, 32 * 32 * 32, 16 * 16 * 64, 16 * 16 * 64, 8 * 8 * 128, 8 * 8 * 128};
-  const uint16_t* src = layer == 6 ? h->l6 : h->act[((layer - 1) & 1) ^ ((h->fuse34 && layer >= 4) ? 1 : 0)];
+  const uint16_t* src = layer == 6 ? h->l6 : act_buf(h, layer);
   HN_CUDA(cudaMemcpyAsync(act_out, src, per_patch[layer] * 2 * static_cast<size_t>(B), cudaMemcpyDeviceToDevice, s));
   return HN_OK;
 }

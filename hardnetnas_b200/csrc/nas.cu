@@ -22,7 +22,6 @@
 #include "handle.h"
 #include "host_common.h"
 #include "tc_conv.cuh"
-#include "nas_resident.cuh"
 #include "nas_tail.cuh"
 
 namespace hn {
@@ -866,16 +865,6 @@ __global__ void __launch_bounds__(256) se_kernel(uint16_t* __restrict__ x, long 
 // ------------------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------------------
-// A run of consecutive ops executed by ONE launch of nas_seg_kernel (nas_resident.cuh) with the activations resident in
-// shared memory; `params` holds everything but the per-call pointers / patch count.
-struct NasSegment {
-  int first = 0, last = 0;   // op range [first, last]
-  int G = 1, minb = 1;
-  size_t smem = 0;
-  SegParams params;
-  uint8_t* blob = nullptr;   // device copy of the weight image
-};
-
 // A run of consecutive ops behind the front stage executed by ONE launch of nas_tail_kernel (nas_tail.cuh), a warpgroup per patch.
 struct NasTail {
   int first = 0, last = 0;   // op range [first, last]
@@ -900,8 +889,6 @@ struct NasState {
   float* headf_b = nullptr;
   int headf_k = 0;
   TcParams headf;
-  std::vector<NasSegment> segs;
-  std::vector<int> seg_of_op;        // index into segs, or -1: the op runs as its own kernel
   std::vector<hn_nas_op> ops;
   std::vector<PwParams> pw;          // one per op (valid for OP_PW)
   std::vector<size_t> w16_off;       // 16-bit weight offset per op (PW / HEAD)
@@ -928,7 +915,6 @@ void nas_state_free(NasState* s) {
   for (auto* p : s->slot) cudaFree(p);
   cudaFree(s->head_in);
   cudaFree(s->front_img);
-  for (auto& sg : s->segs) cudaFree(sg.blob);
   for (auto& tl : s->tails) cudaFree(tl.blob);
   for (auto& tl : s->ftails) cudaFree(tl.blob);
   cudaFree(s->headf_w);
@@ -986,282 +972,10 @@ static int launch_pw(const PwParams& p, int nt, int kcb, int sm_count, cudaStrea
 namespace hn {
 
 // ------------------------------------------------------------------------------------------------------------
-// patch-resident segments (nas_resident.cuh)
-// ------------------------------------------------------------------------------------------------------------
-static bool seg_op_ok(const hn_nas_op& o) {
-  switch (o.kind) {
-    case OP_PW: return o.cin % 16 == 0 && o.cout % 32 == 0 && o.cin <= 512 && o.cout <= 512 && (o.hin * o.hin) % 8 == 0;
-    case OP_DW: return (o.kernel == 3 || o.kernel == 5) && (o.stride == 1 || o.stride == 2) && o.hout % 2 == 0 && o.cin % 8 == 0;
-    case OP_MAXPOOL: return o.hout % 4 == 0 && o.cin % 8 == 0;
-    case OP_SE: return o.cin <= 512 && o.mid <= 128 && o.cin % 8 == 0;
-    default: return false;
-  }
-}
-
-static int seg_pw_nt(int cout) {
-  if (cout <= 256) return cout;
-  if (cout % 128 == 0) return 128;
-  if (cout % 96 == 0) return 96;
-  return 32;
-}
-
-static size_t seg_align(size_t x, size_t a) { return (x + a - 1) / a * a; }
-
-// Shared-memory plan of ops [first, last]: per-patch bytes of the three slot buffers and the layout of the weight blob.
-struct SegPlan {
-  size_t slot_pp[3] = {0, 0, 0};
-  size_t act_pp = 0;
-  size_t blob_bytes = 0;
-  bool has_se = false;
-  std::vector<size_t> w_off, b_off, w2_off, b2_off;   // per op, relative to the blob start
-};
-
-static SegPlan seg_plan(const std::vector<hn_nas_op>& ops, int first, int last, int bf) {
-  const size_t dw_elem = bf ? 4 : 2;   // fp16 activations: fp16 depthwise weights / bias (packed HFMA2 arithmetic)
-  SegPlan pl;
-  const int n = last - first + 1;
-  pl.w_off.assign(n, 0); pl.b_off.assign(n, 0); pl.w2_off.assign(n, 0); pl.b2_off.assign(n, 0);
-  size_t off = 0;
-  auto take = [&](size_t bytes) { const size_t r = off; off = seg_align(off + bytes, 128); return r; };
-  for (int i = first; i <= last; ++i) {
-    const hn_nas_op& o = ops[i];
-    const size_t in_b = static_cast<size_t>(o.cin) * o.hin * o.hin * 2, out_b = static_cast<size_t>(o.cout) * o.hout * o.hout * 2;
-    pl.slot_pp[o.src] = std::max(pl.slot_pp[o.src], in_b);
-    pl.slot_pp[o.dst] = std::max(pl.slot_pp[o.dst], out_b);
-    if (o.kind == OP_PW && o.res >= 0) pl.slot_pp[o.res] = std::max(pl.slot_pp[o.res], out_b);
-    const int k = i - first;
-    switch (o.kind) {
-      case OP_PW: pl.w_off[k] = take(static_cast<size_t>(o.cin) * o.cout * 2); pl.b_off[k] = take(o.cout * 4); break;
-      case OP_DW: pl.w_off[k] = take(static_cast<size_t>(o.kernel) * o.kernel * o.cin * dw_elem); pl.b_off[k] = take(o.cin * dw_elem); break;
-      case OP_SE:
-        pl.has_se = true;
-        pl.w_off[k] = take(static_cast<size_t>(o.mid) * o.cin * 4); pl.b_off[k] = take(o.mid * 4);
-        pl.w2_off[k] = take(static_cast<size_t>(o.mid) * o.cin * 4); pl.b2_off[k] = take(o.cin * 4);
-        break;
-      default: break;
-    }
-  }
-  pl.blob_bytes = off;
-  for (size_t b : pl.slot_pp) pl.act_pp += b;
-  return pl;
-}
-
-constexpr size_t kSegSlack = 2048;      // a partial accumulator tile reads up to 2 KB past the end of a source plane
-constexpr size_t kSegScratch = (512 + 128 + 512) * 4;
-
-// Largest group size that fits `minb` CTAs per SM (shared memory and tensor memory); 0 = does not fit.
-static int seg_fit(const std::vector<hn_nas_op>& ops, int first, int last, const SegPlan& pl, int minb, int gmax) {
-  const size_t budget = (228 * 1024) / minb - 1024 /*reserved per CTA*/ - 1024 /*alignment*/ - 1536 /*rounding of the offsets*/;
-  const size_t fixed = kSegSlack + pl.blob_bytes + (pl.has_se ? kSegScratch : 0) + 64 + 3 * 1024 /*buffer alignment*/;
-  if (fixed + pl.act_pp > budget) return 0;
-  int G = static_cast<int>(std::min<size_t>((budget - fixed) / pl.act_pp, gmax));
-  for (; G >= 1; --G) {
-    int cols = 0;
-    for (int i = first; i <= last; ++i)
-      if (ops[i].kind == OP_PW) cols = std::max(cols, ((G * ops[i].hin * ops[i].hin + kTileM - 1) / kTileM) * ops[i].cout);
-    if (cols <= 512 / minb) break;
-  }
-  return G;
-}
-
-// Finalises segment [first, last]: group size, shared-memory offsets, weight image on the device.
-static int seg_build(hn_handle* h, NasState* st, const float* params, int first, int last, NasSegment& sg) {
-  const SegPlan pl = seg_plan(st->ops, first, last, st->act_bf16);
-  int minb = 0, G = 0;
-  for (int mb : {2, 1}) {
-    if (h->env.nas_minb && h->env.nas_minb != mb) continue;
-    if (mb == 2 && st->act_bf16) continue;   // the fp32 depthwise path of bf16 nets needs > 64 registers per thread
-    G = seg_fit(st->ops, first, last, pl, mb, h->env.nas_gmax);
-    if (G >= 1) { minb = mb; break; }
-  }
-  if (G < 1) return HN_ERR_UNSUPPORTED;
-  sg.first = first; sg.last = last; sg.G = G; sg.minb = minb;
-  SegParams& p = sg.params;
-  memset(&p, 0, sizeof(p));
-  size_t off = 0;
-  size_t slot_off[3];
-  for (int k = 0; k < 3; ++k) { slot_off[k] = off; off = seg_align(off + pl.slot_pp[k] * G, 1024); }
-  off += kSegSlack;
-  p.blob_off = static_cast<int>(off);
-  p.blob_bytes = static_cast<int>(seg_align(pl.blob_bytes, 16));
-  off = seg_align(off + pl.blob_bytes, 128);
-  p.scratch_off = static_cast<int>(off);
-  if (pl.has_se) off += kSegScratch;
-  p.bar_off = static_cast<int>(off);
-  off += 64;
-  sg.smem = off + 1024;
-  p.G = G;
-  p.n_ops = last - first + 1;
-  p.op_base = first;
-  p.seg_id = static_cast<int>(st->segs.size()) & 7;
-  int cols = 32;
-  std::vector<uint8_t> blob(pl.blob_bytes, 0);
-  for (int i = first; i <= last; ++i) {
-    const hn_nas_op& o = st->ops[i];
-    const int k = i - first;
-    SegOp& so = p.ops[k];
-    so.kind = o.kind; so.cin = o.cin; so.cout = o.cout; so.kernel = o.kernel; so.stride = o.stride;
-    so.hin = o.hin; so.hout = o.hout; so.relu = o.relu; so.mid = o.mid;
-    so.src_off = static_cast<int>(slot_off[o.src]);
-    so.dst_off = static_cast<int>(slot_off[o.dst]);
-    so.res_off = (o.kind == OP_PW && o.res >= 0) ? static_cast<int>(slot_off[o.res]) : -1;
-    so.w_off = p.blob_off + static_cast<int>(pl.w_off[k]);
-    so.b_off = p.blob_off + static_cast<int>(pl.b_off[k]);
-    so.w2_off = p.blob_off + static_cast<int>(pl.w2_off[k]);
-    so.b2_off = p.blob_off + static_cast<int>(pl.b2_off[k]);
-    so.nt = o.kind == OP_PW ? seg_pw_nt(o.cout) : 0;
-    so.pitch = static_cast<uint32_t>(G) * o.hin * o.hin * 16;
-    if (o.kind == OP_PW) {
-      so.tiles = (G * o.hin * o.hin + kTileM - 1) / kTileM;
-      so.ksteps = o.cin / 16;
-      so.chunks = o.cout / so.nt;
-      so.idesc = make_idesc_f16(kTileM, so.nt, st->act_bf16);
-      so.b_hi = noswizzle_desc_hi(static_cast<uint32_t>(o.cin) * 16);
-    }
-    if (o.kind == OP_DW) so.sh = 2;
-    uint8_t* b = blob.data();
-    switch (o.kind) {
-      case OP_PW: {
-        // UMMA no-swizzle K-major image of W[cout][cin]: element (n, k) at (n / 8) * (cin * 16) + (k / 8) * 128 + (n % 8) * 16 + (k % 8) * 2
-        uint16_t* w = reinterpret_cast<uint16_t*>(b + pl.w_off[k]);
-        for (int n = 0; n < o.cout; ++n)
-          for (int c = 0; c < o.cin; ++c)
-            w[((n >> 3) * o.cin * 16 + (c >> 3) * 128 + (n & 7) * 16 + (c & 7) * 2) >> 1] = f2h16(params[o.w_off + static_cast<size_t>(n) * o.cin + c], st->act_bf16);
-        memcpy(b + pl.b_off[k], params + o.b_off, o.cout * 4);
-        cols = std::max(cols, ((G * o.hin * o.hin + kTileM - 1) / kTileM) * o.cout);
-        break;
-      }
-      case OP_DW:
-        if (st->act_bf16) {
-          memcpy(b + pl.w_off[k], params + o.w_off, static_cast<size_t>(o.kernel) * o.kernel * o.cin * 4);
-          memcpy(b + pl.b_off[k], params + o.b_off, o.cin * 4);
-        } else {
-          uint16_t* w = reinterpret_cast<uint16_t*>(b + pl.w_off[k]);
-          for (int j = 0; j < o.kernel * o.kernel * o.cin; ++j) w[j] = f2h16(params[o.w_off + j], 0);
-          uint16_t* bb = reinterpret_cast<uint16_t*>(b + pl.b_off[k]);
-          for (int j = 0; j < o.cin; ++j) bb[j] = f2h16(params[o.b_off + j], 0);
-        }
-        break;
-      case OP_SE:
-        memcpy(b + pl.w_off[k], params + o.w_off, static_cast<size_t>(o.mid) * o.cin * 4);
-        memcpy(b + pl.b_off[k], params + o.b_off, o.mid * 4);
-        memcpy(b + pl.w2_off[k], params + o.w2_off, static_cast<size_t>(o.mid) * o.cin * 4);
-        memcpy(b + pl.b2_off[k], params + o.b2_off, o.cin * 4);
-        break;
-      default: break;
-    }
-  }
-  int tc = 32;
-  while (tc < cols) tc <<= 1;
-  p.tmem_cols = tc;
-  HN_CUDA(cudaMalloc(&sg.blob, std::max<size_t>(p.blob_bytes, 16)));
-  blob.resize(std::max<size_t>(p.blob_bytes, 16), 0);
-  HN_CUDA(cudaMemcpy(sg.blob, blob.data(), blob.size(), cudaMemcpyHostToDevice));
-  p.blob = reinterpret_cast<const uint4*>(sg.blob);
-  return HN_OK;
-}
-
-// Partitions the ops behind the front kernel into patch-resident segments. A segment grows while it fits one CTA's shared
-// memory; it is cut at a block boundary (behind a linear pointwise conv, an SE or a max-pool) once the tensor there has
-// shrunk to <= 1 / cut_ratio of the segment's input, so that deeper, smaller stages run with larger groups.
-static int seg_partition(hn_handle* h, NasState* st, const float* params) {
-  const int n_ops = static_cast<int>(st->ops.size());
-  st->seg_of_op.assign(n_ops, -1);
-  st->segs.clear();
-  if (!h->env.nas_resident) return HN_OK;
-  std::vector<char> forced(n_ops, 0);
-  const bool explicit_split = h->env.nas_split[0] != 0;
-  if (explicit_split) {
-    for (const char* c = h->env.nas_split; *c;) {
-      const int v = atoi(c);
-      if (v > 0 && v < n_ops) forced[v] = 1;
-      while (*c && *c != ',') ++c;
-      if (*c == ',') ++c;
-    }
-  }
-  // every tensor an op of [a, b] reads must be the segment's input or produced inside it (a residual from before the
-  // segment that is not its input lives only in HBM)
-  auto reads_ok = [&](int a, int b) {
-    bool defined[3] = {false, false, false};
-    defined[st->ops[a].src] = true;
-    for (int i = a; i <= b; ++i) {
-      const hn_nas_op& o = st->ops[i];
-      if (!defined[o.src] || (o.kind == OP_PW && o.res >= 0 && !defined[o.res])) return false;
-      defined[o.dst] = true;
-    }
-    return true;
-  };
-  // only the last op's output reaches HBM: nothing behind the segment may read another tensor produced inside it
-  auto escapes_ok = [&](int a, int b) {
-    bool inside[3] = {false, false, false};
-    for (int i = a; i <= b; ++i) inside[st->ops[i].dst] = true;
-    inside[st->ops[b].dst] = false;
-    for (int j = b + 1; j < n_ops; ++j) {
-      const hn_nas_op& o = st->ops[j];
-      if (inside[o.src] || (o.kind == OP_PW && o.res >= 0 && inside[o.res])) return false;
-      if (o.kind != OP_HEAD) inside[o.dst] = false;
-    }
-    return true;
-  };
-  auto fits = [&](int a, int b) {
-    if (b - a + 1 > kSegMaxOps || !reads_ok(a, b)) return false;
-    const SegPlan pl = seg_plan(st->ops, a, b, st->act_bf16);
-    return seg_fit(st->ops, a, b, pl, 1, 1) >= 1;
-  };
-  auto close = [&](int a, int b) -> int {
-    while (a <= b) {
-      if (!fits(a, a)) { ++a; continue; }   // e.g. a residual conv cut off from its block input
-      int e = b;
-      while (e > a && !(fits(a, e) && escapes_ok(a, e))) --e;
-      // a lone depthwise / max-pool op gains nothing from residency (same bytes as its own bulk-copy kernel)
-      const bool lone = a == e && (st->ops[a].kind == OP_DW || st->ops[a].kind == OP_MAXPOOL);
-      if (!lone) {
-        NasSegment sg;
-        const int rc = seg_build(h, st, params, a, e, sg);
-        if (rc != HN_OK && rc != HN_ERR_UNSUPPORTED) return rc;
-        if (rc == HN_OK) {
-          for (int i = a; i <= e; ++i) st->seg_of_op[i] = static_cast<int>(st->segs.size());
-          st->segs.push_back(sg);
-        }
-      }
-      a = e + 1;
-    }
-    return HN_OK;
-  };
-  int start = -1;
-  for (int i = st->front_ops; i < n_ops - 1; ++i) {
-    const hn_nas_op& o = st->ops[i];
-    if (!seg_op_ok(o)) {
-      if (start >= 0) HN_TRY(close(start, i - 1));
-      start = -1;
-      continue;
-    }
-    if (start >= 0 && (forced[i] || !fits(start, i))) {
-      HN_TRY(close(start, i - 1));
-      start = -1;
-    }
-    if (start < 0) {
-      if (!fits(i, i)) continue;
-      start = i;
-    }
-    if (!explicit_split && i + 1 < n_ops - 1) {
-      const bool boundary = (o.kind == OP_PW && !o.relu && st->ops[i + 1].kind != OP_SE) || o.kind == OP_SE || o.kind == OP_MAXPOOL;
-      const hn_nas_op& f = st->ops[start];
-      const size_t in_b = static_cast<size_t>(f.cin) * f.hin * f.hin, cut_b = static_cast<size_t>(o.cout) * o.hout * o.hout;
-      if (boundary && cut_b * h->env.nas_cut_ratio <= in_b) {
-        HN_TRY(close(start, i));
-        start = -1;
-      }
-    }
-  }
-  if (start >= 0) HN_TRY(close(start, n_ops - 2));
-  return HN_OK;
-}
-
-
-// ------------------------------------------------------------------------------------------------------------
 // warpgroup-per-patch tail launches (nas_tail.cuh)
 // ------------------------------------------------------------------------------------------------------------
+static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+
 // The ops behind the front stage as a small SSA program over tensor ids (tensor 0 = the front stage's output). Two forms:
 //   plain   one TOp per packed op, a block's residual as an identity second input (activation dumps run this form, so every
 //           packed op's output can still be inspected), and
@@ -1515,7 +1229,7 @@ static bool tail_prog_folded(const std::vector<hn_nas_op>& ops, const float* par
 // Finalises tail launch [first, last] of `pr`: region offsets, warpgroups per CTA, weight image on the device.
 static int tail_build(hn_handle* h, const TProg& pr, int first, int last, int launch_id, NasTail& tl) {
   size_t off = 0;
-  auto take = [&](size_t bytes) { const size_t r = off; off = seg_align(off + bytes, 128); return r; };
+  auto take = [&](size_t bytes) { const size_t r = off; off = align_up(off + bytes, 128); return r; };
   const int n = last - first + 1;
   if (n > kTailMaxOps) return HN_ERR_UNSUPPORTED;
   std::vector<size_t> w_off(n, 0), b_off(n, 0);
@@ -1544,11 +1258,11 @@ static int tail_build(hn_handle* h, const TProg& pr, int first, int last, int la
     if (o.kind == OP_PW) w_off[k] = take(static_cast<size_t>(o.cin + 16 + wc1(o)) * o.cout * 2);   // + 16 K columns: bias as fp16 hi + lo
     if (o.kind == OP_DW) { w_off[k] = take(static_cast<size_t>(o.kernel) * o.kernel * o.cin * 2); b_off[k] = take(o.cin * 2); }
   }
-  const size_t blob_bytes = seg_align(off, 16);
+  const size_t blob_bytes = align_up(off, 16);
   // Three equal regions per warpgroup, assigned by liveness: the run's input sits in region 0 and every output goes to a
   // free region, region 0 last — so region 0 is idle from the last op that touches the input (or a tensor that had to share
   // its region) onwards and the NEXT patch's input is bulk-copied into it while the remaining ops run.
-  region_bytes = seg_align(region_bytes, 1024);
+  region_bytes = align_up(region_bytes, 1024);
   const size_t wg_stride = 3 * region_bytes;
   const int in_t = pr.ops[first].in0;
   auto last_use = [&](int t) {                  // last op of the run that reads tensor t (-1: none); the run's output lives on
@@ -1583,7 +1297,7 @@ static int tail_build(hn_handle* h, const TProg& pr, int first, int last, int la
   }
   // a partial accumulator tile reads up to 2 KB past the end of a source plane: the blob sits behind the last region, so
   // those reads stay inside the CTA's shared memory
-  const size_t fixed = seg_align(std::max<size_t>(blob_bytes, 2048), 128) + 256 + 1024 /*alignment of the base*/;
+  const size_t fixed = align_up(std::max<size_t>(blob_bytes, 2048), 128) + 256 + 1024 /*alignment of the base*/;
   // five or six warpgroups (64 tensor-memory columns and 85 registers each) only for runs without 16 x 16 maps
   int nwg = std::min(h->env.nas_tail_wg, big_map ? 4 : kTailMaxWG);
   while (nwg >= 1 && nwg * wg_stride + fixed > 227 * 1024) --nwg;
@@ -1598,7 +1312,7 @@ static int tail_build(hn_handle* h, const TProg& pr, int first, int last, int la
   p.launch_id = launch_id & 7;
   p.blob_off = static_cast<int>(nwg * wg_stride);
   p.blob_bytes = static_cast<int>(blob_bytes);
-  p.bar_off = static_cast<int>(seg_align(p.blob_off + std::max<size_t>(blob_bytes, 2048), 128));
+  p.bar_off = static_cast<int>(align_up(p.blob_off + std::max<size_t>(blob_bytes, 2048), 128));
   tl.smem = p.bar_off + 256 + 1024;
   tl.dst_off.assign(n, 0);
   std::vector<uint8_t> blob(std::max<size_t>(blob_bytes, 16), 0);
@@ -1750,44 +1464,13 @@ static int launch_tail(const NasTail& tl, const uint16_t* in, uint16_t* out, int
   }
 }
 
-template <int MINB, bool BF16>
-static int launch_seg_cfg(const SegParams& p, size_t smem, int sm_count, cudaStream_t s) {
-  auto kern = nas_seg_kernel<MINB, BF16>;
-  static DeviceOnce attr_once;
-  if (attr_once.first_time()) HN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (228 * 1024) / MINB - 1024));
-  const int groups = (p.n + p.G - 1) / p.G;
-  if (groups <= 0) return HN_OK;
-  kern<<<std::min(groups, sm_count * MINB), kSegThreads, smem, s>>>(p);
-  HN_CUDA(cudaGetLastError());
-  count_launch();
-  return HN_OK;
-}
-
-static int launch_seg(const NasSegment& sg, const uint16_t* in, uint16_t* out, int n, int n_ops, int bf, int sm_count, cudaStream_t s) {
-  SegParams p = sg.params;
-  p.in = in;
-  p.out = out;
-  p.n = n;
-  p.n_ops = n_ops;
-  if (bf) return launch_seg_cfg<1, true>(p, sg.smem, sm_count, s);
-  return sg.minb == 2 ? launch_seg_cfg<2, false>(p, sg.smem, sm_count, s) : launch_seg_cfg<1, false>(p, sg.smem, sm_count, s);
-}
-
-// Runs ops [0, last_op] of the packed program for `n` patches (n <= chunk). With first_op >= 0 only ops [first_op, last_op]
-// run and, if out_override is set, the LAST of them writes there instead of its slot (sub-pass of the front stage below).
-static int run_nas_ops(hn_handle* h, NasState* st, const char* src, int in_dtype, int n, long long off, int last_op,
-                       cudaStream_t s, int first_op = -1, uint16_t* out_override = nullptr) {
+// Runs ops [0, last_op] of the packed program for `n` patches (n <= chunk).
+static int run_nas_ops(hn_handle* h, NasState* st, const char* src, int in_dtype, int n, long long off, int last_op, cudaStream_t s) {
   const int bf = st->act_bf16;
   {
       int first = 0;
-      if (first_op >= 0) {
-        first = first_op;
-      } else if (st->front_img && last_op >= st->front_ops - 1 && h->env.nas_front) {
+      if (st->front_img && last_op >= st->front_ops - 1 && h->env.nas_front) {
         const hn_nas_op &o0 = st->ops[0], &ol = st->ops[st->front_ops - 1];
-        // The front kernel's 64 KB/patch output is the largest tensor of the net and its only reader is the next op (a
-        // stride-2 depthwise conv or max-pool). Both run in sub-passes of `nas_front_chunk` patches over the SAME head of the
-        // slot, so the tensor is produced, consumed and overwritten inside the 126 MB L2 instead of making an HBM round trip
-        // (128 KB/patch of the pass's traffic); the reader writes its 4x smaller output at the sub-pass's offset.
         const int nxt = st->front_ops;
         const hn_nas_op& on = st->ops[nxt];
         if (st->front_fdw && nxt <= last_op) {
@@ -1797,29 +1480,14 @@ static int run_nas_ops(hn_handle* h, NasState* st, const char* src, int in_dtype
                                     /*out_planar=*/nxt < last_op && st->tail_of_op[nxt + 1] >= 0));
           first = nxt + 1;
         } else {
-        const bool sub = h->env.nas_front_chunk > 0 && h->env.nas_front_chunk < n && nxt <= last_op && nxt < static_cast<int>(st->ops.size()) - 1 &&
-                         st->seg_of_op[nxt] < 0 && (on.kind == OP_DW || on.kind == OP_MAXPOOL) && on.src == ol.dst;
-        if (sub) {
-          const size_t in_elem = in_dtype == HN_F32 ? 4 : 1;
-          const size_t out_pp = static_cast<size_t>(on.cout) * on.hout * on.hout;
-          for (int o2 = 0; o2 < n; o2 += h->env.nas_front_chunk) {
-            const int m = std::min(h->env.nas_front_chunk, n - o2);
-            HN_TRY(launch_front_pw(src + static_cast<size_t>(o2) * 1024 * in_elem, in_dtype, st->slot[ol.dst], st->front_tm,
-                                   st->params + o0.w_off, st->params + o0.b_off, st->front_img, st->front_bias2, m, bf, h->sm_count, s));
-            HN_TRY(run_nas_ops(h, st, src, in_dtype, m, off, nxt, s, nxt, st->slot[on.dst] + static_cast<size_t>(o2) * out_pp));
-          }
-          first = nxt + 1;
-        } else {
           HN_TRY(launch_front_pw(src, in_dtype, st->slot[ol.dst], st->front_tm, st->params + o0.w_off, st->params + o0.b_off, st->front_img,
                                  st->front_bias2, n, bf, h->sm_count, s));
           first = st->front_ops;
-        }
         }
       }
       const int n_total = static_cast<int>(st->ops.size());
       for (int i = first; i <= last_op; ++i) {
         const hn_nas_op& o = st->ops[i];
-        uint16_t* const op_out = (out_override && i == last_op && o.kind != OP_HEAD) ? out_override : (o.kind != OP_HEAD ? st->slot[o.dst] : nullptr);
         if (i == st->tail_first && last_op == n_total - 1 && !st->ftails.empty()) {
           // the forward: folded form, launches chained through the slots, the last one writes the head GEMM's rows
           const uint16_t* cur = st->slot[st->ops[i].src];
@@ -1840,23 +1508,11 @@ static int run_nas_ops(hn_handle* h, NasState* st, const char* src, int in_dtype
           const NasTail& tl = st->tails[st->tail_of_op[i]];
           const int end = std::min(tl.last + st->tail_first, last_op);
           const bool to_head = end == n_total - 2 && last_op == n_total - 1;
-          uint16_t* dst = to_head ? st->head_in + static_cast<size_t>(off) * st->head_k : ((out_override && end == last_op) ? out_override : st->slot[st->ops[end].dst]);
+          uint16_t* dst = to_head ? st->head_in + static_cast<size_t>(off) * st->head_k : st->slot[st->ops[end].dst];
           // channel-planar interchange towards the next tail launch / the head GEMM (permuted weight K order); a run that
           // stops here (activation dump) writes NHWC like every per-op kernel
           const int planar = (to_head && st->head_planar) || (end == tl.last + st->tail_first && last_op > end && st->tail_of_op[end + 1] >= 0);
           HN_TRY(launch_tail(tl, st->slot[st->ops[tl.first + st->tail_first].src], dst, planar, n, end - st->tail_first, h->sm_count, s));
-          i = to_head ? end + 1 : end;
-          continue;
-        }
-        if (st->seg_of_op[i] >= 0) {
-          // patch-resident segment: ops [i, end] in one launch; a segment that ends right before the head writes the
-          // head GEMM's input rows directly
-          const NasSegment& sg = st->segs[st->seg_of_op[i]];
-          const int end = std::min(sg.last, last_op);
-          const hn_nas_op& ol = st->ops[end];
-          const bool to_head = end == n_total - 2 && last_op == n_total - 1;
-          uint16_t* dst = to_head ? st->head_in + static_cast<size_t>(off) * st->head_k : st->slot[ol.dst];
-          HN_TRY(launch_seg(sg, st->slot[st->ops[sg.first].src], dst, n, end - sg.first + 1, bf, h->sm_count, s));
           i = to_head ? end + 1 : end;
           continue;
         }
@@ -1877,7 +1533,7 @@ static int run_nas_ops(hn_handle* h, NasState* st, const char* src, int in_dtype
             const long long total = static_cast<long long>(n) * o.hout * (strip ? o.hout / 4 : o.hout) * (o.cin / 8);
             const int grid = static_cast<int>(std::min<long long>((total + 255) / 256, h->sm_count * 16LL));
             const uint16_t* src = st->slot[o.src];
-            uint16_t* dst = op_out;
+            uint16_t* dst = st->slot[o.dst];
             const float* wv = st->params + o.w_off;
             const float* bv = st->params + o.b_off;
             // shared-memory kernel whenever two units of whole maps fit next to the weights (every shape of SEARCH_SPACE2
@@ -1955,14 +1611,14 @@ static int run_nas_ops(hn_handle* h, NasState* st, const char* src, int in_dtype
                   HN_CUDA(cudaFuncSetAttribute(maxpool_smem_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
                   HN_CUDA(cudaFuncSetAttribute(maxpool_smem_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
                 }
-                if (bf) maxpool_smem_kernel<true><<<sgrid, 256, smem, s>>>(st->slot[o.src], op_out, n, o.cin, o.hin, o.hout, G);
-                else maxpool_smem_kernel<false><<<sgrid, 256, smem, s>>>(st->slot[o.src], op_out, n, o.cin, o.hin, o.hout, G);
+                if (bf) maxpool_smem_kernel<true><<<sgrid, 256, smem, s>>>(st->slot[o.src], st->slot[o.dst], n, o.cin, o.hin, o.hout, G);
+                else maxpool_smem_kernel<false><<<sgrid, 256, smem, s>>>(st->slot[o.src], st->slot[o.dst], n, o.cin, o.hin, o.hout, G);
                 HN_CUDA(cudaGetLastError());
                 count_launch();
                 break;
               }
             }
-            maxpool_kernel<<<grid, 256, 0, s>>>(st->slot[o.src], op_out, n, o.cin, o.hin, o.hout, bf);
+            maxpool_kernel<<<grid, 256, 0, s>>>(st->slot[o.src], st->slot[o.dst], n, o.cin, o.hin, o.hout, bf);
             HN_CUDA(cudaGetLastError());
             count_launch();
             break;
@@ -2115,7 +1771,7 @@ extern "C" int hn_pack_nas(hn_handle* h, const hn_nas_op* ops, int n_ops, const 
   }
   // the op behind the front stage, if it is the block's stride-2 depthwise conv (or the Identity's max-pool) on the
   // 32 x 32 x 32 tensor, runs inside the front kernel too (fp16 activations): 64 KB/patch never reach HBM
-  if (!bf && h->env.nas_front_dw && h->env.nas_front && !h->env.nas_resident && st->front_ops < n_ops - 1) {
+  if (!bf && h->env.nas_front_dw && h->env.nas_front && st->front_ops < n_ops - 1) {
     const hn_nas_op& o = ops[st->front_ops];
     const hn_nas_op& prev = ops[st->front_ops - 1];
     const bool shape_ok = o.cin == 32 && o.cout == 32 && o.hin == 32 && o.hout == 16 && o.stride == 2 && o.src == prev.dst;
@@ -2202,8 +1858,7 @@ extern "C" int hn_pack_nas(hn_handle* h, const hn_nas_op* ops, int n_ops, const 
     if (rc != HN_OK) return fail(rc);
   }
   {
-    int rc = seg_partition(h, st, params);
-    if (rc != HN_OK) return fail(rc);
+    int rc = HN_OK;
     // warpgroup-per-patch tail launches behind the fused front stage (fp16 activations, every op of a supported shape)
     st->tail_of_op.assign(n_ops, -1);
     st->tail_first = st->front_ops + 1;
@@ -2310,18 +1965,6 @@ extern "C" int hn_forward_nas(hn_handle* h, const void* patches, int in_dtype, l
   return HN_OK;
 }
 
-#ifdef HN_SEG_TRACE
-extern "C" int hn_debug_seg_trace(unsigned long long* out256, int reset) {
-  HN_CUDA(cudaDeviceSynchronize());
-  HN_CUDA(cudaMemcpyFromSymbol(out256, hn::hn_seg_trace, 256 * sizeof(unsigned long long)));
-  if (reset) {
-    unsigned long long z[256] = {0};
-    HN_CUDA(cudaMemcpyToSymbol(hn::hn_seg_trace, z, sizeof(z)));
-  }
-  return HN_OK;
-}
-#endif
-
 #ifdef HN_TAIL_TRACE
 extern "C" int hn_debug_tail_trace(unsigned long long* out128, int reset) {
   HN_CUDA(cudaDeviceSynchronize());
@@ -2340,11 +1983,7 @@ extern "C" int hn_nas_plan(hn_handle* h, int* out, int cap) {
     set_error("hn_nas_plan: no NAS net packed");
     return HN_ERR_STATE;
   }
-  int n = static_cast<int>(h->nas->segs.size());
-  for (int i = 0; i < n && i < cap && out; ++i) {
-    const NasSegment& sg = h->nas->segs[i];
-    out[4 * i] = sg.first; out[4 * i + 1] = sg.last; out[4 * i + 2] = sg.G; out[4 * i + 3] = sg.minb;
-  }
+  int n = 0;
   // warpgroup-per-patch tail launches of the forward: (first packed op, last packed op, patches in flight per CTA, 0); in the
   // folded form a launch starts / ends at the packed op whose output its first / last op produces
   const bool folded = !h->nas->ftails.empty();

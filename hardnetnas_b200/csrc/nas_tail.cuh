@@ -4,8 +4,8 @@
 // max-pool / 1x1 conv), stacked as in hardnetNAS/supernet_functions/model_supernet.py:70-85 — runs with the patch's
 // activations resident in shared memory.
 //
-// Unlike nas_seg_kernel (nas_resident.cuh: the whole CTA steps through the ops of a group of patches, every step pays a
-// CTA-wide issue -> commit -> wait -> tcgen05.ld -> store -> barrier latency) the unit of execution here is a WARPGROUP:
+// The unit of execution is a WARPGROUP, not the CTA (a CTA that steps through the ops of a group of patches pays a CTA-wide
+// issue -> commit -> wait -> tcgen05.ld -> store -> barrier latency at every step; DESIGN.md section 4):
 // four warps own ONE patch from its load to its store, synchronise only among themselves (named barrier, own mbarrier,
 // own 128 tensor-memory columns) and the 3-4 warpgroups of a CTA run independently, so one warpgroup's latency-bound
 // tensor-core phase overlaps the others' CUDA-core depthwise phases without any hand-written pipeline. All shapes are
@@ -25,7 +25,6 @@
 #pragma once
 
 #include "common.cuh"
-#include "nas_resident.cuh"
 #include "tc_conv.cuh"
 
 namespace hn {

@@ -1,26 +1,14 @@
-// Persistent, warp-specialised tcgen05 kernels for the HardNet conv stack.
+// Shared pieces of the tcgen05 kernels (parameter block, 16-bit packing, channel-planar addressing) and the descriptor head:
 //
-//   conv3x3_kernel : the 3x3 convs (features[6..17], reference hardnet/HardNet.py:287-298) as implicit GEMMs:
-//     M = 128 output pixels per tile, N = C_out, K = 9 taps x C_in, cut into "k-blocks" of one tap x <=64
-//     channels. Activations live in global memory CHANNEL-PLANAR: [patch][plane = c / 8][y][x][c % 8] (16 B per
-//     pixel and plane; stride-2 consumers get the four row/column parity sub-planes [plane][ypar][xpar][y/2][x/2][8]).
-//     The A tile of a k-block is ONE 4-D TMA box (x * 8, y, patch, plane) whose start coordinate carries the tap
-//     shift; out-of-range x / y are zero-filled by TMA, which is exactly the conv's zero padding, and because
-//     x / y are per-patch tensor dimensions nothing bleeds between patches. The box lands in shared memory as
-//     [plane][pixel][8 channels], which is the UMMA no-swizzle K-major layout (core matrix = 8 pixels x 16 B,
-//     SBO = 128 B, LBO = plane pitch). The planar layout is what makes the epilogue's stores coalesce: a warp
-//     writes 32 pixels x 16 B = 512 contiguous bytes per instruction (NHWC rows would touch 32 cache lines).
-//     Weights stay resident in shared memory when they fit (WRES), otherwise they are streamed with the A
-//     tiles. A pipeline stage carries G k-blocks so that one mbarrier round trip feeds G * KCB/32 MMAs.
 //   gemm_l2norm_kernel : the 8x8 head conv (features[19..20] + L2Norm, HardNet.py:300-301,314-315 and
 //     Utils.py:19-22) as a [B, K] x [K, 128] GEMM with bias + L2-normalise in the epilogue (also the NAS
 //     head with K = 2048).
 //
 // Roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM owner + UMMA issuer, warps 2..5 = epilogue
-// (TMEM -> registers -> bias/ReLU/pack or L2-normalise -> global). The producer / issuer loops run
-// warp-uniformly (every lane executes the control flow, elect.sync picks the lane that issues), which
-// lets the compiler keep the loop state in uniform registers. Two accumulator buffers in TMEM let the
-// epilogue of tile i overlap the MMAs of tile i+1.
+// (TMEM -> registers -> bias / L2-normalise -> global). The producer / issuer loops run warp-uniformly (every lane
+// executes the control flow, elect.sync picks the lane that issues), which lets the compiler keep the loop state in
+// uniform registers. Two accumulator buffers in TMEM let the epilogue of tile i overlap the MMAs of tile i+1.
+// The 3x3 convs run on the CTA-pair kernel of tc_conv_pair.cuh.
 #pragma once
 
 #include "common.cuh"
@@ -50,6 +38,18 @@ struct TcParams {
   float* partial;          // [k_splits][num_tiles * 128][128] fp32
 };
 
+// Parameters of the fused conv3 + conv4 kernel (tc_conv34.cuh)
+struct Conv34Params {
+  CUtensorMap tmA[4];   // conv2 output, parity views [ypar * 2 + xpar], box (16 px * 8, 9 rows, 1 patch, 4 planes)
+  CUtensorMap tmB3;     // conv3 weights [64][9 * 32], box (32, 32 rows), 64B swizzle
+  CUtensorMap tmB4;     // conv4 weights [64][9 * 64], box (64, 32 rows), 128B swizzle
+  float bias3[64];      // folded BN shifts, by value (constant bank)
+  float bias4[64];
+  void* out;            // conv4 output, channel-planar parity layout [patch][8 planes][ypar][xpar][8][8][8]
+  int n_patches;
+  int act_bf16;
+};
+
 __device__ __forceinline__ uint32_t pack16(float lo, float hi, int bf16) {
   if (bf16) {
     __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
@@ -65,50 +65,6 @@ __device__ __forceinline__ uint32_t pack16(float lo, float hi, int bf16) {
 constexpr uint32_t tmem_cols_for(int n) {
   return (2 * n <= 32) ? 32u : (2 * n <= 64) ? 64u : (2 * n <= 128) ? 128u : (2 * n <= 256) ? 256u : 512u;
 }
-
-// ------------------------------------------------------------------------------------------------------------
-// 3x3 convolution
-// ------------------------------------------------------------------------------------------------------------
-// ROWSHIFT (stride-1 layers): one TMA load per (kx, channel chunk) fetches the tile's band of image rows plus one
-// halo row above and below; the three ky taps then read that SAME shared-memory tile through UMMA descriptors whose
-// start address is advanced by ky image rows (whole 8-row core matrices). Cuts the L2->SMEM operand traffic from 9x
-// to 3x(R+2)/R. When a tile spans several small patches (8x8 images: two patches) the box is ordered
-// (x, patch, y, plane), so that shared memory holds [plane][y][patch][x] and a ky shift is still one uniform offset;
-// the tile's M rows are then ordered (y, patch, x).
-// TILES: accumulator tiles per pass. With TILES = 2 every streamed weight block feeds two A tiles (halves the weight
-// traffic through the SM's L2 port) and each pipeline stage carries twice the bytes in flight.
-template <int CIN, int COUT, int HOUT, int STRIDE, int G, int STAGES, bool WRES, bool ROWSHIFT = false, int TILES = 1,
-          int KCB_ = 0>
-struct ConvCfg {
-  static constexpr int KCB = KCB_ ? KCB_ : ((CIN >= 64) ? 128 : 64);   // bytes of one pixel's channel chunk
-  static constexpr int KC = KCB / 2;                             // channels per k-block
-  static constexpr int CIN_CHUNKS = CIN / KC;
-  static constexpr int KB = 9 * CIN_CHUNKS;                      // k-blocks per tile
-  static constexpr int PIX = HOUT * HOUT;
-  static constexpr int TILES_PER_PATCH = PIX >= kTileM ? PIX / kTileM : 0;
-  static constexpr int ROWS_PER_TILE = PIX >= kTileM ? kTileM / HOUT : HOUT;
-  static constexpr int PATCHES_PER_TILE = PIX >= kTileM ? 1 : kTileM / PIX;
-  static constexpr int UNITS = ROWSHIFT ? 3 * CIN_CHUNKS : KB;   // TMA loads of A per tile
-  static constexpr int SPT = UNITS / G;                          // stages per tile
-  static constexpr int NPL = KC / 8;                              // 8-channel planes per k-block
-  // one image row (of all the tile's patches when ROWSHIFT) inside one plane of the A tile
-  static constexpr uint32_t ROW_BYTES = (ROWSHIFT ? PATCHES_PER_TILE : 1) * HOUT * 16;
-  static constexpr uint32_t PLANE_BYTES = ROWSHIFT ? (ROWS_PER_TILE + 2) * ROW_BYTES : kTileM * 16;
-  static constexpr uint32_t A_BYTES = NPL * PLANE_BYTES;
-  static constexpr uint32_t B_BYTES = COUT * KCB;
-  static constexpr int B_PER_STAGE = WRES ? 0 : (ROWSHIFT ? 3 : G);   // streamed weight k-blocks per stage
-  static constexpr uint32_t STAGE_BYTES = G * TILES * A_BYTES + B_PER_STAGE * B_BYTES;
-  static constexpr uint32_t W_BYTES = WRES ? KB * B_BYTES : 0u;
-  static_assert(!ROWSHIFT || (STRIDE == 1 && ROW_BYTES % 128 == 0 && (WRES || G == 1)),
-                "ROWSHIFT needs a stride-1 layer whose image rows are whole core matrices");
-  static_assert(UNITS % G == 0, "stage must hold a whole number of loads");
-  static_assert(2 * TILES * COUT <= 512, "two accumulator buffers must fit the tensor memory");
-  static constexpr uint32_t TMEM_COLS = tmem_cols_for(TILES * COUT);
-  static constexpr size_t SMEM = size_t(W_BYTES) + size_t(STAGES) * STAGE_BYTES + 1024 + 256 + COUT * 4;
-  static_assert((G * TILES * A_BYTES) % 1024 == 0 && B_BYTES % 1024 == 0 && STAGE_BYTES % 1024 == 0,
-                "swizzled weight tiles must stay 1024B aligned");
-  static_assert(COUT % 16 == 0 && COUT >= 16 && COUT <= 256, "UMMA M=128 needs N % 16 == 0");
-};
 
 __device__ __forceinline__ uint64_t make_noswizzle_desc(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
   uint64_t d = 0;
@@ -138,260 +94,6 @@ __device__ __forceinline__ uint32_t pack16_plain(float lo, float hi, int bf16) {
   if (bf16) asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
   else asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
   return r;
-}
-
-template <int CIN, int COUT, int HOUT, int STRIDE, int G, int STAGES, bool WRES, int MINB, bool ROWSHIFT, bool OUT_PARITY,
-          int TILES, int KCB_>
-__global__ void __launch_bounds__(kTcThreads, MINB) conv3x3_kernel(const __grid_constant__ TcParams p) {
-  using C = ConvCfg<CIN, COUT, HOUT, STRIDE, G, STAGES, WRES, ROWSHIFT, TILES, KCB_>;
-  static_assert(C::SMEM <= 227 * 1024, "shared memory budget");
-  constexpr int N = COUT;
-  constexpr int PPT = C::PATCHES_PER_TILE;
-
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t raw_addr = smem_u32(smem_raw);
-  const uint32_t base = (raw_addr + 1023u) & ~1023u;
-  const uint32_t w_base = base;
-  const uint32_t ring_base = base + C::W_BYTES;
-  const uint32_t bar_base = ring_base + STAGES * C::STAGE_BYTES;
-  auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (STAGES + s); };
-  auto tfull_bar = [&](int a) { return bar_base + 8u * (2 * STAGES + a); };
-  auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * STAGES + 2 + a); };
-  const uint32_t w_bar = bar_base + 8u * (2 * STAGES + 4);
-  const uint32_t tmem_slot = bar_base + 8u * (2 * STAGES + 5);
-  volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(smem_raw + (tmem_slot - raw_addr));
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int num_groups = (p.num_tiles + TILES - 1) / TILES;   // a pass works on TILES consecutive tiles
-
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&p.tmA[0]);
-    if (STRIDE == 2) {
-      tma_prefetch_desc(&p.tmA[1]);
-      tma_prefetch_desc(&p.tmA[2]);
-      tma_prefetch_desc(&p.tmA[3]);
-    }
-    tma_prefetch_desc(&p.tmB);
-  }
-  if (warp == 1) {
-    if (lane == 0) {
-      for (int s = 0; s < STAGES; ++s) {
-        mbar_init(full_bar(s), 1);
-        mbar_init(empty_bar(s), 1);
-      }
-      for (int a = 0; a < 2; ++a) {
-        mbar_init(tfull_bar(a), 1);
-        mbar_init(tempty_bar(a), 4);  // one arrive per epilogue warp
-      }
-      mbar_init(w_bar, 1);
-      fence_mbar_init();
-    }
-    __syncwarp();
-    tmem_alloc(tmem_slot, C::TMEM_COLS);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot_ptr;
-
-  if (warp == 0) {
-    // ============================== TMA producer (warp-uniform) ==============================
-    if (WRES) {
-      if (elect_one()) {
-        mbar_arrive_expect_tx(w_bar, C::W_BYTES);
-#pragma unroll 1
-        for (int kb = 0; kb < C::KB; ++kb) tma_load_2d(w_base + kb * C::B_BYTES, &p.tmB, w_bar, kb * C::KC, 0);
-      }
-      __syncwarp();
-    }
-    int stage = 0;
-    uint32_t phase = 0;
-    for (int grp = blockIdx.x; grp < num_groups; grp += gridDim.x) {
-      int ky = 0, kx = 0, cc = 0, kb = 0;
-#pragma unroll 1
-      for (int s = 0; s < C::SPT; ++s) {
-        mbar_wait(empty_bar(stage), phase ^ 1u);
-        const uint32_t st_base = ring_base + stage * C::STAGE_BYTES;
-        const bool leader = elect_one();
-        if (leader) mbar_arrive_expect_tx(full_bar(stage), C::STAGE_BYTES);
-#pragma unroll
-        for (int g = 0; g < G; ++g) {
-          if (leader) {
-#pragma unroll
-            for (int tl = 0; tl < TILES; ++tl) {
-              // tiles past the end of the batch read out-of-range patch coordinates: TMA zero-fills them
-              const int tile = grp * TILES + tl;
-              int patch0, y0;
-              if (C::TILES_PER_PATCH >= 1) {
-                patch0 = tile / (C::TILES_PER_PATCH > 0 ? C::TILES_PER_PATCH : 1);
-                y0 = (tile - patch0 * C::TILES_PER_PATCH) * C::ROWS_PER_TILE;
-              } else {
-                patch0 = tile * PPT;
-                y0 = 0;
-              }
-              const uint32_t a_dst = st_base + (g * TILES + tl) * C::A_BYTES;
-              if (ROWSHIFT) {
-                // band of ROWS_PER_TILE + 2 rows starting one row above the tile, shifted by kx - 1 columns;
-                // box order (x, patch, y, plane)
-                tma_load_4d(a_dst, &p.tmA[0], full_bar(stage), (kx - 1) * 8, patch0, y0 - 1, cc * C::NPL);
-              } else if (STRIDE == 1) {
-                tma_load_4d(a_dst, &p.tmA[0], full_bar(stage), (kx - 1) * 8, y0 + ky - 1, patch0, cc * C::NPL);
-              } else {
-                // input x = 2*ox + kx - 1: kx=0 -> odd column ox-1, kx=1 -> even column ox, kx=2 -> odd column ox
-                const int xpar = (kx != 1), ypar = (ky != 1);
-                tma_load_4d(a_dst, &p.tmA[ypar * 2 + xpar], full_bar(stage), (kx == 0) ? -8 : 0,
-                            y0 + ((ky == 0) ? -1 : 0), patch0, cc * C::NPL);
-              }
-            }
-            if (!WRES) {
-              const uint32_t b_dst = st_base + G * TILES * C::A_BYTES;
-              if (ROWSHIFT) {
-#pragma unroll
-                for (int t3 = 0; t3 < 3; ++t3)   // the three ky taps of this (kx, channel chunk) unit
-                  tma_load_2d(b_dst + t3 * C::B_BYTES, &p.tmB, full_bar(stage), ((t3 * 3 + kx) * C::CIN_CHUNKS + cc) * C::KC, 0);
-              } else {
-                tma_load_2d(b_dst + g * C::B_BYTES, &p.tmB, full_bar(stage), kb * C::KC, 0);
-              }
-            }
-          }
-          ++kb;
-          if (++cc == C::CIN_CHUNKS) {
-            cc = 0;
-            if (++kx == 3) { kx = 0; ++ky; }
-          }
-        }
-        __syncwarp();
-        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-      }
-    }
-  } else if (warp == 1) {
-    // ============================== UMMA issuer (warp-uniform) ==============================
-    // The k-loop is fully unrolled: taps, channel chunks and k-steps are compile-time constants, so every descriptor
-    // is `stage base (one multiply-add per stage) + constant` in its lo word; the hi words never change.
-    const uint32_t idesc = make_idesc_f16(kTileM, N, p.act_bf16);
-    constexpr uint32_t A_HI = noswizzle_desc_hi(128);
-    constexpr uint32_t B_HI = kmajor_desc_hi(C::KCB);
-    const uint32_t ring_a_lo = noswizzle_desc_lo(ring_base, C::PLANE_BYTES);
-    const uint32_t ring_b_lo = kmajor_desc_lo(ring_base + G * TILES * C::A_BYTES);   // streamed weights live behind the A tiles
-    const uint32_t w_lo = kmajor_desc_lo(w_base);
-    if (WRES) {
-      mbar_wait(w_bar, 0);
-      tc_fence_after();
-    }
-    int stage = 0;
-    uint32_t phase = 0;
-    int it = 0;
-    for (int grp = blockIdx.x; grp < num_groups; grp += gridDim.x, ++it) {
-      const int acc = it & 1;
-      const uint32_t acc_phase = (it >> 1) & 1;
-      mbar_wait(tempty_bar(acc), acc_phase ^ 1u);
-      tc_fence_after();
-      const uint32_t d_tmem = tmem_base + acc * (TILES * N);
-#pragma unroll
-      for (int s = 0; s < C::SPT; ++s) {
-        mbar_wait(full_bar(stage), phase);
-        tc_fence_after();
-        if (elect_one()) {
-          const uint32_t st_off = static_cast<uint32_t>(stage) * (C::STAGE_BYTES >> 4);
-          const uint32_t a_lo = ring_a_lo + st_off;
-          const uint32_t b_lo = WRES ? w_lo : ring_b_lo + st_off;
-#pragma unroll
-          for (int g = 0; g < G; ++g) {
-            if (ROWSHIFT) {
-              const int u = s * G + g;                              // load unit = (kx, channel chunk)
-              const int kx = u / C::CIN_CHUNKS, cc = u - kx * C::CIN_CHUNKS;
-#pragma unroll
-              for (int ky = 0; ky < 3; ++ky) {
-                const uint32_t b_off = WRES ? ((((ky * 3 + kx) * C::CIN_CHUNKS + cc) * C::B_BYTES) >> 4) : ((ky * C::B_BYTES) >> 4);
-#pragma unroll
-                for (int tl = 0; tl < TILES; ++tl) {
-#pragma unroll
-                  for (int k = 0; k < C::KCB / 32; ++k)
-                    umma_f16_w(d_tmem + tl * N,
-                               a_lo + (((g * TILES + tl) * C::A_BYTES + ky * C::ROW_BYTES + 2 * k * C::PLANE_BYTES) >> 4), A_HI,
-                               b_lo + b_off + 2 * k, B_HI, idesc, (s | g | ky | k) != 0);
-                }
-              }
-            } else {
-#pragma unroll
-              for (int tl = 0; tl < TILES; ++tl) {
-#pragma unroll
-                for (int k = 0; k < C::KCB / 32; ++k) {
-                  // A: 16 K-elements = two 8-channel planes; B: 32 bytes inside the swizzle span = +2 in the (addr >> 4) field
-                  umma_f16_w(d_tmem + tl * N, a_lo + (((g * TILES + tl) * C::A_BYTES + 2 * k * C::PLANE_BYTES) >> 4), A_HI,
-                             b_lo + (((WRES ? (s * G + g) : g) * C::B_BYTES) >> 4) + 2 * k, B_HI, idesc, (s | g | k) != 0);
-                }
-              }
-            }
-          }
-          umma_commit(empty_bar(stage));                        // frees the smem slot once these MMAs have read it
-          if (s == C::SPT - 1) umma_commit(tfull_bar(acc));     // accumulators complete -> epilogue
-        }
-        __syncwarp();
-        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-      }
-    }
-  } else {
-    // ============================== epilogue ==============================
-    const int q = warp & 3;  // TMEM lane quarter this warp may touch
-    const int row_in_tile = q * 32 + lane;
-    const long long total_patches = p.total_rows / C::PIX;
-    int it = 0;
-    for (int grp = blockIdx.x; grp < num_groups; grp += gridDim.x, ++it) {
-      const int acc = it & 1;
-      const uint32_t acc_phase = (it >> 1) & 1;
-      mbar_wait(tfull_bar(acc), acc_phase);
-      tc_fence_after();
-#pragma unroll
-      for (int tl = 0; tl < TILES; ++tl) {
-        const int tile = grp * TILES + tl;
-        const uint32_t t_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + acc * (TILES * N) + tl * N;
-        // which output pixel this accumulator row is
-        long long patch;
-        int pix;
-        if (ROWSHIFT && PPT > 1) {   // rows ordered (y, patch, x)
-          patch = static_cast<long long>(tile) * PPT + (row_in_tile / HOUT) % PPT;
-          pix = (row_in_tile / (HOUT * PPT)) * HOUT + row_in_tile % HOUT;
-        } else {                     // rows ordered (patch, y, x)
-          const long long row = static_cast<long long>(tile) * kTileM + row_in_tile;
-          patch = row / C::PIX;
-          pix = static_cast<int>(row - patch * C::PIX);
-        }
-        const bool valid = patch < total_patches;
-        // channel-planar output: [patch][plane][pixel slot][8]; consecutive lanes = consecutive pixels = consecutive 16 B
-        const int slot = planar_pixel_slot<HOUT, OUT_PARITY>(pix / HOUT, pix % HOUT);
-        uint4* dst = reinterpret_cast<uint4*>(static_cast<uint16_t*>(p.out) + patch * (static_cast<long long>(N) * C::PIX)) + slot;
-#pragma unroll
-        for (int c0 = 0; c0 < N; c0 += 32) {
-          uint32_t r[32];
-          tmem_ld32(t_row + c0, r);
-          tmem_ld_wait();
-          uint32_t o[16];
-#pragma unroll
-          for (int j = 0; j < 16; ++j)
-            o[j] = pack16_relu(__uint_as_float(r[2 * j]) + p.bias_v[c0 + 2 * j], __uint_as_float(r[2 * j + 1]) + p.bias_v[c0 + 2 * j + 1],
-                               p.act_bf16);
-          if (valid) {
-#pragma unroll
-            for (int j = 0; j < 4; ++j) dst[(c0 / 8 + j) * C::PIX] = make_uint4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
-          }
-        }
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(tempty_bar(acc));
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, C::TMEM_COLS);
-  }
 }
 
 // ------------------------------------------------------------------------------------------------------------

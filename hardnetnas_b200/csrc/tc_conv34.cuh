@@ -3,36 +3,30 @@
 // with the 32 KB/patch activation between them resident in shared memory (never written to HBM: the two layers as
 // separate kernels move 96 + 64 KB per patch, this kernel 64 + 32 KB).
 //
-// Two kernels live here. conv34_stack_kernel (second half of the file) is the DEFAULT: conv4's kx taps stacked on N.
-// conv34_pair_kernel (first half, HN_FUSE34=1 / 2) was the first version and is kept as the bit-exact cross-check of the
-// layer arithmetic (mode 1 reproduces the two separate kernels bit for bit) and as the record of why the default looks the
-// way it does: it is bound by the shared-memory pipe.
-//
-// Common to both. Work split: a CTA pair (tcgen05.mma.cta_group::2, M = 256) works on TWO patches at a time, one per CTA. A 16 x 16
+// Work split: a CTA pair (tcgen05.mma.cta_group::2, M = 256) works on TWO patches at a time, one per CTA. A 16 x 16
 // output map is two 128-pixel tiles (image rows 0-7 / 8-15); an MMA covers tile t of both CTAs' patches. Each CTA keeps
-// half of the weight rows of BOTH layers resident (18 + 36 KB), as in conv3x3_pair_kernel.
+// half of the weight rows of BOTH layers resident, as in conv3x3_pair_kernel.
 //
-// conv3 (stride 2) reads the parity-planar conv2 output through TMA exactly like conv3x3_kernel. Two load schemes:
-//   SIX = false: one 8 KB box per tap (9 loads per tile);
-//   SIX = true : one 9 KB box per (row parity, kx) - rows y0-1 .. y0+7 of a parity sub-plane, shifted by the kx column
-//                offset; the ky taps of that parity are descriptor offsets of whole image rows (6 loads per tile, 108
-//                instead of 144 KB per patch through the SM's L2 port).
-// First version (conv34_pair_kernel):
-// conv3's epilogue (bias + ReLU + 16-bit pack) does not store to global memory: it writes the activation into the `mid`
-// region of shared memory in the channel-planar layout = UMMA no-swizzle K-major operand, [plane][row -1..16][16 px][8 ch],
-// THREE times: as is, shifted one pixel right and one pixel left (the halo rows and the border column of the shifted copies
-// are zeroed once and never written = the conv's zero padding). conv4's nine taps are then pure descriptor offsets:
-// copy = kx, start row = ky. (A shifted start address alone cannot express the x taps: a 16-pixel image row is two whole
-// core matrices, so a one-pixel shift would wrap into the neighbouring row.)
+// conv3 (stride 2) reads the parity-planar conv2 output through TMA: one 9 KB box per (row parity, kx) - rows y0-1 .. y0+7
+// of a parity sub-plane, shifted by the kx column offset; the ky taps of that parity are descriptor offsets of whole image
+// rows (6 loads per tile). conv3's epilogue (bias + ReLU + 16-bit pack) does not store to global memory: it writes the
+// activation into shared memory in the channel-planar layout = UMMA no-swizzle K-major operand, [plane][row -1..16][16 px][8 ch]
+// (the halo rows are zeroed once and never written = the conv's zero padding in y).
 //
-// Schedule of the single issuing thread (leader CTA), per pair of patches i:
-//     conv4(i)  [72 MMAs]   then   conv3(i + 2)  [36 MMAs]     (SCHED > 0: that many of conv3's tile-0 load units are dealt
-//                                                               between the six (tile, kx) groups of conv4)
-// and of the eight epilogue warps of each CTA:
-//     wait conv4(i - 1) retired (= mid free)  ->  conv3 epilogue of i (TMEM -> mid)  ->  signal "mid ready"  ->
-//     conv4 epilogue of i - 1 (TMEM -> global)
-// so the conv3 epilogue of patch i runs while the tensor pipe works on conv3(i + 1), and the conv4 epilogue overlaps
-// everything. Tensor memory: 2 x (2 tiles x 64 columns) for conv3 + the same for conv4 = 512 columns.
+// conv4's kx taps are STACKED ON N: the three kx taps share ONE read of the activation. Per ky the weights are a
+// [192 = kx * 64 + c_out][64] tile, an MMA has N = 192 (96 clk of math for 4 KB of A; with one N = 64 MMA per tap the kernel
+// was bound by the shared-memory pipe), and the conv is finished behind the MMAs:  out[y][x] = D0[y][x - 1] + D1[y][x] + D2[y][x + 1].
+// An accumulator lane is a pixel and a 32-lane quarter is two image rows, so D2 is moved one lane down inside tensor memory
+// (tcgen05.shift, a dedicated warp, once the tile's MMAs have retired) and D0 one lane up by warp shuffles in the epilogue;
+// the row ends are masked = the conv's zero padding in x.
+// Shared memory holds the activation double-buffered by patch (the conv3 epilogue of group i + 1 never waits for conv4 of
+// group i) and a TMA ring of 11 boxes. Tensor memory: conv3 2 tiles x 64 columns (a tile's buffer is handed back as soon as
+// the epilogue has read it) + conv4 2 tiles x 192 = 512.
+//
+// Issue order per group i of two patches:  conv3(i + 1) tile 0,  conv4(i) tile 0,  conv3(i + 1) tile 1,  conv4(i) tile 1
+// (the TMA ring drains in bursts of 6 of its 11 boxes).
+// Warps (20): 0 and 3 TMA producers (tile 0 / tile 1 boxes), 1 issuer / TMEM owner, 2 shifter, 4..19 epilogue: (tile, lane
+// quarter, 32-channel half) each.
 #pragma once
 
 #include "common.cuh"
@@ -67,362 +61,6 @@ static __device__ unsigned long long hn_c34_trace[16];
 #define C34_ACC(slot) do { } while (0)
 #endif
 
-constexpr int kC34Threads = 320;   // warp 0: TMA producer, warp 1: issuer / TMEM owner, warps 2..9: epilogue
-
-struct Conv34Params {
-  CUtensorMap tmA[4];   // conv2 output, parity views [ypar * 2 + xpar], box (16 px * 8, ROWS, 1 patch, 4 planes)
-  CUtensorMap tmB3;     // conv3 weights [64][9 * 32], box (32, 32 rows), 64B swizzle
-  CUtensorMap tmB4;     // conv4 weights [64][9 * 64], box (64, 32 rows), 128B swizzle
-  float bias3[64];      // folded BN shifts, by value (constant bank)
-  float bias4[64];
-  void* out;            // conv4 output, channel-planar parity layout [patch][8 planes][ypar][xpar][8][8][8]
-  int n_patches;
-  int act_bf16;
-};
-
-template <bool SIX>
-struct C34Cfg {
-  static constexpr int UNITS = SIX ? 6 : 9;             // TMA loads per conv3 tile
-  static constexpr int ROWS = SIX ? 9 : 8;              // image rows per load
-  static constexpr uint32_t A3_PLANE = ROWS * 256;      // [plane][row][16 px][8 ch]
-  static constexpr uint32_t A3_BYTES = 4 * A3_PLANE;
-  static constexpr int STAGES = 7;
-  static constexpr uint32_t W3_BLK = 32 * 64;           // this CTA's 32 output channels x one tap x 32 input channels
-  static constexpr uint32_t W4_BLK = 32 * 128;          // ... x 64 input channels
-  static constexpr uint32_t W3_BYTES = 9 * W3_BLK, W4_BYTES = 9 * W4_BLK;
-  static constexpr uint32_t MID_PLANE = 18 * 256;       // image rows -1 .. 16
-  static constexpr uint32_t MID_COPY = 8 * MID_PLANE;   // 64 channels
-  static constexpr uint32_t MID_BYTES = 3 * MID_COPY;
-  static constexpr size_t SMEM = size_t(W3_BYTES) + W4_BYTES + MID_BYTES + size_t(STAGES) * A3_BYTES + 1024 + 256;
-  static_assert(SMEM <= 227 * 1024, "shared memory budget");
-};
-
-template <bool SIX, int SCHED>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kC34Threads, 1)
-conv34_pair_kernel(const __grid_constant__ Conv34Params p) {
-  using C = C34Cfg<SIX>;
-  constexpr int STAGES = C::STAGES;
-
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t raw_addr = smem_u32(smem_raw);
-  const uint32_t base = (raw_addr + 1023u) & ~1023u;   // identical in both CTAs
-  const uint32_t w3_base = base;
-  const uint32_t w4_base = w3_base + C::W3_BYTES;
-  const uint32_t mid_base = w4_base + C::W4_BYTES;
-  const uint32_t ring_base = mid_base + C::MID_BYTES;
-  const uint32_t bar_base = ring_base + STAGES * C::A3_BYTES;
-  auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (STAGES + s); };
-  auto t3full_bar = [&](int b) { return bar_base + 8u * (2 * STAGES + b); };
-  auto t4full_bar = [&](int b) { return bar_base + 8u * (2 * STAGES + 2 + b); };
-  auto t4empty_bar = [&](int b) { return bar_base + 8u * (2 * STAGES + 4 + b); };
-  const uint32_t mid_bar = bar_base + 8u * (2 * STAGES + 6);
-  const uint32_t w_bar = bar_base + 8u * (2 * STAGES + 7);
-  const uint32_t tmem_slot = bar_base + 8u * (2 * STAGES + 8);
-  volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(smem_raw + (tmem_slot - raw_addr));
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int pr = blockIdx.x >> 1, num_pairs = gridDim.x >> 1;
-  const int num_groups = (p.n_patches + 1) / 2;                    // a group = two consecutive patches, one per CTA
-  const int n_it = (num_groups - pr + num_pairs - 1) / num_pairs;  // groups of this pair (the host launches <= num_groups pairs)
-
-#ifdef HN_C34_TRACE
-  const long long c34_start = clock64();
-#endif
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&p.tmA[0]);
-    tma_prefetch_desc(&p.tmA[1]);
-    tma_prefetch_desc(&p.tmA[2]);
-    tma_prefetch_desc(&p.tmA[3]);
-    tma_prefetch_desc(&p.tmB3);
-    tma_prefetch_desc(&p.tmB4);
-  }
-  if (warp == 1) {
-    if (lane == 0) {
-      for (int s = 0; s < STAGES; ++s) {
-        mbar_init(full_bar(s), 2);    // one arrive.expect_tx per CTA of the pair (leader's copy)
-        mbar_init(empty_bar(s), 1);   // multicast tcgen05.commit
-      }
-      for (int b = 0; b < 2; ++b) {
-        mbar_init(t3full_bar(b), 1);    // multicast tcgen05.commit
-        mbar_init(t4full_bar(b), 1);    // multicast tcgen05.commit
-        mbar_init(t4empty_bar(b), 16);  // eight epilogue warps of each CTA (leader's copy)
-      }
-      mbar_init(mid_bar, 16);           // eight epilogue warps of each CTA (leader's copy)
-      mbar_init(w_bar, 2);
-      fence_mbar_init();
-    }
-    __syncwarp();
-    tmem_alloc_pair(tmem_slot, 512);
-    tmem_relinquish_pair();
-  }
-  // zero the mid region once: halo rows and the border columns of the shifted copies stay zero for the whole launch
-  {
-    uint4* mid = reinterpret_cast<uint4*>(smem_raw + (mid_base - raw_addr));
-    for (uint32_t i = threadIdx.x; i < C::MID_BYTES / 16; i += kC34Threads) mid[i] = make_uint4(0u, 0u, 0u, 0u);
-    fence_proxy_async_smem();
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();   // the peer's barriers are initialised and its TMEM is allocated before anyone signals it
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot_ptr;
-
-  if (warp == 0) {
-    // ============================== TMA producer (both CTAs, warp-uniform) ==============================
-    const uint32_t lead_w_bar = mapa_cluster(w_bar, 0);
-    if (elect_one()) {
-      mbar_arrive_expect_tx_cluster(lead_w_bar, C::W3_BYTES + C::W4_BYTES);
-#pragma unroll 1
-      for (int kb = 0; kb < 9; ++kb) tma_load_2d_pair(w3_base + kb * C::W3_BLK, &p.tmB3, lead_w_bar, kb * 32, static_cast<int>(rank) * 32);
-#pragma unroll 1
-      for (int kb = 0; kb < 9; ++kb) tma_load_2d_pair(w4_base + kb * C::W4_BLK, &p.tmB4, lead_w_bar, kb * 64, static_cast<int>(rank) * 32);
-    }
-    __syncwarp();
-    int stage = 0;
-    uint32_t phase = 0;
-    for (int it = 0; it < n_it; ++it) {
-      // a patch index past the batch reads stale or out-of-range (zero-filled) data; its results are never stored
-      const int patch = 2 * (pr + it * num_pairs) + static_cast<int>(rank);
-#pragma unroll 1
-      for (int tu = 0; tu < 2 * C::UNITS; ++tu) {
-        const int t = tu / C::UNITS, u = tu - t * C::UNITS;
-        const int y0 = 8 * t;
-        C34_WAIT(9, empty_bar(stage), phase ^ 1u);
-        if (elect_one()) {
-          const uint32_t lead_full = mapa_cluster(full_bar(stage), 0);
-          const uint32_t a_dst = ring_base + stage * C::A3_BYTES;
-          mbar_arrive_expect_tx_cluster(lead_full, C::A3_BYTES);
-          if (SIX) {
-            // u = yp * 3 + kx: yp 0 = odd input rows (taps ky 0 and 2), yp 1 = even input rows (tap ky 1)
-            const int yp = u / 3, kx = u - yp * 3;
-            const int xpar = (kx != 1), ypar = (yp == 0);
-            tma_load_4d_pair(a_dst, &p.tmA[ypar * 2 + xpar], lead_full, (kx == 0) ? -8 : 0, y0 - 1, patch, 0);
-          } else {
-            // input x = 2*ox + kx - 1: kx=0 -> odd column ox-1, kx=1 -> even column ox, kx=2 -> odd column ox
-            const int ky = u / 3, kx = u - ky * 3;
-            const int xpar = (kx != 1), ypar = (ky != 1);
-            tma_load_4d_pair(a_dst, &p.tmA[ypar * 2 + xpar], lead_full, (kx == 0) ? -8 : 0, y0 + ((ky == 0) ? -1 : 0), patch, 0);
-          }
-        }
-        __syncwarp();
-        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-      }
-    }
-  } else if (warp == 1) {
-    // ============================== UMMA issuer (leader CTA only, warp-uniform) ==============================
-    if (rank == 0) {
-      const uint32_t idesc = make_idesc_f16(2 * kTileM, 64, p.act_bf16);
-      constexpr uint32_t A_HI = noswizzle_desc_hi(128);
-      constexpr uint32_t B3_HI = kmajor_desc_hi(64);
-      constexpr uint32_t B4_HI = kmajor_desc_hi(128);
-      const uint32_t ring_a_lo = noswizzle_desc_lo(ring_base, C::A3_PLANE);
-      const uint32_t mid_a_lo = noswizzle_desc_lo(mid_base, C::MID_PLANE);
-      const uint32_t w3_lo = kmajor_desc_lo(w3_base);
-      const uint32_t w4_lo = kmajor_desc_lo(w4_base);
-      mbar_wait(w_bar, 0);
-      tc_fence_after();
-      int stage = 0;
-      uint32_t phase = 0;
-      // one load unit of conv3: wait for its box, issue its 2 - 4 MMAs, hand the slot back
-      auto conv3_unit = [&](auto t_c, auto u_c, int b) {
-        constexpr int t = decltype(t_c)::value, u = decltype(u_c)::value;
-        const uint32_t d_tmem = tmem_base + b * 128 + t * 64;
-        C34_WAIT(0, full_bar(stage), phase);
-        tc_fence_after();
-        if (elect_one()) {
-          const uint32_t a_lo = ring_a_lo + static_cast<uint32_t>(stage) * (C::A3_BYTES >> 4);
-          if constexpr (SIX) {
-            constexpr int yp = u / 3, kx = u - yp * 3;
-            if constexpr (yp == 0) {
-#pragma unroll
-              for (int kyi = 0; kyi < 2; ++kyi) {   // ky = 0 (rows y0-1 ..) and ky = 2 (rows y0 ..)
-                const int ky = 2 * kyi;
-#pragma unroll
-                for (int k = 0; k < 2; ++k)
-                  umma_f16_pair_w(d_tmem, a_lo + ((kyi * 256 + 2 * k * C::A3_PLANE) >> 4), A_HI,
-                                  w3_lo + (((ky * 3 + kx) * C::W3_BLK) >> 4) + 2 * k, B3_HI, idesc, (u | kyi | k) != 0);
-              }
-            } else {
-#pragma unroll
-              for (int k = 0; k < 2; ++k)
-                umma_f16_pair_w(d_tmem, a_lo + ((256 + 2 * k * C::A3_PLANE) >> 4), A_HI, w3_lo + (((3 + kx) * C::W3_BLK) >> 4) + 2 * k,
-                                B3_HI, idesc, 1u);
-            }
-          } else {
-#pragma unroll
-            for (int k = 0; k < 2; ++k)
-              umma_f16_pair_w(d_tmem, a_lo + ((2 * k * C::A3_PLANE) >> 4), A_HI, w3_lo + ((u * C::W3_BLK) >> 4) + 2 * k, B3_HI, idesc,
-                              (u | k) != 0);
-          }
-          umma_commit_pair(empty_bar(stage));
-          if (t == 1 && u == C::UNITS - 1) umma_commit_pair(t3full_bar(b));
-        }
-        __syncwarp();
-        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-      };
-      // one (tile, kx) group of conv4: 12 MMAs on the resident mid copies
-      auto conv4_group = [&](auto g_c, int b) {
-        constexpr int g = decltype(g_c)::value, t = g / 3, kx = g - 3 * t;
-        if (elect_one()) {
-          const uint32_t d_tmem = tmem_base + 256 + b * 128 + t * 64;
-#pragma unroll
-          for (int ky = 0; ky < 3; ++ky) {
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-              umma_f16_pair_w(d_tmem, mid_a_lo + ((kx * C::MID_COPY + (8 * t + ky) * 256 + 2 * k * C::MID_PLANE) >> 4), A_HI,
-                              w4_lo + (((ky * 3 + kx) * C::W4_BLK) >> 4) + 2 * k, B4_HI, idesc, (kx | ky | k) != 0);
-          }
-          if (g == 5) umma_commit_pair(t4full_bar(b));
-        }
-        __syncwarp();
-      };
-      // Virtual iteration j: conv4 of group j (j >= 0) and conv3 of group j + 2. ILV of the conv3 tile-0 load units are dealt
-      // between the six conv4 groups (the TMA ring then drains steadily instead of in one burst of 2 * UNITS boxes); the
-      // rest follows conv4 and covers the conv3 epilogue of group j + 1, which can only start once conv4(j) has retired.
-      constexpr int ILV = SCHED < C::UNITS ? SCHED : C::UNITS;
-      for (int j = -2; j < n_it; ++j) {
-        const int b = j & 1;   // = (j + 2) & 1
-        const bool do4 = j >= 0, do3 = j + 2 < n_it;
-        if (do4) {
-          C34_WAIT(2, t4empty_bar(b), ((j >> 1) & 1) ^ 1u);   // conv4 epilogue of group j - 2 has drained this accumulator
-          C34_WAIT(1, mid_bar, j & 1);                        // conv3 epilogue of group j has written mid (both CTAs)
-          tc_fence_after();
-        }
-        static_for<6>([&](auto g_c) {
-          constexpr int g = decltype(g_c)::value;
-          if (do4) conv4_group(g_c, b);
-          if (do3) {
-            static_for<C::UNITS>([&](auto u_c) {
-              constexpr int u = decltype(u_c)::value;
-              if constexpr (u < ILV && u * 6 / (ILV ? ILV : 1) == g) conv3_unit(std::integral_constant<int, 0>{}, u_c, b);
-            });
-          }
-        });
-        if (do3) {
-          static_for<C::UNITS>([&](auto u_c) {
-            if constexpr (decltype(u_c)::value >= ILV) conv3_unit(std::integral_constant<int, 0>{}, u_c, b);
-          });
-          static_for<C::UNITS>([&](auto u_c) { conv3_unit(std::integral_constant<int, 1>{}, u_c, b); });
-        }
-      }
-    }
-  } else {
-    // ============================== epilogue (both CTAs, each its own patch) ==============================
-    const int e = warp - 2;
-    const int q = warp & 3;    // TMEM lane quarter this warp may touch
-    const int t = e >> 2;      // tile (image rows 8t .. 8t + 7)
-    const int y = 8 * t + 2 * q + (lane >> 4), x = lane & 15;
-    const uint32_t lead_mid_bar = mapa_cluster(mid_bar, 0);
-    uint8_t* mid_px = smem_raw + (mid_base - raw_addr) + (y + 1) * 256 + x * 16;   // this pixel in copy 0 (kx = 0), plane 0
-    const int out_slot = planar_pixel_slot<16, true>(y, x);
-
-    auto epilogue4 = [&](int it) {
-      const int b = it & 1;
-      const long long patch = 2ll * (pr + it * num_pairs) + rank;
-      const bool valid = patch < p.n_patches;
-      const uint32_t t_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + 256 + b * 128 + t * 64;
-      uint4* dst = reinterpret_cast<uint4*>(static_cast<uint16_t*>(p.out) + patch * (64ll * 256)) + out_slot;
-#pragma unroll
-      for (int c0 = 0; c0 < 64; c0 += 32) {
-        uint32_t r[32];
-        tmem_ld32(t_row + c0, r);
-        tmem_ld_wait();
-        uint32_t o[16];
-#pragma unroll
-        for (int j = 0; j < 16; ++j)
-          o[j] = pack16_relu(__uint_as_float(r[2 * j]) + p.bias4[c0 + 2 * j], __uint_as_float(r[2 * j + 1]) + p.bias4[c0 + 2 * j + 1], p.act_bf16);
-        if (valid) {
-#pragma unroll
-          for (int j = 0; j < 4; ++j) dst[(c0 / 8 + j) * 256] = make_uint4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
-        }
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(mapa_cluster(t4empty_bar(b), 0));
-    };
-
-    for (int it = 0; it < n_it; ++it) {
-      const int b = it & 1;
-      if (e == 0) {
-        C34_WAIT(5, t3full_bar(b), (it >> 1) & 1);
-        if (it > 0) C34_WAIT(6, t4full_bar((it - 1) & 1), ((it - 1) >> 1) & 1);
-      }
-      mbar_wait(t3full_bar(b), (it >> 1) & 1);                                  // conv3 accumulators of group `it`
-      if (it > 0) mbar_wait(t4full_bar((it - 1) & 1), ((it - 1) >> 1) & 1);     // conv4 of the previous group retired: mid is free
-      tc_fence_after();
-      C34_T0();
-      {
-        const uint32_t t_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + b * 128 + t * 64;
-#pragma unroll
-        for (int c0 = 0; c0 < 64; c0 += 32) {
-          uint32_t r[32];
-          tmem_ld32(t_row + c0, r);
-          tmem_ld_wait();
-          uint32_t o[16];
-#pragma unroll
-          for (int j = 0; j < 16; ++j)
-            o[j] = pack16_relu(__uint_as_float(r[2 * j]) + p.bias3[c0 + 2 * j], __uint_as_float(r[2 * j + 1]) + p.bias3[c0 + 2 * j + 1], p.act_bf16);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const uint4 v = make_uint4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
-            uint8_t* d = mid_px + (c0 / 8 + j) * C::MID_PLANE;
-            *reinterpret_cast<uint4*>(d + C::MID_COPY) = v;                           // kx = 1: in[x]
-            if (x < 15) *reinterpret_cast<uint4*>(d + 16) = v;                        // kx = 0 reads in[x - 1]
-            if (x > 0) *reinterpret_cast<uint4*>(d + 2 * C::MID_COPY - 16) = v;       // kx = 2 reads in[x + 1]
-          }
-        }
-      }
-      fence_proxy_async_smem();   // generic-proxy writes -> visible to the tensor cores (async proxy)
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(lead_mid_bar);
-      if (e == 0) C34_ACC(7);
-      if (it > 0) epilogue4(it - 1);
-      if (e == 0) C34_ACC(8);
-    }
-    mbar_wait(t4full_bar((n_it - 1) & 1), ((n_it - 1) >> 1) & 1);
-    tc_fence_after();
-    epilogue4(n_it - 1);
-  }
-
-  // nobody leaves (and frees shared / tensor memory) while the peer may still read it or signal its barriers
-  tc_fence_before();
-  __syncthreads();
-#ifdef HN_C34_TRACE
-  if (blockIdx.x == 0 && threadIdx.x == 0) {
-    atomicAdd(&hn_c34_trace[3], static_cast<unsigned long long>(clock64() - c34_start));
-    atomicAdd(&hn_c34_trace[4], static_cast<unsigned long long>(n_it));
-  }
-#endif
-  cluster_sync_all();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc_pair(tmem_base, 512);
-  }
-}
-
-
-// ------------------------------------------------------------------------------------------------------------
-// Second version: conv4's kx taps STACKED ON N.
-// ------------------------------------------------------------------------------------------------------------
-// The kernel above is bound by the shared-memory pipe (~97 % busy): an N = 64 MMA reads 4 KB of A for 32 clk of math, and
-// conv4 reads the resident activation nine times (once per tap). Here the three kx taps share ONE read of the unshifted
-// activation: per ky the weights are a [192 = kx * 64 + c_out][64] tile, an MMA has N = 192 (96 clk of math for the same
-// 4 KB of A), and the conv is finished behind the MMAs:  out[y][x] = D0[y][x - 1] + D1[y][x] + D2[y][x + 1].
-// An accumulator lane is a pixel and a 32-lane quarter is two image rows, so D2 is moved one lane down inside tensor memory
-// (tcgen05.shift, a dedicated warp, once the tile's MMAs have retired) and D0 one lane up by warp shuffles in the epilogue;
-// the row ends are masked = the conv's zero padding in x.
-// Shared memory then holds ONE copy of the activation, double-buffered by patch (the conv3 epilogue of group i + 1 never
-// waits for conv4 of group i), and the TMA ring grows from 7 to 11 boxes. Tensor memory: conv3 2 tiles x 64 columns
-// (a tile's buffer is handed back as soon as the epilogue has read it) + conv4 2 tiles x 192 = 512.
-//
-// Issue order per group i of two patches:  conv3(i + 1) tile 0,  conv4(i) tile 0,  conv3(i + 1) tile 1,  conv4(i) tile 1
-// (the TMA ring drains in bursts of 6 of its 11 boxes).
-// Warps (20): 0 and 3 TMA producers (tile 0 / tile 1 boxes), 1 issuer / TMEM owner, 2 shifter, 4..19 epilogue: (tile, lane
-// quarter, 32-channel half) each.
 constexpr int kC34SThreads = 20 * 32;
 
 __device__ __forceinline__ void tmem_ld16_c34(uint32_t taddr, uint32_t (&r)[16]) {
@@ -447,16 +85,12 @@ struct C34SCfg {
   static constexpr uint32_t MID_PLANE = 18 * 256;       // image rows -1 .. 16
   static constexpr uint32_t MID_BUF = 8 * MID_PLANE;    // 64 channels
   static constexpr uint32_t MID_BYTES = 2 * MID_BUF;
-  static constexpr size_t SMEM = size_t(W3_BYTES) + W4_BYTES + MID_BYTES + size_t(STAGES) * A3_BYTES + 1024 + 320;   // 35 barriers
+  static constexpr size_t SMEM = size_t(W3_BYTES) + W4_BYTES + MID_BYTES + size_t(STAGES) * A3_BYTES + 1024 + 320;   // 34 barriers + TMEM slot
   static_assert(SMEM <= 227 * 1024, "shared memory budget");
 };
 
-// The kernel body as a device function: CTA `blk` of `nblk` (whole pairs) - the stand-alone kernel passes blockIdx.x / gridDim.x,
-// the co-scheduled front + conv3/conv4 launch (front_c34.cuh) gives this role the tail of its grid. ready != nullptr: the conv2
-// output of patch i is being produced by the front role of the SAME launch; the producer warp polls the eight flags
-// ready[i * 8 ..] (acquire at gpu scope) before the patch's first TMA load and clears them for the next launch.
-template <int SHFL16, int NPROD>   // SHFL16 = 1: D0 crosses lanes as fp16 pairs (half the shuffles; fp16 activations only)
-__device__ __forceinline__ void conv34_stack_body(const Conv34Params& p, const int blk, const int nblk, int* __restrict__ ready) {
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kC34SThreads, 1)
+conv34_stack_kernel(const __grid_constant__ Conv34Params p) {
   using C = C34SCfg;
   constexpr int STAGES = C::STAGES;
 
@@ -477,14 +111,13 @@ __device__ __forceinline__ void conv34_stack_body(const Conv34Params& p, const i
   auto mma4_bar = [&](int t) { return bar_base + 8u * (2 * STAGES + 8 + t); };
   const uint32_t mid_bar = bar_base + 8u * (2 * STAGES + 10);
   const uint32_t w_bar = bar_base + 8u * (2 * STAGES + 11);
-  const uint32_t pready_bar = bar_base + 8u * (2 * STAGES + 12);   // co-scheduled launch: producer 0 -> producer 1, "the patch is in global memory"
-  const uint32_t tmem_slot = bar_base + 8u * (2 * STAGES + 13);
+  const uint32_t tmem_slot = bar_base + 8u * (2 * STAGES + 12);
   volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(smem_raw + (tmem_slot - raw_addr));
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
-  const int pr = blk >> 1, num_pairs = nblk >> 1;
+  const int pr = blockIdx.x >> 1, num_pairs = gridDim.x >> 1;
   const int num_groups = (p.n_patches + 1) / 2;                    // a group = two consecutive patches, one per CTA
   const int n_it = pr < num_groups ? (num_groups - pr + num_pairs - 1) / num_pairs : 0;  // groups of this pair
 
@@ -514,7 +147,6 @@ __device__ __forceinline__ void conv34_stack_body(const Conv34Params& p, const i
       }
       mbar_init(mid_bar, 32);            // sixteen epilogue warps of each CTA (leader's copy)
       mbar_init(w_bar, 2);
-      mbar_init(pready_bar, 1);
       fence_mbar_init();
     }
     __syncwarp();
@@ -535,8 +167,8 @@ __device__ __forceinline__ void conv34_stack_body(const Conv34Params& p, const i
 
   if (warp == 0 || warp == 3) {
     // ============================== TMA producers (both CTAs, warp-uniform) ==============================
-    // NPROD = 2: warp 0 loads the boxes of tile 0, warp 3 those of tile 1 (a cp.async.bulk.tensor issue blocks its thread until
-    // the TMA unit has taken the request; two threads keep two requests in flight). Ring slots are dealt in load order.
+    // Warp 0 loads the boxes of tile 0, warp 3 those of tile 1 (a cp.async.bulk.tensor issue blocks its thread until the TMA
+    // unit has taken the request; two threads keep two requests in flight). Ring slots are dealt in load order.
     const int pw = warp == 0 ? 0 : 1;
     if (pw == 0) {
       const uint32_t lead_w_bar = mapa_cluster(w_bar, 0);
@@ -555,60 +187,31 @@ __device__ __forceinline__ void conv34_stack_body(const Conv34Params& p, const i
       }
       __syncwarp();
     }
-    if (pw < NPROD) {
-      int stage = (NPROD == 2 && pw == 1) ? C::UNITS : 0;
-      uint32_t phase = 0;
-      for (int it = 0; it < n_it; ++it) {
-        // a patch index past the batch reads stale or out-of-range (zero-filled) data; its results are never stored
-        const int patch = 2 * (pr + it * num_pairs) + static_cast<int>(rank);
-        if (ready != nullptr) {
-          if (pw == 0) {
-            if (patch < p.n_patches) {
-              const int* f = ready + static_cast<size_t>(patch) * 8 + (lane & 7);
-              const uint64_t t0 = globaltimer_ns();
-              uint32_t spins = 0;
-              for (;;) {
-                int v;
-                asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(f) : "memory");
-                if (!__any_sync(0xffffffffu, v != 1)) break;
-                if ((++spins & 255u) == 0 && globaltimer_ns() - t0 > 4000000000ull) {
-                  if (lane == 0) printf("hardnet_b200: conv2 output of patch %d never became ready (block %d)\n", patch, blockIdx.x);
-                  __trap();
-                }
-              }
-              __syncwarp();
-              if (lane < 8) ready[static_cast<size_t>(patch) * 8 + lane] = 0;   // consumed; the next launch stamps it again
-              asm volatile("fence.proxy.async;" ::: "memory");   // generic-proxy writes of the front role -> this CTA's TMA reads
-            }
-            __syncwarp();
-            if (NPROD == 2 && lane == 0) mbar_arrive(pready_bar);
-          } else {
-            mbar_wait(pready_bar, it & 1);
-          }
-        }
+    int stage = pw * C::UNITS;
+    uint32_t phase = 0;
+    for (int it = 0; it < n_it; ++it) {
+      // a patch index past the batch reads stale or out-of-range (zero-filled) data; its results are never stored
+      const int patch = 2 * (pr + it * num_pairs) + static_cast<int>(rank);
 #pragma unroll 1
-        for (int tu = (NPROD == 2 ? pw * C::UNITS : 0); tu < (NPROD == 2 ? (pw + 1) * C::UNITS : 2 * C::UNITS); ++tu) {
-          const int t = tu / C::UNITS, u = tu - t * C::UNITS;
-          C34_WAIT(9, empty_bar(stage), phase ^ 1u);
-          C34_T0();
-          if (elect_one()) {
-            const uint32_t lead_full = mapa_cluster(full_bar(stage), 0);
-            mbar_arrive_expect_tx_cluster(lead_full, C::A3_BYTES);
-            // u = yp * 3 + kx: yp 0 = odd input rows (taps ky 0 and 2), yp 1 = even input rows (tap ky 1);
-            // input x = 2*ox + kx - 1: kx=0 -> odd column ox-1, kx=1 -> even column ox, kx=2 -> odd column ox
-            const int yp = u / 3, kx = u - yp * 3;
-            const int xpar = (kx != 1), ypar = (yp == 0);
-            tma_load_4d_pair(ring_base + stage * C::A3_BYTES, &p.tmA[ypar * 2 + xpar], lead_full, (kx == 0) ? -8 : 0, 8 * t - 1, patch, 0);
-          }
-          __syncwarp();
-          if (pw == 0) C34_ACC(12);
-          if (++stage >= STAGES) { stage -= STAGES; phase ^= 1u; }
+      for (int u = 0; u < C::UNITS; ++u) {
+        C34_WAIT(9, empty_bar(stage), phase ^ 1u);
+        C34_T0();
+        if (elect_one()) {
+          const uint32_t lead_full = mapa_cluster(full_bar(stage), 0);
+          mbar_arrive_expect_tx_cluster(lead_full, C::A3_BYTES);
+          // u = yp * 3 + kx: yp 0 = odd input rows (taps ky 0 and 2), yp 1 = even input rows (tap ky 1);
+          // input x = 2*ox + kx - 1: kx=0 -> odd column ox-1, kx=1 -> even column ox, kx=2 -> odd column ox
+          const int yp = u / 3, kx = u - yp * 3;
+          const int xpar = (kx != 1), ypar = (yp == 0);
+          tma_load_4d_pair(ring_base + stage * C::A3_BYTES, &p.tmA[ypar * 2 + xpar], lead_full, (kx == 0) ? -8 : 0, 8 * pw - 1, patch, 0);
         }
-        if (NPROD == 2) {   // skip the other producer's six slots
-          stage += C::UNITS;
-          if (stage >= STAGES) { stage -= STAGES; phase ^= 1u; }
-        }
+        __syncwarp();
+        if (pw == 0) C34_ACC(12);
+        if (++stage >= STAGES) { stage -= STAGES; phase ^= 1u; }
       }
+      // skip the other producer's six slots
+      stage += C::UNITS;
+      if (stage >= STAGES) { stage -= STAGES; phase ^= 1u; }
     }
   } else if (warp == 1) {
     // ============================== UMMA issuer (leader CTA only, warp-uniform) ==============================
@@ -751,22 +354,10 @@ __device__ __forceinline__ void conv34_stack_body(const Conv34Params& p, const i
           if (lane == 0) mbar_arrive_cluster(lead_t4empty);
         }
         float v[16];
-        if (SHFL16 && !p.act_bf16) {
-          // the left neighbour's partial sums cross lanes as fp16 pairs: one shuffle moves two values (|D| stays far inside the
-          // fp16 range; 2^-11 relative rounding on one of three addends, below the output's own 16-bit rounding)
 #pragma unroll
-          for (int j = 0; j < 16; j += 2) {
-            const uint32_t lp = __shfl_up_sync(0xffffffffu, pack16_plain(__uint_as_float(r0[j]), __uint_as_float(r0[j + 1]), 0), 1);
-            const float2 lf = __half22float2(*reinterpret_cast<const __half2*>(&lp));
-            v[j] = fmaf(__uint_as_float(r2[j]), m_right, fmaf(lf.x, m_left, __uint_as_float(r1[j]) + p.bias4[32 * h + c0 + j]));
-            v[j + 1] = fmaf(__uint_as_float(r2[j + 1]), m_right, fmaf(lf.y, m_left, __uint_as_float(r1[j + 1]) + p.bias4[32 * h + c0 + j + 1]));
-          }
-        } else {
-#pragma unroll
-          for (int j = 0; j < 16; ++j) {
-            const float from_left = __shfl_up_sync(0xffffffffu, __uint_as_float(r0[j]), 1);
-            v[j] = fmaf(__uint_as_float(r2[j]), m_right, fmaf(from_left, m_left, __uint_as_float(r1[j]) + p.bias4[32 * h + c0 + j]));
-          }
+        for (int j = 0; j < 16; ++j) {
+          const float from_left = __shfl_up_sync(0xffffffffu, __uint_as_float(r0[j]), 1);
+          v[j] = fmaf(__uint_as_float(r2[j]), m_right, fmaf(from_left, m_left, __uint_as_float(r1[j]) + p.bias4[32 * h + c0 + j]));
         }
         if (valid) {
 #pragma unroll
@@ -825,12 +416,6 @@ __device__ __forceinline__ void conv34_stack_body(const Conv34Params& p, const i
     tc_fence_after();
     tmem_dealloc_pair(tmem_base, 512);
   }
-}
-
-template <int SHFL16, int NPROD>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kC34SThreads, 1)
-conv34_stack_kernel(const __grid_constant__ Conv34Params p) {
-  conv34_stack_body<SHFL16, NPROD>(p, static_cast<int>(blockIdx.x), static_cast<int>(gridDim.x), nullptr);
 }
 
 }  // namespace hn

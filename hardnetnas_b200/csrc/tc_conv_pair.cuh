@@ -1,5 +1,14 @@
-// CTA-pair version of the 3x3 implicit-GEMM convolution (features[6..17], reference hardnet/HardNet.py:287-298):
-// two CTAs of one cluster (= the two SMs of a TPC) run tcgen05.mma.cta_group::2 with M = 256: each CTA owns one
+// The 3x3 convs (features[6..17], reference hardnet/HardNet.py:287-298) as persistent, warp-specialised tcgen05 implicit
+// GEMMs: M = 128 output pixels per tile, N = C_out, K = 9 taps x C_in, cut into "k-blocks" of one tap x <=64 channels.
+// Activations live in global memory CHANNEL-PLANAR: [patch][plane = c / 8][y][x][c % 8] (16 B per pixel and plane; stride-2
+// consumers get the four row/column parity sub-planes [plane][ypar][xpar][y/2][x/2][8]). The A tile of a k-block is ONE 4-D
+// TMA box (x * 8, y, patch, plane) whose start coordinate carries the tap shift; out-of-range x / y are zero-filled by TMA,
+// which is exactly the conv's zero padding, and because x / y are per-patch tensor dimensions nothing bleeds between
+// patches. The box lands in shared memory as [plane][pixel][8 channels], which is the UMMA no-swizzle K-major layout (core
+// matrix = 8 pixels x 16 B, SBO = 128 B, LBO = plane pitch). The planar layout is what makes the epilogue's stores
+// coalesce: a warp writes 32 pixels x 16 B = 512 contiguous bytes per instruction (NHWC rows would touch 32 cache lines).
+//
+// Two CTAs of one cluster (= the two SMs of a TPC) run tcgen05.mma.cta_group::2 with M = 256: each CTA owns one
 // 128-pixel tile (A operand + accumulator in its own shared memory / TMEM) and HALF of the weight rows (B operand,
 // C_out / 2 output channels), and the tensor cores of both SMs read B from both halves.
 //
@@ -9,7 +18,8 @@
 // + half of B (N / 8), i.e. 48 per 64 clk at N = 128, and the weights of a layer fit in shared memory
 // (conv6: 2 x 144 KB) so they are loaded once per CTA instead of streamed per tile.
 //
-// Protocol (same ring / double-buffered accumulator structure as conv3x3_kernel):
+// Protocol (a ring of A tiles and two accumulator buffers in TMEM, so the epilogue of tile i overlaps the MMAs of tile i+1;
+// warp 0 = TMA producer, warp 1 = TMEM owner + UMMA issuer, warps 2..5 = epilogue):
 //   * every CTA's TMA loads land in its own shared memory but complete_tx on the LEADER's (cluster rank 0) full
 //     barrier (cp.async.bulk.tensor ... .cta_group::2), which counts one arrive.expect_tx from each producer;
 //   * only the leader issues MMAs; tcgen05.commit ... .multicast::cluster frees the ring slot / publishes the
@@ -87,19 +97,36 @@ __device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
                : "memory");
 }
 
+// ROWSHIFT (stride-1 layers): one TMA load per (kx, channel chunk) fetches the tile's band of image rows plus one
+// halo row above and below; the three ky taps then read that SAME shared-memory tile through UMMA descriptors whose
+// start address is advanced by ky image rows (whole 8-row core matrices). Cuts the L2->SMEM operand traffic from 9x
+// to 3x(R+2)/R. When a tile spans several small patches (8x8 images: two patches) the box is ordered
+// (x, patch, y, plane), so that shared memory holds [plane][y][patch][x] and a ky shift is still one uniform offset;
+// the tile's M rows are then ordered (y, patch, x).
 template <int CIN, int COUT, int HOUT, int STRIDE, int STAGES, bool ROWSHIFT, int KCB_ = 0>
 struct PairCfg {
-  using Base = ConvCfg<CIN, COUT, HOUT, STRIDE, 1, STAGES, true, ROWSHIFT, 1, KCB_>;
-  static constexpr int KCB = Base::KCB, KC = Base::KC, CIN_CHUNKS = Base::CIN_CHUNKS, KB = Base::KB, PIX = Base::PIX;
-  static constexpr int TILES_PER_PATCH = Base::TILES_PER_PATCH, ROWS_PER_TILE = Base::ROWS_PER_TILE;
-  static constexpr int PATCHES_PER_TILE = Base::PATCHES_PER_TILE, SPT = Base::UNITS, NPL = Base::NPL;
-  static constexpr uint32_t ROW_BYTES = Base::ROW_BYTES, PLANE_BYTES = Base::PLANE_BYTES, A_BYTES = Base::A_BYTES;
+  static constexpr int KCB = KCB_ ? KCB_ : ((CIN >= 64) ? 128 : 64);   // bytes of one pixel's channel chunk
+  static constexpr int KC = KCB / 2;                                   // channels per k-block
+  static constexpr int CIN_CHUNKS = CIN / KC;
+  static constexpr int KB = 9 * CIN_CHUNKS;                            // k-blocks per tile
+  static constexpr int PIX = HOUT * HOUT;
+  static constexpr int TILES_PER_PATCH = PIX >= kTileM ? PIX / kTileM : 0;
+  static constexpr int ROWS_PER_TILE = PIX >= kTileM ? kTileM / HOUT : HOUT;
+  static constexpr int PATCHES_PER_TILE = PIX >= kTileM ? 1 : kTileM / PIX;
+  static constexpr int SPT = ROWSHIFT ? 3 * CIN_CHUNKS : KB;           // TMA loads of A (= pipeline stages) per tile
+  static constexpr int NPL = KC / 8;                                   // 8-channel planes per k-block
+  // one image row (of all the tile's patches when ROWSHIFT) inside one plane of the A tile
+  static constexpr uint32_t ROW_BYTES = (ROWSHIFT ? PATCHES_PER_TILE : 1) * HOUT * 16;
+  static constexpr uint32_t PLANE_BYTES = ROWSHIFT ? (ROWS_PER_TILE + 2) * ROW_BYTES : kTileM * 16;
+  static constexpr uint32_t A_BYTES = NPL * PLANE_BYTES;
+  static_assert(!ROWSHIFT || (STRIDE == 1 && ROW_BYTES % 128 == 0),
+                "ROWSHIFT needs a stride-1 layer whose image rows are whole core matrices");
   static constexpr uint32_t BH_BYTES = (COUT / 2) * KCB;       // this CTA's half of one weight k-block
   static constexpr uint32_t W_BYTES = KB * BH_BYTES;           // resident half of the layer's weights
   static constexpr uint32_t STAGE_BYTES = A_BYTES;
   static constexpr uint32_t TMEM_COLS = tmem_cols_for(COUT);
   static constexpr size_t SMEM = size_t(W_BYTES) + size_t(STAGES) * STAGE_BYTES + 1024 + 256 + COUT * 4;
-  static_assert(BH_BYTES % 1024 == 0, "swizzled weight tiles must stay 1024B aligned");
+  static_assert(A_BYTES % 1024 == 0 && BH_BYTES % 1024 == 0, "swizzled weight tiles must stay 1024B aligned");
   static_assert(COUT % 32 == 0 && COUT <= 256, "cta_group::2 UMMA needs N % 16 == 0 and an even split of the rows");
   static_assert(SMEM <= 227 * 1024, "shared memory budget");
 };

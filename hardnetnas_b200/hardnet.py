@@ -253,12 +253,7 @@ class HardNet(_EngineOwner, nn.Module):
         with conv3 + conv4 fused into one kernel (csrc/tc_conv34.cuh, the default) stage 2 carries both layers and stage 3
         launches nothing."""
         names, macs = list(cls.STAGE_NAMES), list(cls.STAGE_MACS)
-        if launches[1] > 0 and launches[2] == 0 and launches[3] == 0 and launches[4] > 0:
-            # HN_COSCHED=1: front kernel and fused conv3 + conv4 kernel are the two roles of one launch (csrc/front_c34.cuh)
-            names[1], macs[1] = "front_conv3_conv4_cosched", macs[1] + macs[2] + macs[3]
-            names[2], macs[2] = "conv3_s2_64 (inside the co-scheduled launch)", 0
-            names[3], macs[3] = "conv4_64 (inside the co-scheduled launch)", 0
-        elif launches[2] > 0 and launches[3] == 0 and launches[4] > 0:
+        if launches[2] > 0 and launches[3] == 0 and launches[4] > 0:
             names[2], macs[2] = "conv3_conv4_fused", macs[2] + macs[3]
             names[3], macs[3] = "conv4_64 (inside the fused kernel)", 0
         return names, macs

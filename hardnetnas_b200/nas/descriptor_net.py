@@ -237,8 +237,8 @@ class SampledDescriptorNet(_EngineOwner, nn.Module):
         self._packed_key = key
 
     def resident_plan(self, device=None):
-        """[(first_op, last_op, patches_per_group, ctas_per_sm)] of the runs of ops that execute patch-resident (one launch,
-        activations in shared memory) on `device`; ops outside every run are one kernel each."""
+        """[(first_op, last_op, patches_in_flight_per_cta, 0)] of the tail launches on `device`: runs of ops that execute
+        patch-resident (one launch, activations in shared memory); ops outside every run are one kernel each."""
         device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
         self._ensure_packed(device)
         buf = (C.c_int * (4 * 32))()

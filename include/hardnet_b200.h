@@ -117,11 +117,11 @@ int hn_pack_nas(hn_handle* h, const hn_nas_op* ops, int n_ops, const float* para
 int hn_forward_nas(hn_handle* h, const void* patches, int in_dtype, long long B, void* desc_out,
                    int out_dtype, void* stream);
 
-/* Execution plan of the packed net: runs of consecutive ops that execute as ONE patch-resident kernel (activations stay in
- * shared memory between the run's first load and last store; hardnetNAS fbnet_builder.py:455-570, an IRFBlock's
- * pw -> dw -> pwl [+x] [+SE] never leaves the SM). Writes up to `cap` entries of 4 ints (first op, last op, patches per group,
- * CTAs per SM) to `out` (HOST memory, may be NULL) and returns the number of runs (>= 0) or a negative hn_status. Ops outside
- * every run execute as one kernel each. */
+/* Execution plan of the packed net: runs of consecutive ops behind the front stage that execute as ONE warpgroup-per-patch
+ * tail launch (activations stay in shared memory between the run's first load and last store; hardnetNAS
+ * fbnet_builder.py:455-570, an IRFBlock's pw -> dw -> pwl [+x] [+SE] never leaves the SM). Writes up to `cap` entries of 4 ints
+ * (first op, last op, patches in flight per CTA, 0) to `out` (HOST memory, may be NULL) and returns the number of runs (>= 0)
+ * or a negative hn_status. Ops outside every run execute as one kernel each. */
 int hn_nas_plan(hn_handle* h, int* out, int cap);
 
 /* Test hook: run ops [0, op_index] for B <= chunk_patches and copy that op's NHWC 16-bit output ([B,H,W,C]). */

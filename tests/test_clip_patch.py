@@ -159,15 +159,14 @@ def test_forward_clip_rejects_cpu_tensors_and_train_mode():
 
 
 @pytest.mark.gpu
-def test_forward_clip_with_front_sub_passes(monkeypatch):
-    """HN_FRONT_CHUNK (read in hn_create) splits a pass into front-kernel sub-passes: the keypoint offset of every sub-pass must
-    follow (hardnet_forward.cu: input_at). 700 keypoints, passes of 512, sub-passes of 200 -> offsets 0, 200, 400, 512, 712..."""
+def test_forward_clip_with_several_passes():
+    """A forward runs in passes of chunk_patches keypoints inside head launches of head_rows: the keypoint offset of every pass
+    must follow (hardnet_forward.cu: input_at). 700 keypoints, passes of 200, head launches of 400 -> offsets 0, 200, 400, 600."""
     from hardnetnas_b200.image_utils import clip_patch
     byxc, scale, ori, im_info, images = clip_oracle.make_clip_inputs(seed=4, B=7, H=150, W=210, k=100)
     args = (byxc.cuda(), scale.cuda(), ori.cuda(), im_info.cuda(), images.cuda())
     ref_model, _ = _hardnet()
     want = ref_model(clip_patch(*args, 32))
-    monkeypatch.setenv("HN_FRONT_CHUNK", "200")
-    model, _ = _hardnet(chunk_patches=512, head_rows=512)
+    model, _ = _hardnet(chunk_patches=200, head_rows=400)
     assert torch.equal(model.forward_clip(*args), model(clip_patch(*args, 32)))
     assert (model.forward_clip(*args) - want).abs().max().item() <= 1e-4   # other pass sizes: same values up to the head's K split

@@ -117,31 +117,6 @@ def test_train_mode_is_stock_torch_and_cpu_eval_fails():
     assert out.requires_grad and out.shape == (8, 128)
 
 
-@pytest.mark.parametrize("arch,env", [("wang2", {}), ("wang2", {"HN_NAS_CUT_RATIO": "2"}), ("wang3", {}), ("wang4", {"HN_NAS_MINB": "1"}),
-                                      ("mixed_se", {}), ("mixed_se", {"HN_NAS_GMAX": "1"})])
-def test_patch_resident_segments(arch, env, monkeypatch):
-    """HN_NAS_RESIDENT=1: runs of ops execute as ONE kernel with the activations resident in shared memory
-    (csrc/nas_resident.cuh; fbnet_builder.py:455-570, an IRFBlock's pw -> dw -> pwl [+x] [+SE] never leaves the SM). The plan
-    must really contain such runs, every stage output and the descriptors must match the oracle, also for a ragged batch that
-    does not fill the last group. (Off by default: measured slower than one kernel per op, DESIGN.md section 4.)"""
-    monkeypatch.setenv("HN_NAS_RESIDENT", "1")
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
-    net, ops, sd = build(arch, chunk_patches=64, head_rows=256)
-    plan = net.resident_plan()
-    assert plan and all(b >= a and g >= 1 and minb in (1, 2) for a, b, g, minb in plan), plan
-    assert any(b > a for a, b, _, _ in plan), f"no multi-op run in {plan}"
-    x = synth.make_patches(203, 6, edge_cases=False)
-    ref, feats = nas_oracle.nas_forward(x, ops, sd, return_features=True)
-    max_abs, cos = _cmp(net(x.cuda()), ref)
-    assert max_abs <= DESC_MAX_ABS and cos >= DESC_MIN_COS, (arch, plan, max_abs, cos)
-    prog = net.compile_program()
-    for stage, op_index in enumerate(prog.stage_end):
-        got = net.forward_op(x[:37].cuda(), op_index).float().cpu().permute(0, 3, 1, 2)
-        r = feats[stage][:37]
-        assert (got - r).abs().max().item() <= 6e-3 * r.abs().max().item() + 1e-5, (arch, stage, op_index)
-
-
 @pytest.mark.parametrize("arch", ["wang2", "wang3", "wang4"])
 def test_front_kernel_with_and_without_the_fused_depthwise_stage(arch, monkeypatch):
     """Default: the stride-2 depthwise conv (wang2: 3x3, wang3: 5x5) or max-pool (wang4) behind the stem runs inside the front

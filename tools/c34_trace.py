@@ -1,10 +1,9 @@
 """Diagnostic: where the roles of the fused conv3 + conv4 kernel (tc_conv34.cuh) wait.
 
     python tools/c34_trace.py --build     # here (no GPU): trace build of the library next to the normal one
-    python tools/c34_trace.py [sched ...] # on the GPU box
+    python tools/c34_trace.py             # on the GPU box
 """
 import ctypes as C
-import os
 import subprocess
 import sys
 from pathlib import Path
@@ -35,19 +34,18 @@ lib.hn_debug_c34_trace.restype = C.c_int
 lib.hn_debug_c34_trace.argtypes = [C.c_void_p, C.c_int]
 x = torch.randn(18944 * 4, 1, 32, 32, device="cuda")
 out = torch.empty(x.size(0), 128, device="cuda")
-names = {0: "issuer: full (loads)", 1: "issuer: mid ready", 2: "issuer: t4empty (v2: t3empty)", 10: "issuer: t4empty (v2)", 11: "shifter: mma4 (v2)", 5: "epi warp 2: t3full", 6: "epi warp 2: t4full (mid free)",
-         7: "epi warp 2: conv3 epilogue", 8: "epi warp 2: conv3 + conv4 epilogue", 9: "producer: empty", 12: "producer 0: issue section"}
-for sched in [a for a in sys.argv[1:] if not a.startswith("-")] or ["2:6", "3:0"]:
-    os.environ["HN_FUSE34"], os.environ["HN_FUSE34_SCHED"] = sched.split(":")
-    m = HardNet().cuda().eval()
-    for _ in range(2):
-        m(x, out=out)
-    buf = (C.c_ulonglong * 16)()
-    lib.hn_debug_c34_trace(buf, 1)
+names = {0: "issuer: full (loads)", 1: "issuer: mid ready", 2: "issuer: t3empty", 10: "issuer: t4empty", 11: "shifter: mma4",
+         5: "epi warp 4: t3full", 6: "epi warp 4: t4full", 7: "epi warp 4: conv3 epilogue", 8: "epi warp 4: conv3 + conv4 epilogue",
+         9: "producer: empty", 12: "producer 0: issue section"}
+m = HardNet().cuda().eval()
+for _ in range(2):
     m(x, out=out)
-    lib.hn_debug_c34_trace(buf, 0)
-    v = list(buf)
-    n = max(v[4], 1)
-    print(f"sched {sched}: CTA 0: {v[3] / n:.0f} cycles per patch over {n} patches")
-    for k, nm in names.items():
-        print(f"  {nm:40s} {v[k] / n:9.0f} cycles/patch")
+buf = (C.c_ulonglong * 16)()
+lib.hn_debug_c34_trace(buf, 1)
+m(x, out=out)
+lib.hn_debug_c34_trace(buf, 0)
+v = list(buf)
+n = max(v[4], 1)
+print(f"CTA 0: {v[3] / n:.0f} cycles per patch over {n} patches")
+for k, nm in names.items():
+    print(f"  {nm:40s} {v[k] / n:9.0f} cycles/patch")

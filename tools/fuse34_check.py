@@ -1,8 +1,8 @@
-"""A/B of the fused conv3 + conv4 kernel (tc_conv34.cuh) against the two separate kernels: stage outputs and descriptors
-bit for bit (same operands, same K order in mode 1) or to the last fp16 bit (mode 2: another accumulation order), then
-throughput and per-stage times of both engines. Run on the GPU box; diagnostic, not a test.
+"""A/B of the fused conv3 + conv4 kernel (tc_conv34.cuh, mode 1 = the default) against the two separate kernels (mode 0,
+HN_FUSE34=0): stage outputs and descriptors to the last fp16 bit (another accumulation order), then throughput and
+per-stage times of both engines. Run on the GPU box; diagnostic, not a test.
 
-    python tools/fuse34_check.py [modes ...]       # default: 0 1 2
+    python tools/fuse34_check.py [modes ...]       # default: 0 1
 """
 import os
 import sys
@@ -16,8 +16,7 @@ from hardnetnas_b200.hardnet import HardNet  # noqa: E402
 
 
 def make(mode, chunk=0):
-    os.environ["HN_FUSE34"] = str(min(mode, 3))        # mode 4 = mode 3 with the front kernel co-scheduled (HN_COSCHED=1)
-    os.environ["HN_COSCHED"] = "1" if mode == 4 else "0"
+    os.environ["HN_FUSE34"] = str(mode)
     w, m, v = synth.hardnet_weights_from_seed(0, 3)
     torch.manual_seed(0)
     model = HardNet(chunk_patches=chunk)
@@ -30,8 +29,8 @@ def make(mode, chunk=0):
 
 
 def main():
-    modes = [int(a) for a in sys.argv[1:] if not a.startswith("-")] or [0, 1, 2]
-    print(torch.cuda.get_device_name(0), "sched", os.environ.get("HN_FUSE34_SCHED"), flush=True)
+    modes = [int(a) for a in sys.argv[1:] if not a.startswith("-")] or [0, 1]
+    print(torch.cuda.get_device_name(0), flush=True)
     for n, chunk in (() if "--time-only" in sys.argv else ((2, 0), (301, 0), (4097, 0), (1000, 256), (18945, 0), (30001, 9472))):
         x = synth.make_patches(n, 77 + n).cuda()
         ref = None
@@ -74,8 +73,7 @@ def main():
         st, nl = model.profile_read()
         model.profile_enable(0)
         print(f"mode {mode}: {B / ms / 1e3:.3f} M patches/s ({ms:.2f} ms per {B}); stage ns/patch "
-              + " ".join(f"{model.STAGE_NAMES[i][:8]}={st[i] * 1e6 / B:.1f}" for i in range(1, 7))
-              + f" | NF={os.environ.get('HN_COSCHED_NF')}", flush=True)
+              + " ".join(f"{model.STAGE_NAMES[i][:8]}={st[i] * 1e6 / B:.1f}" for i in range(1, 7)), flush=True)
 
 
 HardNet._engine_chunk = lambda self: 148 * 128 if self._chunk_patches == 0 else self._chunk_patches

@@ -4,12 +4,11 @@ from pathlib import Path
 import torch
 REPO = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(REPO))
-from tools.nas_resident_check import build, timing  # noqa: E402
+from tools.nas_tail_check import build, timing  # noqa: E402
 from oracle import nas_oracle, synth  # noqa: E402
 
 for arch in ("wang2", "wang3", "wang4", "mixed_se"):
-    os.environ["HN_NAS_FRONT_DW"] = "1"
-    net, ops, sd = build(arch, {}, chunk_patches=64, head_rows=256)
+    net, ops, sd = build(arch, {"HN_NAS_FRONT_DW": "1"}, chunk_patches=64, head_rows=256)
     x = synth.make_patches(203, 6, edge_cases=False)
     ref, feats = nas_oracle.nas_forward(x, ops, sd, return_features=True)
     got = net(x.cuda()).float().cpu()
@@ -25,6 +24,5 @@ for arch in ("wang2", "wang3", "wang4", "mixed_se"):
           torch.nn.functional.cosine_similarity(got, ref, dim=1).min().item(), worst, e8), flush=True)
 for arch in ("wang2", "wang3", "wang4"):
     for v in ("1", "0"):
-        os.environ["HN_NAS_FRONT_DW"] = v
-        r = timing(arch, {})
+        r = timing(arch, {"HN_NAS_FRONT_DW": v})
         print(f"TIMING {arch} front_dw={v}: {r['ms']:.3f} ms {r['patches_per_sec'] / 1e6:.2f} M/s", flush=True)
