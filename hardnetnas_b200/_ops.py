@@ -162,6 +162,53 @@ def match_mutual(q: torch.Tensor, g: torch.Tensor, q16: torch.Tensor | None = No
     return d1, d2, i1, i2, mutual
 
 
+def _require_cuda_f32_batched(name: str, t: torch.Tensor) -> torch.Tensor:
+    if not isinstance(t, torch.Tensor) or not t.is_cuda:
+        raise _lib.HardnetB200Error(f"{name}: the fused path runs on B200 CUDA tensors only (no CPU fallback)")
+    if t.dim() != 3:
+        raise ValueError(f"{name}: descriptors must be a padded batch [B, N, 128], got shape {tuple(t.shape)}")
+    if t.size(2) != 128:
+        raise ValueError(f"{name}: descriptors must be 128-d, got {t.size(2)}")
+    return t.detach().float().contiguous()
+
+
+def _lengths(name: str, t, batch: int, device: torch.device):
+    if t is None:
+        return None
+    if not isinstance(t, torch.Tensor) or t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+        raise ValueError(f"{name}: lengths must be an integer tensor of shape [{batch}]")
+    if tuple(t.shape) != (batch,):
+        raise ValueError(f"{name}: lengths must have shape [{batch}], got {tuple(t.shape)}")
+    return t.to(device=device, dtype=torch.int32).contiguous()
+
+
+def match_batched(q: torch.Tensor, g: torch.Tensor, q_len: torch.Tensor | None = None, g_len: torch.Tensor | None = None,
+                  mutual: bool = False):
+    """(d1, d2, i1, i2[, mutual]), each [B, Nq]: hn_match_batched over the padded batches q [B, Nq, 128] and g [B, Ng, 128].
+    q_len / g_len: integer [B] tensors of valid rows per pair (None = all). Lengths on q's device keep the call free of host
+    synchronisation (and CUDA-graph capturable); a CPU lengths tensor is copied to the device first. Indices are local to the
+    pair; rows past q_len get d = +inf, i = -1 (and mutual = False)."""
+    lib = _lib.load()
+    q = _require_cuda_f32_batched("match_batched", q)
+    g = _require_cuda_f32_batched("match_batched", g)
+    if q.size(0) != g.size(0):
+        raise ValueError(f"match_batched: q and g hold {q.size(0)} and {g.size(0)} pairs")
+    b, nq, ng = q.size(0), q.size(1), g.size(1)
+    dev = q.device
+    ql = _lengths("match_batched q_len", q_len, b, dev)
+    gl = _lengths("match_batched g_len", g_len, b, dev)
+    with torch.cuda.device(dev):
+        ws = _workspace(dev, max(lib.hn_match_batched_workspace_bytes(b, nq, ng, int(mutual)), 1))
+        d1 = torch.empty((b, nq), dtype=torch.float32, device=dev)
+        d2 = torch.empty((b, nq), dtype=torch.float32, device=dev)
+        i1 = torch.empty((b, nq), dtype=torch.int32, device=dev)
+        i2 = torch.empty((b, nq), dtype=torch.int32, device=dev)
+        mu = torch.empty((b, nq), dtype=torch.bool, device=dev) if mutual else None
+        _lib.check(lib.hn_match_batched(_ptr(q), _ptr(g), b, nq, ng, _ptr(ql), _ptr(gl), _ptr(d1), _ptr(d2), _ptr(i1), _ptr(i2),
+                                        _ptr(mu), _ptr(ws), ws.numel(), _stream_ptr()), "hn_match_batched")
+    return (d1, d2, i1, i2, mu) if mutual else (d1, d2, i1, i2)
+
+
 def mutual_claims(i1: torch.Tensor, d1: torch.Tensor, d2: torch.Tensor, q_offset: int, claim: torch.Tensor) -> torch.Tensor:
     """atomicMin of (distance, global row) into claim[int64, Ng] (pre-filled with INT64_MAX = unclaimed); returns the per
     32-row-block minimum of d2 the verification needs."""

@@ -206,6 +206,113 @@ __global__ void __launch_bounds__(128) rerank_kernel(const float* __restrict__ q
   }
 }
 
+// Batched re-rank over the flat [B * nq_pad] query rows of hn_match_batched: row -> pair b = row / nq_pad, whose gallery is
+// rows [0, g_len[b]) of g + b * ng_pad * 128; indices are local to the pair. Rows past q_len[b] get the fill values
+// (d = +inf, i = -1). From the prologue on this is rerank_kernel's body, copied rather than shared so that the single-problem
+// kernel compiles to the same instructions as before: keep the two in step, the bit equality of a batched row with a per-pair
+// hn_match rests on the same candidate threshold and the same summation order (tests/test_matching_batched_gpu.py compares
+// them bit for bit). One difference: the eight distances of a chunk are taken by eight lanes, one sqrtf each, and shuffled to
+// the warp (the same values: every lane holds the same eight dot products). Eight unrolled sqrtf slow-path calls per lane kept
+// the pair's gallery pointer and size live across calls and made ptxas spill.
+__global__ void __launch_bounds__(128) rerank_batched_kernel(const float* __restrict__ q, const float* __restrict__ g_all,
+                                                             const int* __restrict__ cand, const float* __restrict__ cand_val,
+                                                             float margin, long long B, long long nq_pad, long long ng_pad,
+                                                             const int* __restrict__ q_len, const int* __restrict__ g_len, int slots,
+                                                             float* __restrict__ d1, float* __restrict__ d2, int* __restrict__ i1,
+                                                             int* __restrict__ i2) {
+  __shared__ __align__(16) float sq[4][128];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long row = static_cast<long long>(blockIdx.x) * 4 + w;
+  if (row >= B * nq_pad) return;
+  const int b = static_cast<int>(row) / static_cast<int>(nq_pad);   // B * nq_pad < 2^31; element offsets below stay 64-bit
+  if (row - b * nq_pad >= pair_len(q_len, b, nq_pad)) {
+    if (lane == 0) {
+      d1[row] = d2[row] = __int_as_float(0x7f800000);
+      i1[row] = i2[row] = -1;
+    }
+    return;
+  }
+  const float* g = g_all + static_cast<long long>(b) * ng_pad * 128;
+  const long long ng = pair_len(g_len, b, ng_pad);
+  const int* crow = cand + row * slots;
+  const float* cvrow = cand_val + row * slots;
+  reinterpret_cast<float4*>(sq[w])[lane] = reinterpret_cast<const float4*>(q + row * 128)[lane];
+  __syncwarp();
+  // A chunk can hold one of the two nearest columns only if its approximate maximum reaches the second largest
+  // chunk maximum minus twice the error bound of the 16-bit-operand dot product (`margin`, same scaled units).
+  float thr;
+  {
+    float m1 = -__int_as_float(0x7f800000), m2 = m1;
+    for (int c = lane; c < slots; c += 32) {
+      const float v = crow[c] >= 0 ? cvrow[c] : -__int_as_float(0x7f800000);
+      if (v > m1) { m2 = m1; m1 = v; } else if (v > m2) { m2 = v; }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float o1 = __shfl_xor_sync(0xffffffffu, m1, o), o2 = __shfl_xor_sync(0xffffffffu, m2, o);
+      const float lo = fminf(m1, o1);
+      m1 = fmaxf(m1, o1);
+      m2 = fmaxf(fmaxf(m2, o2), lo);
+    }
+    thr = m2 - margin;   // -inf when fewer than two chunks exist: everything is re-ranked
+  }
+  const float inf = __int_as_float(0x7f800000);
+  float b1 = inf, b2 = inf;
+  int j1 = 0x7fffffff, j2 = 0x7fffffff;
+  // The warp walks the surviving chunks together: a gallery row is ONE coalesced 512 B read (lane = float4 index) and
+  // the 128-term dot is finished with a butterfly, so every lane ends up with the same (d, index) stream. Per-lane
+  // row reads (one lane per candidate) cost 32 L1 wavefronts per row instead of 4.
+  const float4 qv = reinterpret_cast<const float4*>(sq[w])[lane];
+  auto eval_chunk = [&](long long chunk) {
+    const long long col0 = chunk * kChunk;
+    float part[kChunk];
+#pragma unroll
+    for (int r = 0; r < kChunk; ++r) {
+      const long long col = col0 + r;
+      part[r] = 0.f;
+      if (col < ng) {
+        const float4 gv = __ldg(reinterpret_cast<const float4*>(g + col * 128) + lane);
+        part[r] = fmaf(qv.x, gv.x, fmaf(qv.y, gv.y, fmaf(qv.z, gv.z, qv.w * gv.w)));
+      }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+      for (int r = 0; r < kChunk; ++r) part[r] += __shfl_xor_sync(0xffffffffu, part[r], o);
+    }
+    float mine = part[0];   // part[lane & 7] without a local-memory array access
+#pragma unroll
+    for (int r = 1; r < kChunk; ++r) mine = (lane & (kChunk - 1)) == r ? part[r] : mine;
+    mine = sqrtf(fminf(fmaxf(2.0f - 2.0f * mine, 1e-8f), 4.0f));
+#pragma unroll
+    for (int r = 0; r < kChunk; ++r) {
+      const long long col = col0 + r;
+      const float d = __shfl_sync(0xffffffffu, mine, r);
+      if (col >= ng) continue;
+      const int ci = static_cast<int>(col);
+      if (d < b1 || (d == b1 && ci < j1)) {
+        b2 = b1; j2 = j1; b1 = d; j1 = ci;
+      } else if (d < b2 || (d == b2 && ci < j2)) {
+        b2 = d; j2 = ci;
+      }
+    }
+  };
+  for (int c = 0; c < slots; ++c) {
+    const int chunk = crow[c];
+    if (chunk < 0 || cvrow[c] < thr) continue;   // warp-uniform
+    eval_chunk(chunk);
+  }
+  // every lane holds the same top-2 now
+  const float m = b1, s = b2;
+  const int mj = j1, sj = j2;
+  if (lane == 0) {
+    d1[row] = m;
+    i1[row] = mj == 0x7fffffff ? -1 : mj;
+    d2[row] = s;
+    i2[row] = sj == 0x7fffffff ? -1 : sj;
+  }
+}
+
 // Optional per-stage CUDA-event timing of hn_match (bench.py: the roofline of the matching GEMM is computed from the kernel's
 // own in-run time): stage 0 = operand packing, 1 = GEMM + shortlist, 2 = exact re-rank.
 struct MatchProfile {
@@ -390,11 +497,178 @@ __global__ void mutual_final_kernel(const int* __restrict__ i1, long long nq, lo
   mutual[i] = m ? 1 : 0;
 }
 
+// Batched column side of hn_match_batched. Claims, beaten flags and block maxima are per pair ([B][ng], [B][ng],
+// [B][ceil(ng / 8)][ceil(nq / 32)]); query rows are local to the pair, so ties resolve to the lowest local row as in a per-pair
+// call. Rows past q_len[b] are never claimants or candidates, and columns past g_len[b] are never claimed.
+// Claims: one thread per (pair, 32-row block slot): a warp is one row block of one pair, padded to whole blocks.
+__global__ void mutual_claim_batched_kernel(const int* __restrict__ i1, const float* __restrict__ d1, const float* __restrict__ d2,
+                                            long long B, long long nq, long long ng, const int* __restrict__ q_len,
+                                            const int* __restrict__ g_len, unsigned long long* __restrict__ claim,
+                                            float* __restrict__ rb_min_d2) {
+  const long long nrb = (nq + 31) / 32;
+  const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (t >= B * nrb * 32) return;   // whole warps
+  const long long b = t / (nrb * 32), r = t - b * nrb * 32;   // 64-bit: B * nrb * 32 may pass 2^31 while B * nq does not
+  const long long i = b * nq + r;
+  const bool valid = r < pair_len(q_len, b, nq);
+  float m = valid ? d2[i] : __int_as_float(0x7f800000);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fminf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0) rb_min_d2[b * nrb + (r >> 5)] = m;
+  if (!valid) return;
+  const long long j = i1[i];
+  if (j < 0 || j >= pair_len(g_len, b, ng)) return;
+  atomicMin(claim + b * ng + j, (static_cast<unsigned long long>(__float_as_uint(d1[i])) << 32) | static_cast<unsigned int>(r));
+}
+
+// One warp per (pair, 8-column chunk), scanning only the pair's valid row blocks. After the prologue (pair pointers and
+// bounds) this is mutual_verify_kernel's body with q_offset = 0 and a block_max row pitch of ceil(nq_pad / 32), copied rather
+// than shared so that the single-problem kernel compiles to the same instructions as before: keep the two in step.
+__global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kernel(const float* __restrict__ q_all, const float* __restrict__ g_all,
+                                                                                 long long B, long long nq_pad, long long ng_pad,
+                                                                                 const int* __restrict__ q_len, const int* __restrict__ g_len,
+                                                                                 const unsigned long long* __restrict__ claim_all,
+                                                                                 const float* __restrict__ block_max_all,
+                                                                                 const float* __restrict__ rb_min_d2_all, float margin_scaled,
+                                                                                 float inv_dot_scale, unsigned char* __restrict__ beaten_all) {
+  extern __shared__ __align__(16) uint8_t vsm[];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  float* s_q = reinterpret_cast<float*>(vsm) + static_cast<size_t>(w) * 32 * kVerifyPitch;                       // [32][132]
+  float4* s_g = reinterpret_cast<float4*>(vsm + static_cast<size_t>(kVerifyWarps) * 32 * kVerifyPitch * 4) + w * kChunk * 32;   // [8][32]
+  const long long chunks = (ng_pad + kChunk - 1) / kChunk, bm_pitch = (nq_pad + 31) / 32;
+  const long long item = static_cast<long long>(blockIdx.x) * kVerifyWarps + w;
+  const long long pair = static_cast<int>(item) / static_cast<int>(chunks), cb = item - pair * chunks;   // B * chunks <= B * ng_pad < 2^31
+  if (pair >= B) return;
+  const long long nq = pair_len(q_len, pair, nq_pad), ng = pair_len(g_len, pair, ng_pad), q_offset = 0;
+  const int n_row_blocks = static_cast<int>((nq + 31) / 32);
+  const float* q = q_all + pair * nq_pad * 128;
+  const float* g = g_all + pair * ng_pad * 128;
+  const unsigned long long* claim = claim_all + pair * ng_pad;
+  const float* block_max = block_max_all + pair * chunks * bm_pitch;
+  const float* rb_min_d2 = rb_min_d2_all + pair * bm_pitch;
+  unsigned char* beaten = beaten_all + pair * ng_pad;
+  if (cb * kChunk >= ng) return;
+  unsigned long long cl = 0x7FFFFFFFFFFFFFFFull;   // unclaimed
+  if (lane < kChunk && cb * kChunk + lane < ng) cl = claim[cb * kChunk + lane];
+  float dcl[kChunk], thr[kChunk];
+  unsigned int icl[kChunk];
+  unsigned undecided = 0, lost = 0;
+  const float ninf = -__int_as_float(0x7f800000);
+#pragma unroll
+  for (int c = 0; c < kChunk; ++c) {
+    const unsigned long long cc = __shfl_sync(0xffffffffu, cl, c);
+    dcl[c] = __uint_as_float(static_cast<unsigned int>(cc >> 32));
+    icl[c] = static_cast<unsigned int>(cc & 0xffffffffu);
+    thr[c] = __int_as_float(0x7f800000);
+    if ((cc >> 32) < 0x7F000000ull) {
+      undecided |= 1u << c;
+      thr[c] = (1.0f - 0.5f * dcl[c] * dcl[c]) * inv_dot_scale - margin_scaled;
+      s_g[c * 32 + lane] = __ldg(reinterpret_cast<const float4*>(g + (cb * kChunk + c) * 128) + lane);
+    }
+  }
+  if (!undecided) return;
+  __syncwarp();
+  const float* bm_row = block_max + cb * bm_pitch;
+
+  // distance of this lane's staged row to column c (arithmetic of rerank_kernel)
+  auto row_distance = [&](int c) {
+    float p[32];
+    const float* qr = s_q + lane * kVerifyPitch;
+#pragma unroll
+    for (int l = 0; l < 32; ++l) {
+      const float4 qv = *reinterpret_cast<const float4*>(qr + 4 * l);
+      const float4 gv = s_g[c * 32 + l];
+      p[l] = fmaf(qv.x, gv.x, fmaf(qv.y, gv.y, fmaf(qv.z, gv.z, qv.w * gv.w)));
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+      for (int l = 0; l < o; ++l) p[l] += p[l + o];
+    }
+    return sqrtf(fminf(fmaxf(2.0f - 2.0f * p[0], 1e-8f), 4.0f));
+  };
+
+  auto evaluate = [&](int rb, float vb, float min_d2) {
+    unsigned need = 0;
+#pragma unroll
+    for (int c = 0; c < kChunk; ++c)
+      if (((undecided >> c) & 1u) && thr[c] <= vb && min_d2 <= dcl[c]) need |= 1u << c;
+    if (!need) return;
+    // stage the cell's 32 rows: one coalesced 512-byte row per iteration
+    const long long k0 = static_cast<long long>(rb) * 32;
+#pragma unroll
+    for (int r0 = 0; r0 < 32; r0 += 8) {   // eight row loads in flight
+      float4 v[8];
+#pragma unroll
+      for (int r = 0; r < 8; ++r) {
+        v[r] = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (k0 + r0 + r < nq) v[r] = __ldg(reinterpret_cast<const float4*>(q + (k0 + r0 + r) * 128) + lane);
+      }
+#pragma unroll
+      for (int r = 0; r < 8; ++r) *reinterpret_cast<float4*>(s_q + (r0 + r) * kVerifyPitch + 4 * lane) = v[r];
+    }
+    __syncwarp();
+    const long long k = k0 + lane;
+    const bool valid = k < nq;
+    const unsigned int gk = static_cast<unsigned int>(k + q_offset);
+#pragma unroll 1
+    for (int c = 0; c < kChunk; ++c) {
+      if (!((need >> c) & 1u)) continue;   // warp-uniform
+      const float d = row_distance(c);
+      const bool beats = valid && gk != icl[c] && (d < dcl[c] || (d == dcl[c] && gk < icl[c]));
+      if (__any_sync(0xffffffffu, beats)) {
+        undecided &= ~(1u << c);
+        lost |= 1u << c;
+      }
+    }
+    __syncwarp();   // the staging tile is reused by the next cell
+  };
+
+  for (int base = 0; base < n_row_blocks && undecided; base += 32) {
+    const int rb = base + lane;
+    const float v = rb < n_row_blocks ? bm_row[rb] : ninf;
+    const float md2 = rb < n_row_blocks ? rb_min_d2[rb] : __int_as_float(0x7f800000);
+    bool mine = false;
+#pragma unroll
+    for (int c = 0; c < kChunk; ++c) mine |= ((undecided >> c) & 1u) && thr[c] <= v && md2 <= dcl[c];
+    unsigned cand = __ballot_sync(0xffffffffu, mine);
+    while (cand && undecided) {
+      const int b = __ffs(cand) - 1;
+      cand &= cand - 1;
+      evaluate(base + b, __shfl_sync(0xffffffffu, v, b), __shfl_sync(0xffffffffu, md2, b));
+    }
+  }
+  if (lane < kChunk && ((lost >> lane) & 1u)) beaten[cb * kChunk + lane] = 1;
+}
+
+
+__global__ void mutual_final_batched_kernel(const int* __restrict__ i1, long long B, long long nq, long long ng,
+                                            const int* __restrict__ q_len, const int* __restrict__ g_len,
+                                            const unsigned long long* __restrict__ claim, const unsigned char* __restrict__ beaten,
+                                            unsigned char* __restrict__ mutual) {
+  const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= B * nq) return;
+  const long long b = static_cast<int>(i) / static_cast<int>(nq), r = i - b * nq;
+  bool m = false;
+  if (r < pair_len(q_len, b, nq)) {
+    const long long j = i1[i];
+    if (j >= 0 && j < pair_len(g_len, b, ng))
+      m = static_cast<unsigned int>(claim[b * ng + j] & 0xffffffffu) == static_cast<unsigned int>(r) && !beaten[b * ng + j];
+  }
+  mutual[i] = m ? 1 : 0;
+}
+
 // Which matching GEMM runs: -1 = by problem size, 0 = single-CTA kernel, 1 = CTA-pair kernel. The initial value comes from
 // HN_MATCH_PAIR, read ONCE when first needed; tests switch it through hn_match_force_kernel instead of the environment.
 static int& match_kernel_mode() {
   static int mode = [] { const char* pe = getenv("HN_MATCH_PAIR"); return pe ? atoi(pe) : -1; }();
   return mode;
+}
+
+// gallery segments of the batched GEMM (hn_match_batched): bounds its candidate lists, [rows][segments][kTopC]
+constexpr int kMaxBatchedSegments = 16;
+static inline long long batched_max_segments(long long Ng) {
+  return std::max<long long>(1, std::min<long long>(kMaxBatchedSegments, (Ng + kDistTile - 1) / kDistTile));
 }
 
 static int make_desc_map(CUtensorMap* tm, const uint16_t* base, long long rows, int K, int box_rows = kDistTile) {
@@ -753,6 +1027,132 @@ extern "C" int hn_match_mutual(const float* q, const float* g, const void* q16, 
   mutual_final_kernel<<<static_cast<unsigned>((Nq + 255) / 256), 256, 0, s>>>(i1, Nq, 0, claim, beaten, Ng, mutual);
   HN_CUDA(cudaGetLastError());
   count_launch();
+  return HN_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// batched matching: B independent padded problems in one launch sequence (hn_match_batched)
+// ------------------------------------------------------------------------------------------------------------
+struct BatchedWs {
+  uint16_t *q16, *g16;
+  int* cand;
+  float* cand_val;
+  float* block_max;          // mutual only
+  unsigned long long* claim;
+  unsigned char* beaten;
+  float* rb_min_d2;
+  size_t bytes;
+};
+
+static BatchedWs carve_batched(void* ws, long long B, long long Nq, long long Ng, bool with_mutual) {
+  BatchedWs w;
+  char* b = static_cast<char*>(ws);
+  size_t off = 0;
+  auto take = [&](size_t n) { char* r = b ? b + off : nullptr; off += align256(n); return r; };
+  const size_t rows_q = static_cast<size_t>(B) * Nq, rows_g = static_cast<size_t>(B) * Ng;
+  w.q16 = reinterpret_cast<uint16_t*>(take(rows_q * 128 * 2));
+  w.g16 = reinterpret_cast<uint16_t*>(take(rows_g * 128 * 2));
+  // candidate lists [rows][segments][kTopC]: a segment holds at least one gallery tile, so at most min(16, tiles) of them
+  const size_t lists = rows_q * batched_max_segments(Ng) * kTopC * 4;
+  w.cand = reinterpret_cast<int*>(take(lists));
+  w.cand_val = reinterpret_cast<float*>(take(lists));
+  w.block_max = nullptr;
+  w.claim = nullptr;
+  w.beaten = nullptr;
+  w.rb_min_d2 = nullptr;
+  if (with_mutual) {
+    w.block_max = reinterpret_cast<float*>(take(static_cast<size_t>(B) * hn_block_max_elems(Nq, Ng) * 4));
+    w.claim = reinterpret_cast<unsigned long long*>(take(rows_g * 8));
+    w.beaten = reinterpret_cast<unsigned char*>(take(rows_g));
+    w.rb_min_d2 = reinterpret_cast<float*>(take(static_cast<size_t>(B) * ((Nq + 31) / 32) * 4));
+  }
+  w.bytes = off;
+  return w;
+}
+
+// {K = 128, N, B} 16-bit operand rows, box {64, 128, 1}: a box never reaches into the next pair, TMA zero-fills past N
+static int make_batched_desc_map(CUtensorMap* tm, const uint16_t* base, long long rows, long long B) {
+  const uint64_t dims[3] = {128, static_cast<uint64_t>(rows), static_cast<uint64_t>(B)};
+  const uint64_t str[2] = {128 * 2, static_cast<uint64_t>(rows) * 128 * 2};
+  const uint32_t box[3] = {64, static_cast<uint32_t>(kDistTile), 1};
+  return make_tmap_16bit(tm, base, 3, dims, str, box, 128);
+}
+
+extern "C" long long hn_match_batched_workspace_bytes(long long B, long long Nq, long long Ng, int with_mutual) {
+  if (B < 0 || Nq < 0 || Ng < 0) return 0;
+  return static_cast<long long>(carve_batched(nullptr, B, Nq, Ng, with_mutual != 0).bytes);
+}
+
+extern "C" int hn_match_batched(const float* q, const float* g, long long B, long long Nq, long long Ng, const int32_t* q_len,
+                                const int32_t* g_len, float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual,
+                                void* workspace, long long workspace_bytes, void* stream) {
+  HN_REQUIRE(q && g && d1 && d2 && i1 && i2 && workspace, "hn_match_batched: NULL argument (q, g, d1, d2, i1, i2 and workspace are required)");
+  HN_REQUIRE(B >= 1 && Nq >= 1 && Ng >= 1, "hn_match_batched: empty input (B=%lld, Nq=%lld, Ng=%lld)", B, Nq, Ng);
+  HN_REQUIRE(Nq < (1LL << 31) / B && Ng < (1LL << 31) / B, "hn_match_batched: B*Nq and B*Ng must stay below 2^31 rows");
+  HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "hn_match_batched: workspace must be 256-byte aligned");
+  HN_REQUIRE(workspace_bytes >= hn_match_batched_workspace_bytes(B, Nq, Ng, mutual != nullptr), "hn_match_batched: workspace too small");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  int sm = 0;
+  HN_TRY(device_sm_count(&sm));
+  const BatchedWs w = carve_batched(workspace, B, Nq, Ng, mutual != nullptr);
+  const long long rows_q = B * Nq, rows_g = B * Ng;
+  const int threads = 256;
+  {
+    MatchTimer timer(0, s);
+    pack_desc_kernel<<<static_cast<unsigned>((rows_q * 32 + threads - 1) / threads), threads, 0, s>>>(q, rows_q, w.q16, 0, 0, nullptr);
+    pack_desc_kernel<<<static_cast<unsigned>((rows_g * 32 + threads - 1) / threads), threads, 0, s>>>(g, rows_g, w.g16, 0, 1, nullptr);
+    HN_CUDA(cudaGetLastError());
+    count_launch(2);
+  }
+  DistParams dp;
+  memset(&dp, 0, sizeof(dp));
+  HN_TRY(make_batched_desc_map(&dp.side[0].tmA, w.q16, Nq, B));
+  HN_TRY(make_batched_desc_map(&dp.side[0].tmB, w.g16, Ng, B));
+  dp.side[0].cand = w.cand;
+  dp.side[0].cand_val = w.cand_val;
+  dp.side[0].block_max = w.block_max;
+  dp.side[0].n_row_blocks = static_cast<int>((Nq + 31) / 32);
+  dp.side[0].Na = Nq;
+  dp.side[0].Nb = Ng;
+  dp.k_blocks = 2;
+  dp.form = HN_FORM_FDL;
+  dp.dot_scale = kDotScale;
+  dp.q_len = q_len;
+  dp.g_len = g_len;
+  dp.batch = static_cast<int>(B);
+  {
+    MatchTimer timer(1, s);
+    // segments from the padded sizes (lengths live on the device): B * ceil(Nq / 256) query blocks over a gallery of Ng
+    const long long m_blocks = (Nq + 2 * kDistTile - 1) / (2 * kDistTile);
+    dp.segments = pick_segments(B * m_blocks * 2 * kDistTile, 2 * kDistTile, Ng, sm, static_cast<int>(batched_max_segments(Ng)));
+    const long long items = B * m_blocks * dp.segments;
+    HN_TRY((launch_dist<2, EPI_SHORTLIST_BATCHED>(dp, static_cast<int>(std::min<long long>(items, sm)), 1, s)));
+  }
+  const float margin = 4.0f * (1.0f / 1024.0f) / kDotScale;   // as hn_match_ex
+  {
+    MatchTimer timer(2, s);
+    rerank_batched_kernel<<<static_cast<unsigned>((rows_q + 3) / 4), 128, 0, s>>>(q, g, w.cand, w.cand_val, margin, B, Nq, Ng, q_len, g_len,
+                                                                                  dp.segments * kTopC, d1, d2, i1, i2);
+    HN_CUDA(cudaGetLastError());
+    count_launch();
+  }
+  if (mutual) {
+    HN_CUDA(cudaMemsetAsync(w.claim, 0x7f, static_cast<size_t>(rows_g) * 8, s));   // "unclaimed"
+    HN_CUDA(cudaMemsetAsync(w.beaten, 0, static_cast<size_t>(rows_g), s));
+    const long long nrb = (Nq + 31) / 32, chunks = (Ng + kChunk - 1) / kChunk;
+    mutual_claim_batched_kernel<<<static_cast<unsigned>((B * nrb * 32 + threads - 1) / threads), threads, 0, s>>>(
+        i1, d1, d2, B, Nq, Ng, q_len, g_len, w.claim, w.rb_min_d2);
+    static DeviceOnce attr_once;
+    if (attr_once.first_time())
+      HN_CUDA(cudaFuncSetAttribute(mutual_verify_batched_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kVerifySmem)));
+    const float vmargin = 2.0f * (1.0f / 1024.0f) / kDotScale;   // as hn_mutual_verify
+    mutual_verify_batched_kernel<<<static_cast<unsigned>((B * chunks + kVerifyWarps - 1) / kVerifyWarps), kVerifyWarps * 32, kVerifySmem, s>>>(
+        q, g, B, Nq, Ng, q_len, g_len, w.claim, w.block_max, w.rb_min_d2, vmargin, 1.0f / kDotScale, w.beaten);
+    mutual_final_batched_kernel<<<static_cast<unsigned>((rows_q + threads - 1) / threads), threads, 0, s>>>(i1, B, Nq, Ng, q_len, g_len,
+                                                                                                        w.claim, w.beaten, mutual);
+    HN_CUDA(cudaGetLastError());
+    count_launch(3);
+  }
   return HN_OK;
 }
 

@@ -12,6 +12,10 @@
 //   EPI_SHORTLIST : single fp16 pass (K = 128). Per row, the TOPC best 8-column chunks by dot product
 //               are kept (max3 trees + a rarely taken sorted insert); a tiny fp32 kernel then re-ranks
 //               those candidates exactly. Used for bulk matching.
+//   EPI_SHORTLIST_BATCHED : EPI_SHORTLIST over B independent padded problems (hn_match_batched). Operands are 3-D tensor maps
+//               {K, N, B} whose boxes never cross into the next pair (TMA zero-fills past N); a work item is (pair, query block,
+//               segment), and each pair has its own row / column counts (q_len / g_len). The batch logic is confined to the
+//               item decode, the TMA coordinates, the per-pair bounds and the output offsets, and compiles away elsewhere.
 #pragma once
 
 #include "../../include/hardnet_b200.h"
@@ -24,7 +28,7 @@ constexpr int kDistStages = 4;
 constexpr int kTopC = 4;     // chunks kept per row and segment
 constexpr int kChunk = 8;    // columns per chunk
 
-enum : int { EPI_EXACT = 0, EPI_SHORTLIST = 1, EPI_EXACT_NEI = 2 };   // EXACT_NEI = EXACT + the keypoint-neighbour masks
+enum : int { EPI_EXACT = 0, EPI_SHORTLIST = 1, EPI_EXACT_NEI = 2, EPI_SHORTLIST_BATCHED = 3 };   // EXACT_NEI = EXACT + the keypoint-neighbour masks
 
 struct DistSide {
   CUtensorMap tmA;             // rows of this launch direction, [Na, K] 16-bit
@@ -54,12 +58,22 @@ struct DistParams {
   int nei_mask;                // diagonal +10 and the neighbour masks (no +1e-8, no duplicate mask): HardNetNeiMask.loss
   float nei_c;                 // neighbour radius C in pixels
   float dot_scale;             // undoes the power-of-two operand scaling
+  // EPI_SHORTLIST_BATCHED only (appended: no parameter of the other kernels moves). side[0].Na / Nb are the padded per-pair
+  // sizes, cand / cand_val hold [batch * Na] rows, block_max is [batch][ceil(Nb / 8)][ceil(Na / 32)].
+  const int* q_len;            // [batch] valid query rows per pair (NULL = all), clamped to [0, Na]
+  const int* g_len;            // [batch] valid gallery rows per pair (NULL = all), clamped to [0, Nb]
+  int batch;
 };
 
 template <int MB>
 constexpr size_t dist_smem_bytes(int k_blocks) {
   return size_t(MB) * k_blocks * (kDistTile * 128) + size_t(kDistStages) * (kDistTile * 128) + 1024 + 256 + 2 * kDistTile * 4 +
          2 * kDistTile * 16 /* column keypoints of the neighbour mask */;
+}
+
+// Valid rows of pair b of a padded batch: len[b] clamped to [0, n], or n when no lengths are given.
+__device__ __forceinline__ long long pair_len(const int* len, long long b, long long n) {
+  return len ? min(max(static_cast<long long>(len[b]), 0ll), n) : n;
 }
 
 __device__ __forceinline__ float max3(float a, float b, float c) { return fmaxf(fmaxf(a, b), c); }
@@ -101,6 +115,8 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
   constexpr int CS = dist_col_split<EPI>();
   static_assert(CS == 1 || MB == 1, "the column split is for the single-M-block loss kernels");
   constexpr bool NEI = EPI == EPI_EXACT_NEI;   // compile-time: the plain loss kernel carries none of the mask code
+  constexpr bool BATCHED = EPI == EPI_SHORTLIST_BATCHED;
+  constexpr bool SHORTLIST = EPI == EPI_SHORTLIST || BATCHED;
   constexpr uint32_t BLK_BYTES = kDistTile * 128;  // 128 rows x 64 fp16
   constexpr uint32_t TMEM_COLS = 2 * MB * kDistTile;
   const DistSide& sd = p.side[blockIdx.y];
@@ -127,10 +143,16 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
 
   const int m_blocks = static_cast<int>((sd.Na + MB * kDistTile - 1) / (MB * kDistTile));
   const int n_tiles = static_cast<int>((sd.Nb + kDistTile - 1) / kDistTile);
-  const int num_items = m_blocks * p.segments;
-  auto seg_range = [&](int seg, int& t0, int& t1) {
-    t0 = static_cast<int>(static_cast<long long>(n_tiles) * seg / p.segments);
-    t1 = static_cast<int>(static_cast<long long>(n_tiles) * (seg + 1) / p.segments);
+  const int num_items = m_blocks * p.segments * (BATCHED ? p.batch : 1);
+  // An item is (pair, query block, segment); a single problem is pair 0. The valid query rows / gallery columns of a pair come
+  // from its lengths: producer, issuer and epilogue read the same ones, so they agree on which items and tiles exist.
+  auto pair_of = [&](int item) { return BATCHED ? item / (m_blocks * p.segments) : 0; };
+  auto pair_rows = [&](int pair) { return BATCHED ? pair_len(p.q_len, pair, sd.Na) : sd.Na; };
+  auto pair_cols = [&](int pair) { return BATCHED ? pair_len(p.g_len, pair, sd.Nb) : sd.Nb; };
+  auto pair_tiles = [&](int pair) { return BATCHED ? static_cast<int>((pair_cols(pair) + kDistTile - 1) / kDistTile) : n_tiles; };
+  auto seg_range = [&](int seg, int tiles, int& t0, int& t1) {
+    t0 = static_cast<int>(static_cast<long long>(tiles) * seg / p.segments);
+    t1 = static_cast<int>(static_cast<long long>(tiles) * (seg + 1) / p.segments);
   };
 
   if (warp == 0 && lane == 0) {
@@ -166,16 +188,22 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
       int stage = 0;
       uint32_t phase = 0, a_phase = 0;
       for (int item = blockIdx.x; item < num_items; item += gridDim.x) {
-        const int mblk = item / p.segments, seg = item - mblk * p.segments;
+        const int pair = pair_of(item), local = item - pair * (m_blocks * p.segments);
+        const int mblk = local / p.segments, seg = local - mblk * p.segments;
         int t0, t1;
-        seg_range(seg, t0, t1);
+        seg_range(seg, pair_tiles(pair), t0, t1);
+        if (BATCHED && (static_cast<long long>(mblk) * MB * kDistTile >= pair_rows(pair) || t0 == t1)) continue;   // as the issuer
         mbar_wait(aempty_bar, a_phase ^ 1u);
         if (elect_one()) {
           mbar_arrive_expect_tx(afull_bar, MB * p.k_blocks * BLK_BYTES);
           for (int mb = 0; mb < MB; ++mb)
-            for (int kb = 0; kb < p.k_blocks; ++kb)
-              tma_load_2d(a_base + (mb * p.k_blocks + kb) * BLK_BYTES, &sd.tmA, afull_bar, kb * 64,
-                          (mblk * MB + mb) * kDistTile);
+            for (int kb = 0; kb < p.k_blocks; ++kb) {
+              if (BATCHED)
+                tma_load_3d(a_base + (mb * p.k_blocks + kb) * BLK_BYTES, &sd.tmA, afull_bar, kb * 64, (mblk * MB + mb) * kDistTile, pair);
+              else
+                tma_load_2d(a_base + (mb * p.k_blocks + kb) * BLK_BYTES, &sd.tmA, afull_bar, kb * 64,
+                            (mblk * MB + mb) * kDistTile);
+            }
         }
         __syncwarp();
         a_phase ^= 1u;
@@ -184,7 +212,8 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
             mbar_wait(empty_bar(stage), phase ^ 1u);
             if (elect_one()) {
               mbar_arrive_expect_tx(full_bar(stage), BLK_BYTES);
-              tma_load_2d(b_base + stage * BLK_BYTES, &sd.tmB, full_bar(stage), kb * 64, t * kDistTile);
+              if (BATCHED) tma_load_3d(b_base + stage * BLK_BYTES, &sd.tmB, full_bar(stage), kb * 64, t * kDistTile, pair);
+              else tma_load_2d(b_base + stage * BLK_BYTES, &sd.tmB, full_bar(stage), kb * 64, t * kDistTile);
             }
             __syncwarp();
             if (++stage == kDistStages) { stage = 0; phase ^= 1u; }
@@ -204,9 +233,11 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
       uint32_t phase = 0, a_phase = 0;
       int it = 0;
       for (int item = blockIdx.x; item < num_items; item += gridDim.x) {
-        const int mblk = item / p.segments, seg = item - mblk * p.segments;
+        const int pair = pair_of(item), local = item - pair * (m_blocks * p.segments);
+        const int mblk = local / p.segments, seg = local - mblk * p.segments;
         int t0, t1;
-        seg_range(seg, t0, t1);
+        seg_range(seg, pair_tiles(pair), t0, t1);
+        if (BATCHED && (static_cast<long long>(mblk) * MB * kDistTile >= pair_rows(pair) || t0 == t1)) continue;   // as the producer
         mbar_wait(afull_bar, a_phase);
         a_phase ^= 1u;
         tc_fence_after();
@@ -246,11 +277,20 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
     const int ep_tid = threadIdx.x - 64;  // 0 .. 128*MB*CS-1
     int it = 0;
     for (int item = blockIdx.x; item < num_items; item += gridDim.x) {
-      const int mblk = item / p.segments, seg = item - mblk * p.segments;
+      const int pair = pair_of(item), local = item - pair * (m_blocks * p.segments);
+      const int mblk = local / p.segments, seg = local - mblk * p.segments;
+      // a single problem reads sd.Na / sd.Nb where it uses them
+      // 32-bit per-pair bounds (B * Na, B * Nb < 2^31): the epilogue runs at the register limit
+      const int rows_b = BATCHED ? static_cast<int>(pair_rows(pair)) : 0, cols_b = BATCHED ? static_cast<int>(pair_cols(pair)) : 0;
+      auto rows = [&] { return BATCHED ? static_cast<long long>(rows_b) : sd.Na; };
+      auto cols = [&] { return BATCHED ? static_cast<long long>(cols_b) : sd.Nb; };
       int t0, t1;
-      seg_range(seg, t0, t1);
+      seg_range(seg, pair_tiles(pair), t0, t1);
+      // a block without valid rows has no tiles in any role; an empty segment (t0 == t1) has none either, but its rows still
+      // get their (empty) candidate lists
+      if (BATCHED && static_cast<long long>(mblk) * MB * kDistTile >= rows()) continue;
       const long long row = static_cast<long long>(mblk * MB + mb) * kDistTile + q * 32 + lane;
-      const bool row_ok = row < sd.Na;
+      const bool row_ok = row < rows();
 
       // per-row running state
       float best = __int_as_float(0x7f800000);
@@ -291,8 +331,8 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
         mbar_wait(tfull_bar(acc), acc_phase);
         tc_fence_after();
         const uint32_t t_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + (acc * MB + mb) * kDistTile;
-        const bool ragged = col0 + kDistTile > sd.Nb;
-        if (EPI == EPI_SHORTLIST) {
+        const bool ragged = col0 + kDistTile > cols();
+        if (SHORTLIST) {
           // all four TMEM loads are issued before the single wait: one exposed round trip per tile instead of four
           uint32_t r[4][32];
 #pragma unroll
@@ -308,13 +348,13 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
             if (ragged) {
 #pragma unroll
               for (int j = 0; j < 32; ++j)
-                if (col0 + c0 + j >= sd.Nb) v[j] = -__int_as_float(0x7f800000);
+                if (col0 + c0 + j >= cols()) v[j] = -__int_as_float(0x7f800000);
             }
 #pragma unroll
             for (int s = 0; s < 32 / kChunk; ++s) {
               const float* w = v + s * kChunk;
               const float m = fmaxf(max3(w[0], w[1], w[2]), max3(max3(w[3], w[4], w[5]), w[6], w[7]));
-              cm[gq * 4 + s] = m;
+              cm[gq * 4 + s] = BATCHED && !row_ok ? -__int_as_float(0x7f800000) : m;   // padding rows stay out of the block maxima
               if (m > tb[kTopC - 1]) {
                 const int id = static_cast<int>((col0 + c0) / kChunk) + s;
                 // sorted insert (descending); strict '>' keeps the earlier chunk on ties
@@ -328,13 +368,15 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
           }
           if (sd.block_max != nullptr) {   // warp-uniform: column side of mutual NN (hn_match_mutual)
             const long long rb = row >> 5;
+            float* const bmax = BATCHED ? sd.block_max + static_cast<long long>(pair) * ((sd.Nb + kChunk - 1) / kChunk) * sd.n_row_blocks
+                                        : nullptr;   // this pair's [ceil(Nb / 8)][n_row_blocks] slice
 #pragma unroll
             for (int hf = 0; hf < 2; ++hf) {
               const float half8[8] = {cm[hf * 8], cm[hf * 8 + 1], cm[hf * 8 + 2], cm[hf * 8 + 3],
                                       cm[hf * 8 + 4], cm[hf * 8 + 5], cm[hf * 8 + 6], cm[hf * 8 + 7]};
               const float bm = warp_chunk_max8(half8, lane);
               const long long cb = col0 / kChunk + hf * 8 + (lane >> 2);
-              if ((lane & 3) == 0 && cb * kChunk < sd.Nb && rb < sd.n_row_blocks) sd.block_max[cb * sd.n_row_blocks + rb] = bm;
+              if ((lane & 3) == 0 && cb * kChunk < cols() && rb < sd.n_row_blocks) (BATCHED ? bmax : sd.block_max)[cb * sd.n_row_blocks + rb] = bm;
             }
           }
         } else {
@@ -421,11 +463,12 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
             atomicMin(sd.row_pack + row, pk);  // distances are positive: bit pattern is order preserving
           }
         } else {
-          int4* dst = reinterpret_cast<int4*>(sd.cand + (row * p.segments + seg) * kTopC);
+          const long long out_row = BATCHED ? pair * sd.Na + row : row;   // chunk ids stay local to the pair
+          int4* dst = reinterpret_cast<int4*>(sd.cand + (out_row * p.segments + seg) * kTopC);
           // unused slots (segment with < kTopC chunks) are marked -1
           *dst = make_int4(tb[0] > -3.0e38f ? tc[0] : -1, tb[1] > -3.0e38f ? tc[1] : -1, tb[2] > -3.0e38f ? tc[2] : -1,
                            tb[3] > -3.0e38f ? tc[3] : -1);
-          *reinterpret_cast<float4*>(sd.cand_val + (row * p.segments + seg) * kTopC) = make_float4(tb[0], tb[1], tb[2], tb[3]);
+          *reinterpret_cast<float4*>(sd.cand_val + (out_row * p.segments + seg) * kTopC) = make_float4(tb[0], tb[1], tb[2], tb[3]);
         }
       }
     }

@@ -101,22 +101,48 @@ def mutual_nearest_neighbors(des1, des2):
     return mutual_nn_ratio(des1, des2)[0]
 
 
+# ---- many image pairs per call ------------------------------------------------------------------------------------------
+# The reference's evaluation matches one image pair at a time (eval_utils.py:85-197). The batched forms take padded batches
+# des1 [B, Nq, 128] / des2 [B, Ng, 128] plus optional integer [B] lengths len1 / len2 (valid rows per pair; device tensors keep
+# the call free of host synchronisation) and run every pair in one launch sequence (hn_match_batched). Per pair and valid row
+# the results equal the per-pair functions on des1[b, :len1[b]], des2[b, :len2[b]]; rows past len1[b], and all rows of a pair
+# without gallery rows, get Da = Db = +inf, Ia = Ib = -1 and are never matched.
+
+def match_top2_batched(des1, des2, len1=None, len2=None):
+    """match_top2 for every pair of a padded batch -> (Da, Db, Ia, Ib), each [B, Nq]; indices int64, local to the pair."""
+    d1, d2, i1, i2 = _ops.match_batched(des1, des2, len1, len2)
+    return d1, d2, i1.long(), i2.long()
+
+
+def mutual_nn_ratio_batched(des1, des2, len1=None, len2=None, threshold=0.7):
+    """mutual_nn_ratio for every pair of a padded batch -> (mutual, ratio_label, Ia, Da, Db), all [B, Nq]. No pair list:
+    compacting it needs its length on the host; mutual[b].nonzero() gives pair b's query rows."""
+    d1, d2, i1, _, mutual = _ops.match_batched(des1, des2, len1, len2, mutual=True)
+    return mutual, (d1 / d2).lt(threshold), i1.long(), d1, d2
+
+
 # ---- match-score counters (FDLNet-master/utils/eval_utils.py:112-197) -----------------------------------------------
 # The callers right behind the hot path in the reference's evaluation: nearest neighbour (or ratio test) on the fused
 # kernel, then "is the matched keypoint within COO_THRSH pixels of the warped keypoint" and two counters. The reference
 # builds an Nq x Nq coordinate distance matrix and takes its diagonal; the same expression is evaluated row-wise here.
 
 def _keypoint_distance(kp1w, nn_kp2):
-    """diag(pairwise_distances(kp1w[:, 1:3], nn_kp2[:, 1:3])) of math_utils.py:22-40: sqrt(clamp(|x|^2 + |y|^2 - 2 x.y, 1e-8))."""
-    x, y = kp1w[:, 1:3].float(), nn_kp2[:, 1:3].float()
-    sq = (x * x).sum(1) + (y * y).sum(1) - 2.0 * (x * y).sum(1)
+    """diag(pairwise_distances(kp1w[..., 1:3], nn_kp2[..., 1:3])) of math_utils.py:22-40: sqrt(clamp(|x|^2 + |y|^2 - 2 x.y, 1e-8)),
+    over the last keypoint dimension (one pair [N, >=3] or a batch of pairs [B, N, >=3])."""
+    x, y = kp1w[..., 1:3].float(), nn_kp2[..., 1:3].float()
+    sq = (x * x).sum(-1) + (y * y).sum(-1) - 2.0 * (x * y).sum(-1)
     return torch.sqrt(sq.clamp(min=1e-8))
 
 
-def _score(predict_label, kp1w, nn_kp2, visible, coo_thrsh, predicted):
+def _counts(predict_label, kp1w, nn_kp2, visible, coo_thrsh, predicted):
+    """(correct, max(#predicted, 1)) as device tensors, counted over the last dimension (per pair)."""
     correspondences = _keypoint_distance(kp1w, nn_kp2).le(coo_thrsh) & visible.bool()
-    correct = (predict_label & correspondences).sum().item()
-    return correct, max(predicted.sum().item(), 1)
+    return (predict_label & correspondences).sum(-1), predicted.sum(-1).clamp(min=1)
+
+
+def _score(predict_label, kp1w, nn_kp2, visible, coo_thrsh, predicted):
+    correct, predict = _counts(predict_label, kp1w, nn_kp2, visible, coo_thrsh, predicted)
+    return correct.item(), predict.item()
 
 
 def nearest_neighbor_match_score(des1, des2, kp1w, kp2, visible, COO_THRSH):
@@ -138,3 +164,35 @@ def nearest_neighbor_distance_ratio_match_score(des1, des2, kp1w, kp2, visible, 
     label, nn_kp2 = nearest_neighbor_distance_ratio_match(des1, des2, kp2, threshold)
     predict = label & visible.bool()
     return _score(predict, kp1w, nn_kp2, visible, COO_THRSH, predict)
+
+
+# Batched counters: kp1w [B, Nq, >=3], kp2 [B, Ng, >=3], visible [B, Nq] are the per-pair arguments with a batch dimension;
+# each returns (correct [B], predicted [B]) int64 device tensors, without host synchronisation. A row without a match (past
+# len1, or in a pair without gallery rows) is neither predicted nor correct.
+
+def _batched_nn_kp2(kp2, ia):
+    """kp2[b, Ia[b, i]] for every pair; rows without a match (Ia = -1) read row 0 and are masked by the caller."""
+    return torch.gather(kp2, 1, ia.clamp(min=0).unsqueeze(-1).expand(-1, -1, kp2.size(-1)))
+
+
+def nearest_neighbor_match_score_batched(des1, des2, kp1w, kp2, visible, COO_THRSH, len1=None, len2=None):
+    """nearest_neighbor_match_score per pair -> (correct [B], predicted = max(#visible, 1) [B])."""
+    _, _, ia, _ = match_top2_batched(des1, des2, len1, len2)
+    vis = visible.bool() & (ia >= 0)
+    return _counts(vis, kp1w, _batched_nn_kp2(kp2, ia), vis, COO_THRSH, vis)
+
+
+def nearest_neighbor_threshold_match_score_batched(des1, des2, kp1w, kp2, visible, DES_THRSH, COO_THRSH, len1=None, len2=None):
+    """nearest_neighbor_threshold_match_score per pair -> (correct [B], predicted = max(#(Da < DES_THRSH and visible), 1) [B])."""
+    da, _, ia, _ = match_top2_batched(des1, des2, len1, len2)
+    predict = da.lt(DES_THRSH) & visible.bool() & (ia >= 0)
+    return _counts(predict, kp1w, _batched_nn_kp2(kp2, ia), visible, COO_THRSH, predict)
+
+
+def nearest_neighbor_distance_ratio_match_score_batched(des1, des2, kp1w, kp2, visible, COO_THRSH, threshold=0.7, len1=None,
+                                                        len2=None):
+    """nearest_neighbor_distance_ratio_match_score per pair -> (correct [B], predicted = max(#(Da / Db < threshold and
+    visible), 1) [B])."""
+    da, db, ia, _ = match_top2_batched(des1, des2, len1, len2)
+    predict = (da / db).lt(threshold) & visible.bool() & (ia >= 0)
+    return _counts(predict, kp1w, _batched_nn_kp2(kp2, ia), visible, COO_THRSH, predict)

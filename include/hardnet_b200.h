@@ -211,11 +211,26 @@ int hn_mutual_verify(const float* q, long long Nq, long long q_offset, const flo
                      const unsigned long long* claim, const float* block_max, const float* rb_min_d2, unsigned char* beaten,
                      void* stream);
 
+/* Batched matching: B independent problems of the shapes hn_match / hn_match_mutual solve, in one launch sequence (the shape
+ * of an evaluation loop over image pairs, FDLNet-master/utils/eval_utils.py:85-197). q:[B,Nq,128], g:[B,Ng,128] fp32 padded
+ * batches with unit-norm rows; q_len / g_len: DEVICE int32 [B] valid row counts per pair (NULL = all rows), clamped to
+ * [0, Nq] / [0, Ng] on the device, so the call reads nothing on the host and is CUDA-graph capturable.
+ * Outputs [B*Nq]: for a valid row r < q_len[b], d1 / d2 / i1 / i2 equal hn_match(q[b, :q_len[b]], g[b, :g_len[b]]) bit for bit
+ * (indices local to the pair) and mutual (optional, NULL = no column side) equals hn_match_mutual on the same slices, wherever
+ * the shortlists are exact (see hn_match). Rows past q_len[b], and every row of a pair with g_len[b] == 0, get d1 = d2 = +inf,
+ * i1 = i2 = -1 and mutual = 0; g_len[b] == 1 gives d2 = +inf, i2 = -1. Padding rows may hold anything (NaN included): they
+ * never influence another row or pair. Requires B*Nq and B*Ng below 2^31 and a 256-byte-aligned workspace of
+ * hn_match_batched_workspace_bytes(B, Nq, Ng, mutual != NULL) bytes. */
+long long hn_match_batched_workspace_bytes(long long B, long long Nq, long long Ng, int with_mutual);
+int hn_match_batched(const float* q, const float* g, long long B, long long Nq, long long Ng, const int32_t* q_len,
+                     const int32_t* g_len, float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual,
+                     void* workspace, long long workspace_bytes, void* stream);
+
 /* Test / measurement switch (process-wide): which matching GEMM hn_match runs: -1 = chosen by problem size (default; the
  * initial value is read once from HN_MATCH_PAIR), 0 = single-CTA kernel, 1 = CTA-pair (cta_group::2) kernel. */
 int hn_match_force_kernel(int mode);
 
-/* Measurement hooks (process-wide): bracket the three stages of every hn_match call (0 = operand packing, 1 = GEMM +
+/* Measurement hooks (process-wide): bracket the three stages of every hn_match / hn_match_batched call (0 = operand packing, 1 = GEMM +
  * shortlist, 2 = exact re-rank) with CUDA events; hn_match_profile_read waits for them, returns the summed milliseconds and
  * launch counts per stage and resets the counters. */
 int hn_match_profile_enable(int on);
