@@ -51,6 +51,9 @@ SIGNATURES = {
     "hn_mutual_verify": (C.c_int, [_P, C.c_longlong, C.c_longlong, _P, C.c_longlong, _P, _P, _P, _P, _P]),
     "hn_match_batched_workspace_bytes": (C.c_longlong, [C.c_longlong, C.c_longlong, C.c_longlong, C.c_int]),
     "hn_match_batched": (C.c_int, [_P, _P, C.c_longlong, C.c_longlong, C.c_longlong, _P, _P, _P, _P, _P, _P, _P, _P, C.c_longlong, _P]),
+    "hn_match_pairs_workspace_bytes": (C.c_longlong, [C.c_longlong, C.c_longlong, C.c_longlong, C.c_int]),
+    "hn_match_pairs": (C.c_int, [_P, _P, C.c_longlong, _P, _P, C.c_longlong, _P, C.c_longlong, C.c_longlong, C.c_longlong, _P, _P, _P,
+                                 _P, _P, _P, C.c_longlong, _P]),
     "hn_match_force_kernel": (C.c_int, [C.c_int]),
     "hn_match_profile_enable": (C.c_int, [C.c_int]),
     "hn_match_profile_read": (C.c_int, [C.POINTER(C.c_double), C.POINTER(C.c_longlong)]),

@@ -209,6 +209,48 @@ def match_batched(q: torch.Tensor, g: torch.Tensor, q_len: torch.Tensor | None =
     return (d1, d2, i1, i2, mu) if mutual else (d1, d2, i1, i2)
 
 
+def _packed(name: str, t: torch.Tensor, n: int) -> torch.Tensor:
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float16 and tuple(t.shape) == (n, 128)
+            and t.is_contiguous()):
+        raise ValueError(f"{name}: packed operands must be contiguous CUDA fp16 [n,128] tensors from pack_descriptors")
+    return t
+
+
+def match_pairs(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, max_q: int, max_g: int, q16: torch.Tensor | None = None,
+                g16: torch.Tensor | None = None, mutual: bool = False):
+    """(d1, d2, i1, i2[, mutual]), each [P, max_q]: hn_match_pairs over the concatenated sets q [Nq_rows, 128] and
+    g [Ng_rows, 128]. pairs: integer [P, 4] table of (q_start, q_len, g_start, g_len), copied to q's device as int32 (a table
+    already there keeps the call free of host synchronisation). q16 / g16: the sets' rows packed by `pack_descriptors`; a set
+    whose packed rows are not given is packed here, once when g is q. Indices are local to the pair's gallery range; rows past
+    q_len get d = +inf, i = -1 (and mutual = False)."""
+    lib = _lib.load()
+    same = g is q
+    q = _require_cuda_f32("match_pairs", q)
+    g = q if same else _require_cuda_f32("match_pairs", g)
+    if not isinstance(pairs, torch.Tensor) or pairs.dtype not in (torch.int32, torch.int64) or pairs.dim() != 2 or pairs.size(1) != 4:
+        raise ValueError("match_pairs: pairs must be an int32 or int64 [P, 4] tensor of (q_start, q_len, g_start, g_len)")
+    dev = q.device
+    if g.device != dev:
+        raise ValueError("match_pairs: q and g must be on the same device")
+    table = pairs.to(device=dev, dtype=torch.int32).contiguous()
+    nq, ng, b = q.size(0), g.size(0), table.size(0)
+    if q16 is None:
+        q16 = g16 if same and g16 is not None else pack_descriptors(q)
+    if g16 is None:
+        g16 = q16 if same else pack_descriptors(g)
+    q16, g16 = _packed("match_pairs", q16, nq), _packed("match_pairs", g16, ng)
+    with torch.cuda.device(dev):
+        ws = _workspace(dev, max(lib.hn_match_pairs_workspace_bytes(b, max_q, max_g, int(mutual)), 1))
+        d1 = torch.empty((b, max_q), dtype=torch.float32, device=dev)
+        d2 = torch.empty((b, max_q), dtype=torch.float32, device=dev)
+        i1 = torch.empty((b, max_q), dtype=torch.int32, device=dev)
+        i2 = torch.empty((b, max_q), dtype=torch.int32, device=dev)
+        mu = torch.empty((b, max_q), dtype=torch.bool, device=dev) if mutual else None
+        _lib.check(lib.hn_match_pairs(_ptr(q), _ptr(q16), nq, _ptr(g), _ptr(g16), ng, _ptr(table), b, max_q, max_g, _ptr(d1),
+                                      _ptr(d2), _ptr(i1), _ptr(i2), _ptr(mu), _ptr(ws), ws.numel(), _stream_ptr()), "hn_match_pairs")
+    return (d1, d2, i1, i2, mu) if mutual else (d1, d2, i1, i2)
+
+
 def mutual_claims(i1: torch.Tensor, d1: torch.Tensor, d2: torch.Tensor, q_offset: int, claim: torch.Tensor) -> torch.Tensor:
     """atomicMin of (distance, global row) into claim[int64, Ng] (pre-filled with INT64_MAX = unclaimed); returns the per
     32-row-block minimum of d2 the verification needs."""

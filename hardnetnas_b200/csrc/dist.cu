@@ -208,35 +208,44 @@ __global__ void __launch_bounds__(128) rerank_kernel(const float* __restrict__ q
 
 // Batched re-rank over the flat [B * nq_pad] query rows of hn_match_batched: row -> pair b = row / nq_pad, whose gallery is
 // rows [0, g_len[b]) of g + b * ng_pad * 128; indices are local to the pair. Rows past q_len[b] get the fill values
-// (d = +inf, i = -1). From the prologue on this is rerank_kernel's body, copied rather than shared so that the single-problem
+// (d = +inf, i = -1). TABLE (hn_match_pairs): pair b's rows are the ranges of the pair table over the concatenated sets instead,
+// query row qs + r of q and gallery rows [gs, gs + gl) of g_all; the padded instantiation keeps the instructions it had before
+// hn_match_pairs existed (reading the padded layout through the table accessor measured 1-2 % slower). From the prologue on this is rerank_kernel's body, copied rather than shared so that the single-problem
 // kernel compiles to the same instructions as before: keep the two in step, the bit equality of a batched row with a per-pair
 // hn_match rests on the same candidate threshold and the same summation order (tests/test_matching_batched_gpu.py compares
 // them bit for bit). One difference: the eight distances of a chunk are taken by eight lanes, one sqrtf each, and shuffled to
 // the warp (the same values: every lane holds the same eight dot products). Eight unrolled sqrtf slow-path calls per lane kept
 // the pair's gallery pointer and size live across calls and made ptxas spill.
+template <bool TABLE>
 __global__ void __launch_bounds__(128) rerank_batched_kernel(const float* __restrict__ q, const float* __restrict__ g_all,
                                                              const int* __restrict__ cand, const float* __restrict__ cand_val,
                                                              float margin, long long B, long long nq_pad, long long ng_pad,
                                                              const int* __restrict__ q_len, const int* __restrict__ g_len, int slots,
                                                              float* __restrict__ d1, float* __restrict__ d2, int* __restrict__ i1,
-                                                             int* __restrict__ i2) {
+                                                             int* __restrict__ i2, const int* __restrict__ pairs, long long q_rows,
+                                                             long long g_rows) {
   __shared__ __align__(16) float sq[4][128];
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long row = static_cast<long long>(blockIdx.x) * 4 + w;
   if (row >= B * nq_pad) return;
   const int b = static_cast<int>(row) / static_cast<int>(nq_pad);   // B * nq_pad < 2^31; element offsets below stay 64-bit
-  if (row - b * nq_pad >= pair_len(q_len, b, nq_pad)) {
+  Span qs{0, 0}, gs{0, 0};
+  if constexpr (TABLE) {
+    qs = table_span(pairs, b, 0, nq_pad, q_rows);
+    gs = table_span(pairs, b, 1, ng_pad, g_rows);
+  }
+  if (row - b * nq_pad >= (TABLE ? qs.len : pair_len(q_len, b, nq_pad))) {
     if (lane == 0) {
       d1[row] = d2[row] = __int_as_float(0x7f800000);
       i1[row] = i2[row] = -1;
     }
     return;
   }
-  const float* g = g_all + static_cast<long long>(b) * ng_pad * 128;
-  const long long ng = pair_len(g_len, b, ng_pad);
+  const float* g = TABLE ? g_all + gs.start * 128 : g_all + static_cast<long long>(b) * ng_pad * 128;
+  const long long ng = TABLE ? gs.len : pair_len(g_len, b, ng_pad);
   const int* crow = cand + row * slots;
   const float* cvrow = cand_val + row * slots;
-  reinterpret_cast<float4*>(sq[w])[lane] = reinterpret_cast<const float4*>(q + row * 128)[lane];
+  reinterpret_cast<float4*>(sq[w])[lane] = reinterpret_cast<const float4*>(q + (TABLE ? qs.start + (row - b * nq_pad) : row) * 128)[lane];
   __syncwarp();
   // A chunk can hold one of the two nearest columns only if its approximate maximum reaches the second largest
   // chunk maximum minus twice the error bound of the 16-bit-operand dot product (`margin`, same scaled units).
@@ -500,37 +509,42 @@ __global__ void mutual_final_kernel(const int* __restrict__ i1, long long nq, lo
 // Batched column side of hn_match_batched. Claims, beaten flags and block maxima are per pair ([B][ng], [B][ng],
 // [B][ceil(ng / 8)][ceil(nq / 32)]); query rows are local to the pair, so ties resolve to the lowest local row as in a per-pair
 // call. Rows past q_len[b] are never claimants or candidates, and columns past g_len[b] are never claimed.
+// TABLE: the lengths come from the pair table (see rerank_batched_kernel); everything else is per pair as above.
 // Claims: one thread per (pair, 32-row block slot): a warp is one row block of one pair, padded to whole blocks.
+template <bool TABLE>
 __global__ void mutual_claim_batched_kernel(const int* __restrict__ i1, const float* __restrict__ d1, const float* __restrict__ d2,
                                             long long B, long long nq, long long ng, const int* __restrict__ q_len,
                                             const int* __restrict__ g_len, unsigned long long* __restrict__ claim,
-                                            float* __restrict__ rb_min_d2) {
+                                            float* __restrict__ rb_min_d2, const int* __restrict__ pairs, long long q_rows,
+                                            long long g_rows) {
   const long long nrb = (nq + 31) / 32;
   const long long t = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (t >= B * nrb * 32) return;   // whole warps
   const long long b = t / (nrb * 32), r = t - b * nrb * 32;   // 64-bit: B * nrb * 32 may pass 2^31 while B * nq does not
   const long long i = b * nq + r;
-  const bool valid = r < pair_len(q_len, b, nq);
+  const bool valid = r < (TABLE ? table_span(pairs, b, 0, nq, q_rows).len : pair_len(q_len, b, nq));
   float m = valid ? d2[i] : __int_as_float(0x7f800000);
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) m = fminf(m, __shfl_xor_sync(0xffffffffu, m, o));
   if ((threadIdx.x & 31) == 0) rb_min_d2[b * nrb + (r >> 5)] = m;
   if (!valid) return;
   const long long j = i1[i];
-  if (j < 0 || j >= pair_len(g_len, b, ng)) return;
+  if (j < 0 || j >= (TABLE ? table_span(pairs, b, 1, ng, g_rows).len : pair_len(g_len, b, ng))) return;
   atomicMin(claim + b * ng + j, (static_cast<unsigned long long>(__float_as_uint(d1[i])) << 32) | static_cast<unsigned int>(r));
 }
 
 // One warp per (pair, 8-column chunk), scanning only the pair's valid row blocks. After the prologue (pair pointers and
 // bounds) this is mutual_verify_kernel's body with q_offset = 0 and a block_max row pitch of ceil(nq_pad / 32), copied rather
 // than shared so that the single-problem kernel compiles to the same instructions as before: keep the two in step.
+template <bool TABLE>
 __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kernel(const float* __restrict__ q_all, const float* __restrict__ g_all,
                                                                                  long long B, long long nq_pad, long long ng_pad,
                                                                                  const int* __restrict__ q_len, const int* __restrict__ g_len,
                                                                                  const unsigned long long* __restrict__ claim_all,
                                                                                  const float* __restrict__ block_max_all,
                                                                                  const float* __restrict__ rb_min_d2_all, float margin_scaled,
-                                                                                 float inv_dot_scale, unsigned char* __restrict__ beaten_all) {
+                                                                                 float inv_dot_scale, unsigned char* __restrict__ beaten_all,
+                                                                                 const int* __restrict__ pairs, long long q_rows, long long g_rows) {
   extern __shared__ __align__(16) uint8_t vsm[];
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* s_q = reinterpret_cast<float*>(vsm) + static_cast<size_t>(w) * 32 * kVerifyPitch;                       // [32][132]
@@ -539,10 +553,15 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kerne
   const long long item = static_cast<long long>(blockIdx.x) * kVerifyWarps + w;
   const long long pair = static_cast<int>(item) / static_cast<int>(chunks), cb = item - pair * chunks;   // B * chunks <= B * ng_pad < 2^31
   if (pair >= B) return;
-  const long long nq = pair_len(q_len, pair, nq_pad), ng = pair_len(g_len, pair, ng_pad), q_offset = 0;
+  Span qs{0, 0}, gs{0, 0};
+  if constexpr (TABLE) {
+    qs = table_span(pairs, pair, 0, nq_pad, q_rows);
+    gs = table_span(pairs, pair, 1, ng_pad, g_rows);
+  }
+  const long long nq = TABLE ? qs.len : pair_len(q_len, pair, nq_pad), ng = TABLE ? gs.len : pair_len(g_len, pair, ng_pad), q_offset = 0;
   const int n_row_blocks = static_cast<int>((nq + 31) / 32);
-  const float* q = q_all + pair * nq_pad * 128;
-  const float* g = g_all + pair * ng_pad * 128;
+  const float* q = TABLE ? q_all + qs.start * 128 : q_all + pair * nq_pad * 128;
+  const float* g = TABLE ? g_all + gs.start * 128 : g_all + pair * ng_pad * 128;
   const unsigned long long* claim = claim_all + pair * ng_pad;
   const float* block_max = block_max_all + pair * chunks * bm_pitch;
   const float* rb_min_d2 = rb_min_d2_all + pair * bm_pitch;
@@ -642,17 +661,19 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kerne
 }
 
 
+template <bool TABLE>
 __global__ void mutual_final_batched_kernel(const int* __restrict__ i1, long long B, long long nq, long long ng,
                                             const int* __restrict__ q_len, const int* __restrict__ g_len,
                                             const unsigned long long* __restrict__ claim, const unsigned char* __restrict__ beaten,
-                                            unsigned char* __restrict__ mutual) {
+                                            unsigned char* __restrict__ mutual, const int* __restrict__ pairs, long long q_rows,
+                                            long long g_rows) {
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= B * nq) return;
   const long long b = static_cast<int>(i) / static_cast<int>(nq), r = i - b * nq;
   bool m = false;
-  if (r < pair_len(q_len, b, nq)) {
+  if (r < (TABLE ? table_span(pairs, b, 0, nq, q_rows).len : pair_len(q_len, b, nq))) {
     const long long j = i1[i];
-    if (j >= 0 && j < pair_len(g_len, b, ng))
+    if (j >= 0 && j < (TABLE ? table_span(pairs, b, 1, ng, g_rows).len : pair_len(g_len, b, ng)))
       m = static_cast<unsigned int>(claim[b * ng + j] & 0xffffffffu) == static_cast<unsigned int>(r) && !beaten[b * ng + j];
   }
   mutual[i] = m ? 1 : 0;
@@ -1031,10 +1052,11 @@ extern "C" int hn_match_mutual(const float* q, const float* g, const void* q16, 
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// batched matching: B independent padded problems in one launch sequence (hn_match_batched)
+// batched matching: B problems in one launch sequence, padded (hn_match_batched) or over row ranges of concatenated sets
+// (hn_match_pairs)
 // ------------------------------------------------------------------------------------------------------------
 struct BatchedWs {
-  uint16_t *q16, *g16;
+  uint16_t *q16, *g16;       // hn_match_batched only: its packed operands
   int* cand;
   float* cand_val;
   float* block_max;          // mutual only
@@ -1044,14 +1066,15 @@ struct BatchedWs {
   size_t bytes;
 };
 
-static BatchedWs carve_batched(void* ws, long long B, long long Nq, long long Ng, bool with_mutual) {
+// Nq / Ng: the per-pair maxima (output pitch). with_packed: room for B*Nq and B*Ng packed rows in front (hn_match_batched).
+static BatchedWs carve_batched(void* ws, long long B, long long Nq, long long Ng, bool with_mutual, bool with_packed) {
   BatchedWs w;
   char* b = static_cast<char*>(ws);
   size_t off = 0;
   auto take = [&](size_t n) { char* r = b ? b + off : nullptr; off += align256(n); return r; };
   const size_t rows_q = static_cast<size_t>(B) * Nq, rows_g = static_cast<size_t>(B) * Ng;
-  w.q16 = reinterpret_cast<uint16_t*>(take(rows_q * 128 * 2));
-  w.g16 = reinterpret_cast<uint16_t*>(take(rows_g * 128 * 2));
+  w.q16 = with_packed ? reinterpret_cast<uint16_t*>(take(rows_q * 128 * 2)) : nullptr;
+  w.g16 = with_packed ? reinterpret_cast<uint16_t*>(take(rows_g * 128 * 2)) : nullptr;
   // candidate lists [rows][segments][kTopC]: a segment holds at least one gallery tile, so at most min(16, tiles) of them
   const size_t lists = rows_q * batched_max_segments(Ng) * kTopC * 4;
   w.cand = reinterpret_cast<int*>(take(lists));
@@ -1078,9 +1101,90 @@ static int make_batched_desc_map(CUtensorMap* tm, const uint16_t* base, long lon
   return make_tmap_16bit(tm, base, 3, dims, str, box, 128);
 }
 
+// Where the pairs of a batched call live. With `pairs` (hn_match_pairs): row ranges [B][4] = (q_start, q_len, g_start, g_len)
+// of the concatenated sets of q_rows / g_rows rows. Without (hn_match_batched): the padded layout, pair b at rows b * max_q /
+// b * max_g with q_len[b] / g_len[b] valid rows (NULL = all), q_rows = B * max_q, g_rows = B * max_g.
+struct PairLayout {
+  const int* pairs;
+  const int* q_len;
+  const int* g_len;
+  long long B, max_q, max_g, q_rows, g_rows;
+};
+
+// The launch sequence of hn_match_pairs (TABLE) and hn_match_batched: GEMM + shortlist, re-rank, and with `mutual` the column
+// side. q16 / g16 are the packed rows of q / g.
+template <bool TABLE>
+static int run_pairs(const float* q, const uint16_t* q16, const float* g, const uint16_t* g16, const PairLayout& L, float* d1,
+                     float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, const BatchedWs& w, cudaStream_t s) {
+  int sm = 0;
+  HN_TRY(device_sm_count(&sm));
+  const long long B = L.B, Nq = L.max_q, Ng = L.max_g, rows_q = B * Nq, rows_g = B * Ng;
+  const int threads = 256;
+  DistParams dp;
+  memset(&dp, 0, sizeof(dp));
+  if (TABLE) {
+    HN_TRY(make_desc_map(&dp.side[0].tmA, q16, L.q_rows, 128));
+    HN_TRY(make_desc_map(&dp.side[0].tmB, g16, L.g_rows, 128));
+  } else {
+    HN_TRY(make_batched_desc_map(&dp.side[0].tmA, q16, Nq, B));
+    HN_TRY(make_batched_desc_map(&dp.side[0].tmB, g16, Ng, B));
+  }
+  dp.side[0].cand = w.cand;
+  dp.side[0].cand_val = w.cand_val;
+  dp.side[0].block_max = w.block_max;
+  dp.side[0].n_row_blocks = static_cast<int>((Nq + 31) / 32);
+  dp.side[0].Na = Nq;
+  dp.side[0].Nb = Ng;
+  dp.k_blocks = 2;
+  dp.form = HN_FORM_FDL;
+  dp.dot_scale = kDotScale;
+  dp.q_len = L.q_len;
+  dp.g_len = L.g_len;
+  dp.batch = static_cast<int>(B);
+  dp.pairs = L.pairs;
+  dp.q_rows = L.q_rows;
+  dp.g_rows = L.g_rows;
+  {
+    MatchTimer timer(1, s);
+    // segments from the per-pair maxima (lengths live on the device): B * ceil(Nq / 256) query blocks over a gallery of Ng
+    const long long m_blocks = (Nq + 2 * kDistTile - 1) / (2 * kDistTile);
+    dp.segments = pick_segments(B * m_blocks * 2 * kDistTile, 2 * kDistTile, Ng, sm, static_cast<int>(batched_max_segments(Ng)));
+    const int grid = static_cast<int>(std::min<long long>(B * m_blocks * dp.segments, sm));
+    if (TABLE) HN_TRY((launch_dist<2, EPI_SHORTLIST_PAIRS>(dp, grid, 1, s)));
+    else HN_TRY((launch_dist<2, EPI_SHORTLIST_BATCHED>(dp, grid, 1, s)));
+  }
+  const float margin = 4.0f * (1.0f / 1024.0f) / kDotScale;   // as hn_match_ex
+  {
+    MatchTimer timer(2, s);
+    rerank_batched_kernel<TABLE><<<static_cast<unsigned>((rows_q + 3) / 4), 128, 0, s>>>(
+        q, g, w.cand, w.cand_val, margin, B, Nq, Ng, L.q_len, L.g_len, dp.segments * kTopC, d1, d2, i1, i2, L.pairs, L.q_rows, L.g_rows);
+    HN_CUDA(cudaGetLastError());
+    count_launch();
+  }
+  if (mutual) {
+    HN_CUDA(cudaMemsetAsync(w.claim, 0x7f, static_cast<size_t>(rows_g) * 8, s));   // "unclaimed"
+    HN_CUDA(cudaMemsetAsync(w.beaten, 0, static_cast<size_t>(rows_g), s));
+    const long long nrb = (Nq + 31) / 32, chunks = (Ng + kChunk - 1) / kChunk;
+    mutual_claim_batched_kernel<TABLE><<<static_cast<unsigned>((B * nrb * 32 + threads - 1) / threads), threads, 0, s>>>(
+        i1, d1, d2, B, Nq, Ng, L.q_len, L.g_len, w.claim, w.rb_min_d2, L.pairs, L.q_rows, L.g_rows);
+    static DeviceOnce attr_once;
+    if (attr_once.first_time())
+      HN_CUDA(cudaFuncSetAttribute(mutual_verify_batched_kernel<TABLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kVerifySmem)));
+    const float vmargin = 2.0f * (1.0f / 1024.0f) / kDotScale;   // as hn_mutual_verify
+    mutual_verify_batched_kernel<TABLE><<<static_cast<unsigned>((B * chunks + kVerifyWarps - 1) / kVerifyWarps), kVerifyWarps * 32, kVerifySmem, s>>>(
+        q, g, B, Nq, Ng, L.q_len, L.g_len, w.claim, w.block_max, w.rb_min_d2, vmargin, 1.0f / kDotScale, w.beaten, L.pairs, L.q_rows,
+        L.g_rows);
+    mutual_final_batched_kernel<TABLE><<<static_cast<unsigned>((rows_q + threads - 1) / threads), threads, 0, s>>>(
+        i1, B, Nq, Ng, L.q_len, L.g_len, w.claim, w.beaten, mutual, L.pairs, L.q_rows, L.g_rows);
+    HN_CUDA(cudaGetLastError());
+    count_launch(3);
+  }
+  return HN_OK;
+}
+
 extern "C" long long hn_match_batched_workspace_bytes(long long B, long long Nq, long long Ng, int with_mutual) {
   if (B < 0 || Nq < 0 || Ng < 0) return 0;
-  return static_cast<long long>(carve_batched(nullptr, B, Nq, Ng, with_mutual != 0).bytes);
+  return static_cast<long long>(carve_batched(nullptr, B, Nq, Ng, with_mutual != 0, true).bytes);
 }
 
 extern "C" int hn_match_batched(const float* q, const float* g, long long B, long long Nq, long long Ng, const int32_t* q_len,
@@ -1092,9 +1196,7 @@ extern "C" int hn_match_batched(const float* q, const float* g, long long B, lon
   HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "hn_match_batched: workspace must be 256-byte aligned");
   HN_REQUIRE(workspace_bytes >= hn_match_batched_workspace_bytes(B, Nq, Ng, mutual != nullptr), "hn_match_batched: workspace too small");
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  int sm = 0;
-  HN_TRY(device_sm_count(&sm));
-  const BatchedWs w = carve_batched(workspace, B, Nq, Ng, mutual != nullptr);
+  const BatchedWs w = carve_batched(workspace, B, Nq, Ng, mutual != nullptr, true);
   const long long rows_q = B * Nq, rows_g = B * Ng;
   const int threads = 256;
   {
@@ -1104,56 +1206,33 @@ extern "C" int hn_match_batched(const float* q, const float* g, long long B, lon
     HN_CUDA(cudaGetLastError());
     count_launch(2);
   }
-  DistParams dp;
-  memset(&dp, 0, sizeof(dp));
-  HN_TRY(make_batched_desc_map(&dp.side[0].tmA, w.q16, Nq, B));
-  HN_TRY(make_batched_desc_map(&dp.side[0].tmB, w.g16, Ng, B));
-  dp.side[0].cand = w.cand;
-  dp.side[0].cand_val = w.cand_val;
-  dp.side[0].block_max = w.block_max;
-  dp.side[0].n_row_blocks = static_cast<int>((Nq + 31) / 32);
-  dp.side[0].Na = Nq;
-  dp.side[0].Nb = Ng;
-  dp.k_blocks = 2;
-  dp.form = HN_FORM_FDL;
-  dp.dot_scale = kDotScale;
-  dp.q_len = q_len;
-  dp.g_len = g_len;
-  dp.batch = static_cast<int>(B);
-  {
-    MatchTimer timer(1, s);
-    // segments from the padded sizes (lengths live on the device): B * ceil(Nq / 256) query blocks over a gallery of Ng
-    const long long m_blocks = (Nq + 2 * kDistTile - 1) / (2 * kDistTile);
-    dp.segments = pick_segments(B * m_blocks * 2 * kDistTile, 2 * kDistTile, Ng, sm, static_cast<int>(batched_max_segments(Ng)));
-    const long long items = B * m_blocks * dp.segments;
-    HN_TRY((launch_dist<2, EPI_SHORTLIST_BATCHED>(dp, static_cast<int>(std::min<long long>(items, sm)), 1, s)));
-  }
-  const float margin = 4.0f * (1.0f / 1024.0f) / kDotScale;   // as hn_match_ex
-  {
-    MatchTimer timer(2, s);
-    rerank_batched_kernel<<<static_cast<unsigned>((rows_q + 3) / 4), 128, 0, s>>>(q, g, w.cand, w.cand_val, margin, B, Nq, Ng, q_len, g_len,
-                                                                                  dp.segments * kTopC, d1, d2, i1, i2);
-    HN_CUDA(cudaGetLastError());
-    count_launch();
-  }
-  if (mutual) {
-    HN_CUDA(cudaMemsetAsync(w.claim, 0x7f, static_cast<size_t>(rows_g) * 8, s));   // "unclaimed"
-    HN_CUDA(cudaMemsetAsync(w.beaten, 0, static_cast<size_t>(rows_g), s));
-    const long long nrb = (Nq + 31) / 32, chunks = (Ng + kChunk - 1) / kChunk;
-    mutual_claim_batched_kernel<<<static_cast<unsigned>((B * nrb * 32 + threads - 1) / threads), threads, 0, s>>>(
-        i1, d1, d2, B, Nq, Ng, q_len, g_len, w.claim, w.rb_min_d2);
-    static DeviceOnce attr_once;
-    if (attr_once.first_time())
-      HN_CUDA(cudaFuncSetAttribute(mutual_verify_batched_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kVerifySmem)));
-    const float vmargin = 2.0f * (1.0f / 1024.0f) / kDotScale;   // as hn_mutual_verify
-    mutual_verify_batched_kernel<<<static_cast<unsigned>((B * chunks + kVerifyWarps - 1) / kVerifyWarps), kVerifyWarps * 32, kVerifySmem, s>>>(
-        q, g, B, Nq, Ng, q_len, g_len, w.claim, w.block_max, w.rb_min_d2, vmargin, 1.0f / kDotScale, w.beaten);
-    mutual_final_batched_kernel<<<static_cast<unsigned>((rows_q + threads - 1) / threads), threads, 0, s>>>(i1, B, Nq, Ng, q_len, g_len,
-                                                                                                        w.claim, w.beaten, mutual);
-    HN_CUDA(cudaGetLastError());
-    count_launch(3);
-  }
-  return HN_OK;
+  const PairLayout L = {nullptr, q_len, g_len, B, Nq, Ng, rows_q, rows_g};
+  return run_pairs<false>(q, w.q16, g, w.g16, L, d1, d2, i1, i2, mutual, w, s);
+}
+
+extern "C" long long hn_match_pairs_workspace_bytes(long long B, long long max_q, long long max_g, int with_mutual) {
+  if (B < 0 || max_q < 0 || max_g < 0) return 0;
+  return static_cast<long long>(carve_batched(nullptr, B, max_q, max_g, with_mutual != 0, false).bytes);
+}
+
+extern "C" int hn_match_pairs(const float* q, const void* q16, long long Nq_rows, const float* g, const void* g16, long long Ng_rows,
+                              const int32_t* pairs, long long B, long long max_q, long long max_g, float* d1, float* d2, int32_t* i1,
+                              int32_t* i2, unsigned char* mutual, void* workspace, long long workspace_bytes, void* stream) {
+  HN_REQUIRE(q && q16 && g && g16 && pairs && d1 && d2 && i1 && i2 && workspace,
+             "hn_match_pairs: NULL argument (q, q16, g, g16, pairs, d1, d2, i1, i2 and workspace are required)");
+  HN_REQUIRE(B >= 1 && max_q >= 1 && max_g >= 1 && Nq_rows >= 1 && Ng_rows >= 1,
+             "hn_match_pairs: empty input (B=%lld, max_q=%lld, max_g=%lld, Nq_rows=%lld, Ng_rows=%lld)", B, max_q, max_g, Nq_rows,
+             Ng_rows);
+  HN_REQUIRE(Nq_rows < (1LL << 31) && Ng_rows < (1LL << 31), "hn_match_pairs: a descriptor set has 2^31 rows or more");
+  HN_REQUIRE(max_q < (1LL << 31) / B && max_g < (1LL << 31) / B, "hn_match_pairs: B*max_q and B*max_g must stay below 2^31 rows");
+  HN_REQUIRE((reinterpret_cast<uintptr_t>(q16) & 15) == 0 && (reinterpret_cast<uintptr_t>(g16) & 15) == 0,
+             "hn_match_pairs: packed operands must be 16-byte aligned");
+  HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "hn_match_pairs: workspace must be 256-byte aligned");
+  HN_REQUIRE(workspace_bytes >= hn_match_pairs_workspace_bytes(B, max_q, max_g, mutual != nullptr), "hn_match_pairs: workspace too small");
+  const BatchedWs w = carve_batched(workspace, B, max_q, max_g, mutual != nullptr, false);
+  const PairLayout L = {pairs, nullptr, nullptr, B, max_q, max_g, Nq_rows, Ng_rows};
+  return run_pairs<true>(q, static_cast<const uint16_t*>(q16), g, static_cast<const uint16_t*>(g16), L, d1, d2, i1, i2, mutual, w,
+                   static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int hn_match_force_kernel(int mode) {

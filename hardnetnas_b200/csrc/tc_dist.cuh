@@ -16,6 +16,13 @@
 //               {K, N, B} whose boxes never cross into the next pair (TMA zero-fills past N); a work item is (pair, query block,
 //               segment), and each pair has its own row / column counts (q_len / g_len). The batch logic is confined to the
 //               item decode, the TMA coordinates, the per-pair bounds and the output offsets, and compiles away elsewhere.
+//   EPI_SHORTLIST_PAIRS : the same over row ranges of concatenated sets (hn_match_pairs): pair b's (start, length) per side comes
+//               from a device table (table_span), operands are 2-D tensor maps over the concatenated rows and the TMA row
+//               coordinate is start + local row. A box may reach past a pair's range into other rows (or past the set, where
+//               TMA zero-fills); the per-pair bounds above keep them out: columns past the length are masked to -inf, rows
+//               past it are neither stored nor part of the cell maxima. A separate instantiation rather than the padded
+//               case of one accessor: reading the padded layout through the table accessor made hn_match_batched 1-2 %
+//               slower (DESIGN.md section 5).
 #pragma once
 
 #include "../../include/hardnet_b200.h"
@@ -28,7 +35,7 @@ constexpr int kDistStages = 4;
 constexpr int kTopC = 4;     // chunks kept per row and segment
 constexpr int kChunk = 8;    // columns per chunk
 
-enum : int { EPI_EXACT = 0, EPI_SHORTLIST = 1, EPI_EXACT_NEI = 2, EPI_SHORTLIST_BATCHED = 3 };   // EXACT_NEI = EXACT + the keypoint-neighbour masks
+enum : int { EPI_EXACT = 0, EPI_SHORTLIST = 1, EPI_EXACT_NEI = 2, EPI_SHORTLIST_BATCHED = 3, EPI_SHORTLIST_PAIRS = 4 };   // EXACT_NEI = EXACT + the keypoint-neighbour masks
 
 struct DistSide {
   CUtensorMap tmA;             // rows of this launch direction, [Na, K] 16-bit
@@ -63,6 +70,10 @@ struct DistParams {
   const int* q_len;            // [batch] valid query rows per pair (NULL = all), clamped to [0, Na]
   const int* g_len;            // [batch] valid gallery rows per pair (NULL = all), clamped to [0, Nb]
   int batch;
+  // EPI_SHORTLIST_PAIRS only: [batch][4] = (q_start, q_len, g_start, g_len) and the rows of the concatenated sets (q_len / g_len
+  // unused; side[0].Na / Nb are the per-pair maxima max_q / max_g)
+  const int* pairs;
+  long long q_rows, g_rows;
 };
 
 template <int MB>
@@ -74,6 +85,16 @@ constexpr size_t dist_smem_bytes(int k_blocks) {
 // Valid rows of pair b of a padded batch: len[b] clamped to [0, n], or n when no lengths are given.
 __device__ __forceinline__ long long pair_len(const int* len, long long b, long long n) {
   return len ? min(max(static_cast<long long>(len[b]), 0ll), n) : n;
+}
+
+// One side (0 = query, 1 = gallery) of pair b of a pair table [B][4] = (q_start, q_len, g_start, g_len): the start clamped to
+// [0, rows], the length to [0, min(max_len, rows - start)].
+struct Span {
+  long long start, len;
+};
+__device__ __forceinline__ Span table_span(const int* pairs, long long b, int side, long long max_len, long long rows) {
+  const long long start = min(max(static_cast<long long>(pairs[4 * b + 2 * side]), 0ll), rows);
+  return {start, min(max(static_cast<long long>(pairs[4 * b + 2 * side + 1]), 0ll), min(max_len, rows - start))};
 }
 
 __device__ __forceinline__ float max3(float a, float b, float c) { return fmaxf(fmaxf(a, b), c); }
@@ -115,7 +136,8 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
   constexpr int CS = dist_col_split<EPI>();
   static_assert(CS == 1 || MB == 1, "the column split is for the single-M-block loss kernels");
   constexpr bool NEI = EPI == EPI_EXACT_NEI;   // compile-time: the plain loss kernel carries none of the mask code
-  constexpr bool BATCHED = EPI == EPI_SHORTLIST_BATCHED;
+  constexpr bool PAIRS = EPI == EPI_SHORTLIST_PAIRS;
+  constexpr bool BATCHED = EPI == EPI_SHORTLIST_BATCHED || PAIRS;
   constexpr bool SHORTLIST = EPI == EPI_SHORTLIST || BATCHED;
   constexpr uint32_t BLK_BYTES = kDistTile * 128;  // 128 rows x 64 fp16
   constexpr uint32_t TMEM_COLS = 2 * MB * kDistTile;
@@ -147,8 +169,12 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
   // An item is (pair, query block, segment); a single problem is pair 0. The valid query rows / gallery columns of a pair come
   // from its lengths: producer, issuer and epilogue read the same ones, so they agree on which items and tiles exist.
   auto pair_of = [&](int item) { return BATCHED ? item / (m_blocks * p.segments) : 0; };
-  auto pair_rows = [&](int pair) { return BATCHED ? pair_len(p.q_len, pair, sd.Na) : sd.Na; };
-  auto pair_cols = [&](int pair) { return BATCHED ? pair_len(p.g_len, pair, sd.Nb) : sd.Nb; };
+  auto pair_rows = [&](int pair) {
+    return PAIRS ? table_span(p.pairs, pair, 0, sd.Na, p.q_rows).len : BATCHED ? pair_len(p.q_len, pair, sd.Na) : sd.Na;
+  };
+  auto pair_cols = [&](int pair) {
+    return PAIRS ? table_span(p.pairs, pair, 1, sd.Nb, p.g_rows).len : BATCHED ? pair_len(p.g_len, pair, sd.Nb) : sd.Nb;
+  };
   auto pair_tiles = [&](int pair) { return BATCHED ? static_cast<int>((pair_cols(pair) + kDistTile - 1) / kDistTile) : n_tiles; };
   auto seg_range = [&](int seg, int tiles, int& t0, int& t1) {
     t0 = static_cast<int>(static_cast<long long>(tiles) * seg / p.segments);
@@ -191,14 +217,25 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
         const int pair = pair_of(item), local = item - pair * (m_blocks * p.segments);
         const int mblk = local / p.segments, seg = local - mblk * p.segments;
         int t0, t1;
-        seg_range(seg, pair_tiles(pair), t0, t1);
-        if (BATCHED && (static_cast<long long>(mblk) * MB * kDistTile >= pair_rows(pair) || t0 == t1)) continue;   // as the issuer
+        int q0 = 0, g0 = 0;   // PAIRS: first row of the pair in each concatenated set; TMA row coordinate = start + local row
+        if constexpr (PAIRS) {   // each span read once (the issuer and epilogue need only the lengths)
+          const Span qsp = table_span(p.pairs, pair, 0, sd.Na, p.q_rows), gsp = table_span(p.pairs, pair, 1, sd.Nb, p.g_rows);
+          seg_range(seg, static_cast<int>((gsp.len + kDistTile - 1) / kDistTile), t0, t1);
+          if (static_cast<long long>(mblk) * MB * kDistTile >= qsp.len || t0 == t1) continue;   // as the issuer
+          q0 = static_cast<int>(qsp.start);
+          g0 = static_cast<int>(gsp.start);
+        } else {
+          seg_range(seg, pair_tiles(pair), t0, t1);
+          if (BATCHED && (static_cast<long long>(mblk) * MB * kDistTile >= pair_rows(pair) || t0 == t1)) continue;   // as the issuer
+        }
         mbar_wait(aempty_bar, a_phase ^ 1u);
         if (elect_one()) {
           mbar_arrive_expect_tx(afull_bar, MB * p.k_blocks * BLK_BYTES);
           for (int mb = 0; mb < MB; ++mb)
             for (int kb = 0; kb < p.k_blocks; ++kb) {
-              if (BATCHED)
+              if (PAIRS)
+                tma_load_2d(a_base + (mb * p.k_blocks + kb) * BLK_BYTES, &sd.tmA, afull_bar, kb * 64, q0 + (mblk * MB + mb) * kDistTile);
+              else if (BATCHED)
                 tma_load_3d(a_base + (mb * p.k_blocks + kb) * BLK_BYTES, &sd.tmA, afull_bar, kb * 64, (mblk * MB + mb) * kDistTile, pair);
               else
                 tma_load_2d(a_base + (mb * p.k_blocks + kb) * BLK_BYTES, &sd.tmA, afull_bar, kb * 64,
@@ -212,7 +249,8 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
             mbar_wait(empty_bar(stage), phase ^ 1u);
             if (elect_one()) {
               mbar_arrive_expect_tx(full_bar(stage), BLK_BYTES);
-              if (BATCHED) tma_load_3d(b_base + stage * BLK_BYTES, &sd.tmB, full_bar(stage), kb * 64, t * kDistTile, pair);
+              if (PAIRS) tma_load_2d(b_base + stage * BLK_BYTES, &sd.tmB, full_bar(stage), kb * 64, g0 + t * kDistTile);
+              else if (BATCHED) tma_load_3d(b_base + stage * BLK_BYTES, &sd.tmB, full_bar(stage), kb * 64, t * kDistTile, pair);
               else tma_load_2d(b_base + stage * BLK_BYTES, &sd.tmB, full_bar(stage), kb * 64, t * kDistTile);
             }
             __syncwarp();

@@ -121,6 +121,64 @@ def mutual_nn_ratio_batched(des1, des2, len1=None, len2=None, threshold=0.7):
     return mutual, (d1 / d2).lt(threshold), i1.long(), d1, d2
 
 
+# ---- pair tables over concatenated descriptor sets -----------------------------------------------------------------------
+# Extraction over a set of images yields one [sum N_i, 128] tensor, and the pairs of an evaluation reuse images (a reference
+# image against the others of its sequence, or every pair of a collection). The pair forms take those sets as they are: a
+# [P, 4] table of (start1, len1, start2, len2) row ranges says which rows of des1 are matched against which rows of des2
+# (hn_match_pairs). Each set is packed once per call, or not at all when its packed rows (pack_descriptors) are passed as
+# des1_16 / des2_16. Outputs are padded per pair to [P, max_len1]; per pair and valid row they equal the per-pair functions on
+# des1[start1:start1 + len1], des2[start2:start2 + len2], with indices local to the gallery range. Rows past len1, and all
+# rows of a pair without gallery rows, get Da = Db = +inf, Ia = Ib = -1 and are never matched. A start is clamped to
+# [0, rows], a length to [0, min(max_len, rows - start)]. max_len1 / max_len2 = None read the largest clamped lengths from the
+# table: one host synchronisation. Passing them (and a table on the device) keeps the call free of host synchronisation and
+# CUDA-graph capturable.
+
+def pair_table(counts1, idx1, idx2, counts2=None):
+    """[P, 4] int32 table for the pair forms, on the device of counts1: pair p matches image idx1[p] of the first set against
+    image idx2[p] of the second. counts1 / counts2: keypoints per image of each set (the sets are the images' descriptors
+    concatenated in image order); counts2 = None means both sides index the same set. Starts are the exclusive cumulative
+    sums of the counts."""
+    c1 = torch.as_tensor(counts1)
+    c2 = c1 if counts2 is None else torch.as_tensor(counts2, device=c1.device)
+    if c1.dim() != 1 or c2.dim() != 1 or c1.dtype.is_floating_point or c2.dtype.is_floating_point:
+        raise ValueError("pair_table: counts must be 1-D integer tensors")
+    i1 = torch.as_tensor(idx1, device=c1.device).long()
+    i2 = torch.as_tensor(idx2, device=c1.device).long()
+    if i1.shape != i2.shape or i1.dim() != 1:
+        raise ValueError("pair_table: idx1 and idx2 must be 1-D of the same length")
+    c1, c2 = c1.long(), c2.long()
+    s1, s2 = torch.cumsum(c1, 0) - c1, torch.cumsum(c2, 0) - c2
+    return torch.stack([s1[i1], c1[i1], s2[i2], c2[i2]], dim=1).to(torch.int32)
+
+
+def _max_lens(pairs, n1, n2, max_len1, max_len2):
+    """The per-pair maxima not given, from the table's clamped lengths (one host synchronisation)."""
+    if max_len1 is not None and max_len2 is not None:
+        return max_len1, max_len2
+    t = pairs.long()
+    m = []
+    for k, n in ((0, n1), (2, n2)):
+        start = t[:, k].clamp(0, n)
+        m.append(torch.minimum(t[:, k + 1], n - start).clamp(min=0).max() if t.size(0) else t.new_zeros(()))
+    m1, m2 = torch.stack(m).tolist()
+    return (max(m1, 1) if max_len1 is None else max_len1), (max(m2, 1) if max_len2 is None else max_len2)
+
+
+def match_top2_pairs(des1, des2, pairs, max_len1=None, max_len2=None, des1_16=None, des2_16=None):
+    """match_top2 for every row-range pair of the table -> (Da, Db, Ia, Ib), each [P, max_len1]; indices int64, local to the
+    pair's gallery range."""
+    max_len1, max_len2 = _max_lens(pairs, des1.size(0), des2.size(0), max_len1, max_len2)
+    d1, d2, i1, i2 = _ops.match_pairs(des1, des2, pairs, max_len1, max_len2, des1_16, des2_16)
+    return d1, d2, i1.long(), i2.long()
+
+
+def mutual_nn_ratio_pairs(des1, des2, pairs, max_len1=None, max_len2=None, threshold=0.7, des1_16=None, des2_16=None):
+    """mutual_nn_ratio for every row-range pair of the table -> (mutual, ratio_label, Ia, Da, Db), all [P, max_len1]."""
+    max_len1, max_len2 = _max_lens(pairs, des1.size(0), des2.size(0), max_len1, max_len2)
+    d1, d2, i1, _, mutual = _ops.match_pairs(des1, des2, pairs, max_len1, max_len2, des1_16, des2_16, mutual=True)
+    return mutual, (d1 / d2).lt(threshold), i1.long(), d1, d2
+
+
 # ---- match-score counters (FDLNet-master/utils/eval_utils.py:112-197) -----------------------------------------------
 # The callers right behind the hot path in the reference's evaluation: nearest neighbour (or ratio test) on the fused
 # kernel, then "is the matched keypoint within COO_THRSH pixels of the warped keypoint" and two counters. The reference
@@ -196,3 +254,42 @@ def nearest_neighbor_distance_ratio_match_score_batched(des1, des2, kp1w, kp2, v
     da, db, ia, _ = match_top2_batched(des1, des2, len1, len2)
     predict = (da / db).lt(threshold) & visible.bool() & (ia >= 0)
     return _counts(predict, kp1w, _batched_nn_kp2(kp2, ia), visible, COO_THRSH, predict)
+
+
+# Pair-table counters: kp1w [P, max_len1, >=3] (each pair's query keypoints warped by its homography) and visible [P, max_len1]
+# are padded per pair, and max_len1 is their second dimension; kp2 [Ng_rows, >=3] holds the keypoints of the concatenated
+# gallery set, read at row g_start + Ia. Each returns (correct [P], predicted [P]) int64 device tensors; a row without a match
+# is neither predicted nor correct.
+
+def _pairs_nn_kp2(kp2, pairs, ia):
+    """kp2[g_start + Ia] for every pair and row; rows without a match (Ia = -1) read a valid row and are masked by the caller."""
+    n = kp2.size(0)
+    start = pairs.to(device=ia.device, dtype=torch.long)[:, 2].clamp(0, n)
+    rows = (start.unsqueeze(1) + ia.clamp(min=0)).clamp(max=max(n - 1, 0))
+    return kp2[rows]
+
+
+def nearest_neighbor_match_score_pairs(des1, des2, pairs, kp1w, kp2, visible, COO_THRSH, max_len2=None, des1_16=None,
+                                       des2_16=None):
+    """nearest_neighbor_match_score per table pair -> (correct [P], predicted = max(#visible, 1) [P])."""
+    _, _, ia, _ = match_top2_pairs(des1, des2, pairs, kp1w.size(1), max_len2, des1_16, des2_16)
+    vis = visible.bool() & (ia >= 0)
+    return _counts(vis, kp1w, _pairs_nn_kp2(kp2, pairs, ia), vis, COO_THRSH, vis)
+
+
+def nearest_neighbor_threshold_match_score_pairs(des1, des2, pairs, kp1w, kp2, visible, DES_THRSH, COO_THRSH, max_len2=None,
+                                                 des1_16=None, des2_16=None):
+    """nearest_neighbor_threshold_match_score per table pair -> (correct [P], predicted = max(#(Da < DES_THRSH and visible), 1)
+    [P])."""
+    da, _, ia, _ = match_top2_pairs(des1, des2, pairs, kp1w.size(1), max_len2, des1_16, des2_16)
+    predict = da.lt(DES_THRSH) & visible.bool() & (ia >= 0)
+    return _counts(predict, kp1w, _pairs_nn_kp2(kp2, pairs, ia), visible, COO_THRSH, predict)
+
+
+def nearest_neighbor_distance_ratio_match_score_pairs(des1, des2, pairs, kp1w, kp2, visible, COO_THRSH, threshold=0.7,
+                                                      max_len2=None, des1_16=None, des2_16=None):
+    """nearest_neighbor_distance_ratio_match_score per table pair -> (correct [P], predicted = max(#(Da / Db < threshold and
+    visible), 1) [P])."""
+    da, db, ia, _ = match_top2_pairs(des1, des2, pairs, kp1w.size(1), max_len2, des1_16, des2_16)
+    predict = (da / db).lt(threshold) & visible.bool() & (ia >= 0)
+    return _counts(predict, kp1w, _pairs_nn_kp2(kp2, pairs, ia), visible, COO_THRSH, predict)

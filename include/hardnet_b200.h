@@ -226,12 +226,30 @@ int hn_match_batched(const float* q, const float* g, long long B, long long Nq, 
                      const int32_t* g_len, float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual,
                      void* workspace, long long workspace_bytes, void* stream);
 
+/* Pair-table matching: B problems over row ranges of two concatenated descriptor sets, in the launch sequence of
+ * hn_match_batched. q:[Nq_rows,128], g:[Ng_rows,128] fp32 unit rows (the
+ * descriptors of several images, concatenated); q16 / g16 their packed rows from hn_pack_descriptors (required, 16-byte
+ * aligned; q may be g and q16 may be g16). pairs: DEVICE int32 [B][4] = (q_start, q_len, g_start, g_len): pair b matches rows
+ * [q_start, q_start + q_len) of q against rows [g_start, g_start + g_len) of g. Clamped on the device: start to [0, N_rows];
+ * len to [0, min(max_q or max_g, N_rows - start)]. The host never reads the table, so the call is CUDA-graph capturable and
+ * a captured graph follows edits of the table.
+ * Outputs are padded per pair like hn_match_batched: d1/d2/i1/i2[/mutual] [B*max_q], row r of pair b at b*max_q + r; for a
+ * valid row they equal hn_match / hn_match_mutual on the two slices bit for bit (indices local to the pair's gallery range);
+ * rows past q_len, and every row of a pair with g_len == 0, get +inf / -1 / 0. Rows outside a pair's ranges never influence
+ * it. Requires Nq_rows, Ng_rows, B*max_q and B*max_g below 2^31 and a 256-byte-aligned workspace of
+ * hn_match_pairs_workspace_bytes(B, max_q, max_g, mutual != NULL) bytes (it does not depend on the set sizes). */
+long long hn_match_pairs_workspace_bytes(long long B, long long max_q, long long max_g, int with_mutual);
+int hn_match_pairs(const float* q, const void* q16, long long Nq_rows, const float* g, const void* g16, long long Ng_rows,
+                   const int32_t* pairs, long long B, long long max_q, long long max_g,
+                   float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual,
+                   void* workspace, long long workspace_bytes, void* stream);
+
 /* Test / measurement switch (process-wide): which matching GEMM hn_match runs: -1 = chosen by problem size (default; the
  * initial value is read once from HN_MATCH_PAIR), 0 = single-CTA kernel, 1 = CTA-pair (cta_group::2) kernel. */
 int hn_match_force_kernel(int mode);
 
-/* Measurement hooks (process-wide): bracket the three stages of every hn_match / hn_match_batched call (0 = operand packing, 1 = GEMM +
- * shortlist, 2 = exact re-rank) with CUDA events; hn_match_profile_read waits for them, returns the summed milliseconds and
+/* Measurement hooks (process-wide): bracket the three stages of every hn_match / hn_match_batched / hn_match_pairs call
+ * (0 = operand packing, not part of hn_match_pairs; 1 = GEMM + shortlist, 2 = exact re-rank) with CUDA events; hn_match_profile_read waits for them, returns the summed milliseconds and
  * launch counts per stage and resets the counters. */
 int hn_match_profile_enable(int on);
 int hn_match_profile_read(double ms_out[3], long long launches_out[3]);
