@@ -55,6 +55,15 @@ SIGNATURES = {
     "hn_match_pairs": (C.c_int, [_P, _P, C.c_longlong, _P, _P, C.c_longlong, _P, C.c_longlong, C.c_longlong, C.c_longlong, _P, _P, _P,
                                  _P, _P, _P, C.c_longlong, _P]),
     "hn_match_force_kernel": (C.c_int, [C.c_int]),
+    "hn_pack_descriptors_typed": (C.c_int, [_P, C.c_int, C.c_longlong, _P, _P]),
+    "hn_match_typed": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_longlong, C.c_longlong, C.c_longlong, _P, _P, _P, _P, _P, _P,
+                                 C.c_longlong, _P, _P]),
+    "hn_match_mutual_typed": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_longlong, C.c_longlong, _P, _P, _P, _P, _P, _P, C.c_longlong,
+                                        _P]),
+    "hn_match_batched_typed": (C.c_int, [_P, _P, C.c_int, C.c_longlong, C.c_longlong, C.c_longlong, _P, _P, _P, _P, _P, _P, _P, _P,
+                                         C.c_longlong, _P]),
+    "hn_match_pairs_typed": (C.c_int, [_P, _P, C.c_longlong, _P, _P, C.c_longlong, C.c_int, _P, C.c_longlong, C.c_longlong,
+                                       C.c_longlong, _P, _P, _P, _P, _P, _P, C.c_longlong, _P]),
     "hn_match_profile_enable": (C.c_int, [C.c_int]),
     "hn_match_profile_read": (C.c_int, [C.POINTER(C.c_double), C.POINTER(C.c_longlong)]),
     "hn_pair_distances": (C.c_int, [_P, _P, C.c_longlong, _P, _P]),

@@ -25,13 +25,30 @@ def _workspace(device: torch.device, nbytes: int) -> torch.Tensor:
     return ws
 
 
-def _require_cuda_f32(name: str, t: torch.Tensor) -> torch.Tensor:
+def _require_cuda_desc(name: str, t: torch.Tensor) -> torch.Tensor:
     if not isinstance(t, torch.Tensor) or not t.is_cuda:
         raise _lib.HardnetB200Error(f"{name}: the fused path runs on B200 CUDA tensors only (no CPU fallback)")
     assert t.dim() == 2, "Inputd must be a 2D matrix."
     if t.size(1) != 128:
         raise ValueError(f"{name}: descriptors must be 128-d, got {t.size(1)}")
-    return t.detach().float().contiguous()
+    return t.detach()
+
+
+def _require_cuda_f32(name: str, t: torch.Tensor) -> torch.Tensor:
+    return _require_cuda_desc(name, t).float().contiguous()
+
+
+_ROW_DTYPES = {torch.float16: _lib.HN_F16, torch.bfloat16: _lib.HN_BF16}
+
+
+def _desc_rows(q: torch.Tensor, g: torch.Tensor | None = None):
+    """(q, g, desc_dtype) for the *_typed matching entry points: fp16 and bf16 rows are read as they are (made contiguous)
+    when both sides share the dtype, so no fp32 copy is made; anything else (fp32, fp64, mixed dtypes) is converted to fp32.
+    The results are the same either way (include/hardnet_b200.h). g = None: a single set."""
+    code = _ROW_DTYPES.get(q.dtype) if g is None or g.dtype == q.dtype else None
+    if code is None:
+        return q.float().contiguous(), (None if g is None else g.float().contiguous()), _lib.HN_F32
+    return q.contiguous(), (None if g is None else g.contiguous()), code
 
 
 def _stream_ptr() -> C.c_void_p:
@@ -88,17 +105,17 @@ def loss_hardnet(anchor: torch.Tensor, positive: torch.Tensor, margin: float, an
 
 
 def pack_descriptors(x: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
-    """[n,128] fp32 unit rows -> the fp16 operand rows of the matching GEMM (x * 2^8), see hn_pack_descriptors.
-    `out`: optional destination (e.g. a symmetric-memory exchange buffer)."""
+    """[n,128] unit rows (fp32, or fp16 / bf16 read as they are) -> the fp16 operand rows of the matching GEMM (x * 2^8), see
+    hn_pack_descriptors. `out`: optional destination (e.g. a symmetric-memory exchange buffer)."""
     lib = _lib.load()
-    x = _require_cuda_f32("pack_descriptors", x)
+    x, _, dt = _desc_rows(_require_cuda_desc("pack_descriptors", x))
     if out is None:
         out = torch.empty((x.size(0), 128), dtype=torch.float16, device=x.device)
     elif not (out.is_cuda and out.dtype == torch.float16 and tuple(out.shape) == (x.size(0), 128) and out.is_contiguous()):
         raise ValueError("pack_descriptors: out must be a contiguous CUDA fp16 [n,128] tensor")
     if x.size(0):
         with torch.cuda.device(x.device):
-            _lib.check(lib.hn_pack_descriptors(_ptr(x), x.size(0), _ptr(out), _stream_ptr()), "hn_pack_descriptors")
+            _lib.check(lib.hn_pack_descriptors_typed(_ptr(x), dt, x.size(0), _ptr(out), _stream_ptr()), "hn_pack_descriptors_typed")
     return out
 
 
@@ -118,10 +135,9 @@ def match_top2(q: torch.Tensor, g: torch.Tensor, g_offset: int = 0, q16: torch.T
     q16 / g16: operands already packed by `pack_descriptors` (skips the packing kernels); g_ready_event: the exact re-rank
     (the only reader of the fp32 gallery `g`) waits for it, so `g` may still be arriving while the GEMM runs.
     block_max: optional fp32 tensor of `block_max_elems(nq, ng)` elements that receives the GEMM's per-cell maxima (column side
-    of mutual NN, see hn_match_mutual)."""
+    of mutual NN, see hn_match_mutual). fp16 / bf16 rows of one dtype are read as they are (hn_match_typed)."""
     lib = _lib.load()
-    q = _require_cuda_f32("match", q)
-    g = _require_cuda_f32("match", g)
+    q, g, dt = _desc_rows(_require_cuda_desc("match", q), _require_cuda_desc("match", g))
     nq, ng = q.size(0), g.size(0)
     for t, n in ((q16, nq), (g16, ng)):
         if t is not None and not (t.is_cuda and t.dtype == torch.float16 and tuple(t.shape) == (n, 128) and t.is_contiguous()):
@@ -134,8 +150,8 @@ def match_top2(q: torch.Tensor, g: torch.Tensor, g_offset: int = 0, q16: torch.T
         i1 = torch.empty(nq, dtype=torch.int32, device=dev)
         i2 = torch.empty(nq, dtype=torch.int32, device=dev)
         ev = C.c_void_p(g_ready_event.cuda_event) if g_ready_event is not None else C.c_void_p(0)
-        _lib.check(lib.hn_match_ex(_ptr(q), _ptr(g), _ptr(q16), _ptr(g16), nq, ng, g_offset, _ptr(d1), _ptr(d2), _ptr(i1),
-                                   _ptr(i2), _ptr(block_max), _ptr(ws), ws.numel(), ev, _stream_ptr()), "hn_match")
+        _lib.check(lib.hn_match_typed(_ptr(q), _ptr(g), dt, _ptr(q16), _ptr(g16), nq, ng, g_offset, _ptr(d1), _ptr(d2), _ptr(i1),
+                                      _ptr(i2), _ptr(block_max), _ptr(ws), ws.numel(), ev, _stream_ptr()), "hn_match_typed")
     return d1, d2, i1, i2
 
 
@@ -144,10 +160,9 @@ def block_max_elems(nq: int, ng: int) -> int:
 
 
 def match_mutual(q: torch.Tensor, g: torch.Tensor, q16: torch.Tensor | None = None, g16: torch.Tensor | None = None):
-    """(d1, d2, i1, i2, mutual bool[Nq]) from ONE matching GEMM: hn_match_mutual."""
+    """(d1, d2, i1, i2, mutual bool[Nq]) from ONE matching GEMM: hn_match_mutual_typed (rows as in match_top2)."""
     lib = _lib.load()
-    q = _require_cuda_f32("match_mutual", q)
-    g = _require_cuda_f32("match_mutual", g)
+    q, g, dt = _desc_rows(_require_cuda_desc("match_mutual", q), _require_cuda_desc("match_mutual", g))
     nq, ng = q.size(0), g.size(0)
     dev = q.device
     with torch.cuda.device(dev):
@@ -157,19 +172,19 @@ def match_mutual(q: torch.Tensor, g: torch.Tensor, q16: torch.Tensor | None = No
         i1 = torch.empty(nq, dtype=torch.int32, device=dev)
         i2 = torch.empty(nq, dtype=torch.int32, device=dev)
         mutual = torch.empty(nq, dtype=torch.bool, device=dev)
-        _lib.check(lib.hn_match_mutual(_ptr(q), _ptr(g), _ptr(q16), _ptr(g16), nq, ng, _ptr(d1), _ptr(d2), _ptr(i1), _ptr(i2),
-                                       _ptr(mutual), _ptr(ws), ws.numel(), _stream_ptr()), "hn_match_mutual")
+        _lib.check(lib.hn_match_mutual_typed(_ptr(q), _ptr(g), dt, _ptr(q16), _ptr(g16), nq, ng, _ptr(d1), _ptr(d2), _ptr(i1),
+                                             _ptr(i2), _ptr(mutual), _ptr(ws), ws.numel(), _stream_ptr()), "hn_match_mutual_typed")
     return d1, d2, i1, i2, mutual
 
 
-def _require_cuda_f32_batched(name: str, t: torch.Tensor) -> torch.Tensor:
+def _require_cuda_desc_batched(name: str, t: torch.Tensor) -> torch.Tensor:
     if not isinstance(t, torch.Tensor) or not t.is_cuda:
         raise _lib.HardnetB200Error(f"{name}: the fused path runs on B200 CUDA tensors only (no CPU fallback)")
     if t.dim() != 3:
         raise ValueError(f"{name}: descriptors must be a padded batch [B, N, 128], got shape {tuple(t.shape)}")
     if t.size(2) != 128:
         raise ValueError(f"{name}: descriptors must be 128-d, got {t.size(2)}")
-    return t.detach().float().contiguous()
+    return t.detach()
 
 
 def _lengths(name: str, t, batch: int, device: torch.device):
@@ -187,10 +202,9 @@ def match_batched(q: torch.Tensor, g: torch.Tensor, q_len: torch.Tensor | None =
     """(d1, d2, i1, i2[, mutual]), each [B, Nq]: hn_match_batched over the padded batches q [B, Nq, 128] and g [B, Ng, 128].
     q_len / g_len: integer [B] tensors of valid rows per pair (None = all). Lengths on q's device keep the call free of host
     synchronisation (and CUDA-graph capturable); a CPU lengths tensor is copied to the device first. Indices are local to the
-    pair; rows past q_len get d = +inf, i = -1 (and mutual = False)."""
+    pair; rows past q_len get d = +inf, i = -1 (and mutual = False). Rows as in match_top2 (hn_match_batched_typed)."""
     lib = _lib.load()
-    q = _require_cuda_f32_batched("match_batched", q)
-    g = _require_cuda_f32_batched("match_batched", g)
+    q, g, dt = _desc_rows(_require_cuda_desc_batched("match_batched", q), _require_cuda_desc_batched("match_batched", g))
     if q.size(0) != g.size(0):
         raise ValueError(f"match_batched: q and g hold {q.size(0)} and {g.size(0)} pairs")
     b, nq, ng = q.size(0), q.size(1), g.size(1)
@@ -204,8 +218,8 @@ def match_batched(q: torch.Tensor, g: torch.Tensor, q_len: torch.Tensor | None =
         i1 = torch.empty((b, nq), dtype=torch.int32, device=dev)
         i2 = torch.empty((b, nq), dtype=torch.int32, device=dev)
         mu = torch.empty((b, nq), dtype=torch.bool, device=dev) if mutual else None
-        _lib.check(lib.hn_match_batched(_ptr(q), _ptr(g), b, nq, ng, _ptr(ql), _ptr(gl), _ptr(d1), _ptr(d2), _ptr(i1), _ptr(i2),
-                                        _ptr(mu), _ptr(ws), ws.numel(), _stream_ptr()), "hn_match_batched")
+        _lib.check(lib.hn_match_batched_typed(_ptr(q), _ptr(g), dt, b, nq, ng, _ptr(ql), _ptr(gl), _ptr(d1), _ptr(d2), _ptr(i1),
+                                              _ptr(i2), _ptr(mu), _ptr(ws), ws.numel(), _stream_ptr()), "hn_match_batched_typed")
     return (d1, d2, i1, i2, mu) if mutual else (d1, d2, i1, i2)
 
 
@@ -222,11 +236,14 @@ def match_pairs(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, max_q: in
     g [Ng_rows, 128]. pairs: integer [P, 4] table of (q_start, q_len, g_start, g_len), copied to q's device as int32 (a table
     already there keeps the call free of host synchronisation). q16 / g16: the sets' rows packed by `pack_descriptors`; a set
     whose packed rows are not given is packed here, once when g is q. Indices are local to the pair's gallery range; rows past
-    q_len get d = +inf, i = -1 (and mutual = False)."""
+    q_len get d = +inf, i = -1 (and mutual = False). Rows as in match_top2 (hn_match_pairs_typed)."""
     lib = _lib.load()
     same = g is q
-    q = _require_cuda_f32("match_pairs", q)
-    g = q if same else _require_cuda_f32("match_pairs", g)
+    if same:
+        q, _, dt = _desc_rows(_require_cuda_desc("match_pairs", q))
+        g = q
+    else:
+        q, g, dt = _desc_rows(_require_cuda_desc("match_pairs", q), _require_cuda_desc("match_pairs", g))
     if not isinstance(pairs, torch.Tensor) or pairs.dtype not in (torch.int32, torch.int64) or pairs.dim() != 2 or pairs.size(1) != 4:
         raise ValueError("match_pairs: pairs must be an int32 or int64 [P, 4] tensor of (q_start, q_len, g_start, g_len)")
     dev = q.device
@@ -246,8 +263,9 @@ def match_pairs(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, max_q: in
         i1 = torch.empty((b, max_q), dtype=torch.int32, device=dev)
         i2 = torch.empty((b, max_q), dtype=torch.int32, device=dev)
         mu = torch.empty((b, max_q), dtype=torch.bool, device=dev) if mutual else None
-        _lib.check(lib.hn_match_pairs(_ptr(q), _ptr(q16), nq, _ptr(g), _ptr(g16), ng, _ptr(table), b, max_q, max_g, _ptr(d1),
-                                      _ptr(d2), _ptr(i1), _ptr(i2), _ptr(mu), _ptr(ws), ws.numel(), _stream_ptr()), "hn_match_pairs")
+        _lib.check(lib.hn_match_pairs_typed(_ptr(q), _ptr(q16), nq, _ptr(g), _ptr(g16), ng, dt, _ptr(table), b, max_q, max_g,
+                                            _ptr(d1), _ptr(d2), _ptr(i1), _ptr(i2), _ptr(mu), _ptr(ws), ws.numel(), _stream_ptr()),
+                   "hn_match_pairs_typed")
     return (d1, d2, i1, i2, mu) if mutual else (d1, d2, i1, i2)
 
 

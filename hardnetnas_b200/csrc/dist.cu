@@ -14,15 +14,36 @@ constexpr float kDotScale = 1.0f / (kOperandScale * kOperandScale);
 
 static inline size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
 
-// fp32 [n,128] -> 16-bit K-major operand rows. split == 0: [hi] (K=128). split == 1: K=384,
+// Descriptor rows of the matching kernels are fp32, fp16 or bf16 (T = float, __half, __nv_bfloat16). A lane reads elements
+// 4 * lane ... 4 * lane + 3 of a row as fp32: one 16-byte load for fp32 rows, one 8-byte load for 16-bit rows, converted on the
+// spot. Every fp16 / bf16 value is an fp32 value, so a kernel on 16-bit rows computes exactly what it computes on x.float().
+__device__ __forceinline__ float4 row4_from_bits(uint2 v, __half) {
+  const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&v.x)), b = __half22float2(*reinterpret_cast<const __half2*>(&v.y));
+  return make_float4(a.x, a.y, b.x, b.y);
+}
+__device__ __forceinline__ float4 row4_from_bits(uint2 v, __nv_bfloat16) {
+  const float2 a = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v.x));
+  const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v.y));
+  return make_float4(a.x, a.y, b.x, b.y);
+}
+__device__ __forceinline__ float4 ld_row4(const float* row, int lane) { return reinterpret_cast<const float4*>(row)[lane]; }
+__device__ __forceinline__ float4 ldg_row4(const float* row, int lane) { return __ldg(reinterpret_cast<const float4*>(row) + lane); }
+template <typename T>
+__device__ __forceinline__ float4 ld_row4(const T* row, int lane) { return row4_from_bits(reinterpret_cast<const uint2*>(row)[lane], T{}); }
+template <typename T>
+__device__ __forceinline__ float4 ldg_row4(const T* row, int lane) { return row4_from_bits(__ldg(reinterpret_cast<const uint2*>(row) + lane), T{}); }
+
+// [n,128] rows -> 16-bit K-major operand rows. split == 0: [hi] (K=128). split == 1 (fp32 rows only): K=384,
 // order 0 = [hi, hi, lo] (row side), order 1 = [hi, lo, hi] (column side), so that the GEMM accumulates
-// hi*hi + hi*lo + lo*hi. Also emits |x|^2 (torch.sum(x*x, dim=1), hardnet/Losses.py:8-9).
-__global__ void pack_desc_kernel(const float* __restrict__ x, long long n, uint16_t* __restrict__ out, int split, int order,
+// hi*hi + hi*lo + lo*hi. Also emits |x|^2 (torch.sum(x*x, dim=1), hardnet/Losses.py:8-9). 16-bit rows are widened to fp32
+// first, so their operand rows equal those of x.float() bit for bit.
+template <typename T>
+__global__ void pack_desc_kernel(const T* __restrict__ x, long long n, uint16_t* __restrict__ out, int split, int order,
                                  float* __restrict__ norm) {
   const long long row = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (row >= n) return;
-  const float4 v = reinterpret_cast<const float4*>(x + row * 128)[lane];
+  const float4 v = ld_row4(x + row * 128, lane);
   const float f[4] = {v.x, v.y, v.z, v.w};
   float ss = (f[0] * f[0] + f[1] * f[1]) + (f[2] * f[2] + f[3] * f[3]);
 #pragma unroll
@@ -124,7 +145,10 @@ __global__ void loss_finalize_kernel(const float* __restrict__ pos, const unsign
 // (|d - d2| within the 2^-9 margin). Scanning the whole segment whenever a list's fourth chunk passes the threshold was
 // measured: it fires on ~5 % of the rows of the BASELINE config-4 set and makes the call 5x slower (0.88 -> 4.2 ms), so the
 // exact remedy has to track the largest DROPPED chunk maximum in the GEMM epilogue instead (not done).
-__global__ void __launch_bounds__(128) rerank_kernel(const float* __restrict__ q, const float* __restrict__ g,
+// T: fp32, fp16 or bf16 rows (ld_row4 / ldg_row4); the fp32 instantiation compiles to the instructions of the kernel before it
+// was a template (checked with cuobjdump), and the 16-bit ones differ only in their loads.
+template <typename T>
+__global__ void __launch_bounds__(128) rerank_kernel(const T* __restrict__ q, const T* __restrict__ g,
                                                      const int* __restrict__ cand, const float* __restrict__ cand_val,
                                                      float margin, long long nq, long long ng, int slots,
                                                      long long g_offset, float* __restrict__ d1, float* __restrict__ d2,
@@ -133,7 +157,7 @@ __global__ void __launch_bounds__(128) rerank_kernel(const float* __restrict__ q
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const long long row = static_cast<long long>(blockIdx.x) * 4 + w;
   if (row >= nq) return;
-  reinterpret_cast<float4*>(sq[w])[lane] = reinterpret_cast<const float4*>(q + row * 128)[lane];
+  reinterpret_cast<float4*>(sq[w])[lane] = ld_row4(q + row * 128, lane);
   __syncwarp();
   // A chunk can hold one of the two nearest columns only if its approximate maximum reaches the second largest
   // chunk maximum minus twice the error bound of the 16-bit-operand dot product (`margin`, same scaled units).
@@ -168,7 +192,7 @@ __global__ void __launch_bounds__(128) rerank_kernel(const float* __restrict__ q
       const long long col = col0 + r;
       part[r] = 0.f;
       if (col < ng) {
-        const float4 gv = __ldg(reinterpret_cast<const float4*>(g + col * 128) + lane);
+        const float4 gv = ldg_row4(g + col * 128, lane);
         part[r] = fmaf(qv.x, gv.x, fmaf(qv.y, gv.y, fmaf(qv.z, gv.z, qv.w * gv.w)));
       }
     }
@@ -216,8 +240,8 @@ __global__ void __launch_bounds__(128) rerank_kernel(const float* __restrict__ q
 // them bit for bit). One difference: the eight distances of a chunk are taken by eight lanes, one sqrtf each, and shuffled to
 // the warp (the same values: every lane holds the same eight dot products). Eight unrolled sqrtf slow-path calls per lane kept
 // the pair's gallery pointer and size live across calls and made ptxas spill.
-template <bool TABLE>
-__global__ void __launch_bounds__(128) rerank_batched_kernel(const float* __restrict__ q, const float* __restrict__ g_all,
+template <bool TABLE, typename T>
+__global__ void __launch_bounds__(128) rerank_batched_kernel(const T* __restrict__ q, const T* __restrict__ g_all,
                                                              const int* __restrict__ cand, const float* __restrict__ cand_val,
                                                              float margin, long long B, long long nq_pad, long long ng_pad,
                                                              const int* __restrict__ q_len, const int* __restrict__ g_len, int slots,
@@ -241,11 +265,11 @@ __global__ void __launch_bounds__(128) rerank_batched_kernel(const float* __rest
     }
     return;
   }
-  const float* g = TABLE ? g_all + gs.start * 128 : g_all + static_cast<long long>(b) * ng_pad * 128;
+  const T* g = TABLE ? g_all + gs.start * 128 : g_all + static_cast<long long>(b) * ng_pad * 128;
   const long long ng = TABLE ? gs.len : pair_len(g_len, b, ng_pad);
   const int* crow = cand + row * slots;
   const float* cvrow = cand_val + row * slots;
-  reinterpret_cast<float4*>(sq[w])[lane] = reinterpret_cast<const float4*>(q + (TABLE ? qs.start + (row - b * nq_pad) : row) * 128)[lane];
+  reinterpret_cast<float4*>(sq[w])[lane] = ld_row4(q + (TABLE ? qs.start + (row - b * nq_pad) : row) * 128, lane);
   __syncwarp();
   // A chunk can hold one of the two nearest columns only if its approximate maximum reaches the second largest
   // chunk maximum minus twice the error bound of the 16-bit-operand dot product (`margin`, same scaled units).
@@ -280,7 +304,7 @@ __global__ void __launch_bounds__(128) rerank_batched_kernel(const float* __rest
       const long long col = col0 + r;
       part[r] = 0.f;
       if (col < ng) {
-        const float4 gv = __ldg(reinterpret_cast<const float4*>(g + col * 128) + lane);
+        const float4 gv = ldg_row4(g + col * 128, lane);
         part[r] = fmaf(qv.x, gv.x, fmaf(qv.y, gv.y, fmaf(qv.z, gv.z, qv.w * gv.w)));
       }
     }
@@ -388,8 +412,9 @@ constexpr int kVerifyWarps = 1;   // one warp per CTA: a chunk with a weakly cla
 constexpr int kVerifyPitch = 132;   // floats per staged query row
 constexpr size_t kVerifySmem = static_cast<size_t>(kVerifyWarps) * (32 * kVerifyPitch * 4 + kChunk * 32 * 16);
 
-__global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_kernel(const float* __restrict__ q, long long nq, long long q_offset,
-                                                                         const float* __restrict__ g, long long ng,
+template <typename T>
+__global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_kernel(const T* __restrict__ q, long long nq, long long q_offset,
+                                                                         const T* __restrict__ g, long long ng,
                                                                          const unsigned long long* __restrict__ claim,
                                                                          const float* __restrict__ block_max,
                                                                          const float* __restrict__ rb_min_d2, int n_row_blocks,
@@ -416,7 +441,7 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_kernel(const 
     if ((cc >> 32) < 0x7F000000ull) {
       undecided |= 1u << c;
       thr[c] = (1.0f - 0.5f * dcl[c] * dcl[c]) * inv_dot_scale - margin_scaled;
-      s_g[c * 32 + lane] = __ldg(reinterpret_cast<const float4*>(g + (cb * kChunk + c) * 128) + lane);
+      s_g[c * 32 + lane] = ldg_row4(g + (cb * kChunk + c) * 128, lane);
     }
   }
   if (!undecided) return;
@@ -455,7 +480,7 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_kernel(const 
 #pragma unroll
       for (int r = 0; r < 8; ++r) {
         v[r] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (k0 + r0 + r < nq) v[r] = __ldg(reinterpret_cast<const float4*>(q + (k0 + r0 + r) * 128) + lane);
+        if (k0 + r0 + r < nq) v[r] = ldg_row4(q + (k0 + r0 + r) * 128, lane);
       }
 #pragma unroll
       for (int r = 0; r < 8; ++r) *reinterpret_cast<float4*>(s_q + (r0 + r) * kVerifyPitch + 4 * lane) = v[r];
@@ -536,8 +561,8 @@ __global__ void mutual_claim_batched_kernel(const int* __restrict__ i1, const fl
 // One warp per (pair, 8-column chunk), scanning only the pair's valid row blocks. After the prologue (pair pointers and
 // bounds) this is mutual_verify_kernel's body with q_offset = 0 and a block_max row pitch of ceil(nq_pad / 32), copied rather
 // than shared so that the single-problem kernel compiles to the same instructions as before: keep the two in step.
-template <bool TABLE>
-__global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kernel(const float* __restrict__ q_all, const float* __restrict__ g_all,
+template <bool TABLE, typename T>
+__global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kernel(const T* __restrict__ q_all, const T* __restrict__ g_all,
                                                                                  long long B, long long nq_pad, long long ng_pad,
                                                                                  const int* __restrict__ q_len, const int* __restrict__ g_len,
                                                                                  const unsigned long long* __restrict__ claim_all,
@@ -560,8 +585,8 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kerne
   }
   const long long nq = TABLE ? qs.len : pair_len(q_len, pair, nq_pad), ng = TABLE ? gs.len : pair_len(g_len, pair, ng_pad), q_offset = 0;
   const int n_row_blocks = static_cast<int>((nq + 31) / 32);
-  const float* q = TABLE ? q_all + qs.start * 128 : q_all + pair * nq_pad * 128;
-  const float* g = TABLE ? g_all + gs.start * 128 : g_all + pair * ng_pad * 128;
+  const T* q = TABLE ? q_all + qs.start * 128 : q_all + pair * nq_pad * 128;
+  const T* g = TABLE ? g_all + gs.start * 128 : g_all + pair * ng_pad * 128;
   const unsigned long long* claim = claim_all + pair * ng_pad;
   const float* block_max = block_max_all + pair * chunks * bm_pitch;
   const float* rb_min_d2 = rb_min_d2_all + pair * bm_pitch;
@@ -582,7 +607,7 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kerne
     if ((cc >> 32) < 0x7F000000ull) {
       undecided |= 1u << c;
       thr[c] = (1.0f - 0.5f * dcl[c] * dcl[c]) * inv_dot_scale - margin_scaled;
-      s_g[c * 32 + lane] = __ldg(reinterpret_cast<const float4*>(g + (cb * kChunk + c) * 128) + lane);
+      s_g[c * 32 + lane] = ldg_row4(g + (cb * kChunk + c) * 128, lane);
     }
   }
   if (!undecided) return;
@@ -621,7 +646,7 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kerne
 #pragma unroll
       for (int r = 0; r < 8; ++r) {
         v[r] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (k0 + r0 + r < nq) v[r] = __ldg(reinterpret_cast<const float4*>(q + (k0 + r0 + r) * 128) + lane);
+        if (k0 + r0 + r < nq) v[r] = ldg_row4(q + (k0 + r0 + r) * 128, lane);
       }
 #pragma unroll
       for (int r = 0; r < 8; ++r) *reinterpret_cast<float4*>(s_q + (r0 + r) * kVerifyPitch + 4 * lane) = v[r];
@@ -756,6 +781,24 @@ static int pick_segments(long long rows, int rows_per_block, long long cols, int
   return best;
 }
 
+// desc_dtype of the matching entry points -> the element type of the row-reading kernels: f(T{}) with T = float, __half or
+// __nv_bfloat16. check_rows has rejected every other value before.
+template <typename F>
+static int with_rows(int desc_dtype, F&& f) {
+  if (desc_dtype == HN_F16) return f(__half{});
+  if (desc_dtype == HN_BF16) return f(__nv_bfloat16{});
+  return f(float{});
+}
+
+// Descriptor rows of a matching call: fp32, fp16 or bf16 (the same for both sides); 16-bit rows are read 8 bytes per lane.
+static int check_rows(const char* fn, int desc_dtype, const void* a, const void* b) {
+  HN_REQUIRE(desc_dtype == HN_F32 || desc_dtype == HN_F16 || desc_dtype == HN_BF16,
+             "%s: desc_dtype must be HN_F32, HN_F16 or HN_BF16 (got %d)", fn, desc_dtype);
+  HN_REQUIRE(desc_dtype == HN_F32 || ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b)) & 7) == 0,
+             "%s: 16-bit descriptor rows must be 8-byte aligned", fn);
+  return HN_OK;
+}
+
 // Shared body of hn_dist_min / hn_loss_hardnet. Leaves packed minima and pos in the workspace.
 static int run_exact(const float* a, const float* p, long long Na, long long Np, int form, int flags, ExactWs& w,
                      cudaStream_t s, const float* a_xy = nullptr, const float* p_xy = nullptr, float nei_c = 0.f) {
@@ -876,15 +919,29 @@ extern "C" int hn_loss_hardnet(const float* anchor, const float* positive, long 
   return HN_OK;
 }
 
-extern "C" int hn_pack_descriptors(const float* x, long long n, void* out16, void* stream) {
-  HN_REQUIRE(x && out16, "hn_pack_descriptors: NULL argument");
-  HN_REQUIRE(n >= 1 && n < (1LL << 31), "hn_pack_descriptors: n out of range (%lld)", n);
+// hn_pack_descriptors / hn_pack_descriptors_typed; fn names the entry point in error messages.
+static int pack_entry(const char* fn, const void* x, int desc_dtype, long long n, void* out16, void* stream) {
+  HN_REQUIRE(x && out16, "%s: NULL argument", fn);
+  HN_TRY(check_rows(fn, desc_dtype, x, x));
+  HN_REQUIRE(n >= 1 && n < (1LL << 31), "%s: n out of range (%lld)", fn, n);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const int threads = 256;
-  pack_desc_kernel<<<static_cast<unsigned>((n * 32 + threads - 1) / threads), threads, 0, s>>>(x, n, static_cast<uint16_t*>(out16), 0, 0, nullptr);
-  HN_CUDA(cudaGetLastError());
-  count_launch();
-  return HN_OK;
+  return with_rows(desc_dtype, [&](auto t) -> int {
+    using T = decltype(t);
+    pack_desc_kernel<<<static_cast<unsigned>((n * 32 + threads - 1) / threads), threads, 0, s>>>(static_cast<const T*>(x), n,
+                                                                                                 static_cast<uint16_t*>(out16), 0, 0, nullptr);
+    HN_CUDA(cudaGetLastError());
+    count_launch();
+    return HN_OK;
+  });
+}
+
+extern "C" int hn_pack_descriptors(const float* x, long long n, void* out16, void* stream) {
+  return pack_entry("hn_pack_descriptors", x, HN_F32, n, out16, stream);
+}
+
+extern "C" int hn_pack_descriptors_typed(const void* x, int desc_dtype, long long n, void* out16, void* stream) {
+  return pack_entry("hn_pack_descriptors_typed", x, desc_dtype, n, out16, stream);
 }
 
 extern "C" int hn_pack_descriptors_multicast(const float* x, long long n, void* mc16, void* mc32, void* stream) {
@@ -900,17 +957,11 @@ extern "C" int hn_pack_descriptors_multicast(const float* x, long long n, void* 
   return HN_OK;
 }
 
-extern "C" int hn_match_ex(const float* q, const float* g, const void* q16_in, const void* g16_in, long long Nq, long long Ng,
-                           long long g_offset, float* d1, float* d2, int32_t* i1, int32_t* i2, float* block_max, void* workspace,
-                           long long workspace_bytes, void* g_ready_event, void* stream) {
-  HN_REQUIRE(q && g && workspace, "hn_match: NULL argument");
-  HN_REQUIRE(Nq >= 1 && Ng >= 1, "hn_match: empty input (Nq=%lld, Ng=%lld)", Nq, Ng);
-  HN_REQUIRE(Nq < (1LL << 31) && Ng + g_offset < (1LL << 31), "hn_match: more than 2^31 rows");
-  HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "hn_match: workspace must be 256-byte aligned");
-  HN_REQUIRE(workspace_bytes >= hn_dist_workspace_bytes(Nq, Ng, 0), "hn_match: workspace too small");
-  HN_REQUIRE((reinterpret_cast<uintptr_t>(q16_in) & 15) == 0 && (reinterpret_cast<uintptr_t>(g16_in) & 15) == 0,
-             "hn_match: packed operands must be 16-byte aligned");
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
+// The launch sequence of hn_match_ex / hn_match_typed on validated arguments.
+template <typename T>
+static int run_match(const T* q, const T* g, const void* q16_in, const void* g16_in, long long Nq, long long Ng, long long g_offset,
+                     float* d1, float* d2, int32_t* i1, int32_t* i2, float* block_max, void* workspace, void* g_ready_event,
+                     cudaStream_t s) {
   int sm = 0;
   HN_TRY(device_sm_count(&sm));
   char* b = static_cast<char*>(workspace);
@@ -963,8 +1014,8 @@ extern "C" int hn_match_ex(const float* q, const float* g, const void* q16_in, c
       HN_TRY((launch_dist<2, EPI_SHORTLIST>(dp, static_cast<int>(std::min<long long>(items, sm)), 1, s)));
     }
   }
-  // The re-rank reads the fp32 gallery rows of the shortlisted columns; a caller that gathered the packed gallery first
-  // (half the bytes) passes the event that marks the fp32 rows' arrival, so that transfer hides behind the GEMM.
+  // The re-rank reads the gallery rows of the shortlisted columns; a caller that gathered the packed gallery first (half the
+  // bytes of fp32 rows) passes the event that marks the rows' arrival, so that transfer hides behind the GEMM.
   if (g_ready_event) HN_CUDA(cudaStreamWaitEvent(s, static_cast<cudaEvent_t>(g_ready_event), 0));
   // |fp16-operand dot - exact dot| <= 2^-10 for rows of norm <= 1 (L2-normalised descriptors, the only input this path
   // is defined for: FDLNet-master/utils/math_utils.py:15-18 clamps 2 - 2ab to [1e-8, 4]); keep 4x that as the margin.
@@ -978,6 +1029,39 @@ extern "C" int hn_match_ex(const float* q, const float* g, const void* q16_in, c
     count_launch();
   }
   return HN_OK;
+}
+
+// hn_match / hn_match_ex / hn_match_typed; fn names the entry point in error messages.
+static int match_entry(const char* fn, const void* q, const void* g, int desc_dtype, const void* q16_in, const void* g16_in,
+                       long long Nq, long long Ng, long long g_offset, float* d1, float* d2, int32_t* i1, int32_t* i2,
+                       float* block_max, void* workspace, long long workspace_bytes, void* g_ready_event, void* stream) {
+  HN_REQUIRE(q && g && workspace, "%s: NULL argument", fn);
+  HN_TRY(check_rows(fn, desc_dtype, q, g));
+  HN_REQUIRE(Nq >= 1 && Ng >= 1, "%s: empty input (Nq=%lld, Ng=%lld)", fn, Nq, Ng);
+  HN_REQUIRE(Nq < (1LL << 31) && Ng + g_offset < (1LL << 31), "%s: more than 2^31 rows", fn);
+  HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "%s: workspace must be 256-byte aligned", fn);
+  HN_REQUIRE(workspace_bytes >= hn_dist_workspace_bytes(Nq, Ng, 0), "%s: workspace too small", fn);
+  HN_REQUIRE((reinterpret_cast<uintptr_t>(q16_in) & 15) == 0 && (reinterpret_cast<uintptr_t>(g16_in) & 15) == 0,
+             "%s: packed operands must be 16-byte aligned", fn);
+  return with_rows(desc_dtype, [&](auto t) -> int {
+    using T = decltype(t);
+    return run_match(static_cast<const T*>(q), static_cast<const T*>(g), q16_in, g16_in, Nq, Ng, g_offset, d1, d2, i1, i2, block_max,
+                     workspace, g_ready_event, static_cast<cudaStream_t>(stream));
+  });
+}
+
+extern "C" int hn_match_ex(const float* q, const float* g, const void* q16_in, const void* g16_in, long long Nq, long long Ng,
+                           long long g_offset, float* d1, float* d2, int32_t* i1, int32_t* i2, float* block_max, void* workspace,
+                           long long workspace_bytes, void* g_ready_event, void* stream) {
+  return match_entry("hn_match", q, g, HN_F32, q16_in, g16_in, Nq, Ng, g_offset, d1, d2, i1, i2, block_max, workspace, workspace_bytes,
+                     g_ready_event, stream);
+}
+
+extern "C" int hn_match_typed(const void* q, const void* g, int desc_dtype, const void* q16, const void* g16, long long Nq, long long Ng,
+                              long long g_offset, float* d1, float* d2, int32_t* i1, int32_t* i2, float* block_max, void* workspace,
+                              long long workspace_bytes, void* g_ready_event, void* stream) {
+  return match_entry("hn_match_typed", q, g, desc_dtype, q16, g16, Nq, Ng, g_offset, d1, d2, i1, i2, block_max, workspace,
+                     workspace_bytes, g_ready_event, stream);
 }
 
 extern "C" int hn_match(const float* q, const float* g, long long Nq, long long Ng, long long g_offset, float* d1,
@@ -1000,22 +1084,28 @@ extern "C" int hn_mutual_claims(const int32_t* i1, const float* d1, const float*
   return HN_OK;
 }
 
-extern "C" int hn_mutual_verify(const float* q, long long Nq, long long q_offset, const float* g, long long Ng,
-                                const unsigned long long* claim, const float* block_max, const float* rb_min_d2,
-                                unsigned char* beaten, void* stream) {
-  HN_REQUIRE(q && g && claim && block_max && rb_min_d2 && beaten, "hn_mutual_verify: NULL argument");
-  HN_REQUIRE(Nq >= 1 && Ng >= 1 && Nq + q_offset < (1LL << 32), "hn_mutual_verify: size out of range");
+template <typename T>
+static int launch_verify(const T* q, long long Nq, long long q_offset, const T* g, long long Ng, const unsigned long long* claim,
+                         const float* block_max, const float* rb_min_d2, unsigned char* beaten, cudaStream_t s) {
   const long long chunks = (Ng + kChunk - 1) / kChunk;
   // twice the 2^-10 error bound of the fp16-operand dot product of unit vectors, in the GEMM's scaled units
   const float margin = 2.0f * (1.0f / 1024.0f) / kDotScale;
   static DeviceOnce attr_once;
   if (attr_once.first_time())
-    HN_CUDA(cudaFuncSetAttribute(mutual_verify_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kVerifySmem)));
-  mutual_verify_kernel<<<static_cast<unsigned>((chunks + kVerifyWarps - 1) / kVerifyWarps), kVerifyWarps * 32, kVerifySmem, static_cast<cudaStream_t>(stream)>>>(
+    HN_CUDA(cudaFuncSetAttribute(mutual_verify_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kVerifySmem)));
+  mutual_verify_kernel<T><<<static_cast<unsigned>((chunks + kVerifyWarps - 1) / kVerifyWarps), kVerifyWarps * 32, kVerifySmem, s>>>(
       q, Nq, q_offset, g, Ng, claim, block_max, rb_min_d2, static_cast<int>((Nq + 31) / 32), margin, 1.0f / kDotScale, beaten);
   HN_CUDA(cudaGetLastError());
   count_launch();
   return HN_OK;
+}
+
+extern "C" int hn_mutual_verify(const float* q, long long Nq, long long q_offset, const float* g, long long Ng,
+                                const unsigned long long* claim, const float* block_max, const float* rb_min_d2,
+                                unsigned char* beaten, void* stream) {
+  HN_REQUIRE(q && g && claim && block_max && rb_min_d2 && beaten, "hn_mutual_verify: NULL argument");
+  HN_REQUIRE(Nq >= 1 && Ng >= 1 && Nq + q_offset < (1LL << 32), "hn_mutual_verify: size out of range");
+  return launch_verify(q, Nq, q_offset, g, Ng, claim, block_max, rb_min_d2, beaten, static_cast<cudaStream_t>(stream));
 }
 
 extern "C" long long hn_mutual_workspace_bytes(long long Nq, long long Ng) {
@@ -1025,11 +1115,13 @@ extern "C" long long hn_mutual_workspace_bytes(long long Nq, long long Ng) {
                                                                          align256(static_cast<size_t>((Nq + 31) / 32) * 4) + 256);
 }
 
-extern "C" int hn_match_mutual(const float* q, const float* g, const void* q16, const void* g16, long long Nq, long long Ng,
-                               float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace,
-                               long long workspace_bytes, void* stream) {
-  HN_REQUIRE(q && g && d1 && d2 && i1 && mutual && workspace, "hn_match_mutual: NULL argument (d1, d2, i1 and mutual are required outputs)");
-  HN_REQUIRE(workspace_bytes >= hn_mutual_workspace_bytes(Nq, Ng), "hn_match_mutual: workspace too small");
+// hn_match_mutual / hn_match_mutual_typed; fn names the entry point in error messages.
+static int mutual_entry(const char* fn, const void* q, const void* g, int desc_dtype, const void* q16, const void* g16, long long Nq,
+                        long long Ng, float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace,
+                        long long workspace_bytes, void* stream) {
+  HN_REQUIRE(q && g && d1 && d2 && i1 && mutual && workspace, "%s: NULL argument (d1, d2, i1 and mutual are required outputs)", fn);
+  HN_TRY(check_rows(fn, desc_dtype, q, g));
+  HN_REQUIRE(workspace_bytes >= hn_mutual_workspace_bytes(Nq, Ng), "%s: workspace too small", fn);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const long long base = hn_dist_workspace_bytes(Nq, Ng, 0);
   char* b = static_cast<char*>(workspace) + align256(static_cast<size_t>(base));
@@ -1040,15 +1132,31 @@ extern "C" int hn_match_mutual(const float* q, const float* g, const void* q16, 
   unsigned char* beaten = reinterpret_cast<unsigned char*>(b);
   b += align256(static_cast<size_t>(Ng));
   float* rbmin = reinterpret_cast<float*>(b);
-  HN_TRY(hn_match_ex(q, g, q16, g16, Nq, Ng, 0, d1, d2, i1, i2, bm, workspace, base, nullptr, stream));
+  HN_TRY(match_entry(fn, q, g, desc_dtype, q16, g16, Nq, Ng, 0, d1, d2, i1, i2, bm, workspace, base, nullptr, stream));
   HN_CUDA(cudaMemsetAsync(claim, 0x7f, static_cast<size_t>(Ng) * 8, s));   // "unclaimed"
   HN_CUDA(cudaMemsetAsync(beaten, 0, static_cast<size_t>(Ng), s));
   HN_TRY(hn_mutual_claims(i1, d1, d2, Nq, 0, claim, Ng, rbmin, stream));
-  HN_TRY(hn_mutual_verify(q, Nq, 0, g, Ng, claim, bm, rbmin, beaten, stream));
+  HN_TRY(with_rows(desc_dtype, [&](auto t) -> int {
+    using T = decltype(t);
+    return launch_verify(static_cast<const T*>(q), Nq, 0, static_cast<const T*>(g), Ng, claim, bm, rbmin, beaten, s);
+  }));
   mutual_final_kernel<<<static_cast<unsigned>((Nq + 255) / 256), 256, 0, s>>>(i1, Nq, 0, claim, beaten, Ng, mutual);
   HN_CUDA(cudaGetLastError());
   count_launch();
   return HN_OK;
+}
+
+extern "C" int hn_match_mutual(const float* q, const float* g, const void* q16, const void* g16, long long Nq, long long Ng,
+                               float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace,
+                               long long workspace_bytes, void* stream) {
+  return mutual_entry("hn_match_mutual", q, g, HN_F32, q16, g16, Nq, Ng, d1, d2, i1, i2, mutual, workspace, workspace_bytes, stream);
+}
+
+extern "C" int hn_match_mutual_typed(const void* q, const void* g, int desc_dtype, const void* q16, const void* g16, long long Nq,
+                                     long long Ng, float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual,
+                                     void* workspace, long long workspace_bytes, void* stream) {
+  return mutual_entry("hn_match_mutual_typed", q, g, desc_dtype, q16, g16, Nq, Ng, d1, d2, i1, i2, mutual, workspace, workspace_bytes,
+                      stream);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -1113,8 +1221,8 @@ struct PairLayout {
 
 // The launch sequence of hn_match_pairs (TABLE) and hn_match_batched: GEMM + shortlist, re-rank, and with `mutual` the column
 // side. q16 / g16 are the packed rows of q / g.
-template <bool TABLE>
-static int run_pairs(const float* q, const uint16_t* q16, const float* g, const uint16_t* g16, const PairLayout& L, float* d1,
+template <bool TABLE, typename T>
+static int run_pairs(const T* q, const uint16_t* q16, const T* g, const uint16_t* g16, const PairLayout& L, float* d1,
                      float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, const BatchedWs& w, cudaStream_t s) {
   int sm = 0;
   HN_TRY(device_sm_count(&sm));
@@ -1156,7 +1264,7 @@ static int run_pairs(const float* q, const uint16_t* q16, const float* g, const 
   const float margin = 4.0f * (1.0f / 1024.0f) / kDotScale;   // as hn_match_ex
   {
     MatchTimer timer(2, s);
-    rerank_batched_kernel<TABLE><<<static_cast<unsigned>((rows_q + 3) / 4), 128, 0, s>>>(
+    rerank_batched_kernel<TABLE, T><<<static_cast<unsigned>((rows_q + 3) / 4), 128, 0, s>>>(
         q, g, w.cand, w.cand_val, margin, B, Nq, Ng, L.q_len, L.g_len, dp.segments * kTopC, d1, d2, i1, i2, L.pairs, L.q_rows, L.g_rows);
     HN_CUDA(cudaGetLastError());
     count_launch();
@@ -1169,9 +1277,9 @@ static int run_pairs(const float* q, const uint16_t* q16, const float* g, const 
         i1, d1, d2, B, Nq, Ng, L.q_len, L.g_len, w.claim, w.rb_min_d2, L.pairs, L.q_rows, L.g_rows);
     static DeviceOnce attr_once;
     if (attr_once.first_time())
-      HN_CUDA(cudaFuncSetAttribute(mutual_verify_batched_kernel<TABLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kVerifySmem)));
+      HN_CUDA(cudaFuncSetAttribute(mutual_verify_batched_kernel<TABLE, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kVerifySmem)));
     const float vmargin = 2.0f * (1.0f / 1024.0f) / kDotScale;   // as hn_mutual_verify
-    mutual_verify_batched_kernel<TABLE><<<static_cast<unsigned>((B * chunks + kVerifyWarps - 1) / kVerifyWarps), kVerifyWarps * 32, kVerifySmem, s>>>(
+    mutual_verify_batched_kernel<TABLE, T><<<static_cast<unsigned>((B * chunks + kVerifyWarps - 1) / kVerifyWarps), kVerifyWarps * 32, kVerifySmem, s>>>(
         q, g, B, Nq, Ng, L.q_len, L.g_len, w.claim, w.block_max, w.rb_min_d2, vmargin, 1.0f / kDotScale, w.beaten, L.pairs, L.q_rows,
         L.g_rows);
     mutual_final_batched_kernel<TABLE><<<static_cast<unsigned>((rows_q + threads - 1) / threads), threads, 0, s>>>(
@@ -1187,15 +1295,9 @@ extern "C" long long hn_match_batched_workspace_bytes(long long B, long long Nq,
   return static_cast<long long>(carve_batched(nullptr, B, Nq, Ng, with_mutual != 0, true).bytes);
 }
 
-extern "C" int hn_match_batched(const float* q, const float* g, long long B, long long Nq, long long Ng, const int32_t* q_len,
-                                const int32_t* g_len, float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual,
-                                void* workspace, long long workspace_bytes, void* stream) {
-  HN_REQUIRE(q && g && d1 && d2 && i1 && i2 && workspace, "hn_match_batched: NULL argument (q, g, d1, d2, i1, i2 and workspace are required)");
-  HN_REQUIRE(B >= 1 && Nq >= 1 && Ng >= 1, "hn_match_batched: empty input (B=%lld, Nq=%lld, Ng=%lld)", B, Nq, Ng);
-  HN_REQUIRE(Nq < (1LL << 31) / B && Ng < (1LL << 31) / B, "hn_match_batched: B*Nq and B*Ng must stay below 2^31 rows");
-  HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "hn_match_batched: workspace must be 256-byte aligned");
-  HN_REQUIRE(workspace_bytes >= hn_match_batched_workspace_bytes(B, Nq, Ng, mutual != nullptr), "hn_match_batched: workspace too small");
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
+template <typename T>
+static int run_batched(const T* q, const T* g, long long B, long long Nq, long long Ng, const int32_t* q_len, const int32_t* g_len,
+                       float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace, cudaStream_t s) {
   const BatchedWs w = carve_batched(workspace, B, Nq, Ng, mutual != nullptr, true);
   const long long rows_q = B * Nq, rows_g = B * Ng;
   const int threads = 256;
@@ -1210,29 +1312,79 @@ extern "C" int hn_match_batched(const float* q, const float* g, long long B, lon
   return run_pairs<false>(q, w.q16, g, w.g16, L, d1, d2, i1, i2, mutual, w, s);
 }
 
+// hn_match_batched / hn_match_batched_typed; fn names the entry point in error messages.
+static int batched_entry(const char* fn, const void* q, const void* g, int desc_dtype, long long B, long long Nq, long long Ng,
+                         const int32_t* q_len, const int32_t* g_len, float* d1, float* d2, int32_t* i1, int32_t* i2,
+                         unsigned char* mutual, void* workspace, long long workspace_bytes, void* stream) {
+  HN_REQUIRE(q && g && d1 && d2 && i1 && i2 && workspace, "%s: NULL argument (q, g, d1, d2, i1, i2 and workspace are required)", fn);
+  HN_TRY(check_rows(fn, desc_dtype, q, g));
+  HN_REQUIRE(B >= 1 && Nq >= 1 && Ng >= 1, "%s: empty input (B=%lld, Nq=%lld, Ng=%lld)", fn, B, Nq, Ng);
+  HN_REQUIRE(Nq < (1LL << 31) / B && Ng < (1LL << 31) / B, "%s: B*Nq and B*Ng must stay below 2^31 rows", fn);
+  HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "%s: workspace must be 256-byte aligned", fn);
+  HN_REQUIRE(workspace_bytes >= hn_match_batched_workspace_bytes(B, Nq, Ng, mutual != nullptr), "%s: workspace too small", fn);
+  return with_rows(desc_dtype, [&](auto t) -> int {
+    using T = decltype(t);
+    return run_batched(static_cast<const T*>(q), static_cast<const T*>(g), B, Nq, Ng, q_len, g_len, d1, d2, i1, i2, mutual, workspace,
+                       static_cast<cudaStream_t>(stream));
+  });
+}
+
+extern "C" int hn_match_batched(const float* q, const float* g, long long B, long long Nq, long long Ng, const int32_t* q_len,
+                                const int32_t* g_len, float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual,
+                                void* workspace, long long workspace_bytes, void* stream) {
+  return batched_entry("hn_match_batched", q, g, HN_F32, B, Nq, Ng, q_len, g_len, d1, d2, i1, i2, mutual, workspace, workspace_bytes,
+                       stream);
+}
+
+extern "C" int hn_match_batched_typed(const void* q, const void* g, int desc_dtype, long long B, long long Nq, long long Ng,
+                                      const int32_t* q_len, const int32_t* g_len, float* d1, float* d2, int32_t* i1, int32_t* i2,
+                                      unsigned char* mutual, void* workspace, long long workspace_bytes, void* stream) {
+  return batched_entry("hn_match_batched_typed", q, g, desc_dtype, B, Nq, Ng, q_len, g_len, d1, d2, i1, i2, mutual, workspace,
+                       workspace_bytes, stream);
+}
+
 extern "C" long long hn_match_pairs_workspace_bytes(long long B, long long max_q, long long max_g, int with_mutual) {
   if (B < 0 || max_q < 0 || max_g < 0) return 0;
   return static_cast<long long>(carve_batched(nullptr, B, max_q, max_g, with_mutual != 0, false).bytes);
 }
 
+// hn_match_pairs / hn_match_pairs_typed; fn names the entry point in error messages.
+static int pairs_entry(const char* fn, const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16, long long Ng_rows,
+                       int desc_dtype, const int32_t* pairs, long long B, long long max_q, long long max_g, float* d1, float* d2,
+                       int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace, long long workspace_bytes, void* stream) {
+  HN_REQUIRE(q && q16 && g && g16 && pairs && d1 && d2 && i1 && i2 && workspace,
+             "%s: NULL argument (q, q16, g, g16, pairs, d1, d2, i1, i2 and workspace are required)", fn);
+  HN_TRY(check_rows(fn, desc_dtype, q, g));
+  HN_REQUIRE(B >= 1 && max_q >= 1 && max_g >= 1 && Nq_rows >= 1 && Ng_rows >= 1,
+             "%s: empty input (B=%lld, max_q=%lld, max_g=%lld, Nq_rows=%lld, Ng_rows=%lld)", fn, B, max_q, max_g, Nq_rows, Ng_rows);
+  HN_REQUIRE(Nq_rows < (1LL << 31) && Ng_rows < (1LL << 31), "%s: a descriptor set has 2^31 rows or more", fn);
+  HN_REQUIRE(max_q < (1LL << 31) / B && max_g < (1LL << 31) / B, "%s: B*max_q and B*max_g must stay below 2^31 rows", fn);
+  HN_REQUIRE((reinterpret_cast<uintptr_t>(q16) & 15) == 0 && (reinterpret_cast<uintptr_t>(g16) & 15) == 0,
+             "%s: packed operands must be 16-byte aligned", fn);
+  HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "%s: workspace must be 256-byte aligned", fn);
+  HN_REQUIRE(workspace_bytes >= hn_match_pairs_workspace_bytes(B, max_q, max_g, mutual != nullptr), "%s: workspace too small", fn);
+  const BatchedWs w = carve_batched(workspace, B, max_q, max_g, mutual != nullptr, false);
+  const PairLayout L = {pairs, nullptr, nullptr, B, max_q, max_g, Nq_rows, Ng_rows};
+  return with_rows(desc_dtype, [&](auto t) -> int {
+    using T = decltype(t);
+    return run_pairs<true>(static_cast<const T*>(q), static_cast<const uint16_t*>(q16), static_cast<const T*>(g),
+                           static_cast<const uint16_t*>(g16), L, d1, d2, i1, i2, mutual, w, static_cast<cudaStream_t>(stream));
+  });
+}
+
 extern "C" int hn_match_pairs(const float* q, const void* q16, long long Nq_rows, const float* g, const void* g16, long long Ng_rows,
                               const int32_t* pairs, long long B, long long max_q, long long max_g, float* d1, float* d2, int32_t* i1,
                               int32_t* i2, unsigned char* mutual, void* workspace, long long workspace_bytes, void* stream) {
-  HN_REQUIRE(q && q16 && g && g16 && pairs && d1 && d2 && i1 && i2 && workspace,
-             "hn_match_pairs: NULL argument (q, q16, g, g16, pairs, d1, d2, i1, i2 and workspace are required)");
-  HN_REQUIRE(B >= 1 && max_q >= 1 && max_g >= 1 && Nq_rows >= 1 && Ng_rows >= 1,
-             "hn_match_pairs: empty input (B=%lld, max_q=%lld, max_g=%lld, Nq_rows=%lld, Ng_rows=%lld)", B, max_q, max_g, Nq_rows,
-             Ng_rows);
-  HN_REQUIRE(Nq_rows < (1LL << 31) && Ng_rows < (1LL << 31), "hn_match_pairs: a descriptor set has 2^31 rows or more");
-  HN_REQUIRE(max_q < (1LL << 31) / B && max_g < (1LL << 31) / B, "hn_match_pairs: B*max_q and B*max_g must stay below 2^31 rows");
-  HN_REQUIRE((reinterpret_cast<uintptr_t>(q16) & 15) == 0 && (reinterpret_cast<uintptr_t>(g16) & 15) == 0,
-             "hn_match_pairs: packed operands must be 16-byte aligned");
-  HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "hn_match_pairs: workspace must be 256-byte aligned");
-  HN_REQUIRE(workspace_bytes >= hn_match_pairs_workspace_bytes(B, max_q, max_g, mutual != nullptr), "hn_match_pairs: workspace too small");
-  const BatchedWs w = carve_batched(workspace, B, max_q, max_g, mutual != nullptr, false);
-  const PairLayout L = {pairs, nullptr, nullptr, B, max_q, max_g, Nq_rows, Ng_rows};
-  return run_pairs<true>(q, static_cast<const uint16_t*>(q16), g, static_cast<const uint16_t*>(g16), L, d1, d2, i1, i2, mutual, w,
-                   static_cast<cudaStream_t>(stream));
+  return pairs_entry("hn_match_pairs", q, q16, Nq_rows, g, g16, Ng_rows, HN_F32, pairs, B, max_q, max_g, d1, d2, i1, i2, mutual,
+                     workspace, workspace_bytes, stream);
+}
+
+extern "C" int hn_match_pairs_typed(const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16,
+                                    long long Ng_rows, int desc_dtype, const int32_t* pairs, long long B, long long max_q,
+                                    long long max_g, float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual,
+                                    void* workspace, long long workspace_bytes, void* stream) {
+  return pairs_entry("hn_match_pairs_typed", q, q16, Nq_rows, g, g16, Ng_rows, desc_dtype, pairs, B, max_q, max_g, d1, d2, i1, i2,
+                     mutual, workspace, workspace_bytes, stream);
 }
 
 extern "C" int hn_match_force_kernel(int mode) {

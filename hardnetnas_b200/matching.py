@@ -3,6 +3,9 @@
 The reference materialises the full distance matrix and then takes `min` (eval_utils.py:113-114) or a full
 row `sort` (:168-175). Here one fused pass (tensor-core GEMM + in-register shortlist, exact fp32 re-rank)
 returns the nearest and second-nearest gallery row per query; nothing of size Nq x Ng is ever stored.
+Descriptors may be fp32, fp16 or bf16: fp16 / bf16 tensors of one dtype (e.g. `HardNet.forward(x, out_dtype=torch.float16)`) are
+matched as they are, without an fp32 copy, with results bit-identical to the same call on their `.float()`; mixed or other dtypes
+are converted to fp32 first.
 """
 from __future__ import annotations
 

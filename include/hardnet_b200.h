@@ -248,6 +248,33 @@ int hn_match_pairs(const float* q, const void* q16, long long Nq_rows, const flo
  * initial value is read once from HN_MATCH_PAIR), 0 = single-CTA kernel, 1 = CTA-pair (cta_group::2) kernel. */
 int hn_match_force_kernel(int mode);
 
+/* ---- matching on fp16 / bf16 descriptor rows -------------------------------------------------------------------------------
+ * Typed twins of the row-reading matching entry points: descriptor rows are `const void*` of desc_dtype HN_F32, HN_F16 or
+ * HN_BF16 (e.g. the out_dtype output of hn_forward / hn_forward_nas / hn_forward_clip), the same type on both sides of a call;
+ * the other arguments, the outputs and the preconditions are those of the fp32 function named. Every kernel widens a 16-bit
+ * element to fp32 where it loads it and then runs the fp32 arithmetic: the packed operand is __float2half_rn(float(x) * 2^8)
+ * as for fp32 rows, and the re-rank and the mutual verification sum the same fp32 products in the same order. So a call on
+ * 16-bit rows returns exactly what the fp32 call returns on the rows converted to fp32 (distances, indices, ties, mutual
+ * flags, bit for bit), without that fp32 copy: the re-rank and verification read 256 instead of 512 bytes per row.
+ * The workspace does not depend on the row type: hn_dist_workspace_bytes, hn_mutual_workspace_bytes,
+ * hn_match_batched_workspace_bytes and hn_match_pairs_workspace_bytes size the typed calls too. Validation as the fp32
+ * function, plus: a desc_dtype other than HN_F32 / HN_F16 / HN_BF16 (HN_U8 included) and 16-bit rows that are not 8-byte
+ * aligned are rejected with HN_ERR_INVALID before any device work. The fp32 functions are these calls with HN_F32. */
+int hn_pack_descriptors_typed(const void* x, int desc_dtype, long long n, void* out16, void* stream);          /* hn_pack_descriptors */
+int hn_match_typed(const void* q, const void* g, int desc_dtype, const void* q16, const void* g16, long long Nq, long long Ng,
+                   long long g_offset, float* d1, float* d2, int32_t* i1, int32_t* i2, float* block_max, void* workspace,
+                   long long workspace_bytes, void* g_ready_event, void* stream);                              /* hn_match_ex */
+int hn_match_mutual_typed(const void* q, const void* g, int desc_dtype, const void* q16, const void* g16, long long Nq,
+                          long long Ng, float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace,
+                          long long workspace_bytes, void* stream);                                            /* hn_match_mutual */
+int hn_match_batched_typed(const void* q, const void* g, int desc_dtype, long long B, long long Nq, long long Ng,
+                           const int32_t* q_len, const int32_t* g_len, float* d1, float* d2, int32_t* i1, int32_t* i2,
+                           unsigned char* mutual, void* workspace, long long workspace_bytes, void* stream);  /* hn_match_batched */
+int hn_match_pairs_typed(const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16, long long Ng_rows,
+                         int desc_dtype, const int32_t* pairs, long long B, long long max_q, long long max_g, float* d1, float* d2,
+                         int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace, long long workspace_bytes,
+                         void* stream);                                                                        /* hn_match_pairs */
+
 /* Measurement hooks (process-wide): bracket the three stages of every hn_match / hn_match_batched / hn_match_pairs call
  * (0 = operand packing, not part of hn_match_pairs; 1 = GEMM + shortlist, 2 = exact re-rank) with CUDA events; hn_match_profile_read waits for them, returns the summed milliseconds and
  * launch counts per stage and resets the counters. */
