@@ -11,6 +11,11 @@ namespace hn {
 
 constexpr float kOperandScale = 256.0f;  // descriptors are unit vectors: x256 keeps the fp16 hi/lo split clear of subnormals
 constexpr float kDotScale = 1.0f / (kOperandScale * kOperandScale);
+// |fp16-operand dot - exact dot| <= 2^-10 for rows of norm <= 1 (L2-normalised descriptors, the only input matching is defined
+// for: FDLNet-master/utils/math_utils.py:15-18 clamps 2 - 2ab to [1e-8, 4]). In the GEMM's scaled units, the re-rank keeps 4x
+// that bound as the margin of its candidate threshold and the mutual verification 2x as the margin of its cell test.
+constexpr float kRerankMargin = 4.0f * (1.0f / 1024.0f) / kDotScale;
+constexpr float kVerifyMargin = 2.0f * (1.0f / 1024.0f) / kDotScale;
 
 static inline size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
 
@@ -137,35 +142,35 @@ __global__ void loss_finalize_kernel(const float* __restrict__ pos, const unsign
   }
 }
 
-// Exact fp32 re-rank of the shortlisted chunks: one warp per query row, one candidate gallery row per lane.
-// Distances in the FDLNet form; ties resolve to the lower gallery index like torch.min / a stable sort.
+// Top-2 of one query row: distances d1 <= d2 and their gallery columns (0x7fffffff: fewer columns than that).
+struct Top2 {
+  float d1, d2;
+  int i1, i2;
+};
+
+// Exact fp32 re-rank of the shortlisted chunks of one query row: one warp per row, whose staged query row is sqw. crow / cvrow
+// are the row's `slots` candidate chunks and their approximate maxima, g / ng its gallery. Distances in the FDLNet form; ties
+// resolve to the lower gallery index like torch.min / a stable sort. rerank_kernel and rerank_batched_kernel both run this
+// body, so a batched or pair-table row equals the per-pair hn_match row bit for bit.
 // Known limit (documented precondition of hn_match): the GEMM keeps the kTopC = 4 best chunks per row and list (a list = one
 // gallery segment, or one 64-column half of it in the CTA-pair kernel). Should five or more chunks of ONE list reach the
 // threshold, the fifth is not re-ranked; with 15-30 lists per row this needs five near-tied best candidates inside one list
 // (|d - d2| within the 2^-9 margin). Scanning the whole segment whenever a list's fourth chunk passes the threshold was
 // measured: it fires on ~5 % of the rows of the BASELINE config-4 set and makes the call 5x slower (0.88 -> 4.2 ms), so the
 // exact remedy has to track the largest DROPPED chunk maximum in the GEMM epilogue instead (not done).
-// T: fp32, fp16 or bf16 rows (ld_row4 / ldg_row4); the fp32 instantiation compiles to the instructions of the kernel before it
-// was a template (checked with cuobjdump), and the 16-bit ones differ only in their loads.
+// Both re-rank kernels ask for 10 CTAs per SM, i.e. at most 48 registers, which this body fits without spilling. Left to its
+// own choice ptxas spilled 8 bytes in some instantiations to stay within 48 or 56 registers.
+constexpr int kRerankCtasPerSm = 10;
 template <typename T>
-__global__ void __launch_bounds__(128) rerank_kernel(const T* __restrict__ q, const T* __restrict__ g,
-                                                     const int* __restrict__ cand, const float* __restrict__ cand_val,
-                                                     float margin, long long nq, long long ng, int slots,
-                                                     long long g_offset, float* __restrict__ d1, float* __restrict__ d2,
-                                                     int* __restrict__ i1, int* __restrict__ i2) {
-  __shared__ __align__(16) float sq[4][128];
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long long row = static_cast<long long>(blockIdx.x) * 4 + w;
-  if (row >= nq) return;
-  reinterpret_cast<float4*>(sq[w])[lane] = ld_row4(q + row * 128, lane);
-  __syncwarp();
+__device__ __forceinline__ Top2 rerank_row(const float* sqw, const T* g, long long ng, const int* crow, const float* cvrow, int slots,
+                                           float margin, int lane) {
   // A chunk can hold one of the two nearest columns only if its approximate maximum reaches the second largest
   // chunk maximum minus twice the error bound of the 16-bit-operand dot product (`margin`, same scaled units).
   float thr;
   {
     float m1 = -__int_as_float(0x7f800000), m2 = m1;
     for (int c = lane; c < slots; c += 32) {
-      const float v = cand[row * slots + c] >= 0 ? cand_val[row * slots + c] : -__int_as_float(0x7f800000);
+      const float v = crow[c] >= 0 ? cvrow[c] : -__int_as_float(0x7f800000);
       if (v > m1) { m2 = m1; m1 = v; } else if (v > m2) { m2 = v; }
     }
 #pragma unroll
@@ -183,16 +188,15 @@ __global__ void __launch_bounds__(128) rerank_kernel(const T* __restrict__ q, co
   // The warp walks the surviving chunks together: a gallery row is ONE coalesced 512 B read (lane = float4 index) and
   // the 128-term dot is finished with a butterfly, so every lane ends up with the same (d, index) stream. Per-lane
   // row reads (one lane per candidate) cost 32 L1 wavefronts per row instead of 4.
-  const float4 qv = reinterpret_cast<const float4*>(sq[w])[lane];
+  const float4 qv = reinterpret_cast<const float4*>(sqw)[lane];
   auto eval_chunk = [&](long long chunk) {
-    const long long col0 = chunk * kChunk;
+    const long long col0 = chunk * kChunk, left = ng - col0;   // column col0 + r exists iff r < left
     float part[kChunk];
 #pragma unroll
     for (int r = 0; r < kChunk; ++r) {
-      const long long col = col0 + r;
       part[r] = 0.f;
-      if (col < ng) {
-        const float4 gv = ldg_row4(g + col * 128, lane);
+      if (r < left) {
+        const float4 gv = ldg_row4(g + (col0 + r) * 128, lane);
         part[r] = fmaf(qv.x, gv.x, fmaf(qv.y, gv.y, fmaf(qv.z, gv.z, qv.w * gv.w)));
       }
     }
@@ -201,12 +205,18 @@ __global__ void __launch_bounds__(128) rerank_kernel(const T* __restrict__ q, co
 #pragma unroll
       for (int r = 0; r < kChunk; ++r) part[r] += __shfl_xor_sync(0xffffffffu, part[r], o);
     }
+    // The eight distances are taken by eight lanes, one sqrtf each, and shuffled to the warp (every lane holds the same eight
+    // dot products). Eight unrolled sqrtf per lane are eight slow-path calls, across which the gallery pointer and size stay
+    // live: that made ptxas spill.
+    float mine = part[0];   // part[lane & 7] without a local-memory array access
+#pragma unroll
+    for (int r = 1; r < kChunk; ++r) mine = (lane & (kChunk - 1)) == r ? part[r] : mine;
+    mine = sqrtf(fminf(fmaxf(2.0f - 2.0f * mine, 1e-8f), 4.0f));
 #pragma unroll
     for (int r = 0; r < kChunk; ++r) {
-      const long long col = col0 + r;
-      if (col >= ng) continue;
-      const float d = sqrtf(fminf(fmaxf(2.0f - 2.0f * part[r], 1e-8f), 4.0f));
-      const int ci = static_cast<int>(col);
+      const float d = __shfl_sync(0xffffffffu, mine, r);
+      if (r >= left) continue;
+      const int ci = static_cast<int>(col0) + r;   // ng < 2^31
       if (d < b1 || (d == b1 && ci < j1)) {
         b2 = b1; j2 = j1; b1 = d; j1 = ci;
       } else if (d < b2 || (d == b2 && ci < j2)) {
@@ -215,33 +225,44 @@ __global__ void __launch_bounds__(128) rerank_kernel(const T* __restrict__ q, co
     }
   };
   for (int c = 0; c < slots; ++c) {
-    const int chunk = cand[row * slots + c];
-    if (chunk < 0 || cand_val[row * slots + c] < thr) continue;   // warp-uniform
+    const int chunk = crow[c];
+    if (chunk < 0 || cvrow[c] < thr) continue;   // warp-uniform
     eval_chunk(chunk);
   }
-  // every lane holds the same top-2 now
-  const float m = b1, s = b2;
-  const int mj = j1, sj = j2;
+  return {b1, b2, j1, j2};   // the same on every lane
+}
+
+// Re-rank of hn_match: query row `row` of q against g; optional outputs, indices shifted by g_offset.
+// T: fp32, fp16 or bf16 rows (ld_row4 / ldg_row4).
+template <typename T>
+__global__ void __launch_bounds__(128, kRerankCtasPerSm) rerank_kernel(const T* __restrict__ q, const T* __restrict__ g,
+                                                     const int* __restrict__ cand, const float* __restrict__ cand_val,
+                                                     float margin, long long nq, long long ng, int slots,
+                                                     long long g_offset, float* __restrict__ d1, float* __restrict__ d2,
+                                                     int* __restrict__ i1, int* __restrict__ i2) {
+  __shared__ __align__(16) float sq[4][128];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int row = static_cast<int>(blockIdx.x * 4 + w);   // nq < 2^31; widened where it scales an element offset
+  if (row >= nq) return;
+  reinterpret_cast<float4*>(sq[w])[lane] = ld_row4(q + static_cast<long long>(row) * 128, lane);
+  __syncwarp();
+  const Top2 t = rerank_row(sq[w], g, ng, cand + static_cast<long long>(row) * slots, cand_val + static_cast<long long>(row) * slots,
+                            slots, margin, lane);
   if (lane == 0) {
-    if (d1) d1[row] = m;
-    if (i1) i1[row] = mj == 0x7fffffff ? -1 : static_cast<int>(mj + g_offset);
-    if (d2) d2[row] = s;
-    if (i2) i2[row] = sj == 0x7fffffff ? -1 : static_cast<int>(sj + g_offset);
+    if (d1) d1[row] = t.d1;
+    if (i1) i1[row] = t.i1 == 0x7fffffff ? -1 : static_cast<int>(t.i1 + g_offset);
+    if (d2) d2[row] = t.d2;
+    if (i2) i2[row] = t.i2 == 0x7fffffff ? -1 : static_cast<int>(t.i2 + g_offset);
   }
 }
 
 // Batched re-rank over the flat [B * nq_pad] query rows of hn_match_batched: row -> pair b = row / nq_pad, whose gallery is
 // rows [0, g_len[b]) of g + b * ng_pad * 128; indices are local to the pair. Rows past q_len[b] get the fill values
 // (d = +inf, i = -1). TABLE (hn_match_pairs): pair b's rows are the ranges of the pair table over the concatenated sets instead,
-// query row qs + r of q and gallery rows [gs, gs + gl) of g_all; the padded instantiation keeps the instructions it had before
-// hn_match_pairs existed (reading the padded layout through the table accessor measured 1-2 % slower). From the prologue on this is rerank_kernel's body, copied rather than shared so that the single-problem
-// kernel compiles to the same instructions as before: keep the two in step, the bit equality of a batched row with a per-pair
-// hn_match rests on the same candidate threshold and the same summation order (tests/test_matching_batched_gpu.py compares
-// them bit for bit). One difference: the eight distances of a chunk are taken by eight lanes, one sqrtf each, and shuffled to
-// the warp (the same values: every lane holds the same eight dot products). Eight unrolled sqrtf slow-path calls per lane kept
-// the pair's gallery pointer and size live across calls and made ptxas spill.
+// query row qs + r of q and gallery rows [gs, gs + gl) of g_all. The padded instantiation does not read its layout through the
+// table accessor: that measured 1-2 % slower.
 template <bool TABLE, typename T>
-__global__ void __launch_bounds__(128) rerank_batched_kernel(const T* __restrict__ q, const T* __restrict__ g_all,
+__global__ void __launch_bounds__(128, kRerankCtasPerSm) rerank_batched_kernel(const T* __restrict__ q, const T* __restrict__ g_all,
                                                              const int* __restrict__ cand, const float* __restrict__ cand_val,
                                                              float margin, long long B, long long nq_pad, long long ng_pad,
                                                              const int* __restrict__ q_len, const int* __restrict__ g_len, int slots,
@@ -271,78 +292,12 @@ __global__ void __launch_bounds__(128) rerank_batched_kernel(const T* __restrict
   const float* cvrow = cand_val + row * slots;
   reinterpret_cast<float4*>(sq[w])[lane] = ld_row4(q + (TABLE ? qs.start + (row - b * nq_pad) : row) * 128, lane);
   __syncwarp();
-  // A chunk can hold one of the two nearest columns only if its approximate maximum reaches the second largest
-  // chunk maximum minus twice the error bound of the 16-bit-operand dot product (`margin`, same scaled units).
-  float thr;
-  {
-    float m1 = -__int_as_float(0x7f800000), m2 = m1;
-    for (int c = lane; c < slots; c += 32) {
-      const float v = crow[c] >= 0 ? cvrow[c] : -__int_as_float(0x7f800000);
-      if (v > m1) { m2 = m1; m1 = v; } else if (v > m2) { m2 = v; }
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      const float o1 = __shfl_xor_sync(0xffffffffu, m1, o), o2 = __shfl_xor_sync(0xffffffffu, m2, o);
-      const float lo = fminf(m1, o1);
-      m1 = fmaxf(m1, o1);
-      m2 = fmaxf(fmaxf(m2, o2), lo);
-    }
-    thr = m2 - margin;   // -inf when fewer than two chunks exist: everything is re-ranked
-  }
-  const float inf = __int_as_float(0x7f800000);
-  float b1 = inf, b2 = inf;
-  int j1 = 0x7fffffff, j2 = 0x7fffffff;
-  // The warp walks the surviving chunks together: a gallery row is ONE coalesced 512 B read (lane = float4 index) and
-  // the 128-term dot is finished with a butterfly, so every lane ends up with the same (d, index) stream. Per-lane
-  // row reads (one lane per candidate) cost 32 L1 wavefronts per row instead of 4.
-  const float4 qv = reinterpret_cast<const float4*>(sq[w])[lane];
-  auto eval_chunk = [&](long long chunk) {
-    const long long col0 = chunk * kChunk;
-    float part[kChunk];
-#pragma unroll
-    for (int r = 0; r < kChunk; ++r) {
-      const long long col = col0 + r;
-      part[r] = 0.f;
-      if (col < ng) {
-        const float4 gv = ldg_row4(g + col * 128, lane);
-        part[r] = fmaf(qv.x, gv.x, fmaf(qv.y, gv.y, fmaf(qv.z, gv.z, qv.w * gv.w)));
-      }
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-#pragma unroll
-      for (int r = 0; r < kChunk; ++r) part[r] += __shfl_xor_sync(0xffffffffu, part[r], o);
-    }
-    float mine = part[0];   // part[lane & 7] without a local-memory array access
-#pragma unroll
-    for (int r = 1; r < kChunk; ++r) mine = (lane & (kChunk - 1)) == r ? part[r] : mine;
-    mine = sqrtf(fminf(fmaxf(2.0f - 2.0f * mine, 1e-8f), 4.0f));
-#pragma unroll
-    for (int r = 0; r < kChunk; ++r) {
-      const long long col = col0 + r;
-      const float d = __shfl_sync(0xffffffffu, mine, r);
-      if (col >= ng) continue;
-      const int ci = static_cast<int>(col);
-      if (d < b1 || (d == b1 && ci < j1)) {
-        b2 = b1; j2 = j1; b1 = d; j1 = ci;
-      } else if (d < b2 || (d == b2 && ci < j2)) {
-        b2 = d; j2 = ci;
-      }
-    }
-  };
-  for (int c = 0; c < slots; ++c) {
-    const int chunk = crow[c];
-    if (chunk < 0 || cvrow[c] < thr) continue;   // warp-uniform
-    eval_chunk(chunk);
-  }
-  // every lane holds the same top-2 now
-  const float m = b1, s = b2;
-  const int mj = j1, sj = j2;
+  const Top2 t = rerank_row(sq[w], g, ng, crow, cvrow, slots, margin, lane);
   if (lane == 0) {
-    d1[row] = m;
-    i1[row] = mj == 0x7fffffff ? -1 : mj;
-    d2[row] = s;
-    i2[row] = sj == 0x7fffffff ? -1 : sj;
+    d1[row] = t.d1;
+    i1[row] = t.i1 == 0x7fffffff ? -1 : t.i1;
+    d2[row] = t.d2;
+    i2[row] = t.i2 == 0x7fffffff ? -1 : t.i2;
   }
 }
 
@@ -406,25 +361,22 @@ __global__ void mutual_claim_kernel(const int* __restrict__ i1, const float* __r
 // A cell's 32 query rows are staged ONCE in shared memory with coalesced loads (row pitch 132 floats: the per-row reads below
 // are bank-conflict free; per-lane global reads at a 512-byte stride cost 32 L1 wavefronts per instruction and made this
 // kernel slower than a whole second GEMM) and serve every column of the chunk that needs the cell, two columns per sweep.
-// The dot product is summed in the order of rerank_kernel (32 float4 partials, then the xor-butterfly tree), so a distance
+// The dot product is summed in the order of rerank_row (32 float4 partials, then the xor-butterfly tree), so a distance
 // computed here is bit-identical to the one a second (gallery x queries) matching pass would produce.
 constexpr int kVerifyWarps = 1;   // one warp per CTA: a chunk with a weakly claimed column evaluates ~20 cells one after the other (~70 us), so CTAs must be small and many (10 per SM by shared memory) for the hardware to balance them
 constexpr int kVerifyPitch = 132;   // floats per staged query row
 constexpr size_t kVerifySmem = static_cast<size_t>(kVerifyWarps) * (32 * kVerifyPitch * 4 + kChunk * 32 * 16);
 
+// Verification of the claims of column chunk cb of one problem (see above; nothing to do for a chunk past ng): q / nq, g / ng
+// and the claims, cell maxima (row pitch bm_pitch, n_row_blocks of them per chunk), row blocks' minimum d2 and beaten flags of
+// that problem; q_offset shifts its query rows to the rows of the claims. s_q / s_g: the warp's staging tiles.
+// mutual_verify_kernel and mutual_verify_batched_kernel both run this body, so a batched or pair-table flag equals the
+// per-pair one bit for bit.
 template <typename T>
-__global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_kernel(const T* __restrict__ q, long long nq, long long q_offset,
-                                                                         const T* __restrict__ g, long long ng,
-                                                                         const unsigned long long* __restrict__ claim,
-                                                                         const float* __restrict__ block_max,
-                                                                         const float* __restrict__ rb_min_d2, int n_row_blocks,
-                                                                         float margin_scaled, float inv_dot_scale,
-                                                                         unsigned char* __restrict__ beaten) {
-  extern __shared__ __align__(16) uint8_t vsm[];
-  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  float* s_q = reinterpret_cast<float*>(vsm) + static_cast<size_t>(w) * 32 * kVerifyPitch;                       // [32][132]
-  float4* s_g = reinterpret_cast<float4*>(vsm + static_cast<size_t>(kVerifyWarps) * 32 * kVerifyPitch * 4) + w * kChunk * 32;   // [8][32]
-  const long long cb = static_cast<long long>(blockIdx.x) * kVerifyWarps + w;
+__device__ __forceinline__ void verify_chunk(const T* q, long long nq, long long q_offset, const T* g, long long ng,
+                                             const unsigned long long* claim, const float* block_max, long long bm_pitch,
+                                             const float* rb_min_d2, int n_row_blocks, float margin_scaled, float inv_dot_scale, unsigned char* beaten,
+                                             long long cb, float* s_q, float4* s_g, int lane) {
   if (cb * kChunk >= ng) return;
   unsigned long long cl = 0x7FFFFFFFFFFFFFFFull;   // unclaimed
   if (lane < kChunk && cb * kChunk + lane < ng) cl = claim[cb * kChunk + lane];
@@ -446,9 +398,9 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_kernel(const 
   }
   if (!undecided) return;
   __syncwarp();
-  const float* bm_row = block_max + cb * n_row_blocks;
+  const float* bm_row = block_max + cb * bm_pitch;
 
-  // distance of this lane's staged row to column c (arithmetic of rerank_kernel)
+  // distance of this lane's staged row to column c (arithmetic of rerank_row)
   auto row_distance = [&](int c) {
     float p[32];
     const float* qr = s_q + lane * kVerifyPitch;
@@ -517,6 +469,23 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_kernel(const 
     }
   }
   if (lane < kChunk && ((lost >> lane) & 1u)) beaten[cb * kChunk + lane] = 1;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_kernel(const T* __restrict__ q, long long nq, long long q_offset,
+                                                                         const T* __restrict__ g, long long ng,
+                                                                         const unsigned long long* __restrict__ claim,
+                                                                         const float* __restrict__ block_max,
+                                                                         const float* __restrict__ rb_min_d2, int n_row_blocks,
+                                                                         float margin_scaled, float inv_dot_scale,
+                                                                         unsigned char* __restrict__ beaten) {
+  extern __shared__ __align__(16) uint8_t vsm[];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  float* s_q = reinterpret_cast<float*>(vsm) + static_cast<size_t>(w) * 32 * kVerifyPitch;                       // [32][132]
+  float4* s_g = reinterpret_cast<float4*>(vsm + static_cast<size_t>(kVerifyWarps) * 32 * kVerifyPitch * 4) + w * kChunk * 32;   // [8][32]
+  const long long cb = static_cast<long long>(blockIdx.x) * kVerifyWarps + w;
+  verify_chunk(q, nq, q_offset, g, ng, claim, block_max, n_row_blocks, rb_min_d2, n_row_blocks, margin_scaled, inv_dot_scale,
+               beaten, cb, s_q, s_g, lane);
 }
 
 // mutual[i] = the best claimant of my nearest column is me, and nobody beat it
@@ -558,9 +527,8 @@ __global__ void mutual_claim_batched_kernel(const int* __restrict__ i1, const fl
   atomicMin(claim + b * ng + j, (static_cast<unsigned long long>(__float_as_uint(d1[i])) << 32) | static_cast<unsigned int>(r));
 }
 
-// One warp per (pair, 8-column chunk), scanning only the pair's valid row blocks. After the prologue (pair pointers and
-// bounds) this is mutual_verify_kernel's body with q_offset = 0 and a block_max row pitch of ceil(nq_pad / 32), copied rather
-// than shared so that the single-problem kernel compiles to the same instructions as before: keep the two in step.
+// One warp per (pair, 8-column chunk), scanning only the pair's valid row blocks: verify_chunk on the pair's rows, with local
+// query rows (q_offset = 0) and a block_max row pitch of ceil(nq_pad / 32).
 template <bool TABLE, typename T>
 __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kernel(const T* __restrict__ q_all, const T* __restrict__ g_all,
                                                                                  long long B, long long nq_pad, long long ng_pad,
@@ -583,7 +551,7 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kerne
     qs = table_span(pairs, pair, 0, nq_pad, q_rows);
     gs = table_span(pairs, pair, 1, ng_pad, g_rows);
   }
-  const long long nq = TABLE ? qs.len : pair_len(q_len, pair, nq_pad), ng = TABLE ? gs.len : pair_len(g_len, pair, ng_pad), q_offset = 0;
+  const long long nq = TABLE ? qs.len : pair_len(q_len, pair, nq_pad), ng = TABLE ? gs.len : pair_len(g_len, pair, ng_pad);
   const int n_row_blocks = static_cast<int>((nq + 31) / 32);
   const T* q = TABLE ? q_all + qs.start * 128 : q_all + pair * nq_pad * 128;
   const T* g = TABLE ? g_all + gs.start * 128 : g_all + pair * ng_pad * 128;
@@ -591,98 +559,8 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_batched_kerne
   const float* block_max = block_max_all + pair * chunks * bm_pitch;
   const float* rb_min_d2 = rb_min_d2_all + pair * bm_pitch;
   unsigned char* beaten = beaten_all + pair * ng_pad;
-  if (cb * kChunk >= ng) return;
-  unsigned long long cl = 0x7FFFFFFFFFFFFFFFull;   // unclaimed
-  if (lane < kChunk && cb * kChunk + lane < ng) cl = claim[cb * kChunk + lane];
-  float dcl[kChunk], thr[kChunk];
-  unsigned int icl[kChunk];
-  unsigned undecided = 0, lost = 0;
-  const float ninf = -__int_as_float(0x7f800000);
-#pragma unroll
-  for (int c = 0; c < kChunk; ++c) {
-    const unsigned long long cc = __shfl_sync(0xffffffffu, cl, c);
-    dcl[c] = __uint_as_float(static_cast<unsigned int>(cc >> 32));
-    icl[c] = static_cast<unsigned int>(cc & 0xffffffffu);
-    thr[c] = __int_as_float(0x7f800000);
-    if ((cc >> 32) < 0x7F000000ull) {
-      undecided |= 1u << c;
-      thr[c] = (1.0f - 0.5f * dcl[c] * dcl[c]) * inv_dot_scale - margin_scaled;
-      s_g[c * 32 + lane] = ldg_row4(g + (cb * kChunk + c) * 128, lane);
-    }
-  }
-  if (!undecided) return;
-  __syncwarp();
-  const float* bm_row = block_max + cb * bm_pitch;
-
-  // distance of this lane's staged row to column c (arithmetic of rerank_kernel)
-  auto row_distance = [&](int c) {
-    float p[32];
-    const float* qr = s_q + lane * kVerifyPitch;
-#pragma unroll
-    for (int l = 0; l < 32; ++l) {
-      const float4 qv = *reinterpret_cast<const float4*>(qr + 4 * l);
-      const float4 gv = s_g[c * 32 + l];
-      p[l] = fmaf(qv.x, gv.x, fmaf(qv.y, gv.y, fmaf(qv.z, gv.z, qv.w * gv.w)));
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-#pragma unroll
-      for (int l = 0; l < o; ++l) p[l] += p[l + o];
-    }
-    return sqrtf(fminf(fmaxf(2.0f - 2.0f * p[0], 1e-8f), 4.0f));
-  };
-
-  auto evaluate = [&](int rb, float vb, float min_d2) {
-    unsigned need = 0;
-#pragma unroll
-    for (int c = 0; c < kChunk; ++c)
-      if (((undecided >> c) & 1u) && thr[c] <= vb && min_d2 <= dcl[c]) need |= 1u << c;
-    if (!need) return;
-    // stage the cell's 32 rows: one coalesced 512-byte row per iteration
-    const long long k0 = static_cast<long long>(rb) * 32;
-#pragma unroll
-    for (int r0 = 0; r0 < 32; r0 += 8) {   // eight row loads in flight
-      float4 v[8];
-#pragma unroll
-      for (int r = 0; r < 8; ++r) {
-        v[r] = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (k0 + r0 + r < nq) v[r] = ldg_row4(q + (k0 + r0 + r) * 128, lane);
-      }
-#pragma unroll
-      for (int r = 0; r < 8; ++r) *reinterpret_cast<float4*>(s_q + (r0 + r) * kVerifyPitch + 4 * lane) = v[r];
-    }
-    __syncwarp();
-    const long long k = k0 + lane;
-    const bool valid = k < nq;
-    const unsigned int gk = static_cast<unsigned int>(k + q_offset);
-#pragma unroll 1
-    for (int c = 0; c < kChunk; ++c) {
-      if (!((need >> c) & 1u)) continue;   // warp-uniform
-      const float d = row_distance(c);
-      const bool beats = valid && gk != icl[c] && (d < dcl[c] || (d == dcl[c] && gk < icl[c]));
-      if (__any_sync(0xffffffffu, beats)) {
-        undecided &= ~(1u << c);
-        lost |= 1u << c;
-      }
-    }
-    __syncwarp();   // the staging tile is reused by the next cell
-  };
-
-  for (int base = 0; base < n_row_blocks && undecided; base += 32) {
-    const int rb = base + lane;
-    const float v = rb < n_row_blocks ? bm_row[rb] : ninf;
-    const float md2 = rb < n_row_blocks ? rb_min_d2[rb] : __int_as_float(0x7f800000);
-    bool mine = false;
-#pragma unroll
-    for (int c = 0; c < kChunk; ++c) mine |= ((undecided >> c) & 1u) && thr[c] <= v && md2 <= dcl[c];
-    unsigned cand = __ballot_sync(0xffffffffu, mine);
-    while (cand && undecided) {
-      const int b = __ffs(cand) - 1;
-      cand &= cand - 1;
-      evaluate(base + b, __shfl_sync(0xffffffffu, v, b), __shfl_sync(0xffffffffu, md2, b));
-    }
-  }
-  if (lane < kChunk && ((lost >> lane) & 1u)) beaten[cb * kChunk + lane] = 1;
+  verify_chunk(q, nq, 0, g, ng, claim, block_max, bm_pitch, rb_min_d2, n_row_blocks, margin_scaled, inv_dot_scale,
+               beaten, cb, s_q, s_g, lane);
 }
 
 
@@ -1017,13 +895,10 @@ static int run_match(const T* q, const T* g, const void* q16_in, const void* g16
   // The re-rank reads the gallery rows of the shortlisted columns; a caller that gathered the packed gallery first (half the
   // bytes of fp32 rows) passes the event that marks the rows' arrival, so that transfer hides behind the GEMM.
   if (g_ready_event) HN_CUDA(cudaStreamWaitEvent(s, static_cast<cudaEvent_t>(g_ready_event), 0));
-  // |fp16-operand dot - exact dot| <= 2^-10 for rows of norm <= 1 (L2-normalised descriptors, the only input this path
-  // is defined for: FDLNet-master/utils/math_utils.py:15-18 clamps 2 - 2ab to [1e-8, 4]); keep 4x that as the margin.
-  const float margin = 4.0f * (1.0f / 1024.0f) / kDotScale;
   {
     MatchTimer timer(2, s);
     // the CTA-pair kernel keeps two top-kTopC lists per row and segment (one per 64-column half of its tiles)
-    rerank_kernel<<<static_cast<unsigned>((Nq + 3) / 4), 128, 0, s>>>(q, g, cand, cand_val, margin, Nq, Ng,
+    rerank_kernel<<<static_cast<unsigned>((Nq + 3) / 4), 128, 0, s>>>(q, g, cand, cand_val, kRerankMargin, Nq, Ng,
                                                                      dp.segments * kTopC * (use_pair ? 2 : 1), g_offset, d1, d2, i1, i2);
     HN_CUDA(cudaGetLastError());
     count_launch();
@@ -1088,13 +963,11 @@ template <typename T>
 static int launch_verify(const T* q, long long Nq, long long q_offset, const T* g, long long Ng, const unsigned long long* claim,
                          const float* block_max, const float* rb_min_d2, unsigned char* beaten, cudaStream_t s) {
   const long long chunks = (Ng + kChunk - 1) / kChunk;
-  // twice the 2^-10 error bound of the fp16-operand dot product of unit vectors, in the GEMM's scaled units
-  const float margin = 2.0f * (1.0f / 1024.0f) / kDotScale;
   static DeviceOnce attr_once;
   if (attr_once.first_time())
     HN_CUDA(cudaFuncSetAttribute(mutual_verify_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kVerifySmem)));
   mutual_verify_kernel<T><<<static_cast<unsigned>((chunks + kVerifyWarps - 1) / kVerifyWarps), kVerifyWarps * 32, kVerifySmem, s>>>(
-      q, Nq, q_offset, g, Ng, claim, block_max, rb_min_d2, static_cast<int>((Nq + 31) / 32), margin, 1.0f / kDotScale, beaten);
+      q, Nq, q_offset, g, Ng, claim, block_max, rb_min_d2, static_cast<int>((Nq + 31) / 32), kVerifyMargin, 1.0f / kDotScale, beaten);
   HN_CUDA(cudaGetLastError());
   count_launch();
   return HN_OK;
@@ -1261,11 +1134,10 @@ static int run_pairs(const T* q, const uint16_t* q16, const T* g, const uint16_t
     if (TABLE) HN_TRY((launch_dist<2, EPI_SHORTLIST_PAIRS>(dp, grid, 1, s)));
     else HN_TRY((launch_dist<2, EPI_SHORTLIST_BATCHED>(dp, grid, 1, s)));
   }
-  const float margin = 4.0f * (1.0f / 1024.0f) / kDotScale;   // as hn_match_ex
   {
     MatchTimer timer(2, s);
     rerank_batched_kernel<TABLE, T><<<static_cast<unsigned>((rows_q + 3) / 4), 128, 0, s>>>(
-        q, g, w.cand, w.cand_val, margin, B, Nq, Ng, L.q_len, L.g_len, dp.segments * kTopC, d1, d2, i1, i2, L.pairs, L.q_rows, L.g_rows);
+        q, g, w.cand, w.cand_val, kRerankMargin, B, Nq, Ng, L.q_len, L.g_len, dp.segments * kTopC, d1, d2, i1, i2, L.pairs, L.q_rows, L.g_rows);
     HN_CUDA(cudaGetLastError());
     count_launch();
   }
@@ -1278,9 +1150,8 @@ static int run_pairs(const T* q, const uint16_t* q16, const T* g, const uint16_t
     static DeviceOnce attr_once;
     if (attr_once.first_time())
       HN_CUDA(cudaFuncSetAttribute(mutual_verify_batched_kernel<TABLE, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kVerifySmem)));
-    const float vmargin = 2.0f * (1.0f / 1024.0f) / kDotScale;   // as hn_mutual_verify
     mutual_verify_batched_kernel<TABLE, T><<<static_cast<unsigned>((B * chunks + kVerifyWarps - 1) / kVerifyWarps), kVerifyWarps * 32, kVerifySmem, s>>>(
-        q, g, B, Nq, Ng, L.q_len, L.g_len, w.claim, w.block_max, w.rb_min_d2, vmargin, 1.0f / kDotScale, w.beaten, L.pairs, L.q_rows,
+        q, g, B, Nq, Ng, L.q_len, L.g_len, w.claim, w.block_max, w.rb_min_d2, kVerifyMargin, 1.0f / kDotScale, w.beaten, L.pairs, L.q_rows,
         L.g_rows);
     mutual_final_batched_kernel<TABLE><<<static_cast<unsigned>((rows_q + threads - 1) / threads), threads, 0, s>>>(
         i1, B, Nq, Ng, L.q_len, L.g_len, w.claim, w.beaten, mutual, L.pairs, L.q_rows, L.g_rows);
