@@ -1536,8 +1536,9 @@ static int run_nas_ops(hn_handle* h, NasState* st, const char* src, int in_dtype
             uint16_t* dst = st->slot[o.dst];
             const float* wv = st->params + o.w_off;
             const float* bv = st->params + o.b_off;
-            // shared-memory kernel whenever two units of whole maps fit next to the weights (every shape of SEARCH_SPACE2
-            // with expansion 1); wider expansions fall through to the register-strip kernel below
+            // shared-memory kernel whenever one unit of two whole maps fits next to the weights (227 KB): every depthwise
+            // shape of SEARCH_SPACE2 except the 32 x 32 input maps of a layer-0 block wider than 32 channels (e3 / s4 / e6:
+            // 96-192 channels, 388-788 KB), which fall through to the register-strip kernel below
             if (strip && h->env.nas_dw_smem) {
               const size_t map_bytes = static_cast<size_t>(o.hin) * o.hin * o.cin * 2;
               // 5x5 stride 1 is bound by the fp32 pipe + unpack instructions: strips of 8 rows re-use each loaded and

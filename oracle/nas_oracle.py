@@ -88,3 +88,70 @@ def nas_forward(x: torch.Tensor, op_names, sd: dict, return_features: bool = Fal
         y = y.reshape(y.size(0), -1)
         y = y / torch.norm(y, p=2, dim=-1, keepdim=True)                   # model_supernet.py:84
     return (y, feats) if return_features else y
+
+
+def state_dict_f64(sd: dict) -> dict:
+    """The state_dict with every floating tensor in float64 (for nas_forward as a float64 reference)."""
+    return {k: (v.double() if v.dtype.is_floating_point else v) for k, v in sd.items()}
+
+
+OP_STEM, OP_PW, OP_DW, OP_MAXPOOL, OP_SE, OP_HEAD = 0, 1, 2, 3, 4, 5
+
+
+def run_program(x: torch.Tensor, ops, params: torch.Tensor):
+    """Float64 interpreter of exactly what hn_pack_nas receives: the `hn_nas_op` list of
+    SampledDescriptorNet.compile_program() and the flat parameter blob (torch.cat(prog.params)). It knows nothing of the
+    module tree, so it checks every host-side transformation in front of the C ABI (BatchNorm folding, shuffle folding,
+    grouped-to-dense expansion, weight layouts, slot assignment).
+
+    x [B,1,32,32] -> (descriptors [B,128], outs) with outs[i] the NCHW tensor in op i's dst slot after op i ran."""
+    p = params.double()
+    x = x.double()
+    B = x.size(0)
+    slots = [None, None, None]
+    outs = []
+    desc = None
+
+    def take(off, n):
+        assert 0 <= off and off + n <= p.numel(), "parameter range outside the blob"
+        return p[off:off + n]
+
+    with torch.no_grad():
+        for o in ops:
+            if o.kind == OP_STEM:                               # [9][32] taps-major, + shift, ReLU
+                w = take(o.w_off, 9 * o.cout).view(9, o.cout).t().reshape(o.cout, 1, 3, 3)
+                y = F.conv2d(x, w, take(o.b_off, o.cout), padding=1)
+                y = F.relu(y) if o.relu else y
+            elif o.kind == OP_PW:                               # dense [cout][cin] (+ res slot), optional ReLU
+                w = take(o.w_off, o.cout * o.cin).view(o.cout, o.cin, 1, 1)
+                y = F.conv2d(slots[o.src], w, take(o.b_off, o.cout))
+                if o.res >= 0:
+                    y = y + slots[o.res]
+                y = F.relu(y) if o.relu else y
+            elif o.kind == OP_DW:                               # [k*k][C], pad k // 2
+                k = o.kernel
+                w = take(o.w_off, k * k * o.cin).view(k * k, o.cin).t().reshape(o.cin, 1, k, k)
+                y = F.conv2d(slots[o.src], w, take(o.b_off, o.cin), stride=o.stride, padding=k // 2, groups=o.cin)
+                y = F.relu(y) if o.relu else y
+            elif o.kind == OP_MAXPOOL:
+                y = F.max_pool2d(slots[o.src], 3, 2, 1)
+            elif o.kind == OP_SE:                               # fc1 [mid][C], fc2 [C][mid], in place
+                v = slots[o.src]
+                s = v.mean(dim=(2, 3))
+                s = F.relu(s @ take(o.w_off, o.mid * o.cin).view(o.mid, o.cin).t() + take(o.b_off, o.mid))
+                s = torch.sigmoid(s @ take(o.w2_off, o.cin * o.mid).view(o.cin, o.mid).t() + take(o.b2_off, o.cin))
+                y = v * s[:, :, None, None]
+            elif o.kind == OP_HEAD:                             # [128][(y*k + x)*C + c], + shift, L2 norm
+                v = slots[o.src]
+                assert v.shape[1:] == (o.cin, o.kernel, o.kernel)
+                w = take(o.w_off, o.cout * o.kernel * o.kernel * o.cin).view(o.cout, -1)
+                y = v.permute(0, 2, 3, 1).reshape(B, -1) @ w.t() + take(o.b_off, o.cout)
+                desc = y / torch.norm(y, p=2, dim=-1, keepdim=True)
+                outs.append(desc)
+                continue
+            else:
+                raise ValueError(f"unknown op kind {o.kind}")
+            assert y.shape[1:] == (o.cout, o.hout, o.hout), (o.kind, tuple(y.shape))
+            slots[o.dst] = y
+            outs.append(y)
+    return desc, outs
