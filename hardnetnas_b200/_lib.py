@@ -11,7 +11,7 @@ from pathlib import Path
 _HERE = Path(__file__).resolve().parent
 LIB_PATH = _HERE / "libhardnet_b200.so"
 
-HN_F32, HN_F16, HN_BF16, HN_U8 = 0, 1, 2, 3
+HN_F32, HN_F16, HN_BF16, HN_U8, HN_F8E4M3 = 0, 1, 2, 3, 5
 HN_FORM_HARDNET, HN_FORM_FDL = 0, 1
 HN_FLAG_LOSS_MASK, HN_FLAG_SWAP, HN_FLAG_NEI_MASK = 1, 2, 4
 

@@ -38,13 +38,14 @@ def _require_cuda_f32(name: str, t: torch.Tensor) -> torch.Tensor:
     return _require_cuda_desc(name, t).float().contiguous()
 
 
-_ROW_DTYPES = {torch.float16: _lib.HN_F16, torch.bfloat16: _lib.HN_BF16}
+_ROW_DTYPES = {torch.float16: _lib.HN_F16, torch.bfloat16: _lib.HN_BF16, torch.float8_e4m3fn: _lib.HN_F8E4M3}
 
 
 def _desc_rows(q: torch.Tensor, g: torch.Tensor | None = None):
-    """(q, g, desc_dtype) for the *_typed matching entry points: fp16 and bf16 rows are read as they are (made contiguous)
-    when both sides share the dtype, so no fp32 copy is made; anything else (fp32, fp64, mixed dtypes) is converted to fp32.
-    The results are the same either way (include/hardnet_b200.h). g = None: a single set."""
+    """(q, g, desc_dtype) for the *_typed matching entry points: fp16, bf16 and fp8 e4m3 (torch.float8_e4m3fn) rows are read
+    as they are (made contiguous) when both sides share the dtype, so no fp32 copy is made; anything else (fp32, fp64,
+    float8_e5m2, mixed dtypes) is converted to fp32. The results are the same either way (include/hardnet_b200.h).
+    g = None: a single set."""
     code = _ROW_DTYPES.get(q.dtype) if g is None or g.dtype == q.dtype else None
     if code is None:
         return q.float().contiguous(), (None if g is None else g.float().contiguous()), _lib.HN_F32
@@ -104,15 +105,22 @@ def loss_hardnet(anchor: torch.Tensor, positive: torch.Tensor, margin: float, an
     return out
 
 
+def _packed_dtype(desc_dtype: int) -> torch.dtype:
+    """dtype of the packed operand rows of a matching call on rows of desc_dtype: e4m3 for e4m3 rows, fp16 otherwise."""
+    return torch.float8_e4m3fn if desc_dtype == _lib.HN_F8E4M3 else torch.float16
+
+
 def pack_descriptors(x: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
-    """[n,128] unit rows (fp32, or fp16 / bf16 read as they are) -> the fp16 operand rows of the matching GEMM (x * 2^8), see
-    hn_pack_descriptors. `out`: optional destination (e.g. a symmetric-memory exchange buffer)."""
+    """[n,128] unit rows (fp32, or fp16 / bf16 / fp8 e4m3 read as they are) -> the operand rows of the matching GEMM (x * 2^8),
+    see hn_pack_descriptors_typed: fp16 rows, or e4m3 rows for e4m3 input (exact: |x| <= 1). `out`: optional destination
+    (e.g. a symmetric-memory exchange buffer) of that dtype."""
     lib = _lib.load()
     x, _, dt = _desc_rows(_require_cuda_desc("pack_descriptors", x))
+    pdt = _packed_dtype(dt)
     if out is None:
-        out = torch.empty((x.size(0), 128), dtype=torch.float16, device=x.device)
-    elif not (out.is_cuda and out.dtype == torch.float16 and tuple(out.shape) == (x.size(0), 128) and out.is_contiguous()):
-        raise ValueError("pack_descriptors: out must be a contiguous CUDA fp16 [n,128] tensor")
+        out = torch.empty((x.size(0), 128), dtype=pdt, device=x.device)
+    elif not (out.is_cuda and out.dtype == pdt and tuple(out.shape) == (x.size(0), 128) and out.is_contiguous()):
+        raise ValueError(f"pack_descriptors: out must be a contiguous CUDA {pdt} [n,128] tensor")
     if x.size(0):
         with torch.cuda.device(x.device):
             _lib.check(lib.hn_pack_descriptors_typed(_ptr(x), dt, x.size(0), _ptr(out), _stream_ptr()), "hn_pack_descriptors_typed")
@@ -135,13 +143,14 @@ def match_top2(q: torch.Tensor, g: torch.Tensor, g_offset: int = 0, q16: torch.T
     q16 / g16: operands already packed by `pack_descriptors` (skips the packing kernels); g_ready_event: the exact re-rank
     (the only reader of the fp32 gallery `g`) waits for it, so `g` may still be arriving while the GEMM runs.
     block_max: optional fp32 tensor of `block_max_elems(nq, ng)` elements that receives the GEMM's per-cell maxima (column side
-    of mutual NN, see hn_match_mutual). fp16 / bf16 rows of one dtype are read as they are (hn_match_typed)."""
+    of mutual NN, see hn_match_mutual). fp16 / bf16 / fp8 e4m3 rows of one dtype are read as they are (hn_match_typed); packed
+    operands are then of the dtype pack_descriptors gives for them (e4m3 for e4m3 rows, fp16 otherwise)."""
     lib = _lib.load()
     q, g, dt = _desc_rows(_require_cuda_desc("match", q), _require_cuda_desc("match", g))
     nq, ng = q.size(0), g.size(0)
     for t, n in ((q16, nq), (g16, ng)):
-        if t is not None and not (t.is_cuda and t.dtype == torch.float16 and tuple(t.shape) == (n, 128) and t.is_contiguous()):
-            raise ValueError("match: packed operands must be contiguous CUDA fp16 [n,128] tensors from pack_descriptors")
+        if t is not None:
+            _packed("match", t, n, dt)
     dev = q.device
     with torch.cuda.device(dev):
         ws = _workspace(dev, lib.hn_dist_workspace_bytes(nq, ng, 0))
@@ -223,10 +232,13 @@ def match_batched(q: torch.Tensor, g: torch.Tensor, q_len: torch.Tensor | None =
     return (d1, d2, i1, i2, mu) if mutual else (d1, d2, i1, i2)
 
 
-def _packed(name: str, t: torch.Tensor, n: int) -> torch.Tensor:
-    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.float16 and tuple(t.shape) == (n, 128)
-            and t.is_contiguous()):
-        raise ValueError(f"{name}: packed operands must be contiguous CUDA fp16 [n,128] tensors from pack_descriptors")
+def _packed(name: str, t: torch.Tensor, n: int, desc_dtype: int) -> torch.Tensor:
+    """Checks packed operand rows against the rows they were made from: the C ABI receives a bare pointer and cannot tell an
+    fp16 operand from an e4m3 one."""
+    pdt = _packed_dtype(desc_dtype)
+    if not (isinstance(t, torch.Tensor) and t.dtype == pdt and t.is_cuda and tuple(t.shape) == (n, 128) and t.is_contiguous()):
+        raise ValueError(f"{name}: packed operands must be contiguous CUDA {pdt} [n,128] tensors from pack_descriptors "
+                         f"(e4m3 for e4m3 rows, fp16 otherwise)")
     return t
 
 
@@ -235,7 +247,7 @@ def match_pairs(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, max_q: in
     """(d1, d2, i1, i2[, mutual]), each [P, max_q]: hn_match_pairs over the concatenated sets q [Nq_rows, 128] and
     g [Ng_rows, 128]. pairs: integer [P, 4] table of (q_start, q_len, g_start, g_len), copied to q's device as int32 (a table
     already there keeps the call free of host synchronisation). q16 / g16: the sets' rows packed by `pack_descriptors`; a set
-    whose packed rows are not given is packed here, once when g is q. Indices are local to the pair's gallery range; rows past
+    whose packed rows are not given is packed here (per row dtype, see pack_descriptors), once when g is q. Indices are local to the pair's gallery range; rows past
     q_len get d = +inf, i = -1 (and mutual = False). Rows as in match_top2 (hn_match_pairs_typed)."""
     lib = _lib.load()
     same = g is q
@@ -255,7 +267,7 @@ def match_pairs(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, max_q: in
         q16 = g16 if same and g16 is not None else pack_descriptors(q)
     if g16 is None:
         g16 = q16 if same else pack_descriptors(g)
-    q16, g16 = _packed("match_pairs", q16, nq), _packed("match_pairs", g16, ng)
+    q16, g16 = _packed("match_pairs", q16, nq, dt), _packed("match_pairs", g16, ng, dt)
     with torch.cuda.device(dev):
         ws = _workspace(dev, max(lib.hn_match_pairs_workspace_bytes(b, max_q, max_g, int(mutual)), 1))
         d1 = torch.empty((b, max_q), dtype=torch.float32, device=dev)

@@ -5,6 +5,7 @@
 #include <cuda.h>          // CUtensorMap (types only; the driver entry point is resolved at run time)
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
+#include <cuda_fp8.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -27,6 +28,15 @@ __device__ __forceinline__ bool elect_one() {
       "selp.u32 %0, 1, 0, p;\n\t}"
       : "=r"(pred));
   return pred != 0;
+}
+
+// {a, b, c, d} -> four e4m3 bytes (a lowest), round to nearest even like torch's .to(torch.float8_e4m3fn), two
+// F2FP.SATFINITE.E4M3 instructions. Unit descriptors never reach the saturation bound (448).
+__device__ __forceinline__ uint32_t pack_e4m3x4(float a, float b, float c, float d) {
+  uint16_t lo, hi;
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(lo) : "f"(b), "f"(a));
+  asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(hi) : "f"(d), "f"(c));
+  return static_cast<uint32_t>(lo) | (static_cast<uint32_t>(hi) << 16);
 }
 
 __device__ __forceinline__ uint64_t globaltimer_ns() {
@@ -179,6 +189,20 @@ __device__ __forceinline__ void umma_f16_w(uint32_t d_tmem, uint32_t a_lo, uint3
       "mov.b64 da, {%1, %2};\n\t"
       "mov.b64 db, {%3, %4};\n\t"
       "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n\t}"
+      ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// kind::f8f6f4 twin of umma_f16_w (UTCQMMA): one MMA takes K = 32 one-byte elements, i.e. the same 32 bytes of a K-major row
+// as a K = 16 fp16 MMA, so the descriptors advance exactly as in the fp16 loops. The A / B format fields of the instruction
+// descriptor are 0 for E4M3, so make_idesc_f16(m, n, 0) is also the E4M3 x E4M3 -> fp32 descriptor.
+__device__ __forceinline__ void umma_f8_w(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
+                                          uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
+      "setp.ne.b32 p, %6, 0;\n\t"
+      "mov.b64 da, {%1, %2};\n\t"
+      "mov.b64 db, {%3, %4};\n\t"
+      "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], da, db, %5, p;\n\t}"
       ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
       : "memory");
 }

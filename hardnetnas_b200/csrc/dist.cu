@@ -1,6 +1,7 @@
 // C ABI for the distance / hardest-in-batch / matching path: operand packing, the fused tcgen05
 // distance kernels (tc_dist.cuh), fp32 re-ranking of shortlisted candidates and the small finalisers.
 #include <algorithm>
+#include <type_traits>
 #include <vector>
 
 #include "host_common.h"
@@ -14,6 +15,17 @@ constexpr float kDotScale = 1.0f / (kOperandScale * kOperandScale);
 // |fp16-operand dot - exact dot| <= 2^-10 for rows of norm <= 1 (L2-normalised descriptors, the only input matching is defined
 // for: FDLNet-master/utils/math_utils.py:15-18 clamps 2 - 2ab to [1e-8, 4]). In the GEMM's scaled units, the re-rank keeps 4x
 // that bound as the margin of its candidate threshold and the mutual verification 2x as the margin of its cell test.
+// e4m3 rows (packed as exact e4m3 x * 2^8, kind::f8f6f4 GEMM): every product is exact, so the dot error is the tensor core's
+// accumulation alone, which PTX does not specify. The bound relied on, and its assumption: each MMA (K = 32) adds its 32
+// products to the fp32 accumulator with an error of at most 2^-18 times the largest magnitude involved (a product or the
+// running sum) per term, i.e. it keeps at least 18 bits below the leading bit of the aligned sum (true fp32 accumulation keeps
+// 23; with scaled operands every partial sum is a multiple of 2^-2 below 2^17, so fp32 accumulation is exact). Rows rounded to
+// e4m3 have norm <= (1 + 2^-4) + sqrt(128) * 2^-10 < 1.074 (relative rounding 2^-4 plus the subnormal spacing), so every
+// product and partial sum is <= 1.074^2 < 1.16 and the error of a 128-term dot is <= 4 MMAs * 33 terms * 2^-18 * 1.16 < 5.9e-4
+// < 2^-10. The fp16 bound holds, and the same margins keep the same factor of two. tests/test_matching_fp8_gpu.py checks the
+// bound (kF8DotBound below, in unscaled units) against float64 cell maxima of adversarial e4m3 rows.
+constexpr float kF8DotBound = 5.9e-4f;
+static_assert(kF8DotBound <= 1.0f / 1024.0f, "the fp8 GEMM's error must stay within the bound the margins are made of");
 constexpr float kRerankMargin = 4.0f * (1.0f / 1024.0f) / kDotScale;
 constexpr float kVerifyMargin = 2.0f * (1.0f / 1024.0f) / kDotScale;
 
@@ -31,7 +43,20 @@ __device__ __forceinline__ float4 row4_from_bits(uint2 v, __nv_bfloat16) {
   const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v.y));
   return make_float4(a.x, a.y, b.x, b.y);
 }
+// e4m3 rows (HN_F8E4M3): one 4-byte load per lane, four exact e4m3 -> fp16 -> fp32 conversions.
+__device__ __forceinline__ float4 row4_from_bits(uint32_t v, __nv_fp8_e4m3) {
+  const __half2_raw a = __nv_cvt_fp8x2_to_halfraw2(static_cast<__nv_fp8x2_storage_t>(v & 0xffffu), __NV_E4M3);
+  const __half2_raw b = __nv_cvt_fp8x2_to_halfraw2(static_cast<__nv_fp8x2_storage_t>(v >> 16), __NV_E4M3);
+  const float2 fa = __half22float2(__half2(a)), fb = __half22float2(__half2(b));
+  return make_float4(fa.x, fa.y, fb.x, fb.y);
+}
 __device__ __forceinline__ float4 ld_row4(const float* row, int lane) { return reinterpret_cast<const float4*>(row)[lane]; }
+__device__ __forceinline__ float4 ld_row4(const __nv_fp8_e4m3* row, int lane) {
+  return row4_from_bits(reinterpret_cast<const uint32_t*>(row)[lane], __nv_fp8_e4m3{});
+}
+__device__ __forceinline__ float4 ldg_row4(const __nv_fp8_e4m3* row, int lane) {
+  return row4_from_bits(__ldg(reinterpret_cast<const unsigned int*>(row) + lane), __nv_fp8_e4m3{});
+}
 __device__ __forceinline__ float4 ldg_row4(const float* row, int lane) { return __ldg(reinterpret_cast<const float4*>(row) + lane); }
 template <typename T>
 __device__ __forceinline__ float4 ld_row4(const T* row, int lane) { return row4_from_bits(reinterpret_cast<const uint2*>(row)[lane], T{}); }
@@ -72,6 +97,15 @@ __global__ void pack_desc_kernel(const T* __restrict__ x, long long n, uint16_t*
     *reinterpret_cast<uint2*>(dst + 128) = order == 0 ? H : L;
     *reinterpret_cast<uint2*>(dst + 256) = order == 0 ? L : H;
   }
+}
+
+// [n,128] e4m3 rows -> e4m3 operand rows x * 2^8 (exact for |x| <= 1, see the margin comment), one 4-byte word per lane.
+__global__ void pack_desc_f8_kernel(const __nv_fp8_e4m3* __restrict__ x, long long n, uint32_t* __restrict__ out) {
+  const long long row = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (row >= n) return;
+  const float4 v = ld_row4(x + row * 128, lane);
+  out[row * 32 + lane] = pack_e4m3x4(v.x * kOperandScale, v.y * kOperandScale, v.z * kOperandScale, v.w * kOperandScale);
 }
 
 // Push all-gather over NVSwitch multicast: a rank packs its shard and writes BOTH forms (fp16 operand rows for the GEMM, fp32
@@ -233,7 +267,7 @@ __device__ __forceinline__ Top2 rerank_row(const float* sqw, const T* g, long lo
 }
 
 // Re-rank of hn_match: query row `row` of q against g; optional outputs, indices shifted by g_offset.
-// T: fp32, fp16 or bf16 rows (ld_row4 / ldg_row4).
+// T: fp32, fp16, bf16 or e4m3 rows (ld_row4 / ldg_row4).
 template <typename T>
 __global__ void __launch_bounds__(128, kRerankCtasPerSm) rerank_kernel(const T* __restrict__ q, const T* __restrict__ g,
                                                      const int* __restrict__ cand, const float* __restrict__ cand_val,
@@ -601,10 +635,17 @@ static int make_desc_map(CUtensorMap* tm, const uint16_t* base, long long rows, 
   const uint32_t box[2] = {64, static_cast<uint32_t>(box_rows)};
   return make_tmap_16bit(tm, base, 2, dims, str, box, 128);
 }
+// e4m3 twin: [rows, 128] operand rows of 128 bytes, box {128, box_rows} = one 128B-swizzle atom per row
+static int make_desc_map_f8(CUtensorMap* tm, const uint8_t* base, long long rows, int box_rows = kDistTile) {
+  const uint64_t dims[2] = {128, static_cast<uint64_t>(rows)};
+  const uint64_t str[1] = {128};
+  const uint32_t box[2] = {128, static_cast<uint32_t>(box_rows)};
+  return make_tmap_8bit(tm, base, 2, dims, str, box, 128);
+}
 
-template <int MB, int EPI>
+template <int MB, int EPI, bool F8 = false>
 static int launch_dist(const DistParams& p, int grid_x, int grid_y, cudaStream_t s) {
-  auto kern = dist_kernel<MB, EPI>;
+  auto kern = dist_kernel<MB, EPI, F8>;
   const size_t smem = dist_smem_bytes<MB>(p.k_blocks);
   // the size depends on k_blocks (MB = 1: up to 6 for the 3-way split, MB = 2: always 2): raise the limit once per device
   static DeviceOnce attr_once;
@@ -659,22 +700,37 @@ static int pick_segments(long long rows, int rows_per_block, long long cols, int
   return best;
 }
 
-// desc_dtype of the matching entry points -> the element type of the row-reading kernels: f(T{}) with T = float, __half or
-// __nv_bfloat16. check_rows has rejected every other value before.
+// desc_dtype of the matching entry points -> the element type of the row-reading kernels: f(T{}) with T = float, __half,
+// __nv_bfloat16 or __nv_fp8_e4m3. check_rows has rejected every other value before.
 template <typename F>
 static int with_rows(int desc_dtype, F&& f) {
   if (desc_dtype == HN_F16) return f(__half{});
   if (desc_dtype == HN_BF16) return f(__nv_bfloat16{});
+  if (desc_dtype == HN_F8E4M3) return f(__nv_fp8_e4m3{});
   return f(float{});
 }
+// Rows of type T are matched on e4m3 operands by the fp8 GEMM (e4m3 rows) or on fp16 operands (every other row type).
+template <typename T>
+constexpr bool kF8Rows = std::is_same<T, __nv_fp8_e4m3>::value;
 
-// Descriptor rows of a matching call: fp32, fp16 or bf16 (the same for both sides); 16-bit rows are read 8 bytes per lane.
+// Descriptor rows of a matching call: fp32, fp16, bf16 or e4m3 (the same for both sides); 16-bit rows are read 8 bytes per
+// lane, e4m3 rows 4 bytes.
 static int check_rows(const char* fn, int desc_dtype, const void* a, const void* b) {
-  HN_REQUIRE(desc_dtype == HN_F32 || desc_dtype == HN_F16 || desc_dtype == HN_BF16,
-             "%s: desc_dtype must be HN_F32, HN_F16 or HN_BF16 (got %d)", fn, desc_dtype);
-  HN_REQUIRE(desc_dtype == HN_F32 || ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b)) & 7) == 0,
-             "%s: 16-bit descriptor rows must be 8-byte aligned", fn);
+  HN_REQUIRE(desc_dtype == HN_F32 || desc_dtype == HN_F16 || desc_dtype == HN_BF16 || desc_dtype == HN_F8E4M3,
+             "%s: desc_dtype must be HN_F32, HN_F16 or HN_BF16, or HN_F8E4M3 (got %d)", fn, desc_dtype);
+  const uintptr_t bits = reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b);
+  HN_REQUIRE(desc_dtype != HN_F16 && desc_dtype != HN_BF16 || (bits & 7) == 0, "%s: 16-bit descriptor rows must be 8-byte aligned", fn);
+  HN_REQUIRE(desc_dtype != HN_F8E4M3 || (bits & 3) == 0, "%s: e4m3 descriptor rows must be 4-byte aligned", fn);
   return HN_OK;
+}
+
+// n rows of x -> their packed operand rows (fp16 [n,128], or e4m3 [n,128] for e4m3 rows). order: see pack_desc_kernel.
+template <typename T>
+static void launch_pack(const T* x, long long n, void* out, int order, cudaStream_t s) {
+  const int threads = 256;
+  const unsigned blocks = static_cast<unsigned>((n * 32 + threads - 1) / threads);
+  if constexpr (kF8Rows<T>) pack_desc_f8_kernel<<<blocks, threads, 0, s>>>(x, n, static_cast<uint32_t*>(out));
+  else pack_desc_kernel<<<blocks, threads, 0, s>>>(x, n, static_cast<uint16_t*>(out), 0, order, nullptr);
 }
 
 // Shared body of hn_dist_min / hn_loss_hardnet. Leaves packed minima and pos in the workspace.
@@ -803,11 +859,9 @@ static int pack_entry(const char* fn, const void* x, int desc_dtype, long long n
   HN_TRY(check_rows(fn, desc_dtype, x, x));
   HN_REQUIRE(n >= 1 && n < (1LL << 31), "%s: n out of range (%lld)", fn, n);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const int threads = 256;
   return with_rows(desc_dtype, [&](auto t) -> int {
     using T = decltype(t);
-    pack_desc_kernel<<<static_cast<unsigned>((n * 32 + threads - 1) / threads), threads, 0, s>>>(static_cast<const T*>(x), n,
-                                                                                                 static_cast<uint16_t*>(out16), 0, 0, nullptr);
+    launch_pack(static_cast<const T*>(x), n, out16, 0, s);
     HN_CUDA(cudaGetLastError());
     count_launch();
     return HN_OK;
@@ -842,18 +896,19 @@ static int run_match(const T* q, const T* g, const void* q16_in, const void* g16
                      cudaStream_t s) {
   int sm = 0;
   HN_TRY(device_sm_count(&sm));
+  constexpr bool F8 = kF8Rows<T>;
   char* b = static_cast<char*>(workspace);
-  uint16_t* q16 = reinterpret_cast<uint16_t*>(b);
-  uint16_t* g16 = reinterpret_cast<uint16_t*>(b + align256(static_cast<size_t>(Nq) * 256));
+  // packed operand slots of 256 bytes per row (fp16); e4m3 operands use the first half of each
+  void* q16 = b;
+  void* g16 = b + align256(static_cast<size_t>(Nq) * 256);
   int* cand = reinterpret_cast<int*>(b + align256(static_cast<size_t>(Nq) * 256) + align256(static_cast<size_t>(Ng) * 256));
   float* cand_val = reinterpret_cast<float*>(reinterpret_cast<char*>(cand) + align256(static_cast<size_t>(Nq) * 32 * kTopC * 4));
-  const int threads = 256;
   {
     MatchTimer timer(0, s);
-    if (q16_in) q16 = const_cast<uint16_t*>(static_cast<const uint16_t*>(q16_in));
-    else pack_desc_kernel<<<static_cast<unsigned>((Nq * 32 + threads - 1) / threads), threads, 0, s>>>(q, Nq, q16, 0, 0, nullptr);
-    if (g16_in) g16 = const_cast<uint16_t*>(static_cast<const uint16_t*>(g16_in));
-    else pack_desc_kernel<<<static_cast<unsigned>((Ng * 32 + threads - 1) / threads), threads, 0, s>>>(g, Ng, g16, 0, 1, nullptr);
+    if (q16_in) q16 = const_cast<void*>(q16_in);
+    else launch_pack(q, Nq, q16, 0, s);
+    if (g16_in) g16 = const_cast<void*>(g16_in);
+    else launch_pack(g, Ng, g16, 1, s);
     HN_CUDA(cudaGetLastError());
     count_launch((q16_in ? 0 : 1) + (g16_in ? 0 : 1));
   }
@@ -862,15 +917,20 @@ static int run_match(const T* q, const T* g, const void* q16_in, const void* g16
   // CTA pairs (tc_dist_pair.cuh) once the problem is large enough to fill the machine with 512-row query blocks
   const int pair_mode = match_kernel_mode();
   const bool use_pair = pair_mode >= 0 ? pair_mode != 0 : (Nq >= 8192 && Ng >= 1024);
-  HN_TRY(make_desc_map(&dp.side[0].tmA, q16, Nq, 128));
-  HN_TRY(make_desc_map(&dp.side[0].tmB, g16, Ng, 128, use_pair ? 64 : kDistTile));
+  if (F8) {
+    HN_TRY(make_desc_map_f8(&dp.side[0].tmA, static_cast<const uint8_t*>(q16), Nq));
+    HN_TRY(make_desc_map_f8(&dp.side[0].tmB, static_cast<const uint8_t*>(g16), Ng, use_pair ? 64 : kDistTile));
+  } else {
+    HN_TRY(make_desc_map(&dp.side[0].tmA, static_cast<const uint16_t*>(q16), Nq, 128));
+    HN_TRY(make_desc_map(&dp.side[0].tmB, static_cast<const uint16_t*>(g16), Ng, 128, use_pair ? 64 : kDistTile));
+  }
   dp.side[0].cand = cand;
   dp.side[0].cand_val = cand_val;
   dp.side[0].block_max = block_max;
   dp.side[0].n_row_blocks = static_cast<int>((Nq + 31) / 32);
   dp.side[0].Na = Nq;
   dp.side[0].Nb = Ng;
-  dp.k_blocks = 2;
+  dp.k_blocks = F8 ? 1 : 2;
   dp.form = HN_FORM_FDL;
   dp.dot_scale = kDotScale;
   {
@@ -881,15 +941,15 @@ static int run_match(const T* q, const T* g, const void* q16_in, const void* g16
       const long long items = ((Nq + 4 * kDistTile - 1) / (4 * kDistTile)) * dp.segments;
       static DeviceOnce attr_once;
       if (attr_once.first_time()) {
-        HN_CUDA(cudaFuncSetAttribute(match_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kMpSmem)));
+        HN_CUDA(cudaFuncSetAttribute(match_pair_kernel<F8>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(mp_smem_bytes<F8>())));
       }
-      match_pair_kernel<<<2 * static_cast<int>(std::min<long long>(items, pairs)), kMpThreads, kMpSmem, s>>>(dp);
+      match_pair_kernel<F8><<<2 * static_cast<int>(std::min<long long>(items, pairs)), kMpThreads, mp_smem_bytes<F8>(), s>>>(dp);
       HN_CUDA(cudaGetLastError());
       count_launch();
     } else {
       dp.segments = pick_segments(Nq, 2 * kDistTile, Ng, sm, 16);
       const long long items = ((Nq + 2 * kDistTile - 1) / (2 * kDistTile)) * dp.segments;
-      HN_TRY((launch_dist<2, EPI_SHORTLIST>(dp, static_cast<int>(std::min<long long>(items, sm)), 1, s)));
+      HN_TRY((launch_dist<2, EPI_SHORTLIST, F8>(dp, static_cast<int>(std::min<long long>(items, sm)), 1, s)));
     }
   }
   // The re-rank reads the gallery rows of the shortlisted columns; a caller that gathered the packed gallery first (half the
@@ -1037,7 +1097,7 @@ extern "C" int hn_match_mutual_typed(const void* q, const void* g, int desc_dtyp
 // (hn_match_pairs)
 // ------------------------------------------------------------------------------------------------------------
 struct BatchedWs {
-  uint16_t *q16, *g16;       // hn_match_batched only: its packed operands
+  uint16_t *q16, *g16;       // hn_match_batched only: its packed operands (fp16; e4m3 rows use the first half of each slot)
   int* cand;
   float* cand_val;
   float* block_max;          // mutual only
@@ -1074,12 +1134,14 @@ static BatchedWs carve_batched(void* ws, long long B, long long Nq, long long Ng
   return w;
 }
 
-// {K = 128, N, B} 16-bit operand rows, box {64, 128, 1}: a box never reaches into the next pair, TMA zero-fills past N
-static int make_batched_desc_map(CUtensorMap* tm, const uint16_t* base, long long rows, long long B) {
+// {K = 128, N, B} 16-bit operand rows, box {64, 128, 1}: a box never reaches into the next pair, TMA zero-fills past N.
+// F8: e4m3 operand rows, box {128, 128, 1}.
+static int make_batched_desc_map(CUtensorMap* tm, const void* base, long long rows, long long B, bool f8) {
+  const uint64_t esz = f8 ? 1 : 2;
   const uint64_t dims[3] = {128, static_cast<uint64_t>(rows), static_cast<uint64_t>(B)};
-  const uint64_t str[2] = {128 * 2, static_cast<uint64_t>(rows) * 128 * 2};
-  const uint32_t box[3] = {64, static_cast<uint32_t>(kDistTile), 1};
-  return make_tmap_16bit(tm, base, 3, dims, str, box, 128);
+  const uint64_t str[2] = {128 * esz, static_cast<uint64_t>(rows) * 128 * esz};
+  const uint32_t box[3] = {f8 ? 128u : 64u, static_cast<uint32_t>(kDistTile), 1};
+  return f8 ? make_tmap_8bit(tm, base, 3, dims, str, box, 128) : make_tmap_16bit(tm, base, 3, dims, str, box, 128);
 }
 
 // Where the pairs of a batched call live. With `pairs` (hn_match_pairs): row ranges [B][4] = (q_start, q_len, g_start, g_len)
@@ -1095,20 +1157,24 @@ struct PairLayout {
 // The launch sequence of hn_match_pairs (TABLE) and hn_match_batched: GEMM + shortlist, re-rank, and with `mutual` the column
 // side. q16 / g16 are the packed rows of q / g.
 template <bool TABLE, typename T>
-static int run_pairs(const T* q, const uint16_t* q16, const T* g, const uint16_t* g16, const PairLayout& L, float* d1,
+static int run_pairs(const T* q, const void* q16, const T* g, const void* g16, const PairLayout& L, float* d1,
                      float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, const BatchedWs& w, cudaStream_t s) {
+  constexpr bool F8 = kF8Rows<T>;
   int sm = 0;
   HN_TRY(device_sm_count(&sm));
   const long long B = L.B, Nq = L.max_q, Ng = L.max_g, rows_q = B * Nq, rows_g = B * Ng;
   const int threads = 256;
   DistParams dp;
   memset(&dp, 0, sizeof(dp));
-  if (TABLE) {
-    HN_TRY(make_desc_map(&dp.side[0].tmA, q16, L.q_rows, 128));
-    HN_TRY(make_desc_map(&dp.side[0].tmB, g16, L.g_rows, 128));
+  if (TABLE && F8) {
+    HN_TRY(make_desc_map_f8(&dp.side[0].tmA, static_cast<const uint8_t*>(q16), L.q_rows));
+    HN_TRY(make_desc_map_f8(&dp.side[0].tmB, static_cast<const uint8_t*>(g16), L.g_rows));
+  } else if (TABLE) {
+    HN_TRY(make_desc_map(&dp.side[0].tmA, static_cast<const uint16_t*>(q16), L.q_rows, 128));
+    HN_TRY(make_desc_map(&dp.side[0].tmB, static_cast<const uint16_t*>(g16), L.g_rows, 128));
   } else {
-    HN_TRY(make_batched_desc_map(&dp.side[0].tmA, q16, Nq, B));
-    HN_TRY(make_batched_desc_map(&dp.side[0].tmB, g16, Ng, B));
+    HN_TRY(make_batched_desc_map(&dp.side[0].tmA, q16, Nq, B, F8));
+    HN_TRY(make_batched_desc_map(&dp.side[0].tmB, g16, Ng, B, F8));
   }
   dp.side[0].cand = w.cand;
   dp.side[0].cand_val = w.cand_val;
@@ -1116,7 +1182,7 @@ static int run_pairs(const T* q, const uint16_t* q16, const T* g, const uint16_t
   dp.side[0].n_row_blocks = static_cast<int>((Nq + 31) / 32);
   dp.side[0].Na = Nq;
   dp.side[0].Nb = Ng;
-  dp.k_blocks = 2;
+  dp.k_blocks = F8 ? 1 : 2;
   dp.form = HN_FORM_FDL;
   dp.dot_scale = kDotScale;
   dp.q_len = L.q_len;
@@ -1131,8 +1197,8 @@ static int run_pairs(const T* q, const uint16_t* q16, const T* g, const uint16_t
     const long long m_blocks = (Nq + 2 * kDistTile - 1) / (2 * kDistTile);
     dp.segments = pick_segments(B * m_blocks * 2 * kDistTile, 2 * kDistTile, Ng, sm, static_cast<int>(batched_max_segments(Ng)));
     const int grid = static_cast<int>(std::min<long long>(B * m_blocks * dp.segments, sm));
-    if (TABLE) HN_TRY((launch_dist<2, EPI_SHORTLIST_PAIRS>(dp, grid, 1, s)));
-    else HN_TRY((launch_dist<2, EPI_SHORTLIST_BATCHED>(dp, grid, 1, s)));
+    if (TABLE) HN_TRY((launch_dist<2, EPI_SHORTLIST_PAIRS, F8>(dp, grid, 1, s)));
+    else HN_TRY((launch_dist<2, EPI_SHORTLIST_BATCHED, F8>(dp, grid, 1, s)));
   }
   {
     MatchTimer timer(2, s);
@@ -1171,11 +1237,10 @@ static int run_batched(const T* q, const T* g, long long B, long long Nq, long l
                        float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace, cudaStream_t s) {
   const BatchedWs w = carve_batched(workspace, B, Nq, Ng, mutual != nullptr, true);
   const long long rows_q = B * Nq, rows_g = B * Ng;
-  const int threads = 256;
   {
     MatchTimer timer(0, s);
-    pack_desc_kernel<<<static_cast<unsigned>((rows_q * 32 + threads - 1) / threads), threads, 0, s>>>(q, rows_q, w.q16, 0, 0, nullptr);
-    pack_desc_kernel<<<static_cast<unsigned>((rows_g * 32 + threads - 1) / threads), threads, 0, s>>>(g, rows_g, w.g16, 0, 1, nullptr);
+    launch_pack(q, rows_q, w.q16, 0, s);
+    launch_pack(g, rows_g, w.g16, 1, s);
     HN_CUDA(cudaGetLastError());
     count_launch(2);
   }
@@ -1238,8 +1303,8 @@ static int pairs_entry(const char* fn, const void* q, const void* q16, long long
   const PairLayout L = {pairs, nullptr, nullptr, B, max_q, max_g, Nq_rows, Ng_rows};
   return with_rows(desc_dtype, [&](auto t) -> int {
     using T = decltype(t);
-    return run_pairs<true>(static_cast<const T*>(q), static_cast<const uint16_t*>(q16), static_cast<const T*>(g),
-                           static_cast<const uint16_t*>(g16), L, d1, d2, i1, i2, mutual, w, static_cast<cudaStream_t>(stream));
+    return run_pairs<true>(static_cast<const T*>(q), q16, static_cast<const T*>(g), g16, L, d1, d2, i1, i2, mutual, w,
+                           static_cast<cudaStream_t>(stream));
   });
 }
 

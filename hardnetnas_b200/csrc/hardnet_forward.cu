@@ -621,7 +621,7 @@ extern "C" int hn_forward(hn_handle* h, const void* patches, int in_dtype, long 
   }
   HN_REQUIRE(B >= 0, "hn_forward: negative batch");
   HN_REQUIRE(in_dtype == HN_F32 || in_dtype == HN_U8, "hn_forward: in_dtype must be HN_F32 or HN_U8");
-  HN_REQUIRE(out_dtype == HN_F32 || out_dtype == HN_F16 || out_dtype == HN_BF16, "hn_forward: bad out_dtype");
+  HN_REQUIRE(out_dtype == HN_F32 || out_dtype == HN_F16 || out_dtype == HN_BF16 || out_dtype == HN_F8E4M3, "hn_forward: bad out_dtype");
   if (B == 0) return HN_OK;
   HN_REQUIRE(patches && desc_out, "hn_forward: NULL data pointer");
   return forward_passes(h, patches, in_dtype, B, desc_out, out_dtype, static_cast<cudaStream_t>(stream));
@@ -638,7 +638,7 @@ extern "C" int hn_forward_clip(hn_handle* h, const void* images, int img_dtype, 
     return HN_ERR_STATE;
   }
   HN_REQUIRE(img_dtype == HN_F32 || img_dtype == HN_U8, "hn_forward_clip: img_dtype must be HN_F32 or HN_U8");
-  HN_REQUIRE(out_dtype == HN_F32 || out_dtype == HN_F16 || out_dtype == HN_BF16, "hn_forward_clip: bad out_dtype");
+  HN_REQUIRE(out_dtype == HN_F32 || out_dtype == HN_F16 || out_dtype == HN_BF16 || out_dtype == HN_F8E4M3, "hn_forward_clip: bad out_dtype");
   HN_REQUIRE(B >= 1 && H >= 1 && W >= 1 && static_cast<long long>(H) * W < (1ll << 31), "hn_forward_clip: bad image size");
   HN_REQUIRE(N >= 0 && N % B == 0, "hn_forward_clip: the reference's view(B, -1) needs N (%lld) to be a multiple of B (%lld)", N, B);
   if (N == 0) return HN_OK;
@@ -659,7 +659,7 @@ extern "C" int hn_forward_clip(hn_handle* h, const void* images, int img_dtype, 
 }
 
 static int forward_passes(hn_handle* h, const void* patches, int in_dtype, long long B, void* desc_out, int out_dtype, cudaStream_t s) {
-  const size_t out_elem = out_dtype == HN_F32 ? 4 : 2;
+  const size_t out_elem = out_dtype == HN_F32 ? 4 : out_dtype == HN_F8E4M3 ? 1 : 2;
   for (long long base = 0; base < B; base += h->head_rows) {
     const long long nb = std::min<long long>(h->head_rows, B - base);
     for (long long off = 0; off < nb; off += h->chunk) {

@@ -28,8 +28,8 @@ static EncodeTiledFn resolve_encode() {
   return fn;
 }
 
-int make_tmap_16bit(CUtensorMap* tm, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                    const uint32_t* box, int swizzle_bytes) {
+static int make_tmap(CUtensorMap* tm, CUtensorMapDataType dtype, const void* base, int rank, const uint64_t* dims,
+                     const uint64_t* strides_bytes, const uint32_t* box, int swizzle_bytes) {
   EncodeTiledFn fn = resolve_encode();
   if (!fn) {
     set_error("cuTensorMapEncodeTiled is not available (no CUDA driver?)");
@@ -49,8 +49,7 @@ int make_tmap_16bit(CUtensorMap* tm, const void* base, int rank, const uint64_t*
                                 : swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B
                                 : swizzle_bytes == 32 ? CU_TENSOR_MAP_SWIZZLE_32B
                                                       : CU_TENSOR_MAP_SWIZZLE_NONE;
-  // FLOAT16 vs BFLOAT16 only matters for OOB NaN fill, which is not used: tiles are moved as raw 16-bit.
-  CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, static_cast<cuuint32_t>(rank), const_cast<void*>(base), gdim,
+  CUresult r = fn(tm, dtype, static_cast<cuuint32_t>(rank), const_cast<void*>(base), gdim,
                   gstr, bdim, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -60,6 +59,18 @@ int make_tmap_16bit(CUtensorMap* tm, const void* base, int rank, const uint64_t*
     return HN_ERR_CUDA;
   }
   return HN_OK;
+}
+
+int make_tmap_16bit(CUtensorMap* tm, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
+                    const uint32_t* box, int swizzle_bytes) {
+  // FLOAT16 vs BFLOAT16 only matters for OOB NaN fill, which is not used: tiles are moved as raw 16-bit.
+  return make_tmap(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, base, rank, dims, strides_bytes, box, swizzle_bytes);
+}
+
+int make_tmap_8bit(CUtensorMap* tm, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
+                   const uint32_t* box, int swizzle_bytes) {
+  // raw bytes (e4m3 operand rows): out-of-bounds boxes are zero-filled as for the 16-bit maps
+  return make_tmap(tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, base, rank, dims, strides_bytes, box, swizzle_bytes);
 }
 
 static std::atomic<long long> g_launch_count{0};

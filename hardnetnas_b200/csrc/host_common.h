@@ -49,6 +49,9 @@ inline void set_error(const char* fmt, ...) {
 // (dims 1..rank-1). swizzle_bytes is 32 / 64 / 128 (and must equal box[0] * 2) or 0 for a dense, unswizzled box.
 int make_tmap_16bit(CUtensorMap* tm, const void* base, int rank, const uint64_t* dims,
                     const uint64_t* strides_bytes, const uint32_t* box, int swizzle_bytes);
+// The same for 1-byte elements (swizzle_bytes = box[0]).
+int make_tmap_8bit(CUtensorMap* tm, const void* base, int rank, const uint64_t* dims,
+                   const uint64_t* strides_bytes, const uint32_t* box, int swizzle_bytes);
 
 int device_sm_count(int* out);
 

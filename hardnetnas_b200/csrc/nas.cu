@@ -1940,13 +1940,13 @@ extern "C" int hn_forward_nas(hn_handle* h, const void* patches, int in_dtype, l
   }
   HN_REQUIRE(B >= 0, "hn_forward_nas: negative batch");
   HN_REQUIRE(in_dtype == HN_F32 || in_dtype == HN_U8, "hn_forward_nas: in_dtype must be HN_F32 or HN_U8");
-  HN_REQUIRE(out_dtype == HN_F32 || out_dtype == HN_F16 || out_dtype == HN_BF16, "hn_forward_nas: bad out_dtype");
+  HN_REQUIRE(out_dtype == HN_F32 || out_dtype == HN_F16 || out_dtype == HN_BF16 || out_dtype == HN_F8E4M3, "hn_forward_nas: bad out_dtype");
   if (B == 0) return HN_OK;
   HN_REQUIRE(patches && desc_out, "hn_forward_nas: NULL data pointer");
   NasState* st = h->nas;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const size_t in_elem = in_dtype == HN_F32 ? 4 : 1;
-  const size_t out_elem = out_dtype == HN_F32 ? 4 : 2;
+  const size_t out_elem = out_dtype == HN_F32 ? 4 : out_dtype == HN_F8E4M3 ? 1 : 2;
   const int n_ops = static_cast<int>(st->ops.size());
   for (long long base = 0; base < B; base += h->head_rows) {
     const long long nb = std::min<long long>(h->head_rows, B - base);

@@ -18,7 +18,7 @@ namespace hn {
 constexpr int kTileM = 128;
 constexpr int kTcThreads = 192;
 
-enum : int { DT_F32 = 0, DT_F16 = 1, DT_BF16 = 2, DT_U8 = 3 };
+enum : int { DT_F32 = 0, DT_F16 = 1, DT_BF16 = 2, DT_U8 = 3, DT_F8E4M3 = 5 };   // = hn_dtype
 
 struct TcParams {
   CUtensorMap tmA[4];      // conv stride 1 / gemm: [0]; conv stride 2: parity views [ypar * 2 + xpar]
@@ -26,12 +26,12 @@ struct TcParams {
   const float* bias;       // [N] folded BatchNorm shift
   float bias_v[128];       // conv kernels: the same values BY VALUE - parameters sit in the constant bank, so the epilogue's
                            // `acc + bias` is an FADD with a constant operand instead of shared-memory loads on the busy L1 pipe
-  void* out;               // conv: 16-bit channel-planar (see above); head: f32/f16/bf16 [rows, N]
+  void* out;               // conv: 16-bit channel-planar (see above); head: f32/f16/bf16/e4m3 [rows, N]
   long long total_rows;    // valid output rows (pixels or patches)
   int num_tiles;
   int num_k_stages;        // gemm only: K / (G * 64)
   int act_bf16;            // 16-bit activation flavour: 0 = fp16, 1 = bf16
-  int out_dtype;           // head only: DT_F32 / DT_F16 / DT_BF16
+  int out_dtype;           // head only: DT_F32 / DT_F16 / DT_BF16 / DT_F8E4M3
   float l2_eps;            // head only: 1e-10 (Utils.py:18); 0 for the NAS head
   int k_splits;            // head only: > 1 = split-K (small batches): a CTA reduces num_k_stages / k_splits stages of one row tile
                            // and writes raw fp32 partial sums to `partial`; head_finalize_kernel adds them, the bias and the norm
@@ -289,6 +289,14 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_l2norm_kernel(const __grid
             float4* dst = reinterpret_cast<float4*>(static_cast<float*>(p.out) + row * N + c0);
 #pragma unroll
             for (int j = 0; j < 8; ++j) dst[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+          } else if (p.out_dtype == DT_F8E4M3) {
+            uint4* dst = reinterpret_cast<uint4*>(static_cast<uint8_t*>(p.out) + row * N + c0);
+#pragma unroll
+            for (int j = 0; j < 2; ++j)
+              dst[j] = make_uint4(pack_e4m3x4(v[16 * j], v[16 * j + 1], v[16 * j + 2], v[16 * j + 3]),
+                                  pack_e4m3x4(v[16 * j + 4], v[16 * j + 5], v[16 * j + 6], v[16 * j + 7]),
+                                  pack_e4m3x4(v[16 * j + 8], v[16 * j + 9], v[16 * j + 10], v[16 * j + 11]),
+                                  pack_e4m3x4(v[16 * j + 12], v[16 * j + 13], v[16 * j + 14], v[16 * j + 15]));
           } else {
             uint4* dst = reinterpret_cast<uint4*>(static_cast<uint16_t*>(p.out) + row * N + c0);
             const int bf = p.out_dtype == DT_BF16;
@@ -334,6 +342,8 @@ static __global__ void __launch_bounds__(256) head_finalize_kernel(const float* 
   v.x *= inv; v.y *= inv; v.z *= inv; v.w *= inv;
   if (out_dtype == DT_F32) {
     *reinterpret_cast<float4*>(static_cast<float*>(out) + row * 128 + lane * 4) = v;
+  } else if (out_dtype == DT_F8E4M3) {
+    *reinterpret_cast<uint32_t*>(static_cast<uint8_t*>(out) + row * 128 + lane * 4) = pack_e4m3x4(v.x, v.y, v.z, v.w);
   } else {
     const int bf = out_dtype == DT_BF16;
     *reinterpret_cast<uint2*>(static_cast<uint16_t*>(out) + row * 128 + lane * 4) = make_uint2(pack16(v.x, v.y, bf), pack16(v.z, v.w, bf));

@@ -90,6 +90,18 @@ __device__ __forceinline__ void umma_f16_pair_w(uint32_t d_tmem, uint32_t a_lo, 
       ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// kind::f8f6f4 twin (UTCQMMA.2CTA), see umma_f8_w
+__device__ __forceinline__ void umma_f8_pair_w(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
+                                               uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
+      "setp.ne.b32 p, %6, 0;\n\t"
+      "mov.b64 da, {%1, %2};\n\t"
+      "mov.b64 db, {%3, %4};\n\t"
+      "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], da, db, %5, p;\n\t}"
+      ::"r"(d_tmem), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // Arrives on the barrier at this shared-memory offset in BOTH CTAs once the previously issued MMAs have retired.
 __device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),

@@ -23,6 +23,10 @@
 //               past it are neither stored nor part of the cell maxima. A separate instantiation rather than the padded
 //               case of one accessor: reading the padded layout through the table accessor made hn_match_batched 1-2 %
 //               slower (DESIGN.md section 5).
+//
+// F8: the shortlist kernels on e4m3 operand rows (matching on HN_F8E4M3 rows, dist.cu). A K = 128 e4m3 row is 128 bytes, one
+// 128B-swizzle atom, so an fp8 operand is the fp16 case with k_blocks = 1: the same shared-memory blocks, tensor maps with the
+// same box in bytes, the same descriptor steps; only the MMA kind changes (umma_f8_w, kind::f8f6f4, K = 32 per MMA).
 #pragma once
 
 #include "../../include/hardnet_b200.h"
@@ -38,7 +42,7 @@ constexpr int kChunk = 8;    // columns per chunk
 enum : int { EPI_EXACT = 0, EPI_SHORTLIST = 1, EPI_EXACT_NEI = 2, EPI_SHORTLIST_BATCHED = 3, EPI_SHORTLIST_PAIRS = 4 };   // EXACT_NEI = EXACT + the keypoint-neighbour masks
 
 struct DistSide {
-  CUtensorMap tmA;             // rows of this launch direction, [Na, K] 16-bit
+  CUtensorMap tmA;             // rows of this launch direction, [Na, K] 16-bit (e4m3 in the F8 kernels)
   CUtensorMap tmB;             // columns, [Nb, K]
   const float* norm_a;         // |a_i|^2 (hardnet form)
   const float* norm_b;
@@ -58,7 +62,7 @@ struct DistSide {
 
 struct DistParams {
   DistSide side[2];            // [1] = transposed problem (anchor swap / column minima)
-  int k_blocks;                // K / 64
+  int k_blocks;                // 128-byte K blocks per row: K / 64 (16-bit operands), 1 (e4m3 operands)
   int segments;
   int form;                    // HN_FORM_*
   int loss_mask;               // apply +1e-8, diagonal +10, (<0.008) +10
@@ -130,7 +134,7 @@ __device__ __forceinline__ float warp_chunk_max8(const float (&c)[8], int lane) 
 template <int EPI>
 constexpr int dist_col_split() { return (EPI == EPI_EXACT || EPI == EPI_EXACT_NEI) ? 4 : 1; }
 
-template <int MB, int EPI>
+template <int MB, int EPI, bool F8 = false>
 __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist_kernel(const __grid_constant__ DistParams p) {
   constexpr bool EXACT = EPI == EPI_EXACT || EPI == EPI_EXACT_NEI;
   constexpr int CS = dist_col_split<EPI>();
@@ -139,7 +143,8 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
   constexpr bool PAIRS = EPI == EPI_SHORTLIST_PAIRS;
   constexpr bool BATCHED = EPI == EPI_SHORTLIST_BATCHED || PAIRS;
   constexpr bool SHORTLIST = EPI == EPI_SHORTLIST || BATCHED;
-  constexpr uint32_t BLK_BYTES = kDistTile * 128;  // 128 rows x 64 fp16
+  static_assert(!F8 || (SHORTLIST && MB == 2), "e4m3 operands are for the matching GEMMs");
+  constexpr uint32_t BLK_BYTES = kDistTile * 128;  // 128 rows x 64 fp16 (F8: x 128 e4m3)
   constexpr uint32_t TMEM_COLS = 2 * MB * kDistTile;
   const DistSide& sd = p.side[blockIdx.y];
 
@@ -294,7 +299,10 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
                 const uint32_t a_lo = a_lo0 + static_cast<uint32_t>(mb * p.k_blocks + kb) * (BLK_BYTES >> 4);
                 const uint32_t d_tmem = tmem_base + (acc * MB + mb) * kDistTile;
 #pragma unroll
-                for (int k = 0; k < 4; ++k) umma_f16_w(d_tmem, a_lo + 2u * k, HI, b_lo + 2u * k, HI, idesc, (kb | k) != 0);
+                for (int k = 0; k < 4; ++k) {
+                  if constexpr (F8) umma_f8_w(d_tmem, a_lo + 2u * k, HI, b_lo + 2u * k, HI, idesc, (kb | k) != 0);
+                  else umma_f16_w(d_tmem, a_lo + 2u * k, HI, b_lo + 2u * k, HI, idesc, (kb | k) != 0);
+                }
               }
               umma_commit(empty_bar(stage));
               if (kb == p.k_blocks - 1) umma_commit(tfull_bar(acc));

@@ -5,6 +5,9 @@
 // which takes the N = 128 GEMM off the shared-memory port limit, and the gallery streams through each SM's L2 port once
 // per 512 query rows instead of once per 256. The epilogue (top-4 chunks per row + their maxima) and the output format
 // are those of dist_kernel<2, EPI_SHORTLIST>; the signalling protocol is the one of tc_conv_pair.cuh.
+// F8: e4m3 operand rows (see tc_dist.cuh): an A block is one 128-byte K block instead of two and a stage is one 8 KB half-tile
+// instead of two k-blocks, with kind::f8f6f4 MMAs (umma_f8_pair_w). The stage count stays kMpStages: the same number of
+// gallery tiles in flight, in half the shared memory.
 #pragma once
 
 #include "tc_conv_pair.cuh"
@@ -12,25 +15,32 @@
 
 namespace hn {
 
-constexpr int kMpStages = 6;                       // gallery half-tiles (both k-blocks, 16 KB) in flight per CTA
-constexpr uint32_t kMpABlk = kDistTile * 128;      // one 128-row x 64-element A block
-constexpr uint32_t kMpBBlk = 64 * 128;             // this CTA's 64-row x 64-element half of a B k-block
-constexpr uint32_t kMpStage = 2 * kMpBBlk;         // both k-blocks of a half tile
-constexpr size_t kMpSmem = 4 * kMpABlk + kMpStages * kMpStage + 1024 + 256;
+constexpr int kMpStages = 6;                       // gallery half-tiles (both k-blocks, 16 KB; F8: 8 KB) in flight per CTA
+constexpr uint32_t kMpABlk = kDistTile * 128;      // one 128-row x 64-element A block (F8: 128 e4m3)
+constexpr uint32_t kMpBBlk = 64 * 128;             // this CTA's 64-row x 64-element half of a B k-block (F8: 128 e4m3)
+template <bool F8>
+constexpr int mp_k_blocks() { return F8 ? 1 : 2; }
+template <bool F8>
+constexpr uint32_t mp_stage_bytes() { return mp_k_blocks<F8>() * kMpBBlk; }   // all k-blocks of a half tile
+template <bool F8>
+constexpr size_t mp_smem_bytes() { return 2 * mp_k_blocks<F8>() * kMpABlk + kMpStages * mp_stage_bytes<F8>() + 1024 + 256; }
 // The epilogue (per row: maxima of sixteen 8-column chunks per tile + a sorted insert) is the longest step per tile, so
 // every 32-row lane quarter of an accumulator is shared by TWO warps, each reducing 64 of the 128 columns into its own
 // top-kTopC list (the lists of the two halves are separate slots of the candidate table).
 constexpr int kMpEpiWarps = 16;
 constexpr int kMpThreads = 64 + kMpEpiWarps * 32;
 
+template <bool F8>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kMpThreads, 1) match_pair_kernel(const __grid_constant__ DistParams p) {
   constexpr int MB = 2;
+  constexpr int KB = mp_k_blocks<F8>();
+  constexpr uint32_t kMpStage = mp_stage_bytes<F8>();
   const DistSide& sd = p.side[0];
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_addr = smem_u32(smem_raw);
   const uint32_t base = (raw_addr + 1023u) & ~1023u;
   const uint32_t a_base = base;                              // [mb][kb] blocks
-  const uint32_t b_base = base + 4 * kMpABlk;
+  const uint32_t b_base = base + MB * KB * kMpABlk;
   const uint32_t bar_base = b_base + kMpStages * kMpStage;
   auto full_bar = [&](int s) { return bar_base + 8u * s; };
   auto empty_bar = [&](int s) { return bar_base + 8u * (kMpStages + s); };
@@ -93,13 +103,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kMpThreads, 1) match
       seg_range(seg, t0, t1);
       mbar_wait(aempty_bar, a_phase ^ 1u);
       if (elect_one()) {
-        mbar_arrive_expect_tx_cluster(lead_afull, 4 * kMpABlk);
+        mbar_arrive_expect_tx_cluster(lead_afull, MB * KB * kMpABlk);
         const int row0 = (mblk * 2 + static_cast<int>(rank)) * MB * kDistTile;
 #pragma unroll
         for (int mb = 0; mb < MB; ++mb)
 #pragma unroll
-          for (int kb = 0; kb < 2; ++kb)
-            tma_load_2d_pair(a_base + (mb * 2 + kb) * kMpABlk, &sd.tmA, lead_afull, kb * 64, row0 + mb * kDistTile);
+          for (int kb = 0; kb < KB; ++kb)
+            tma_load_2d_pair(a_base + (mb * KB + kb) * kMpABlk, &sd.tmA, lead_afull, kb * 64, row0 + mb * kDistTile);
       }
       __syncwarp();
       a_phase ^= 1u;
@@ -109,8 +119,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kMpThreads, 1) match
           const uint32_t lead_full = mapa_cluster(full_bar(stage), 0);
           mbar_arrive_expect_tx_cluster(lead_full, kMpStage);
           const int grow = t * kDistTile + static_cast<int>(rank) * 64;
-          tma_load_2d_pair(b_base + stage * kMpStage, &sd.tmB, lead_full, 0, grow);
-          tma_load_2d_pair(b_base + stage * kMpStage + kMpBBlk, &sd.tmB, lead_full, 64, grow);
+#pragma unroll
+          for (int kb = 0; kb < KB; ++kb) tma_load_2d_pair(b_base + stage * kMpStage + kb * kMpBBlk, &sd.tmB, lead_full, kb * 64, grow);
         }
         __syncwarp();
         if (++stage == kMpStages) { stage = 0; phase ^= 1u; }
@@ -145,11 +155,13 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kMpThreads, 1) match
             for (int mb = 0; mb < MB; ++mb) {
               const uint32_t d_tmem = tmem_base + (acc * MB + mb) * kDistTile;
 #pragma unroll
-              for (int kb = 0; kb < 2; ++kb) {
+              for (int kb = 0; kb < KB; ++kb) {
 #pragma unroll
-                for (int k = 0; k < 4; ++k)
-                  umma_f16_pair_w(d_tmem, a_lo0 + (((mb * 2 + kb) * kMpABlk) >> 4) + 2u * k, HI,
-                                  b_lo + ((kb * kMpBBlk) >> 4) + 2u * k, HI, idesc, (kb | k) != 0);
+                for (int k = 0; k < 4; ++k) {
+                  const uint32_t a_lo = a_lo0 + (((mb * KB + kb) * kMpABlk) >> 4) + 2u * k, b_lo_k = b_lo + ((kb * kMpBBlk) >> 4) + 2u * k;
+                  if constexpr (F8) umma_f8_pair_w(d_tmem, a_lo, HI, b_lo_k, HI, idesc, (kb | k) != 0);
+                  else umma_f16_pair_w(d_tmem, a_lo, HI, b_lo_k, HI, idesc, (kb | k) != 0);
+                }
               }
             }
             umma_commit_pair(empty_bar(stage));

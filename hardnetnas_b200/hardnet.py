@@ -19,7 +19,8 @@ import torch.nn as nn
 from . import _lib
 
 _DTYPES = {"fp16": _lib.HN_F16, "bf16": _lib.HN_BF16}
-_OUT_DTYPES = {torch.float32: _lib.HN_F32, torch.float16: _lib.HN_F16, torch.bfloat16: _lib.HN_BF16}
+_OUT_DTYPES = {torch.float32: _lib.HN_F32, torch.float16: _lib.HN_F16, torch.bfloat16: _lib.HN_BF16,
+               torch.float8_e4m3fn: _lib.HN_F8E4M3}
 
 
 class L2Norm(nn.Module):

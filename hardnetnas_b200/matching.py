@@ -3,9 +3,10 @@
 The reference materialises the full distance matrix and then takes `min` (eval_utils.py:113-114) or a full
 row `sort` (:168-175). Here one fused pass (tensor-core GEMM + in-register shortlist, exact fp32 re-rank)
 returns the nearest and second-nearest gallery row per query; nothing of size Nq x Ng is ever stored.
-Descriptors may be fp32, fp16 or bf16: fp16 / bf16 tensors of one dtype (e.g. `HardNet.forward(x, out_dtype=torch.float16)`) are
-matched as they are, without an fp32 copy, with results bit-identical to the same call on their `.float()`; mixed or other dtypes
-are converted to fp32 first.
+Descriptors may be fp32, fp16, bf16 or fp8 e4m3 (torch.float8_e4m3fn): fp16 / bf16 / e4m3 tensors of one dtype (e.g.
+`HardNet.forward(x, out_dtype=torch.float16)`) are matched as they are, without an fp32 copy, with results bit-identical to the
+same call on their `.float()`; e4m3 rows are matched on the fp8 tensor core. Mixed or other dtypes (float8_e5m2 included) are
+converted to fp32 first.
 """
 from __future__ import annotations
 
@@ -18,7 +19,9 @@ def assert_unit_norm(des, tol: float = 1e-3):
     """Precondition of the fused matching kernels (include/hardnet_b200.h, hn_match): rows are L2-normalised descriptors, the
     only input the FDLNet distance form `sqrt(2 - 2 a.b)` is defined for. The kernels do not check it (their fp16 operand
     packing and the re-rank margin assume |x| <= 1); call this once on descriptors of unknown origin - one device
-    synchronisation, raises ValueError naming the first offending row."""
+    synchronisation, raises ValueError naming the first offending row. Unit descriptors rounded to e4m3
+    (torch.float8_e4m3fn) keep their norm within (2^-4 + sqrt(128) * 2^-10) < 0.074 of 1 (random unit rows: within about
+    0.006), so check those with tol=0.075."""
     n = des.float().norm(dim=1)
     bad = ((n - 1.0).abs() > tol) & (n > 0)        # all-zero rows (constant patches) are legal and match nothing
     if bool(bad.any()):

@@ -35,7 +35,8 @@ typedef enum hn_status {
   HN_ERR_UNSUPPORTED = -4
 } hn_status;
 
-typedef enum hn_dtype { HN_F32 = 0, HN_F16 = 1, HN_BF16 = 2, HN_U8 = 3 } hn_dtype;
+/* HN_F8E4M3: fp8 E4M3 (torch.float8_e4m3fn), descriptor outputs and matching rows only. 4 is not a dtype. */
+typedef enum hn_dtype { HN_F32 = 0, HN_F16 = 1, HN_BF16 = 2, HN_U8 = 3, HN_F8E4M3 = 5 } hn_dtype;
 
 /* distance forms */
 #define HN_FORM_HARDNET 0 /* sqrt(|a|^2 + |p|^2 - 2ab + 1e-6)           hardnet/Losses.py:5-13            */
@@ -74,7 +75,8 @@ int hn_pack_hardnet(hn_handle* h, const float* const w[7], const float* const bn
 int hn_set_hardnet_eps(hn_handle* h, float input_norm_eps, float l2_eps);
 
 /* HardNet.forward in eval mode: input_norm -> 7 conv/BN/ReLU stages -> L2Norm.
- * patches: [B,1,32,32] (HN_F32 or HN_U8); desc_out: [B,128] (HN_F32 / HN_F16 / HN_BF16). */
+ * patches: [B,1,32,32] (HN_F32 or HN_U8); desc_out: [B,128] (HN_F32 / HN_F16 / HN_BF16 / HN_F8E4M3). Every output dtype is the
+ * fp32 descriptor rounded to nearest even (HN_F8E4M3: 128 bytes per row, equal to .to(torch.float8_e4m3fn) of the fp32 output). */
 int hn_forward(hn_handle* h, const void* patches, int in_dtype, long long B, void* desc_out,
                int out_dtype, void* stream);
 
@@ -248,7 +250,7 @@ int hn_match_pairs(const float* q, const void* q16, long long Nq_rows, const flo
  * initial value is read once from HN_MATCH_PAIR), 0 = single-CTA kernel, 1 = CTA-pair (cta_group::2) kernel. */
 int hn_match_force_kernel(int mode);
 
-/* ---- matching on fp16 / bf16 descriptor rows -------------------------------------------------------------------------------
+/* ---- matching on fp16 / bf16 / fp8 E4M3 descriptor rows --------------------------------------------------------------------
  * Typed twins of the row-reading matching entry points: descriptor rows are `const void*` of desc_dtype HN_F32, HN_F16 or
  * HN_BF16 (e.g. the out_dtype output of hn_forward / hn_forward_nas / hn_forward_clip), the same type on both sides of a call;
  * the other arguments, the outputs and the preconditions are those of the fp32 function named. Every kernel widens a 16-bit
@@ -259,7 +261,15 @@ int hn_match_force_kernel(int mode);
  * The workspace does not depend on the row type: hn_dist_workspace_bytes, hn_mutual_workspace_bytes,
  * hn_match_batched_workspace_bytes and hn_match_pairs_workspace_bytes size the typed calls too. Validation as the fp32
  * function, plus: a desc_dtype other than HN_F32 / HN_F16 / HN_BF16 (HN_U8 included) and 16-bit rows that are not 8-byte
- * aligned are rejected with HN_ERR_INVALID before any device work. The fp32 functions are these calls with HN_F32. */
+ * aligned are rejected with HN_ERR_INVALID before any device work. The fp32 functions are these calls with HN_F32.
+ * HN_F8E4M3 rows (128 bytes per row, 4-byte aligned) follow the same contract: every output equals the fp32 call on the rows
+ * converted to fp32, bit for bit. Their packed operand is e4m3 x * 2^8 ([n,128], 128 bytes per row), which is exact: a row
+ * element of a unit row has |x| <= 1, so |x * 2^8| <= 256 < 448, and the smallest e4m3 subnormal 2^-9 becomes the normal
+ * 2^-1. The matching GEMM then runs on the fp8 tensor core (kind::f8f6f4); its products are exact and only the accumulation can
+ * differ from the fp16 GEMM (dist.cu states the bound the re-rank and verification margins rely on). Packed operands given by the
+ * caller (q16 / g16) must come from hn_pack_descriptors_typed on rows of the call's dtype: e4m3 for HN_F8E4M3 rows, fp16
+ * otherwise; the Python wrappers check this. An fp8 call needs no more workspace than the fp32 call the *_workspace_bytes
+ * functions size. hn_pack_descriptors_multicast, hn_dist_min and hn_loss_hardnet take fp32 rows only. */
 int hn_pack_descriptors_typed(const void* x, int desc_dtype, long long n, void* out16, void* stream);          /* hn_pack_descriptors */
 int hn_match_typed(const void* q, const void* g, int desc_dtype, const void* q16, const void* g16, long long Nq, long long Ng,
                    long long g_offset, float* d1, float* d2, int32_t* i1, int32_t* i2, float* block_max, void* workspace,
