@@ -369,19 +369,28 @@ struct MatchTimer {
 // claimant of a column can be its mutual partner. `claim` must be initialised to an "unclaimed" value: any word whose upper
 // half is >= 0x7F000000 (no real distance has such bits): bytes of 0x7F, or INT64_MAX - positive as a signed integer too, so
 // that an all_reduce(MIN) over int64 orders claims like the unsigned atomicMin does.
+// The claim of one query row, shared by mutual_claim_kernel and mutual_claim_batched_kernel: a warp is one 32-row block of one
+// problem, whose minimum d2 over its valid rows goes to rb_min_d2[rb] (lane 0, if store_min). Row i of i1 / d1 / d2 is valid iff
+// it is a row of the problem; it then claims its nearest column j < ng() of `claim` as row number id.
+template <typename Cols>
+__device__ __forceinline__ void claim_row(const int* i1, const float* d1, const float* d2, long long i, bool valid, float* rb_min_d2,
+                                          long long rb, bool store_min, unsigned long long* claim, Cols ng, unsigned int id) {
+  // a warp is one 32-row block: its smallest second-nearest distance bounds every d(k, j) with j not the nearest column of k
+  float m = valid ? d2[i] : __int_as_float(0x7f800000);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fminf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0 && store_min) rb_min_d2[rb] = m;
+  if (!valid) return;
+  const long long j = i1[i];
+  if (j < 0 || j >= ng()) return;
+  atomicMin(claim + j, (static_cast<unsigned long long>(__float_as_uint(d1[i])) << 32) | id);
+}
+
 __global__ void mutual_claim_kernel(const int* __restrict__ i1, const float* __restrict__ d1, const float* __restrict__ d2,
                                     long long nq, long long q_offset, unsigned long long* __restrict__ claim, long long ng,
                                     float* __restrict__ rb_min_d2) {
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  // a warp is one 32-row block: its smallest second-nearest distance bounds every d(k, j) with j not the nearest column of k
-  float m = i < nq ? d2[i] : __int_as_float(0x7f800000);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) m = fminf(m, __shfl_xor_sync(0xffffffffu, m, o));
-  if ((threadIdx.x & 31) == 0 && i < nq) rb_min_d2[i >> 5] = m;
-  if (i >= nq) return;
-  const long long j = i1[i];
-  if (j < 0 || j >= ng) return;
-  atomicMin(claim + j, (static_cast<unsigned long long>(__float_as_uint(d1[i])) << 32) | static_cast<unsigned int>(i + q_offset));
+  claim_row(i1, d1, d2, i, i < nq, rb_min_d2, i >> 5, i < nq, claim, [&] { return ng; }, static_cast<unsigned int>(i + q_offset));
 }
 
 // Is the claimant of column j really the nearest query of g_j (lowest row wins ties, like torch.min)? A query row k can beat
@@ -522,16 +531,21 @@ __global__ void __launch_bounds__(kVerifyWarps * 32) mutual_verify_kernel(const 
                beaten, cb, s_q, s_g, lane);
 }
 
-// mutual[i] = the best claimant of my nearest column is me, and nobody beat it
+// mutual flag of query row `row` of a problem whose nearest column is j: the best claimant of column j < ng() is the row
+// (number row + q_offset in the claims), and nobody beat it. Shared by mutual_final_kernel and mutual_final_batched_kernel.
+template <typename Cols>
+__device__ __forceinline__ bool is_mutual(long long j, Cols ng, const unsigned long long* claim, const unsigned char* beaten,
+                                          long long row, long long q_offset) {
+  return j >= 0 && j < ng() && static_cast<unsigned int>(claim[j] & 0xffffffffu) == static_cast<unsigned int>(row + q_offset) &&
+         !beaten[j];
+}
+
 __global__ void mutual_final_kernel(const int* __restrict__ i1, long long nq, long long q_offset,
                                     const unsigned long long* __restrict__ claim, const unsigned char* __restrict__ beaten,
                                     long long ng, unsigned char* __restrict__ mutual) {
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= nq) return;
-  const long long j = i1[i];
-  bool m = false;
-  if (j >= 0 && j < ng) m = static_cast<unsigned int>(claim[j] & 0xffffffffu) == static_cast<unsigned int>(i + q_offset) && !beaten[j];
-  mutual[i] = m ? 1 : 0;
+  mutual[i] = is_mutual(i1[i], [&] { return ng; }, claim, beaten, i, q_offset) ? 1 : 0;
 }
 
 // Batched column side of hn_match_batched. Claims, beaten flags and block maxima are per pair ([B][ng], [B][ng],
@@ -551,14 +565,8 @@ __global__ void mutual_claim_batched_kernel(const int* __restrict__ i1, const fl
   const long long b = t / (nrb * 32), r = t - b * nrb * 32;   // 64-bit: B * nrb * 32 may pass 2^31 while B * nq does not
   const long long i = b * nq + r;
   const bool valid = r < (TABLE ? table_span(pairs, b, 0, nq, q_rows).len : pair_len(q_len, b, nq));
-  float m = valid ? d2[i] : __int_as_float(0x7f800000);
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) m = fminf(m, __shfl_xor_sync(0xffffffffu, m, o));
-  if ((threadIdx.x & 31) == 0) rb_min_d2[b * nrb + (r >> 5)] = m;
-  if (!valid) return;
-  const long long j = i1[i];
-  if (j < 0 || j >= (TABLE ? table_span(pairs, b, 1, ng, g_rows).len : pair_len(g_len, b, ng))) return;
-  atomicMin(claim + b * ng + j, (static_cast<unsigned long long>(__float_as_uint(d1[i])) << 32) | static_cast<unsigned int>(r));
+  const auto ng_b = [&] { return TABLE ? table_span(pairs, b, 1, ng, g_rows).len : pair_len(g_len, b, ng); };
+  claim_row(i1, d1, d2, i, valid, rb_min_d2, b * nrb + (r >> 5), true, claim + b * ng, ng_b, static_cast<unsigned int>(r));
 }
 
 // One warp per (pair, 8-column chunk), scanning only the pair's valid row blocks: verify_chunk on the pair's rows, with local
@@ -607,13 +615,9 @@ __global__ void mutual_final_batched_kernel(const int* __restrict__ i1, long lon
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= B * nq) return;
   const long long b = static_cast<int>(i) / static_cast<int>(nq), r = i - b * nq;
-  bool m = false;
-  if (r < (TABLE ? table_span(pairs, b, 0, nq, q_rows).len : pair_len(q_len, b, nq))) {
-    const long long j = i1[i];
-    if (j >= 0 && j < (TABLE ? table_span(pairs, b, 1, ng, g_rows).len : pair_len(g_len, b, ng)))
-      m = static_cast<unsigned int>(claim[b * ng + j] & 0xffffffffu) == static_cast<unsigned int>(r) && !beaten[b * ng + j];
-  }
-  mutual[i] = m ? 1 : 0;
+  const bool valid = r < (TABLE ? table_span(pairs, b, 0, nq, q_rows).len : pair_len(q_len, b, nq));
+  const auto ng_b = [&] { return TABLE ? table_span(pairs, b, 1, ng, g_rows).len : pair_len(g_len, b, ng); };
+  mutual[i] = valid && is_mutual(i1[i], ng_b, claim + b * ng, beaten + b * ng, r, 0) ? 1 : 0;
 }
 
 // Which matching GEMM runs: -1 = by problem size, 0 = single-CTA kernel, 1 = CTA-pair kernel. The initial value comes from
@@ -629,18 +633,34 @@ static inline long long batched_max_segments(long long Ng) {
   return std::max<long long>(1, std::min<long long>(kMaxBatchedSegments, (Ng + kDistTile - 1) / kDistTile));
 }
 
-static int make_desc_map(CUtensorMap* tm, const uint16_t* base, long long rows, int K, int box_rows = kDistTile) {
-  const uint64_t dims[2] = {static_cast<uint64_t>(K), static_cast<uint64_t>(rows)};
-  const uint64_t str[1] = {static_cast<uint64_t>(K) * 2};
-  const uint32_t box[2] = {64, static_cast<uint32_t>(box_rows)};
-  return make_tmap_16bit(tm, base, 2, dims, str, box, 128);
+// Tensor map over packed operand rows of K elements: fp16 (K = 128 or 384) or, with f8, e4m3 (K = 128). 2-D [rows][K], or with
+// B > 0 3-D [B][rows][K] (hn_match_batched: a box never reaches into the next pair, TMA zero-fills past `rows`). A box is one
+// 128-byte K block, i.e. one 128B-swizzle atom per row, of box_rows rows.
+static int make_operand_map(CUtensorMap* tm, const void* base, bool f8, int K, long long rows, long long B, int box_rows) {
+  const uint64_t esz = f8 ? 1 : 2;
+  const uint64_t dims[3] = {static_cast<uint64_t>(K), static_cast<uint64_t>(rows), static_cast<uint64_t>(B)};
+  const uint64_t str[2] = {K * esz, static_cast<uint64_t>(rows) * K * esz};
+  const uint32_t box[3] = {static_cast<uint32_t>(128 / esz), static_cast<uint32_t>(box_rows), 1};
+  const int rank = B > 0 ? 3 : 2;
+  return f8 ? make_tmap_8bit(tm, base, rank, dims, str, box, 128) : make_tmap_16bit(tm, base, rank, dims, str, box, 128);
 }
-// e4m3 twin: [rows, 128] operand rows of 128 bytes, box {128, box_rows} = one 128B-swizzle atom per row
-static int make_desc_map_f8(CUtensorMap* tm, const uint8_t* base, long long rows, int box_rows = kDistTile) {
-  const uint64_t dims[2] = {128, static_cast<uint64_t>(rows)};
-  const uint64_t str[1] = {128};
-  const uint32_t box[2] = {128, static_cast<uint32_t>(box_rows)};
-  return make_tmap_8bit(tm, base, 2, dims, str, box, 128);
+
+// The shortlist GEMM's part of DistParams (hn_match, hn_match_batched, hn_match_pairs): candidate lists, optional cell maxima
+// (mutual NN), Na query rows against Nb gallery rows (per-pair maxima in a batched call) and f8 = e4m3 operands. The tensor maps,
+// the segment count and the batch fields are the caller's.
+static DistParams shortlist_params(bool f8, long long Na, long long Nb, int* cand, float* cand_val, float* block_max) {
+  DistParams dp;
+  memset(&dp, 0, sizeof(dp));
+  dp.side[0].cand = cand;
+  dp.side[0].cand_val = cand_val;
+  dp.side[0].block_max = block_max;
+  dp.side[0].n_row_blocks = static_cast<int>((Na + 31) / 32);
+  dp.side[0].Na = Na;
+  dp.side[0].Nb = Nb;
+  dp.k_blocks = f8 ? 1 : 2;
+  dp.form = HN_FORM_FDL;
+  dp.dot_scale = kDotScale;
+  return dp;
 }
 
 template <int MB, int EPI, bool F8 = false>
@@ -676,6 +696,42 @@ static ExactWs carve_exact(void* ws, long long Na, long long Np) {
   w.pos = reinterpret_cast<float*>(take(static_cast<size_t>(std::max(Na, Np)) * 4));
   w.row_pack = reinterpret_cast<unsigned long long*>(take(static_cast<size_t>(Na) * 8));
   w.col_pack = reinterpret_cast<unsigned long long*>(take(static_cast<size_t>(Np) * 8));
+  w.bytes = off;
+  return w;
+}
+
+// Workspace of a matching call: carve_match (hn_match, hn_match_mutual) or carve_batched (hn_match_batched, hn_match_pairs).
+struct MatchWs {
+  void *q16, *g16;           // packed operand slots of 256 bytes per row (fp16; e4m3 operands use the first half of each)
+  int* cand;
+  float* cand_val;
+  float* block_max;          // mutual only
+  unsigned long long* claim;
+  unsigned char* beaten;
+  float* rb_min_d2;
+  size_t bytes;
+};
+
+// hn_match: packed operands and candidate lists [Nq][<= 16 segments][2 lists in the CTA-pair kernel][kTopC]. One workspace
+// serves this layout and carve_exact (hn_dist_workspace_bytes), plus 256 bytes. with_mutual (hn_match_mutual): the column side's
+// cell maxima, claims, beaten flags and row blocks' minimum d2 follow that size, plus 256 bytes.
+static MatchWs carve_match(void* ws, long long Nq, long long Ng, bool with_mutual) {
+  MatchWs w{};
+  char* b = static_cast<char*>(ws);
+  size_t off = 0;
+  auto take = [&](size_t n) { char* r = b ? b + off : nullptr; off += align256(n); return r; };
+  w.q16 = take(static_cast<size_t>(Nq) * 128 * 2);
+  w.g16 = take(static_cast<size_t>(Ng) * 128 * 2);
+  w.cand = reinterpret_cast<int*>(take(static_cast<size_t>(Nq) * 32 * kTopC * 4));
+  w.cand_val = reinterpret_cast<float*>(take(static_cast<size_t>(Nq) * 32 * kTopC * 4));
+  off = std::max(off, carve_exact(nullptr, Nq, Ng).bytes) + 256;
+  if (with_mutual) {
+    w.block_max = reinterpret_cast<float*>(take(static_cast<size_t>(hn_block_max_elems(Nq, Ng)) * 4));
+    w.claim = reinterpret_cast<unsigned long long*>(take(static_cast<size_t>(Ng) * 8));
+    w.beaten = reinterpret_cast<unsigned char*>(take(static_cast<size_t>(Ng)));
+    w.rb_min_d2 = reinterpret_cast<float*>(take(static_cast<size_t>((Nq + 31) / 32) * 4));
+    off += 256;
+  }
   w.bytes = off;
   return w;
 }
@@ -748,8 +804,8 @@ static int run_exact(const float* a, const float* p, long long Na, long long Np,
   if (swap) HN_CUDA(cudaMemsetAsync(w.col_pack, 0xff, static_cast<size_t>(Np) * 8, s));
   DistParams dp;
   memset(&dp, 0, sizeof(dp));
-  HN_TRY(make_desc_map(&dp.side[0].tmA, w.a16, Na, 384));
-  HN_TRY(make_desc_map(&dp.side[0].tmB, w.p16, Np, 384));
+  HN_TRY(make_operand_map(&dp.side[0].tmA, w.a16, false, 384, Na, 0, kDistTile));
+  HN_TRY(make_operand_map(&dp.side[0].tmB, w.p16, false, 384, Np, 0, kDistTile));
   dp.side[0].norm_a = w.na;
   dp.side[0].norm_b = w.np;
   dp.side[0].row_pack = w.row_pack;
@@ -792,10 +848,7 @@ using namespace hn;
 extern "C" long long hn_dist_workspace_bytes(long long Na, long long Np, int split) {
   if (Na < 0 || Np < 0) return 0;
   (void)split;
-  ExactWs w = carve_exact(nullptr, Na, Np);
-  const size_t shortlist = align256(static_cast<size_t>(Na) * 128 * 2) + align256(static_cast<size_t>(Np) * 128 * 2) +
-                           2 * align256(static_cast<size_t>(Na) * 32 * kTopC * 4);
-  return static_cast<long long>(std::max(w.bytes, shortlist) + 256);
+  return static_cast<long long>(carve_match(nullptr, Na, Np, false).bytes);
 }
 
 extern "C" int hn_dist_min_ex(const float* a, const float* p, long long Na, long long Np, int form, int flags, const float* a_xy,
@@ -892,47 +945,26 @@ extern "C" int hn_pack_descriptors_multicast(const float* x, long long n, void* 
 // The launch sequence of hn_match_ex / hn_match_typed on validated arguments.
 template <typename T>
 static int run_match(const T* q, const T* g, const void* q16_in, const void* g16_in, long long Nq, long long Ng, long long g_offset,
-                     float* d1, float* d2, int32_t* i1, int32_t* i2, float* block_max, void* workspace, void* g_ready_event,
+                     float* d1, float* d2, int32_t* i1, int32_t* i2, float* block_max, const MatchWs& w, void* g_ready_event,
                      cudaStream_t s) {
   int sm = 0;
   HN_TRY(device_sm_count(&sm));
   constexpr bool F8 = kF8Rows<T>;
-  char* b = static_cast<char*>(workspace);
-  // packed operand slots of 256 bytes per row (fp16); e4m3 operands use the first half of each
-  void* q16 = b;
-  void* g16 = b + align256(static_cast<size_t>(Nq) * 256);
-  int* cand = reinterpret_cast<int*>(b + align256(static_cast<size_t>(Nq) * 256) + align256(static_cast<size_t>(Ng) * 256));
-  float* cand_val = reinterpret_cast<float*>(reinterpret_cast<char*>(cand) + align256(static_cast<size_t>(Nq) * 32 * kTopC * 4));
+  const void* q16 = q16_in ? q16_in : w.q16;
+  const void* g16 = g16_in ? g16_in : w.g16;
   {
     MatchTimer timer(0, s);
-    if (q16_in) q16 = const_cast<void*>(q16_in);
-    else launch_pack(q, Nq, q16, 0, s);
-    if (g16_in) g16 = const_cast<void*>(g16_in);
-    else launch_pack(g, Ng, g16, 1, s);
+    if (!q16_in) launch_pack(q, Nq, w.q16, 0, s);
+    if (!g16_in) launch_pack(g, Ng, w.g16, 1, s);
     HN_CUDA(cudaGetLastError());
     count_launch((q16_in ? 0 : 1) + (g16_in ? 0 : 1));
   }
-  DistParams dp;
-  memset(&dp, 0, sizeof(dp));
+  DistParams dp = shortlist_params(F8, Nq, Ng, w.cand, w.cand_val, block_max);
   // CTA pairs (tc_dist_pair.cuh) once the problem is large enough to fill the machine with 512-row query blocks
   const int pair_mode = match_kernel_mode();
   const bool use_pair = pair_mode >= 0 ? pair_mode != 0 : (Nq >= 8192 && Ng >= 1024);
-  if (F8) {
-    HN_TRY(make_desc_map_f8(&dp.side[0].tmA, static_cast<const uint8_t*>(q16), Nq));
-    HN_TRY(make_desc_map_f8(&dp.side[0].tmB, static_cast<const uint8_t*>(g16), Ng, use_pair ? 64 : kDistTile));
-  } else {
-    HN_TRY(make_desc_map(&dp.side[0].tmA, static_cast<const uint16_t*>(q16), Nq, 128));
-    HN_TRY(make_desc_map(&dp.side[0].tmB, static_cast<const uint16_t*>(g16), Ng, 128, use_pair ? 64 : kDistTile));
-  }
-  dp.side[0].cand = cand;
-  dp.side[0].cand_val = cand_val;
-  dp.side[0].block_max = block_max;
-  dp.side[0].n_row_blocks = static_cast<int>((Nq + 31) / 32);
-  dp.side[0].Na = Nq;
-  dp.side[0].Nb = Ng;
-  dp.k_blocks = F8 ? 1 : 2;
-  dp.form = HN_FORM_FDL;
-  dp.dot_scale = kDotScale;
+  HN_TRY(make_operand_map(&dp.side[0].tmA, q16, F8, 128, Nq, 0, kDistTile));
+  HN_TRY(make_operand_map(&dp.side[0].tmB, g16, F8, 128, Ng, 0, use_pair ? 64 : kDistTile));
   {
     MatchTimer timer(1, s);
     if (use_pair) {
@@ -958,7 +990,7 @@ static int run_match(const T* q, const T* g, const void* q16_in, const void* g16
   {
     MatchTimer timer(2, s);
     // the CTA-pair kernel keeps two top-kTopC lists per row and segment (one per 64-column half of its tiles)
-    rerank_kernel<<<static_cast<unsigned>((Nq + 3) / 4), 128, 0, s>>>(q, g, cand, cand_val, kRerankMargin, Nq, Ng,
+    rerank_kernel<<<static_cast<unsigned>((Nq + 3) / 4), 128, 0, s>>>(q, g, w.cand, w.cand_val, kRerankMargin, Nq, Ng,
                                                                      dp.segments * kTopC * (use_pair ? 2 : 1), g_offset, d1, d2, i1, i2);
     HN_CUDA(cudaGetLastError());
     count_launch();
@@ -981,7 +1013,7 @@ static int match_entry(const char* fn, const void* q, const void* g, int desc_dt
   return with_rows(desc_dtype, [&](auto t) -> int {
     using T = decltype(t);
     return run_match(static_cast<const T*>(q), static_cast<const T*>(g), q16_in, g16_in, Nq, Ng, g_offset, d1, d2, i1, i2, block_max,
-                     workspace, g_ready_event, static_cast<cudaStream_t>(stream));
+                     carve_match(workspace, Nq, Ng, false), g_ready_event, static_cast<cudaStream_t>(stream));
   });
 }
 
@@ -1043,9 +1075,7 @@ extern "C" int hn_mutual_verify(const float* q, long long Nq, long long q_offset
 
 extern "C" long long hn_mutual_workspace_bytes(long long Nq, long long Ng) {
   if (Nq < 0 || Ng < 0) return 0;
-  return hn_dist_workspace_bytes(Nq, Ng, 0) + static_cast<long long>(align256(static_cast<size_t>(hn_block_max_elems(Nq, Ng)) * 4) +
-                                                                         align256(static_cast<size_t>(Ng) * 8) + align256(static_cast<size_t>(Ng)) +
-                                                                         align256(static_cast<size_t>((Nq + 31) / 32) * 4) + 256);
+  return static_cast<long long>(carve_match(nullptr, Nq, Ng, true).bytes);
 }
 
 // hn_match_mutual / hn_match_mutual_typed; fn names the entry point in error messages.
@@ -1055,25 +1085,18 @@ static int mutual_entry(const char* fn, const void* q, const void* g, int desc_d
   HN_REQUIRE(q && g && d1 && d2 && i1 && mutual && workspace, "%s: NULL argument (d1, d2, i1 and mutual are required outputs)", fn);
   HN_TRY(check_rows(fn, desc_dtype, q, g));
   HN_REQUIRE(workspace_bytes >= hn_mutual_workspace_bytes(Nq, Ng), "%s: workspace too small", fn);
+  HN_REQUIRE(Nq >= 1 && Ng >= 1, "%s: empty input (Nq=%lld, Ng=%lld)", fn, Nq, Ng);   // sizes the carve below relies on
   cudaStream_t s = static_cast<cudaStream_t>(stream);
-  const long long base = hn_dist_workspace_bytes(Nq, Ng, 0);
-  char* b = static_cast<char*>(workspace) + align256(static_cast<size_t>(base));
-  float* bm = reinterpret_cast<float*>(b);
-  b += align256(static_cast<size_t>(hn_block_max_elems(Nq, Ng)) * 4);
-  unsigned long long* claim = reinterpret_cast<unsigned long long*>(b);
-  b += align256(static_cast<size_t>(Ng) * 8);
-  unsigned char* beaten = reinterpret_cast<unsigned char*>(b);
-  b += align256(static_cast<size_t>(Ng));
-  float* rbmin = reinterpret_cast<float*>(b);
-  HN_TRY(match_entry(fn, q, g, desc_dtype, q16, g16, Nq, Ng, 0, d1, d2, i1, i2, bm, workspace, base, nullptr, stream));
-  HN_CUDA(cudaMemsetAsync(claim, 0x7f, static_cast<size_t>(Ng) * 8, s));   // "unclaimed"
-  HN_CUDA(cudaMemsetAsync(beaten, 0, static_cast<size_t>(Ng), s));
-  HN_TRY(hn_mutual_claims(i1, d1, d2, Nq, 0, claim, Ng, rbmin, stream));
+  const MatchWs w = carve_match(workspace, Nq, Ng, true);
+  HN_TRY(match_entry(fn, q, g, desc_dtype, q16, g16, Nq, Ng, 0, d1, d2, i1, i2, w.block_max, workspace, workspace_bytes, nullptr, stream));
+  HN_CUDA(cudaMemsetAsync(w.claim, 0x7f, static_cast<size_t>(Ng) * 8, s));   // "unclaimed"
+  HN_CUDA(cudaMemsetAsync(w.beaten, 0, static_cast<size_t>(Ng), s));
+  HN_TRY(hn_mutual_claims(i1, d1, d2, Nq, 0, w.claim, Ng, w.rb_min_d2, stream));
   HN_TRY(with_rows(desc_dtype, [&](auto t) -> int {
     using T = decltype(t);
-    return launch_verify(static_cast<const T*>(q), Nq, 0, static_cast<const T*>(g), Ng, claim, bm, rbmin, beaten, s);
+    return launch_verify(static_cast<const T*>(q), Nq, 0, static_cast<const T*>(g), Ng, w.claim, w.block_max, w.rb_min_d2, w.beaten, s);
   }));
-  mutual_final_kernel<<<static_cast<unsigned>((Nq + 255) / 256), 256, 0, s>>>(i1, Nq, 0, claim, beaten, Ng, mutual);
+  mutual_final_kernel<<<static_cast<unsigned>((Nq + 255) / 256), 256, 0, s>>>(i1, Nq, 0, w.claim, w.beaten, Ng, mutual);
   HN_CUDA(cudaGetLastError());
   count_launch();
   return HN_OK;
@@ -1096,34 +1119,19 @@ extern "C" int hn_match_mutual_typed(const void* q, const void* g, int desc_dtyp
 // batched matching: B problems in one launch sequence, padded (hn_match_batched) or over row ranges of concatenated sets
 // (hn_match_pairs)
 // ------------------------------------------------------------------------------------------------------------
-struct BatchedWs {
-  uint16_t *q16, *g16;       // hn_match_batched only: its packed operands (fp16; e4m3 rows use the first half of each slot)
-  int* cand;
-  float* cand_val;
-  float* block_max;          // mutual only
-  unsigned long long* claim;
-  unsigned char* beaten;
-  float* rb_min_d2;
-  size_t bytes;
-};
-
 // Nq / Ng: the per-pair maxima (output pitch). with_packed: room for B*Nq and B*Ng packed rows in front (hn_match_batched).
-static BatchedWs carve_batched(void* ws, long long B, long long Nq, long long Ng, bool with_mutual, bool with_packed) {
-  BatchedWs w;
+static MatchWs carve_batched(void* ws, long long B, long long Nq, long long Ng, bool with_mutual, bool with_packed) {
+  MatchWs w{};
   char* b = static_cast<char*>(ws);
   size_t off = 0;
   auto take = [&](size_t n) { char* r = b ? b + off : nullptr; off += align256(n); return r; };
   const size_t rows_q = static_cast<size_t>(B) * Nq, rows_g = static_cast<size_t>(B) * Ng;
-  w.q16 = with_packed ? reinterpret_cast<uint16_t*>(take(rows_q * 128 * 2)) : nullptr;
-  w.g16 = with_packed ? reinterpret_cast<uint16_t*>(take(rows_g * 128 * 2)) : nullptr;
+  w.q16 = with_packed ? take(rows_q * 128 * 2) : nullptr;
+  w.g16 = with_packed ? take(rows_g * 128 * 2) : nullptr;
   // candidate lists [rows][segments][kTopC]: a segment holds at least one gallery tile, so at most min(16, tiles) of them
   const size_t lists = rows_q * batched_max_segments(Ng) * kTopC * 4;
   w.cand = reinterpret_cast<int*>(take(lists));
   w.cand_val = reinterpret_cast<float*>(take(lists));
-  w.block_max = nullptr;
-  w.claim = nullptr;
-  w.beaten = nullptr;
-  w.rb_min_d2 = nullptr;
   if (with_mutual) {
     w.block_max = reinterpret_cast<float*>(take(static_cast<size_t>(B) * hn_block_max_elems(Nq, Ng) * 4));
     w.claim = reinterpret_cast<unsigned long long*>(take(rows_g * 8));
@@ -1132,16 +1140,6 @@ static BatchedWs carve_batched(void* ws, long long B, long long Nq, long long Ng
   }
   w.bytes = off;
   return w;
-}
-
-// {K = 128, N, B} 16-bit operand rows, box {64, 128, 1}: a box never reaches into the next pair, TMA zero-fills past N.
-// F8: e4m3 operand rows, box {128, 128, 1}.
-static int make_batched_desc_map(CUtensorMap* tm, const void* base, long long rows, long long B, bool f8) {
-  const uint64_t esz = f8 ? 1 : 2;
-  const uint64_t dims[3] = {128, static_cast<uint64_t>(rows), static_cast<uint64_t>(B)};
-  const uint64_t str[2] = {128 * esz, static_cast<uint64_t>(rows) * 128 * esz};
-  const uint32_t box[3] = {f8 ? 128u : 64u, static_cast<uint32_t>(kDistTile), 1};
-  return f8 ? make_tmap_8bit(tm, base, 3, dims, str, box, 128) : make_tmap_16bit(tm, base, 3, dims, str, box, 128);
 }
 
 // Where the pairs of a batched call live. With `pairs` (hn_match_pairs): row ranges [B][4] = (q_start, q_len, g_start, g_len)
@@ -1158,33 +1156,16 @@ struct PairLayout {
 // side. q16 / g16 are the packed rows of q / g.
 template <bool TABLE, typename T>
 static int run_pairs(const T* q, const void* q16, const T* g, const void* g16, const PairLayout& L, float* d1,
-                     float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, const BatchedWs& w, cudaStream_t s) {
+                     float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, const MatchWs& w, cudaStream_t s) {
   constexpr bool F8 = kF8Rows<T>;
   int sm = 0;
   HN_TRY(device_sm_count(&sm));
   const long long B = L.B, Nq = L.max_q, Ng = L.max_g, rows_q = B * Nq, rows_g = B * Ng;
   const int threads = 256;
-  DistParams dp;
-  memset(&dp, 0, sizeof(dp));
-  if (TABLE && F8) {
-    HN_TRY(make_desc_map_f8(&dp.side[0].tmA, static_cast<const uint8_t*>(q16), L.q_rows));
-    HN_TRY(make_desc_map_f8(&dp.side[0].tmB, static_cast<const uint8_t*>(g16), L.g_rows));
-  } else if (TABLE) {
-    HN_TRY(make_desc_map(&dp.side[0].tmA, static_cast<const uint16_t*>(q16), L.q_rows, 128));
-    HN_TRY(make_desc_map(&dp.side[0].tmB, static_cast<const uint16_t*>(g16), L.g_rows, 128));
-  } else {
-    HN_TRY(make_batched_desc_map(&dp.side[0].tmA, q16, Nq, B, F8));
-    HN_TRY(make_batched_desc_map(&dp.side[0].tmB, g16, Ng, B, F8));
-  }
-  dp.side[0].cand = w.cand;
-  dp.side[0].cand_val = w.cand_val;
-  dp.side[0].block_max = w.block_max;
-  dp.side[0].n_row_blocks = static_cast<int>((Nq + 31) / 32);
-  dp.side[0].Na = Nq;
-  dp.side[0].Nb = Ng;
-  dp.k_blocks = F8 ? 1 : 2;
-  dp.form = HN_FORM_FDL;
-  dp.dot_scale = kDotScale;
+  DistParams dp = shortlist_params(F8, Nq, Ng, w.cand, w.cand_val, w.block_max);
+  // the table form's maps run over the concatenated sets, the padded form's over [B][N] rows
+  HN_TRY(make_operand_map(&dp.side[0].tmA, q16, F8, 128, TABLE ? L.q_rows : Nq, TABLE ? 0 : B, kDistTile));
+  HN_TRY(make_operand_map(&dp.side[0].tmB, g16, F8, 128, TABLE ? L.g_rows : Ng, TABLE ? 0 : B, kDistTile));
   dp.q_len = L.q_len;
   dp.g_len = L.g_len;
   dp.batch = static_cast<int>(B);
@@ -1235,7 +1216,7 @@ extern "C" long long hn_match_batched_workspace_bytes(long long B, long long Nq,
 template <typename T>
 static int run_batched(const T* q, const T* g, long long B, long long Nq, long long Ng, const int32_t* q_len, const int32_t* g_len,
                        float* d1, float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace, cudaStream_t s) {
-  const BatchedWs w = carve_batched(workspace, B, Nq, Ng, mutual != nullptr, true);
+  const MatchWs w = carve_batched(workspace, B, Nq, Ng, mutual != nullptr, true);
   const long long rows_q = B * Nq, rows_g = B * Ng;
   {
     MatchTimer timer(0, s);
@@ -1299,7 +1280,7 @@ static int pairs_entry(const char* fn, const void* q, const void* q16, long long
              "%s: packed operands must be 16-byte aligned", fn);
   HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "%s: workspace must be 256-byte aligned", fn);
   HN_REQUIRE(workspace_bytes >= hn_match_pairs_workspace_bytes(B, max_q, max_g, mutual != nullptr), "%s: workspace too small", fn);
-  const BatchedWs w = carve_batched(workspace, B, max_q, max_g, mutual != nullptr, false);
+  const MatchWs w = carve_batched(workspace, B, max_q, max_g, mutual != nullptr, false);
   const PairLayout L = {pairs, nullptr, nullptr, B, max_q, max_g, Nq_rows, Ng_rows};
   return with_rows(desc_dtype, [&](auto t) -> int {
     using T = decltype(t);

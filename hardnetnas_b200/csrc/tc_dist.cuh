@@ -127,6 +127,15 @@ __device__ __forceinline__ float warp_chunk_max8(const float (&c)[8], int lane) 
   return v;
 }
 
+// A row's candidate list (one segment; in the CTA-pair kernel one 64-column half of it) at list index `list` of cand /
+// cand_val: the kTopC chunk ids, -1 in unused slots (a segment with fewer than kTopC chunks), and the chunks' maxima.
+__device__ __forceinline__ void store_cand_list(int* cand, float* cand_val, long long list, const float (&tb)[kTopC],
+                                                const int (&tc)[kTopC]) {
+  *reinterpret_cast<int4*>(cand + list * kTopC) = make_int4(tb[0] > -3.0e38f ? tc[0] : -1, tb[1] > -3.0e38f ? tc[1] : -1,
+                                                            tb[2] > -3.0e38f ? tc[2] : -1, tb[3] > -3.0e38f ? tc[3] : -1);
+  *reinterpret_cast<float4*>(cand_val + list * kTopC) = make_float4(tb[0], tb[1], tb[2], tb[3]);
+}
+
 // Epilogue warps per accumulator lane quarter. The exact epilogues (loss kernels) cost ~80 instructions per column and a loss-sized
 // problem (N = 1024) gives every CTA exactly ONE 128 x 128 tile: with one warp per quarter a thread walked 128 columns alone
 // (~10 k dependent instructions = 13 us of a 28 us kernel). Four warps per quarter take 32 columns each and merge through the
@@ -377,8 +386,8 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
         mbar_wait(tfull_bar(acc), acc_phase);
         tc_fence_after();
         const uint32_t t_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + (acc * MB + mb) * kDistTile;
-        const bool ragged = col0 + kDistTile > cols();
         if (SHORTLIST) {
+          const bool ragged = col0 + kDistTile > cols();
           // all four TMEM loads are issued before the single wait: one exposed round trip per tile instead of four
           uint32_t r[4][32];
 #pragma unroll
@@ -426,15 +435,14 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
             }
           }
         } else {
-        // NOT unrolled: the exact epilogue is ~80 instructions per column and a loss-sized problem (N = 1024) runs it ONCE per CTA,
-        // so four unrolled copies were 10 k instructions of straight-line code fetched cold - the instruction fetch (stall reason
-        // no_inst in ncu) was most of the kernel's 28 us; one copy of the 32-column body stays in the instruction cache.
+          // NOT unrolled: the exact epilogue is ~80 instructions per column and a loss-sized problem (N = 1024) runs it ONCE per CTA,
+          // so four unrolled copies were 10 k instructions of straight-line code fetched cold - the instruction fetch (stall reason
+          // no_inst in ncu) was most of the kernel's 28 us; one copy of the 32-column body stays in the instruction cache.
 #pragma unroll 1
-        for (int c0 = CS == 1 ? 0 : cs * 32; c0 < (CS == 1 ? kDistTile : cs * 32 + 32); c0 += 32) {
-          uint32_t r[32];
-          tmem_ld32(t_row + c0, r);
-          tmem_ld_wait();
-          if (EXACT) {
+          for (int c0 = CS == 1 ? 0 : cs * 32; c0 < (CS == 1 ? kDistTile : cs * 32 + 32); c0 += 32) {
+            uint32_t r[32];
+            tmem_ld32(t_row + c0, r);
+            tmem_ld_wait();
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
               const long long col = col0 + c0 + j;
@@ -470,31 +478,7 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
               }
               if (col < sd.Nb && d < best) { best = d; best_col = static_cast<int>(col); }
             }
-          } else {
-            float v[32];
-#pragma unroll
-            for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
-            if (ragged) {
-#pragma unroll
-              for (int j = 0; j < 32; ++j)
-                if (col0 + c0 + j >= sd.Nb) v[j] = -__int_as_float(0x7f800000);
-            }
-#pragma unroll
-            for (int s = 0; s < 32 / kChunk; ++s) {
-              const float* w = v + s * kChunk;
-              const float m = fmaxf(max3(w[0], w[1], w[2]), max3(max3(w[3], w[4], w[5]), w[6], w[7]));
-              if (m > tb[kTopC - 1]) {
-                const int id = static_cast<int>((col0 + c0) / kChunk) + s;
-                // sorted insert (descending); strict '>' keeps the earlier chunk on ties
-                const bool g0 = m > tb[0], g1 = m > tb[1], g2 = m > tb[2];
-                tb[3] = g2 ? tb[2] : m;               tc[3] = g2 ? tc[2] : id;
-                tb[2] = g2 ? (g1 ? tb[1] : m) : tb[2]; tc[2] = g2 ? (g1 ? tc[1] : id) : tc[2];
-                tb[1] = g1 ? (g0 ? tb[0] : m) : tb[1]; tc[1] = g1 ? (g0 ? tc[0] : id) : tc[1];
-                tb[0] = g0 ? m : tb[0];               tc[0] = g0 ? id : tc[0];
-              }
-            }
           }
-        }
         }
         tc_fence_before();
         __syncwarp();
@@ -510,11 +494,7 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
           }
         } else {
           const long long out_row = BATCHED ? pair * sd.Na + row : row;   // chunk ids stay local to the pair
-          int4* dst = reinterpret_cast<int4*>(sd.cand + (out_row * p.segments + seg) * kTopC);
-          // unused slots (segment with < kTopC chunks) are marked -1
-          *dst = make_int4(tb[0] > -3.0e38f ? tc[0] : -1, tb[1] > -3.0e38f ? tc[1] : -1, tb[2] > -3.0e38f ? tc[2] : -1,
-                           tb[3] > -3.0e38f ? tc[3] : -1);
-          *reinterpret_cast<float4*>(sd.cand_val + (out_row * p.segments + seg) * kTopC) = make_float4(tb[0], tb[1], tb[2], tb[3]);
+          store_cand_list(sd.cand, sd.cand_val, out_row * p.segments + seg, tb, tc);
         }
       }
     }

@@ -240,12 +240,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kMpThreads, 1) match
           if ((lane & 3) == 0 && cb * kChunk < sd.Nb && rb < sd.n_row_blocks) sd.block_max[cb * sd.n_row_blocks + rb] = bm;
         }
       }
-      if (row_ok) {
-        int4* dst = reinterpret_cast<int4*>(sd.cand + ((row * p.segments + seg) * 2 + half) * kTopC);
-        *dst = make_int4(tb[0] > -3.0e38f ? tc[0] : -1, tb[1] > -3.0e38f ? tc[1] : -1, tb[2] > -3.0e38f ? tc[2] : -1,
-                         tb[3] > -3.0e38f ? tc[3] : -1);
-        *reinterpret_cast<float4*>(sd.cand_val + ((row * p.segments + seg) * 2 + half) * kTopC) = make_float4(tb[0], tb[1], tb[2], tb[3]);
-      }
+      if (row_ok) store_cand_list(sd.cand, sd.cand_val, (row * p.segments + seg) * 2 + half, tb, tc);
     }
   }
 
