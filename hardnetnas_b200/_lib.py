@@ -64,6 +64,13 @@ SIGNATURES = {
                                          C.c_longlong, _P]),
     "hn_match_pairs_typed": (C.c_int, [_P, _P, C.c_longlong, _P, _P, C.c_longlong, C.c_int, _P, C.c_longlong, C.c_longlong,
                                        C.c_longlong, _P, _P, _P, _P, _P, _P, C.c_longlong, _P]),
+    "hn_match_topk_workspace_bytes": (C.c_longlong, [C.c_longlong, C.c_longlong]),
+    "hn_match_topk_typed": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_longlong, C.c_longlong, C.c_int, _P, _P, _P, C.c_longlong, _P]),
+    "hn_match_pairs_topk_workspace_bytes": (C.c_longlong, [C.c_longlong, C.c_longlong, C.c_longlong]),
+    "hn_match_pairs_topk_typed": (C.c_int, [_P, _P, C.c_longlong, _P, _P, C.c_longlong, C.c_int, _P, C.c_longlong, C.c_longlong,
+                                            C.c_longlong, C.c_int, _P, _P, _P, C.c_longlong, _P]),
+    "hn_match_topk_fallback_enable": (C.c_int, [C.c_int]),
+    "hn_match_topk_fallback_read": (C.c_int, [C.POINTER(C.c_longlong)]),
     "hn_match_profile_enable": (C.c_int, [C.c_int]),
     "hn_match_profile_read": (C.c_int, [C.POINTER(C.c_double), C.POINTER(C.c_longlong)]),
     "hn_pair_distances": (C.c_int, [_P, _P, C.c_longlong, _P, _P]),

@@ -242,6 +242,29 @@ def _packed(name: str, t: torch.Tensor, n: int, desc_dtype: int) -> torch.Tensor
     return t
 
 
+def _pair_operands(name: str, q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, q16: torch.Tensor | None,
+                   g16: torch.Tensor | None):
+    """(q, g, desc_dtype, device int32 table, q16, g16) of a pair-table call: rows as _desc_rows, the sets packed here unless
+    their packed rows are given (once when g is q), packed rows checked against the rows."""
+    same = g is q
+    if same:
+        q, _, dt = _desc_rows(_require_cuda_desc(name, q))
+        g = q
+    else:
+        q, g, dt = _desc_rows(_require_cuda_desc(name, q), _require_cuda_desc(name, g))
+    if not isinstance(pairs, torch.Tensor) or pairs.dtype not in (torch.int32, torch.int64) or pairs.dim() != 2 or pairs.size(1) != 4:
+        raise ValueError(f"{name}: pairs must be an int32 or int64 [P, 4] tensor of (q_start, q_len, g_start, g_len)")
+    dev = q.device
+    if g.device != dev:
+        raise ValueError(f"{name}: q and g must be on the same device")
+    table = pairs.to(device=dev, dtype=torch.int32).contiguous()
+    if q16 is None:
+        q16 = g16 if same and g16 is not None else pack_descriptors(q)
+    if g16 is None:
+        g16 = q16 if same else pack_descriptors(g)
+    return q, g, dt, table, _packed(name, q16, q.size(0), dt), _packed(name, g16, g.size(0), dt)
+
+
 def match_pairs(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, max_q: int, max_g: int, q16: torch.Tensor | None = None,
                 g16: torch.Tensor | None = None, mutual: bool = False):
     """(d1, d2, i1, i2[, mutual]), each [P, max_q]: hn_match_pairs over the concatenated sets q [Nq_rows, 128] and
@@ -250,24 +273,9 @@ def match_pairs(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, max_q: in
     whose packed rows are not given is packed here (per row dtype, see pack_descriptors), once when g is q. Indices are local to the pair's gallery range; rows past
     q_len get d = +inf, i = -1 (and mutual = False). Rows as in match_top2 (hn_match_pairs_typed)."""
     lib = _lib.load()
-    same = g is q
-    if same:
-        q, _, dt = _desc_rows(_require_cuda_desc("match_pairs", q))
-        g = q
-    else:
-        q, g, dt = _desc_rows(_require_cuda_desc("match_pairs", q), _require_cuda_desc("match_pairs", g))
-    if not isinstance(pairs, torch.Tensor) or pairs.dtype not in (torch.int32, torch.int64) or pairs.dim() != 2 or pairs.size(1) != 4:
-        raise ValueError("match_pairs: pairs must be an int32 or int64 [P, 4] tensor of (q_start, q_len, g_start, g_len)")
-    dev = q.device
-    if g.device != dev:
-        raise ValueError("match_pairs: q and g must be on the same device")
-    table = pairs.to(device=dev, dtype=torch.int32).contiguous()
+    q, g, dt, table, q16, g16 = _pair_operands("match_pairs", q, g, pairs, q16, g16)
     nq, ng, b = q.size(0), g.size(0), table.size(0)
-    if q16 is None:
-        q16 = g16 if same and g16 is not None else pack_descriptors(q)
-    if g16 is None:
-        g16 = q16 if same else pack_descriptors(g)
-    q16, g16 = _packed("match_pairs", q16, nq, dt), _packed("match_pairs", g16, ng, dt)
+    dev = q.device
     with torch.cuda.device(dev):
         ws = _workspace(dev, max(lib.hn_match_pairs_workspace_bytes(b, max_q, max_g, int(mutual)), 1))
         d1 = torch.empty((b, max_q), dtype=torch.float32, device=dev)
@@ -279,6 +287,53 @@ def match_pairs(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, max_q: in
                                             _ptr(d1), _ptr(d2), _ptr(i1), _ptr(i2), _ptr(mu), _ptr(ws), ws.numel(), _stream_ptr()),
                    "hn_match_pairs_typed")
     return (d1, d2, i1, i2, mu) if mutual else (d1, d2, i1, i2)
+
+
+TOPK_MAX = 8
+
+
+def _check_k(name: str, k) -> int:
+    if isinstance(k, bool) or not isinstance(k, int) or not 1 <= k <= TOPK_MAX:
+        raise ValueError(f"{name}: k must be an integer in [1, {TOPK_MAX}], got {k!r}")
+    return k
+
+
+def match_topk(q: torch.Tensor, g: torch.Tensor, k: int, q16: torch.Tensor | None = None, g16: torch.Tensor | None = None):
+    """(dist [Nq, k] fp32, idx [Nq, k] int32): the k nearest gallery rows per query, sorted by (distance, index), exact
+    (hn_match_topk_typed). Rows and packed operands as in match_top2; missing slots (Ng < k) are +inf / -1."""
+    k = _check_k("match_topk", k)
+    lib = _lib.load()
+    q, g, dt = _desc_rows(_require_cuda_desc("match_topk", q), _require_cuda_desc("match_topk", g))
+    nq, ng = q.size(0), g.size(0)
+    for t, n in ((q16, nq), (g16, ng)):
+        if t is not None:
+            _packed("match_topk", t, n, dt)
+    dev = q.device
+    with torch.cuda.device(dev):
+        ws = _workspace(dev, lib.hn_match_topk_workspace_bytes(nq, ng))
+        dist = torch.empty((nq, k), dtype=torch.float32, device=dev)
+        idx = torch.empty((nq, k), dtype=torch.int32, device=dev)
+        _lib.check(lib.hn_match_topk_typed(_ptr(q), _ptr(g), dt, _ptr(q16), _ptr(g16), nq, ng, k, _ptr(dist), _ptr(idx), _ptr(ws),
+                                           ws.numel(), _stream_ptr()), "hn_match_topk_typed")
+    return dist, idx
+
+
+def match_pairs_topk(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, k: int, max_q: int, max_g: int,
+                     q16: torch.Tensor | None = None, g16: torch.Tensor | None = None):
+    """(dist, idx), each [P, max_q, k]: hn_match_pairs_topk_typed over the pair table (arguments as in match_pairs)."""
+    k = _check_k("match_pairs_topk", k)
+    lib = _lib.load()
+    q, g, dt, table, q16, g16 = _pair_operands("match_pairs_topk", q, g, pairs, q16, g16)
+    nq, ng, b = q.size(0), g.size(0), table.size(0)
+    dev = q.device
+    with torch.cuda.device(dev):
+        ws = _workspace(dev, max(lib.hn_match_pairs_topk_workspace_bytes(b, max_q, max_g), 1))
+        dist = torch.empty((b, max_q, k), dtype=torch.float32, device=dev)
+        idx = torch.empty((b, max_q, k), dtype=torch.int32, device=dev)
+        _lib.check(lib.hn_match_pairs_topk_typed(_ptr(q), _ptr(q16), nq, _ptr(g), _ptr(g16), ng, dt, _ptr(table), b, max_q, max_g, k,
+                                                 _ptr(dist), _ptr(idx), _ptr(ws), ws.numel(), _stream_ptr()),
+                   "hn_match_pairs_topk_typed")
+    return dist, idx
 
 
 def mutual_claims(i1: torch.Tensor, d1: torch.Tensor, d2: torch.Tensor, q_offset: int, claim: torch.Tensor) -> torch.Tensor:

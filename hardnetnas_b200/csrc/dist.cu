@@ -182,6 +182,37 @@ struct Top2 {
   int i1, i2;
 };
 
+// Exact fp32 distances of the kChunk columns col0 ... col0 + 7 of g to one query row, for a warp whose lane holds elements
+// 4 * lane ... 4 * lane + 3 of that row in qv: lane r < kChunk (and every lane r + 8 j) returns the distance of column col0 + r,
+// for r < left (the columns that exist). The warp reads a gallery row as ONE coalesced 512 B read (lane = float4 index) and
+// finishes the 128-term dot with a butterfly, so every lane holds the same dot products. Per-lane row reads (one lane per
+// candidate) cost 32 L1 wavefronts per row instead of 4. rerank_row and rerank_topk_row both evaluate chunks here, so their
+// distances agree bit for bit.
+template <typename T>
+__device__ __forceinline__ float chunk_distance(float4 qv, const T* g, long long col0, long long left, int lane) {
+  float part[kChunk];
+#pragma unroll
+  for (int r = 0; r < kChunk; ++r) {
+    part[r] = 0.f;
+    if (r < left) {
+      const float4 gv = ldg_row4(g + (col0 + r) * 128, lane);
+      part[r] = fmaf(qv.x, gv.x, fmaf(qv.y, gv.y, fmaf(qv.z, gv.z, qv.w * gv.w)));
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+    for (int r = 0; r < kChunk; ++r) part[r] += __shfl_xor_sync(0xffffffffu, part[r], o);
+  }
+  // The eight distances are taken by eight lanes, one sqrtf each, and shuffled to the warp by the caller (every lane holds the
+  // same eight dot products). Eight unrolled sqrtf per lane are eight slow-path calls, across which the gallery pointer and size
+  // stay live: that made ptxas spill.
+  float mine = part[0];   // part[lane & 7] without a local-memory array access
+#pragma unroll
+  for (int r = 1; r < kChunk; ++r) mine = (lane & (kChunk - 1)) == r ? part[r] : mine;
+  return sqrtf(fminf(fmaxf(2.0f - 2.0f * mine, 1e-8f), 4.0f));
+}
+
 // Exact fp32 re-rank of the shortlisted chunks of one query row: one warp per row, whose staged query row is sqw. crow / cvrow
 // are the row's `slots` candidate chunks and their approximate maxima, g / ng its gallery. Distances in the FDLNet form; ties
 // resolve to the lower gallery index like torch.min / a stable sort. rerank_kernel and rerank_batched_kernel both run this
@@ -195,6 +226,9 @@ struct Top2 {
 // Both re-rank kernels ask for 10 CTAs per SM, i.e. at most 48 registers, which this body fits without spilling. Left to its
 // own choice ptxas spilled 8 bytes in some instantiations to stay within 48 or 56 registers.
 constexpr int kRerankCtasPerSm = 10;
+// gallery segments of the batched GEMM (hn_match_batched) and of the top-k GEMMs: bounds their candidate lists,
+// [rows][segments][kTopC or kTopKC]
+constexpr int kMaxBatchedSegments = 16;
 template <typename T>
 __device__ __forceinline__ Top2 rerank_row(const float* sqw, const T* g, long long ng, const int* crow, const float* cvrow, int slots,
                                            float margin, int lane) {
@@ -219,33 +253,11 @@ __device__ __forceinline__ Top2 rerank_row(const float* sqw, const T* g, long lo
   const float inf = __int_as_float(0x7f800000);
   float b1 = inf, b2 = inf;
   int j1 = 0x7fffffff, j2 = 0x7fffffff;
-  // The warp walks the surviving chunks together: a gallery row is ONE coalesced 512 B read (lane = float4 index) and
-  // the 128-term dot is finished with a butterfly, so every lane ends up with the same (d, index) stream. Per-lane
-  // row reads (one lane per candidate) cost 32 L1 wavefronts per row instead of 4.
+  // the warp walks the surviving chunks together, every lane sees the same (d, index) stream
   const float4 qv = reinterpret_cast<const float4*>(sqw)[lane];
   auto eval_chunk = [&](long long chunk) {
     const long long col0 = chunk * kChunk, left = ng - col0;   // column col0 + r exists iff r < left
-    float part[kChunk];
-#pragma unroll
-    for (int r = 0; r < kChunk; ++r) {
-      part[r] = 0.f;
-      if (r < left) {
-        const float4 gv = ldg_row4(g + (col0 + r) * 128, lane);
-        part[r] = fmaf(qv.x, gv.x, fmaf(qv.y, gv.y, fmaf(qv.z, gv.z, qv.w * gv.w)));
-      }
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-#pragma unroll
-      for (int r = 0; r < kChunk; ++r) part[r] += __shfl_xor_sync(0xffffffffu, part[r], o);
-    }
-    // The eight distances are taken by eight lanes, one sqrtf each, and shuffled to the warp (every lane holds the same eight
-    // dot products). Eight unrolled sqrtf per lane are eight slow-path calls, across which the gallery pointer and size stay
-    // live: that made ptxas spill.
-    float mine = part[0];   // part[lane & 7] without a local-memory array access
-#pragma unroll
-    for (int r = 1; r < kChunk; ++r) mine = (lane & (kChunk - 1)) == r ? part[r] : mine;
-    mine = sqrtf(fminf(fmaxf(2.0f - 2.0f * mine, 1e-8f), 4.0f));
+    const float mine = chunk_distance(qv, g, col0, left, lane);
 #pragma unroll
     for (int r = 0; r < kChunk; ++r) {
       const float d = __shfl_sync(0xffffffffu, mine, r);
@@ -333,6 +345,199 @@ __global__ void __launch_bounds__(128, kRerankCtasPerSm) rerank_batched_kernel(c
     d2[row] = t.d2;
     i2[row] = t.i2 == 0x7fffffff ? -1 : t.i2;
   }
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// k nearest neighbours (hn_match_topk, hn_match_pairs_topk), k <= kTopKMax
+// ------------------------------------------------------------------------------------------------------------
+// The GEMM keeps kTopKC = 8 chunks per row and list (a list = one gallery segment) and each list's dropped maximum: the
+// largest approximate chunk maximum that did not make the list. The re-rank of a row then
+//   - takes M_k, the k-th largest kept chunk maximum over all of the row's lists (-inf with fewer than k kept chunks), and the
+//     threshold thr = M_k - kRerankMargin;
+//   - evaluates every kept chunk whose maximum is >= thr, and
+//   - for every list whose dropped maximum is >= thr evaluates every chunk of that list's column range instead (fallback).
+// Why this is exact. Let eps = 2^-10 bound the error of the approximate (fp16- or e4m3-operand) dot product, as for the
+// margins above (kF8DotBound). The k distinct columns behind the k largest kept maxima have approximate dots >= M_k, hence
+// exact dots >= M_k - eps: the k-th best exact dot is at least M_k - eps, and every column of the exact top-k has an
+// approximate dot >= M_k - 2 eps. A kept chunk, or the dropped part of a list, whose maximum is below M_k - 2 eps therefore
+// holds none of them; whatever holds one is evaluated. The margin is twice that, 4 eps: the second factor of two covers the
+// fp32 summation of the re-rank (its error is some 1e-6 of a dot product) and distances that round to the same fp32 value, so
+// the columns evaluated include the top k of a brute-force fp32 evaluation sorted by (distance, index). Nothing depends on how
+// many of a list's chunks come close: a list whose ninth chunk reaches the threshold is scanned whole, and with up to
+// kMaxBatchedSegments lists per row a scan covers at most 1/16 of the gallery (plus one tile).
+// The running top-k lives in the warp's registers: lane j < k holds the j-th best (distance, column); a candidate finds its
+// place with one ballot and the entries behind it move one lane up with a shuffle.
+constexpr int kTopKMax = 8;
+constexpr int kRerankTopkCtasPerSm = 6;   // up to 80 registers: at 48 (kRerankCtasPerSm) or 64 the top-k re-rank spilled
+static_assert(kMaxBatchedSegments * kTopKC <= 4 * 32, "rerank_topk_row holds a row's list maxima in four registers per lane");
+
+struct TopkEntry {
+  float d;
+  int i;   // 0x7fffffff: fewer columns than that
+};
+
+// One query row (staged in sqw, lanes as rerank_row): its gallery g / ng, its `segments` lists crow / cvrow ([segments][kTopKC])
+// and their dropped maxima drow. Returns the lane's entry of the row's top k; `scanned` tells whether a list was scanned whole.
+template <typename T>
+__device__ __forceinline__ TopkEntry rerank_topk_row(const float* sqw, const T* g, long long ng, const int* crow, const float* cvrow,
+                                                     const float* drow, int segments, int k, float margin, int lane, bool& scanned) {
+  const float inf = __int_as_float(0x7f800000);
+  const int slots = segments * kTopKC;
+  // slot c = lane + 32 j of the row's lists (list c / kTopKC) is held by this lane: chunk id and maximum (-inf: unused)
+  int cid[4];
+  float v[4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const int c = lane + 32 * j;
+    cid[j] = c < slots ? crow[c] : -1;
+    v[j] = cid[j] >= 0 ? cvrow[c] : -inf;
+  }
+  // M_k, counting equal maxima: each round takes the largest value below the previous one and how many slots hold it
+  float mk = -inf, below = inf;
+  int need = k;
+  for (int it = 0; it < k; ++it) {
+    float m = -inf;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) m = v[j] < below ? fmaxf(m, v[j]) : m;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+    if (m == -inf) break;   // fewer than k kept chunks: thr = -inf, every kept chunk is evaluated
+    int cnt = 0;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) cnt += v[j] == m ? 1 : 0;
+    cnt = static_cast<int>(__reduce_add_sync(0xffffffffu, static_cast<unsigned>(cnt)));
+    if (cnt >= need) { mk = m; break; }
+    need -= cnt;
+    below = m;
+  }
+  const float thr = mk - margin;
+  // lists whose dropped maximum reaches the threshold may hide one of the k nearest columns: their whole column range
+  // (seg_range of the GEMM) is evaluated instead of their kept chunks
+  const float dl = lane < segments ? drow[lane] : -inf;
+  const unsigned scan = __ballot_sync(0xffffffffu, dl > -inf && dl >= thr);
+  scanned = scan != 0;
+  unsigned take[4];   // per j, the lanes whose slot j is a kept chunk to evaluate
+#pragma unroll
+  for (int j = 0; j < 4; ++j)
+    take[j] = __ballot_sync(0xffffffffu, cid[j] >= 0 && v[j] >= thr && !((scan >> ((lane + 32 * j) / kTopKC)) & 1u));
+
+  TopkEntry e{inf, 0x7fffffff};
+  const float4 qv = reinterpret_cast<const float4*>(sqw)[lane];
+  auto eval_chunk = [&](long long chunk) {
+    const long long col0 = chunk * kChunk, left = ng - col0;   // column col0 + r exists iff r < left
+    const float mine = chunk_distance(qv, g, col0, left, lane);
+#pragma unroll
+    for (int r = 0; r < kChunk; ++r) {
+      const float d = __shfl_sync(0xffffffffu, mine, r);
+      if (r >= left) continue;
+      const int ci = static_cast<int>(col0) + r;   // ng < 2^31
+      // the entries the candidate precedes in (d, column) order: a suffix of the k lanes, starting at its place
+      const unsigned behind = __ballot_sync(0xffffffffu, lane < k && (d < e.d || (d == e.d && ci < e.i)));
+      if (behind) {   // warp-uniform
+        const int pos = __ffs(behind) - 1;
+        const float ud = __shfl_up_sync(0xffffffffu, e.d, 1);
+        const int ui = __shfl_up_sync(0xffffffffu, e.i, 1);
+        if (lane > pos) e = {ud, ui};
+        else if (lane == pos) e = {d, ci};
+      }
+    }
+  };
+  // One walk over the work, so that eval_chunk has one call site: the kept chunks of take[0..3], then the scanned lists'
+  // ranges. Every branch is warp-uniform.
+  const long long tiles = (ng + kDistTile - 1) / kDistTile, chunks = (ng + kChunk - 1) / kChunk;
+  int j = 0;
+  unsigned lists = scan;
+  long long c = 0, c1 = 0;   // the scanned list's chunks still to evaluate
+  for (;;) {
+    long long chunk;
+    if (j < 4) {
+      const unsigned t = j == 0 ? take[0] : j == 1 ? take[1] : j == 2 ? take[2] : take[3];
+      if (!t) { ++j; continue; }
+      const int src = __ffs(t) - 1;
+      const int held = j == 0 ? cid[0] : j == 1 ? cid[1] : j == 2 ? cid[2] : cid[3];
+      if (j == 0) take[0] &= t - 1; else if (j == 1) take[1] &= t - 1; else if (j == 2) take[2] &= t - 1; else take[3] &= t - 1;
+      chunk = __shfl_sync(0xffffffffu, held, src);
+    } else if (c < c1) {
+      chunk = c++;
+    } else if (lists) {
+      const int l = __ffs(lists) - 1;
+      lists &= lists - 1;
+      c = tiles * l / segments * (kDistTile / kChunk);
+      c1 = std::min(tiles * (l + 1) / segments * (kDistTile / kChunk), chunks);
+      continue;
+    } else {
+      break;
+    }
+    eval_chunk(chunk);
+  }
+  return e;
+}
+
+// Output of one top-k row: lane j < k writes entry j; rows that scanned a list are counted when `fallback_rows` is set.
+__device__ __forceinline__ void store_topk_row(const TopkEntry& e, long long row, int k, bool scanned, float* dist, int* idx,
+                                               unsigned long long* fallback_rows, int lane) {
+  if (lane < k) {
+    dist[row * k + lane] = e.d;
+    idx[row * k + lane] = e.i == 0x7fffffff ? -1 : e.i;
+  }
+  if (fallback_rows && scanned && lane == 0) atomicAdd(fallback_rows, 1ull);
+}
+
+// Re-rank of hn_match_topk: query row `row` of q against g, lists [nq][segments][kTopKC] and dropped maxima [nq][segments].
+template <typename T>
+__global__ void __launch_bounds__(128, kRerankTopkCtasPerSm) rerank_topk_kernel(const T* __restrict__ q, const T* __restrict__ g,
+                                                          const int* __restrict__ cand, const float* __restrict__ cand_val,
+                                                          const float* __restrict__ cand_drop, float margin, long long nq,
+                                                          long long ng, int segments, int k, float* __restrict__ dist,
+                                                          int* __restrict__ idx, unsigned long long* fallback_rows) {
+  __shared__ __align__(16) float sq[4][128];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long row = static_cast<long long>(blockIdx.x) * 4 + w;
+  if (row >= nq) return;
+  reinterpret_cast<float4*>(sq[w])[lane] = ld_row4(q + row * 128, lane);
+  __syncwarp();
+  bool scanned = false;
+  const TopkEntry e = rerank_topk_row(sq[w], g, ng, cand + row * segments * kTopKC, cand_val + row * segments * kTopKC,
+                                      cand_drop + row * segments, segments, k, margin, lane, scanned);
+  store_topk_row(e, row, k, scanned, dist, idx, fallback_rows, lane);
+}
+
+// Re-rank of hn_match_pairs_topk over the flat [B * nq_pad] rows: pair b = row / nq_pad matches query row qs + r of q against
+// gallery rows [gs, gs + gl) of g_all (table_span, as rerank_batched_kernel); rows past the pair's length get +inf / -1.
+template <typename T>
+__global__ void __launch_bounds__(128, kRerankTopkCtasPerSm) rerank_topk_pairs_kernel(const T* __restrict__ q, const T* __restrict__ g_all,
+                                                                const int* __restrict__ cand, const float* __restrict__ cand_val,
+                                                                const float* __restrict__ cand_drop, float margin, long long B,
+                                                                long long nq_pad, long long ng_pad, const int* __restrict__ pairs,
+                                                                long long q_rows, long long g_rows, int segments, int k,
+                                                                float* __restrict__ dist, int* __restrict__ idx,
+                                                                unsigned long long* fallback_rows) {
+  __shared__ __align__(16) float sq[4][128];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long row = static_cast<long long>(blockIdx.x) * 4 + w;
+  if (row >= B * nq_pad) return;
+  const int b = static_cast<int>(row) / static_cast<int>(nq_pad);   // B * nq_pad < 2^31
+  const Span qs = table_span(pairs, b, 0, nq_pad, q_rows), gs = table_span(pairs, b, 1, ng_pad, g_rows);
+  if (row - b * nq_pad >= qs.len) {
+    store_topk_row(TopkEntry{__int_as_float(0x7f800000), 0x7fffffff}, row, k, false, dist, idx, nullptr, lane);
+    return;
+  }
+  reinterpret_cast<float4*>(sq[w])[lane] = ld_row4(q + (qs.start + (row - b * nq_pad)) * 128, lane);
+  __syncwarp();
+  bool scanned = false;
+  const TopkEntry e = rerank_topk_row(sq[w], g_all + gs.start * 128, gs.len, cand + row * segments * kTopKC,
+                                      cand_val + row * segments * kTopKC, cand_drop + row * segments, segments, k, margin, lane,
+                                      scanned);
+  store_topk_row(e, row, k, scanned, dist, idx, fallback_rows, lane);
+}
+
+// Process-wide count of top-k rows that scanned a list (hn_match_topk_fallback_*): off by default (nullptr), else a device word
+// of the device that was current when it was enabled. Not a __device__ variable: that would move the constant-bank addresses
+// every other kernel of this file uses.
+static unsigned long long* g_topk_fallback_rows = nullptr;
+static int topk_fallback_counter(unsigned long long** p) {
+  *p = g_topk_fallback_rows;
+  return HN_OK;
 }
 
 // Optional per-stage CUDA-event timing of hn_match (bench.py: the roofline of the matching GEMM is computed from the kernel's
@@ -627,8 +832,6 @@ static int& match_kernel_mode() {
   return mode;
 }
 
-// gallery segments of the batched GEMM (hn_match_batched): bounds its candidate lists, [rows][segments][kTopC]
-constexpr int kMaxBatchedSegments = 16;
 static inline long long batched_max_segments(long long Ng) {
   return std::max<long long>(1, std::min<long long>(kMaxBatchedSegments, (Ng + kDistTile - 1) / kDistTile));
 }
@@ -663,9 +866,9 @@ static DistParams shortlist_params(bool f8, long long Na, long long Nb, int* can
   return dp;
 }
 
-template <int MB, int EPI, bool F8 = false>
+template <int MB, int EPI, bool F8 = false, int TOPC = kTopC>
 static int launch_dist(const DistParams& p, int grid_x, int grid_y, cudaStream_t s) {
-  auto kern = dist_kernel<MB, EPI, F8>;
+  auto kern = dist_kernel<MB, EPI, F8, TOPC>;
   const size_t smem = dist_smem_bytes<MB>(p.k_blocks);
   // the size depends on k_blocks (MB = 1: up to 6 for the 3-way split, MB = 2: always 2): raise the limit once per device
   static DeviceOnce attr_once;
@@ -705,6 +908,7 @@ struct MatchWs {
   void *q16, *g16;           // packed operand slots of 256 bytes per row (fp16; e4m3 operands use the first half of each)
   int* cand;
   float* cand_val;
+  float* cand_drop;          // top-k only: the lists' dropped maxima
   float* block_max;          // mutual only
   unsigned long long* claim;
   unsigned char* beaten;
@@ -714,16 +918,19 @@ struct MatchWs {
 
 // hn_match: packed operands and candidate lists [Nq][<= 16 segments][2 lists in the CTA-pair kernel][kTopC]. One workspace
 // serves this layout and carve_exact (hn_dist_workspace_bytes), plus 256 bytes. with_mutual (hn_match_mutual): the column side's
-// cell maxima, claims, beaten flags and row blocks' minimum d2 follow that size, plus 256 bytes.
-static MatchWs carve_match(void* ws, long long Nq, long long Ng, bool with_mutual) {
+// cell maxima, claims, beaten flags and row blocks' minimum d2 follow that size, plus 256 bytes. width = kTopKC (hn_match_topk):
+// lists [Nq][<= 16 segments][kTopKC] (single-CTA kernel only) and their dropped maxima [Nq][<= 16 segments] instead.
+static MatchWs carve_match(void* ws, long long Nq, long long Ng, bool with_mutual, int width = kTopC) {
   MatchWs w{};
   char* b = static_cast<char*>(ws);
   size_t off = 0;
   auto take = [&](size_t n) { char* r = b ? b + off : nullptr; off += align256(n); return r; };
+  const size_t lists = static_cast<size_t>(Nq) * (width == kTopC ? 2 * kMaxBatchedSegments : kMaxBatchedSegments);
   w.q16 = take(static_cast<size_t>(Nq) * 128 * 2);
   w.g16 = take(static_cast<size_t>(Ng) * 128 * 2);
-  w.cand = reinterpret_cast<int*>(take(static_cast<size_t>(Nq) * 32 * kTopC * 4));
-  w.cand_val = reinterpret_cast<float*>(take(static_cast<size_t>(Nq) * 32 * kTopC * 4));
+  w.cand = reinterpret_cast<int*>(take(lists * width * 4));
+  w.cand_val = reinterpret_cast<float*>(take(lists * width * 4));
+  if (width == kTopKC) w.cand_drop = reinterpret_cast<float*>(take(lists * 4));
   off = std::max(off, carve_exact(nullptr, Nq, Ng).bytes) + 256;
   if (with_mutual) {
     w.block_max = reinterpret_cast<float*>(take(static_cast<size_t>(hn_block_max_elems(Nq, Ng)) * 4));
@@ -942,6 +1149,19 @@ extern "C" int hn_pack_descriptors_multicast(const float* x, long long n, void* 
   return HN_OK;
 }
 
+// Operand packing of a single-problem call (stage 0): the packed rows the caller gave (q16_in / g16_in), else those of q / g
+// packed into w.
+template <typename T>
+static int pack_operands(const T* q, const T* g, const void* q16_in, const void* g16_in, long long Nq, long long Ng, const MatchWs& w,
+                         cudaStream_t s) {
+  MatchTimer timer(0, s);
+  if (!q16_in) launch_pack(q, Nq, w.q16, 0, s);
+  if (!g16_in) launch_pack(g, Ng, w.g16, 1, s);
+  HN_CUDA(cudaGetLastError());
+  count_launch((q16_in ? 0 : 1) + (g16_in ? 0 : 1));
+  return HN_OK;
+}
+
 // The launch sequence of hn_match_ex / hn_match_typed on validated arguments.
 template <typename T>
 static int run_match(const T* q, const T* g, const void* q16_in, const void* g16_in, long long Nq, long long Ng, long long g_offset,
@@ -952,13 +1172,7 @@ static int run_match(const T* q, const T* g, const void* q16_in, const void* g16
   constexpr bool F8 = kF8Rows<T>;
   const void* q16 = q16_in ? q16_in : w.q16;
   const void* g16 = g16_in ? g16_in : w.g16;
-  {
-    MatchTimer timer(0, s);
-    if (!q16_in) launch_pack(q, Nq, w.q16, 0, s);
-    if (!g16_in) launch_pack(g, Ng, w.g16, 1, s);
-    HN_CUDA(cudaGetLastError());
-    count_launch((q16_in ? 0 : 1) + (g16_in ? 0 : 1));
-  }
+  HN_TRY(pack_operands(q, g, q16_in, g16_in, Nq, Ng, w, s));
   DistParams dp = shortlist_params(F8, Nq, Ng, w.cand, w.cand_val, block_max);
   // CTA pairs (tc_dist_pair.cuh) once the problem is large enough to fill the machine with 512-row query blocks
   const int pair_mode = match_kernel_mode();
@@ -999,14 +1213,21 @@ static int run_match(const T* q, const T* g, const void* q16_in, const void* g16
 }
 
 // hn_match / hn_match_ex / hn_match_typed; fn names the entry point in error messages.
-static int match_entry(const char* fn, const void* q, const void* g, int desc_dtype, const void* q16_in, const void* g16_in,
-                       long long Nq, long long Ng, long long g_offset, float* d1, float* d2, int32_t* i1, int32_t* i2,
-                       float* block_max, void* workspace, long long workspace_bytes, void* g_ready_event, void* stream) {
-  HN_REQUIRE(q && g && workspace, "%s: NULL argument", fn);
+// Argument checks of a single-problem matching call (hn_match_typed, hn_match_topk_typed) up to the workspace size.
+static int check_match(const char* fn, int desc_dtype, const void* q, const void* g, long long Nq, long long Ng, long long g_offset,
+                       const void* workspace) {
   HN_TRY(check_rows(fn, desc_dtype, q, g));
   HN_REQUIRE(Nq >= 1 && Ng >= 1, "%s: empty input (Nq=%lld, Ng=%lld)", fn, Nq, Ng);
   HN_REQUIRE(Nq < (1LL << 31) && Ng + g_offset < (1LL << 31), "%s: more than 2^31 rows", fn);
   HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "%s: workspace must be 256-byte aligned", fn);
+  return HN_OK;
+}
+
+static int match_entry(const char* fn, const void* q, const void* g, int desc_dtype, const void* q16_in, const void* g16_in,
+                       long long Nq, long long Ng, long long g_offset, float* d1, float* d2, int32_t* i1, int32_t* i2,
+                       float* block_max, void* workspace, long long workspace_bytes, void* g_ready_event, void* stream) {
+  HN_REQUIRE(q && g && workspace, "%s: NULL argument", fn);
+  HN_TRY(check_match(fn, desc_dtype, q, g, Nq, Ng, g_offset, workspace));
   HN_REQUIRE(workspace_bytes >= hn_dist_workspace_bytes(Nq, Ng, 0), "%s: workspace too small", fn);
   HN_REQUIRE((reinterpret_cast<uintptr_t>(q16_in) & 15) == 0 && (reinterpret_cast<uintptr_t>(g16_in) & 15) == 0,
              "%s: packed operands must be 16-byte aligned", fn);
@@ -1120,7 +1341,8 @@ extern "C" int hn_match_mutual_typed(const void* q, const void* g, int desc_dtyp
 // (hn_match_pairs)
 // ------------------------------------------------------------------------------------------------------------
 // Nq / Ng: the per-pair maxima (output pitch). with_packed: room for B*Nq and B*Ng packed rows in front (hn_match_batched).
-static MatchWs carve_batched(void* ws, long long B, long long Nq, long long Ng, bool with_mutual, bool with_packed) {
+// width = kTopKC (hn_match_pairs_topk): lists of kTopKC chunks and their dropped maxima.
+static MatchWs carve_batched(void* ws, long long B, long long Nq, long long Ng, bool with_mutual, bool with_packed, int width = kTopC) {
   MatchWs w{};
   char* b = static_cast<char*>(ws);
   size_t off = 0;
@@ -1128,10 +1350,11 @@ static MatchWs carve_batched(void* ws, long long B, long long Nq, long long Ng, 
   const size_t rows_q = static_cast<size_t>(B) * Nq, rows_g = static_cast<size_t>(B) * Ng;
   w.q16 = with_packed ? take(rows_q * 128 * 2) : nullptr;
   w.g16 = with_packed ? take(rows_g * 128 * 2) : nullptr;
-  // candidate lists [rows][segments][kTopC]: a segment holds at least one gallery tile, so at most min(16, tiles) of them
-  const size_t lists = rows_q * batched_max_segments(Ng) * kTopC * 4;
-  w.cand = reinterpret_cast<int*>(take(lists));
-  w.cand_val = reinterpret_cast<float*>(take(lists));
+  // candidate lists [rows][segments][width]: a segment holds at least one gallery tile, so at most min(16, tiles) of them
+  const size_t lists = rows_q * batched_max_segments(Ng);
+  w.cand = reinterpret_cast<int*>(take(lists * width * 4));
+  w.cand_val = reinterpret_cast<float*>(take(lists * width * 4));
+  if (width == kTopKC) w.cand_drop = reinterpret_cast<float*>(take(lists * 4));
   if (with_mutual) {
     w.block_max = reinterpret_cast<float*>(take(static_cast<size_t>(B) * hn_block_max_elems(Nq, Ng) * 4));
     w.claim = reinterpret_cast<unsigned long long*>(take(rows_g * 8));
@@ -1154,6 +1377,23 @@ struct PairLayout {
 
 // The launch sequence of hn_match_pairs (TABLE) and hn_match_batched: GEMM + shortlist, re-rank, and with `mutual` the column
 // side. q16 / g16 are the packed rows of q / g.
+// The shortlist GEMM's parameters of a batched call (everything but the segment count): lists of w, operand maps over q16 /
+// g16 laid out as L says.
+static int pairs_params(bool f8, bool table, const void* q16, const void* g16, const PairLayout& L, const MatchWs& w, DistParams* dp) {
+  *dp = shortlist_params(f8, L.max_q, L.max_g, w.cand, w.cand_val, w.block_max);
+  // the table form's maps run over the concatenated sets, the padded form's over [B][N] rows
+  HN_TRY(make_operand_map(&dp->side[0].tmA, q16, f8, 128, table ? L.q_rows : L.max_q, table ? 0 : L.B, kDistTile));
+  HN_TRY(make_operand_map(&dp->side[0].tmB, g16, f8, 128, table ? L.g_rows : L.max_g, table ? 0 : L.B, kDistTile));
+  dp->q_len = L.q_len;
+  dp->g_len = L.g_len;
+  dp->batch = static_cast<int>(L.B);
+  dp->pairs = L.pairs;
+  dp->q_rows = L.q_rows;
+  dp->g_rows = L.g_rows;
+  dp->cand_drop = w.cand_drop;
+  return HN_OK;
+}
+
 template <bool TABLE, typename T>
 static int run_pairs(const T* q, const void* q16, const T* g, const void* g16, const PairLayout& L, float* d1,
                      float* d2, int32_t* i1, int32_t* i2, unsigned char* mutual, const MatchWs& w, cudaStream_t s) {
@@ -1162,16 +1402,8 @@ static int run_pairs(const T* q, const void* q16, const T* g, const void* g16, c
   HN_TRY(device_sm_count(&sm));
   const long long B = L.B, Nq = L.max_q, Ng = L.max_g, rows_q = B * Nq, rows_g = B * Ng;
   const int threads = 256;
-  DistParams dp = shortlist_params(F8, Nq, Ng, w.cand, w.cand_val, w.block_max);
-  // the table form's maps run over the concatenated sets, the padded form's over [B][N] rows
-  HN_TRY(make_operand_map(&dp.side[0].tmA, q16, F8, 128, TABLE ? L.q_rows : Nq, TABLE ? 0 : B, kDistTile));
-  HN_TRY(make_operand_map(&dp.side[0].tmB, g16, F8, 128, TABLE ? L.g_rows : Ng, TABLE ? 0 : B, kDistTile));
-  dp.q_len = L.q_len;
-  dp.g_len = L.g_len;
-  dp.batch = static_cast<int>(B);
-  dp.pairs = L.pairs;
-  dp.q_rows = L.q_rows;
-  dp.g_rows = L.g_rows;
+  DistParams dp;
+  HN_TRY(pairs_params(F8, TABLE, q16, g16, L, w, &dp));
   {
     MatchTimer timer(1, s);
     // segments from the per-pair maxima (lengths live on the device): B * ceil(Nq / 256) query blocks over a gallery of Ng
@@ -1265,12 +1497,9 @@ extern "C" long long hn_match_pairs_workspace_bytes(long long B, long long max_q
   return static_cast<long long>(carve_batched(nullptr, B, max_q, max_g, with_mutual != 0, false).bytes);
 }
 
-// hn_match_pairs / hn_match_pairs_typed; fn names the entry point in error messages.
-static int pairs_entry(const char* fn, const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16, long long Ng_rows,
-                       int desc_dtype, const int32_t* pairs, long long B, long long max_q, long long max_g, float* d1, float* d2,
-                       int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace, long long workspace_bytes, void* stream) {
-  HN_REQUIRE(q && q16 && g && g16 && pairs && d1 && d2 && i1 && i2 && workspace,
-             "%s: NULL argument (q, q16, g, g16, pairs, d1, d2, i1, i2 and workspace are required)", fn);
+// Argument checks of a pair-table call (hn_match_pairs_typed, hn_match_pairs_topk_typed) up to the workspace size.
+static int check_pairs(const char* fn, int desc_dtype, const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16,
+                       long long Ng_rows, long long B, long long max_q, long long max_g, const void* workspace) {
   HN_TRY(check_rows(fn, desc_dtype, q, g));
   HN_REQUIRE(B >= 1 && max_q >= 1 && max_g >= 1 && Nq_rows >= 1 && Ng_rows >= 1,
              "%s: empty input (B=%lld, max_q=%lld, max_g=%lld, Nq_rows=%lld, Ng_rows=%lld)", fn, B, max_q, max_g, Nq_rows, Ng_rows);
@@ -1279,6 +1508,16 @@ static int pairs_entry(const char* fn, const void* q, const void* q16, long long
   HN_REQUIRE((reinterpret_cast<uintptr_t>(q16) & 15) == 0 && (reinterpret_cast<uintptr_t>(g16) & 15) == 0,
              "%s: packed operands must be 16-byte aligned", fn);
   HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "%s: workspace must be 256-byte aligned", fn);
+  return HN_OK;
+}
+
+// hn_match_pairs / hn_match_pairs_typed; fn names the entry point in error messages.
+static int pairs_entry(const char* fn, const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16, long long Ng_rows,
+                       int desc_dtype, const int32_t* pairs, long long B, long long max_q, long long max_g, float* d1, float* d2,
+                       int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace, long long workspace_bytes, void* stream) {
+  HN_REQUIRE(q && q16 && g && g16 && pairs && d1 && d2 && i1 && i2 && workspace,
+             "%s: NULL argument (q, q16, g, g16, pairs, d1, d2, i1, i2 and workspace are required)", fn);
+  HN_TRY(check_pairs(fn, desc_dtype, q, q16, Nq_rows, g, g16, Ng_rows, B, max_q, max_g, workspace));
   HN_REQUIRE(workspace_bytes >= hn_match_pairs_workspace_bytes(B, max_q, max_g, mutual != nullptr), "%s: workspace too small", fn);
   const MatchWs w = carve_batched(workspace, B, max_q, max_g, mutual != nullptr, false);
   const PairLayout L = {pairs, nullptr, nullptr, B, max_q, max_g, Nq_rows, Ng_rows};
@@ -1304,6 +1543,115 @@ extern "C" int hn_match_pairs_typed(const void* q, const void* q16, long long Nq
                      mutual, workspace, workspace_bytes, stream);
 }
 
+// ---- k nearest neighbours ----------------------------------------------------------------------------------------------
+
+extern "C" long long hn_match_topk_workspace_bytes(long long Nq, long long Ng) {
+  if (Nq < 0 || Ng < 0) return 0;
+  return static_cast<long long>(carve_match(nullptr, Nq, Ng, false, kTopKC).bytes);
+}
+
+extern "C" long long hn_match_pairs_topk_workspace_bytes(long long B, long long max_q, long long max_g) {
+  if (B < 0 || max_q < 0 || max_g < 0) return 0;
+  return static_cast<long long>(carve_batched(nullptr, B, max_q, max_g, false, false, kTopKC).bytes);
+}
+
+// The launch sequence of hn_match_topk_typed on validated arguments: the single-CTA GEMM with top-kTopKC lists over (up to)
+// kMaxBatchedSegments segments, so that a list spans at most 1/16 of the gallery (the bound on a fallback scan), then the re-rank.
+template <typename T>
+static int run_match_topk(const T* q, const T* g, const void* q16_in, const void* g16_in, long long Nq, long long Ng, int k, float* dist,
+                          int32_t* idx, const MatchWs& w, cudaStream_t s) {
+  int sm = 0;
+  HN_TRY(device_sm_count(&sm));
+  constexpr bool F8 = kF8Rows<T>;
+  HN_TRY(pack_operands(q, g, q16_in, g16_in, Nq, Ng, w, s));
+  DistParams dp = shortlist_params(F8, Nq, Ng, w.cand, w.cand_val, nullptr);
+  dp.cand_drop = w.cand_drop;
+  HN_TRY(make_operand_map(&dp.side[0].tmA, q16_in ? q16_in : w.q16, F8, 128, Nq, 0, kDistTile));
+  HN_TRY(make_operand_map(&dp.side[0].tmB, g16_in ? g16_in : w.g16, F8, 128, Ng, 0, kDistTile));
+  dp.segments = static_cast<int>(batched_max_segments(Ng));
+  {
+    MatchTimer timer(1, s);
+    const long long items = ((Nq + 2 * kDistTile - 1) / (2 * kDistTile)) * dp.segments;
+    HN_TRY((launch_dist<2, EPI_SHORTLIST, F8, kTopKC>(dp, static_cast<int>(std::min<long long>(items, sm)), 1, s)));
+  }
+  unsigned long long* fallback_rows = nullptr;
+  HN_TRY(topk_fallback_counter(&fallback_rows));
+  {
+    MatchTimer timer(2, s);
+    rerank_topk_kernel<T><<<static_cast<unsigned>((Nq + 3) / 4), 128, 0, s>>>(q, g, w.cand, w.cand_val, w.cand_drop, kRerankMargin, Nq,
+                                                                                Ng, dp.segments, k, dist, idx, fallback_rows);
+    HN_CUDA(cudaGetLastError());
+    count_launch();
+  }
+  return HN_OK;
+}
+
+extern "C" int hn_match_topk_typed(const void* q, const void* g, int desc_dtype, const void* q16, const void* g16, long long Nq,
+                                   long long Ng, int k, float* dist, int32_t* idx, void* workspace, long long workspace_bytes,
+                                   void* stream) {
+  const char* fn = "hn_match_topk_typed";
+  HN_REQUIRE(q && g && dist && idx && workspace, "%s: NULL argument (q, g, dist, idx and workspace are required)", fn);
+  HN_REQUIRE(k >= 1 && k <= kTopKMax, "%s: k must be in [1, %d] (got %d)", fn, kTopKMax, k);
+  HN_TRY(check_match(fn, desc_dtype, q, g, Nq, Ng, 0, workspace));
+  HN_REQUIRE(workspace_bytes >= hn_match_topk_workspace_bytes(Nq, Ng), "%s: workspace too small", fn);
+  HN_REQUIRE((reinterpret_cast<uintptr_t>(q16) & 15) == 0 && (reinterpret_cast<uintptr_t>(g16) & 15) == 0,
+             "%s: packed operands must be 16-byte aligned", fn);
+  return with_rows(desc_dtype, [&](auto t) -> int {
+    using T = decltype(t);
+    return run_match_topk(static_cast<const T*>(q), static_cast<const T*>(g), q16, g16, Nq, Ng, k, dist, idx,
+                          carve_match(workspace, Nq, Ng, false, kTopKC), static_cast<cudaStream_t>(stream));
+  });
+}
+
+// The launch sequence of hn_match_pairs_topk_typed on validated arguments: the pair-table GEMM with top-kTopKC lists over
+// (up to) kMaxBatchedSegments segments of each pair's gallery, then the re-rank.
+template <typename T>
+static int run_pairs_topk(const T* q, const void* q16, const T* g, const void* g16, const PairLayout& L, int k, float* dist, int32_t* idx,
+                          const MatchWs& w, cudaStream_t s) {
+  constexpr bool F8 = kF8Rows<T>;
+  int sm = 0;
+  HN_TRY(device_sm_count(&sm));
+  DistParams dp;
+  HN_TRY(pairs_params(F8, true, q16, g16, L, w, &dp));
+  dp.segments = static_cast<int>(batched_max_segments(L.max_g));
+  {
+    MatchTimer timer(1, s);
+    const long long m_blocks = (L.max_q + 2 * kDistTile - 1) / (2 * kDistTile);
+    const int grid = static_cast<int>(std::min<long long>(L.B * m_blocks * dp.segments, sm));
+    HN_TRY((launch_dist<2, EPI_SHORTLIST_PAIRS, F8, kTopKC>(dp, grid, 1, s)));
+  }
+  unsigned long long* fallback_rows = nullptr;
+  HN_TRY(topk_fallback_counter(&fallback_rows));
+  {
+    MatchTimer timer(2, s);
+    rerank_topk_pairs_kernel<T><<<static_cast<unsigned>((L.B * L.max_q + 3) / 4), 128, 0, s>>>(
+        q, g, w.cand, w.cand_val, w.cand_drop, kRerankMargin, L.B, L.max_q, L.max_g, L.pairs, L.q_rows, L.g_rows, dp.segments, k, dist,
+        idx, fallback_rows);
+    HN_CUDA(cudaGetLastError());
+    count_launch();
+  }
+  return HN_OK;
+}
+
+extern "C" int hn_match_pairs_topk_typed(const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16,
+                                         long long Ng_rows, int desc_dtype, const int32_t* pairs, long long B, long long max_q,
+                                         long long max_g, int k, float* dist, int32_t* idx, void* workspace, long long workspace_bytes,
+                                         void* stream) {
+  const char* fn = "hn_match_pairs_topk_typed";
+  HN_REQUIRE(q && q16 && g && g16 && pairs && dist && idx && workspace,
+             "%s: NULL argument (q, q16, g, g16, pairs, dist, idx and workspace are required)", fn);
+  HN_REQUIRE(k >= 1 && k <= kTopKMax, "%s: k must be in [1, %d] (got %d)", fn, kTopKMax, k);
+  HN_TRY(check_pairs(fn, desc_dtype, q, q16, Nq_rows, g, g16, Ng_rows, B, max_q, max_g, workspace));
+  HN_REQUIRE(workspace_bytes >= hn_match_pairs_topk_workspace_bytes(B, max_q, max_g), "%s: workspace too small", fn);
+  const MatchWs w = carve_batched(workspace, B, max_q, max_g, false, false, kTopKC);
+  const PairLayout L = {pairs, nullptr, nullptr, B, max_q, max_g, Nq_rows, Ng_rows};
+  return with_rows(desc_dtype, [&](auto t) -> int {
+    using T = decltype(t);
+    return run_pairs_topk(static_cast<const T*>(q), q16, static_cast<const T*>(g), g16, L, k, dist, idx, w,
+                          static_cast<cudaStream_t>(stream));
+  });
+}
+
 extern "C" int hn_match_force_kernel(int mode) {
   HN_REQUIRE(mode >= -1 && mode <= 1, "hn_match_force_kernel: mode must be -1 (by size), 0 (single CTA) or 1 (CTA pair)");
   match_kernel_mode() = mode;
@@ -1313,6 +1661,26 @@ extern "C" int hn_match_force_kernel(int mode) {
 extern "C" int hn_match_profile_enable(int on) {
   g_match_profile.on = on != 0;
   for (size_t& u : g_match_profile.used) u = 0;
+  return HN_OK;
+}
+
+extern "C" int hn_match_topk_fallback_enable(int on) {
+  if (g_topk_fallback_rows) HN_CUDA(cudaFree(g_topk_fallback_rows));
+  g_topk_fallback_rows = nullptr;
+  if (on) {
+    HN_CUDA(cudaMalloc(&g_topk_fallback_rows, sizeof(unsigned long long)));
+    HN_CUDA(cudaMemset(g_topk_fallback_rows, 0, sizeof(unsigned long long)));
+  }
+  return HN_OK;
+}
+
+extern "C" int hn_match_topk_fallback_read(long long* rows_out) {
+  HN_REQUIRE(rows_out, "hn_match_topk_fallback_read: NULL argument");
+  HN_REQUIRE(g_topk_fallback_rows, "hn_match_topk_fallback_read: the count is not enabled (hn_match_topk_fallback_enable(1))");
+  unsigned long long v = 0;
+  HN_CUDA(cudaMemcpy(&v, g_topk_fallback_rows, sizeof(v), cudaMemcpyDeviceToHost));
+  *rows_out = static_cast<long long>(v);
+  HN_CUDA(cudaMemset(g_topk_fallback_rows, 0, sizeof(unsigned long long)));
   return HN_OK;
 }
 

@@ -37,6 +37,7 @@ namespace hn {
 constexpr int kDistTile = 128;
 constexpr int kDistStages = 4;
 constexpr int kTopC = 4;     // chunks kept per row and segment
+constexpr int kTopKC = 8;    // the same for the k-nearest-neighbour lists (hn_match_topk), which also keep a dropped maximum
 constexpr int kChunk = 8;    // columns per chunk
 
 enum : int { EPI_EXACT = 0, EPI_SHORTLIST = 1, EPI_EXACT_NEI = 2, EPI_SHORTLIST_BATCHED = 3, EPI_SHORTLIST_PAIRS = 4 };   // EXACT_NEI = EXACT + the keypoint-neighbour masks
@@ -78,6 +79,9 @@ struct DistParams {
   // unused; side[0].Na / Nb are the per-pair maxima max_q / max_g)
   const int* pairs;
   long long q_rows, g_rows;
+  // TOPC = kTopKC lists only (appended like the batch fields): [lists] the largest approximate chunk maximum of each list that
+  // did not make it (-inf when every chunk of the list was kept)
+  float* cand_drop;
 };
 
 template <int MB>
@@ -128,12 +132,17 @@ __device__ __forceinline__ float warp_chunk_max8(const float (&c)[8], int lane) 
 }
 
 // A row's candidate list (one segment; in the CTA-pair kernel one 64-column half of it) at list index `list` of cand /
-// cand_val: the kTopC chunk ids, -1 in unused slots (a segment with fewer than kTopC chunks), and the chunks' maxima.
-__device__ __forceinline__ void store_cand_list(int* cand, float* cand_val, long long list, const float (&tb)[kTopC],
-                                                const int (&tc)[kTopC]) {
-  *reinterpret_cast<int4*>(cand + list * kTopC) = make_int4(tb[0] > -3.0e38f ? tc[0] : -1, tb[1] > -3.0e38f ? tc[1] : -1,
-                                                            tb[2] > -3.0e38f ? tc[2] : -1, tb[3] > -3.0e38f ? tc[3] : -1);
-  *reinterpret_cast<float4*>(cand_val + list * kTopC) = make_float4(tb[0], tb[1], tb[2], tb[3]);
+// cand_val: the C chunk ids (C = kTopC or kTopKC), -1 in unused slots (a segment with fewer than C chunks), and the chunks'
+// maxima.
+template <int C>
+__device__ __forceinline__ void store_cand_list(int* cand, float* cand_val, long long list, const float (&tb)[C], const int (&tc)[C]) {
+  static_assert(C % 4 == 0, "lists are stored in 16-byte pieces");
+#pragma unroll
+  for (int h = 0; h < C; h += 4) {
+    *reinterpret_cast<int4*>(cand + list * C + h) = make_int4(tb[h] > -3.0e38f ? tc[h] : -1, tb[h + 1] > -3.0e38f ? tc[h + 1] : -1,
+                                                              tb[h + 2] > -3.0e38f ? tc[h + 2] : -1, tb[h + 3] > -3.0e38f ? tc[h + 3] : -1);
+    *reinterpret_cast<float4*>(cand_val + list * C + h) = make_float4(tb[h], tb[h + 1], tb[h + 2], tb[h + 3]);
+  }
 }
 
 // Epilogue warps per accumulator lane quarter. The exact epilogues (loss kernels) cost ~80 instructions per column and a loss-sized
@@ -143,7 +152,10 @@ __device__ __forceinline__ void store_cand_list(int* cand, float* cand_val, long
 template <int EPI>
 constexpr int dist_col_split() { return (EPI == EPI_EXACT || EPI == EPI_EXACT_NEI) ? 4 : 1; }
 
-template <int MB, int EPI, bool F8 = false>
+// TOPC: chunks per candidate list of the shortlist epilogues. kTopC for hn_match and its batched forms; kTopKC for the k-nearest-
+// neighbour lists, which also record each list's dropped maximum (p.cand_drop) so that the re-rank can tell when a list may
+// hide one of the k nearest columns (rerank_topk_row).
+template <int MB, int EPI, bool F8 = false, int TOPC = kTopC>
 __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist_kernel(const __grid_constant__ DistParams p) {
   constexpr bool EXACT = EPI == EPI_EXACT || EPI == EPI_EXACT_NEI;
   constexpr int CS = dist_col_split<EPI>();
@@ -153,6 +165,8 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
   constexpr bool BATCHED = EPI == EPI_SHORTLIST_BATCHED || PAIRS;
   constexpr bool SHORTLIST = EPI == EPI_SHORTLIST || BATCHED;
   static_assert(!F8 || (SHORTLIST && MB == 2), "e4m3 operands are for the matching GEMMs");
+  constexpr bool DROP = TOPC == kTopKC;
+  static_assert(TOPC == kTopC || (DROP && (EPI == EPI_SHORTLIST || EPI == EPI_SHORTLIST_PAIRS)), "top-k lists: single problems and pair tables");
   constexpr uint32_t BLK_BYTES = kDistTile * 128;  // 128 rows x 64 fp16 (F8: x 128 e4m3)
   constexpr uint32_t TMEM_COLS = 2 * MB * kDistTile;
   const DistSide& sd = p.side[blockIdx.y];
@@ -351,15 +365,16 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
       float best = __int_as_float(0x7f800000);
       int best_col = 0x7fffffff;
       float na = 0.f;
-      float tb[kTopC];
-      int tc[kTopC];
+      float tb[TOPC];
+      int tc[TOPC];
+      float drop = -__int_as_float(0x7f800000);   // DROP only
       float2 r_axy = make_float2(0.f, 0.f), r_pxy = make_float2(0.f, 0.f);
       if (EXACT) {
         if (p.form == HN_FORM_HARDNET && row_ok) na = sd.norm_a[row];
         if (NEI && row_ok) { r_axy = sd.xy_a_rows[row]; r_pxy = sd.xy_p_rows[row]; }
       } else {
 #pragma unroll
-        for (int i = 0; i < kTopC; ++i) { tb[i] = -__int_as_float(0x7f800000); tc[i] = 0; }
+        for (int i = 0; i < TOPC; ++i) { tb[i] = -__int_as_float(0x7f800000); tc[i] = 0; }
       }
 
       for (int t = t0; t < t1; ++t, ++it) {
@@ -388,36 +403,57 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
         const uint32_t t_row = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + (acc * MB + mb) * kDistTile;
         if (SHORTLIST) {
           const bool ragged = col0 + kDistTile > cols();
-          // all four TMEM loads are issued before the single wait: one exposed round trip per tile instead of four
-          uint32_t r[4][32];
-#pragma unroll
-          for (int gq = 0; gq < 4; ++gq) tmem_ld32(t_row + gq * 32, r[gq]);
-          tmem_ld_wait();
+          // all four TMEM loads are issued before the single wait: one exposed round trip per tile instead of four. The top-k
+          // lists (DROP) hold 8 + 8 more registers; there two loads per wait keep the epilogue clear of spills.
+          constexpr int LDS = DROP ? 2 : 4;
           float cm[16];   // this row's maxima of the tile's sixteen chunks
 #pragma unroll
-          for (int gq = 0; gq < 4; ++gq) {
-            const int c0 = gq * 32;
-            float v[32];
+          for (int h = 0; h < 4; h += LDS) {
+            uint32_t r[LDS][32];
 #pragma unroll
-            for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[gq][j]);
-            if (ragged) {
+            for (int gq = 0; gq < LDS; ++gq) tmem_ld32(t_row + (h + gq) * 32, r[gq]);
+            tmem_ld_wait();
 #pragma unroll
-              for (int j = 0; j < 32; ++j)
-                if (col0 + c0 + j >= cols()) v[j] = -__int_as_float(0x7f800000);
-            }
+            for (int gq = h; gq < h + LDS; ++gq) {
+              const int c0 = gq * 32;
+              float v[32];
 #pragma unroll
-            for (int s = 0; s < 32 / kChunk; ++s) {
-              const float* w = v + s * kChunk;
-              const float m = fmaxf(max3(w[0], w[1], w[2]), max3(max3(w[3], w[4], w[5]), w[6], w[7]));
-              cm[gq * 4 + s] = BATCHED && !row_ok ? -__int_as_float(0x7f800000) : m;   // padding rows stay out of the block maxima
-              if (m > tb[kTopC - 1]) {
-                const int id = static_cast<int>((col0 + c0) / kChunk) + s;
-                // sorted insert (descending); strict '>' keeps the earlier chunk on ties
-                const bool g0 = m > tb[0], g1 = m > tb[1], g2 = m > tb[2];
-                tb[3] = g2 ? tb[2] : m;               tc[3] = g2 ? tc[2] : id;
-                tb[2] = g2 ? (g1 ? tb[1] : m) : tb[2]; tc[2] = g2 ? (g1 ? tc[1] : id) : tc[2];
-                tb[1] = g1 ? (g0 ? tb[0] : m) : tb[1]; tc[1] = g1 ? (g0 ? tc[0] : id) : tc[1];
-                tb[0] = g0 ? m : tb[0];               tc[0] = g0 ? id : tc[0];
+              for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[gq - h][j]);
+              if (ragged) {
+#pragma unroll
+                for (int j = 0; j < 32; ++j)
+                  if (col0 + c0 + j >= cols()) v[j] = -__int_as_float(0x7f800000);
+              }
+#pragma unroll
+              for (int s = 0; s < 32 / kChunk; ++s) {
+                const float* w = v + s * kChunk;
+                const float m = fmaxf(max3(w[0], w[1], w[2]), max3(max3(w[3], w[4], w[5]), w[6], w[7]));
+                cm[gq * 4 + s] = BATCHED && !row_ok ? -__int_as_float(0x7f800000) : m;   // padding rows stay out of the block maxima
+                // the chunk that leaves the list, this one or the evicted last entry, is the smaller of the two
+                if constexpr (DROP) drop = fmaxf(drop, fminf(m, tb[TOPC - 1]));
+                if (m > tb[TOPC - 1]) {
+                  const int id = static_cast<int>((col0 + c0) / kChunk) + s;
+                  // sorted insert (descending); strict '>' keeps the earlier chunk on ties
+                  if constexpr (TOPC == kTopC) {   // hn_match's lists, written out: the loop below compiles differently
+                    const bool g0 = m > tb[0], g1 = m > tb[1], g2 = m > tb[2];
+                    tb[3] = g2 ? tb[2] : m;               tc[3] = g2 ? tc[2] : id;
+                    tb[2] = g2 ? (g1 ? tb[1] : m) : tb[2]; tc[2] = g2 ? (g1 ? tc[1] : id) : tc[2];
+                    tb[1] = g1 ? (g0 ? tb[0] : m) : tb[1]; tc[1] = g1 ? (g0 ? tc[0] : id) : tc[1];
+                    tb[0] = g0 ? m : tb[0];               tc[0] = g0 ? id : tc[0];
+                  } else {
+                    // slot i takes the entry above it when m beats both, m when it beats slot i only (always true of the last)
+                    bool gt[TOPC - 1];
+#pragma unroll
+                    for (int i = 0; i < TOPC - 1; ++i) gt[i] = m > tb[i];
+                    tb[TOPC - 1] = gt[TOPC - 2] ? tb[TOPC - 2] : m; tc[TOPC - 1] = gt[TOPC - 2] ? tc[TOPC - 2] : id;
+#pragma unroll
+                    for (int i = TOPC - 2; i > 0; --i) {
+                      tb[i] = gt[i] ? (gt[i - 1] ? tb[i - 1] : m) : tb[i];
+                      tc[i] = gt[i] ? (gt[i - 1] ? tc[i - 1] : id) : tc[i];
+                    }
+                    tb[0] = gt[0] ? m : tb[0];               tc[0] = gt[0] ? id : tc[0];
+                  }
+                }
               }
             }
           }
@@ -495,6 +531,7 @@ __global__ void __launch_bounds__(64 + 128 * MB * dist_col_split<EPI>(), 1) dist
         } else {
           const long long out_row = BATCHED ? pair * sd.Na + row : row;   // chunk ids stay local to the pair
           store_cand_list(sd.cand, sd.cand_val, out_row * p.segments + seg, tb, tc);
+          if constexpr (DROP) p.cand_drop[out_row * p.segments + seg] = drop;
         }
       }
     }

@@ -72,6 +72,14 @@ def match_top2(des1, des2):
     return d1, d2, i1.long(), i2.long()
 
 
+def match_topk(des1, des2, k):
+    """(D [Nq, k] fp32, I [Nq, k] int64) = sorted[:, :k], indices[:, :k] of eval_utils.py:170-171 for k in [1, 8]: the k nearest
+    gallery rows of every query, ascending by (distance, index), exact (hn_match_topk_typed); without the Nq x Ng matrix.
+    Rows with fewer than k gallery rows get +inf / -1 in the missing slots."""
+    d, i = _ops.match_topk(des1, des2, k)
+    return d, i.long()
+
+
 def mutual_nn_ratio(des1, des2, threshold=0.7, return_pairs=True):
     """Mutual nearest neighbours AND the ratio test of BASELINE config 4 in one call:
     (pairs [M,2] int64 or None, mutual bool[Nq], ratio_label bool[Nq], Ia int64[Nq], Da, Db).
@@ -183,6 +191,16 @@ def mutual_nn_ratio_pairs(des1, des2, pairs, max_len1=None, max_len2=None, thres
     max_len1, max_len2 = _max_lens(pairs, des1.size(0), des2.size(0), max_len1, max_len2)
     d1, d2, i1, _, mutual = _ops.match_pairs(des1, des2, pairs, max_len1, max_len2, des1_16, des2_16, mutual=True)
     return mutual, (d1 / d2).lt(threshold), i1.long(), d1, d2
+
+
+def match_topk_pairs(des1, des2, pairs, k, max_len1=None, max_len2=None, des1_16=None, des2_16=None):
+    """match_topk for every row-range pair of the table -> (D, I), each [P, max_len1, k]; indices int64, local to the pair's
+    gallery range; rows past len1 and pairs without gallery rows get +inf / -1. A padded batch des1 [B, N1, 128],
+    des2 [B, N2, 128] with lengths len1 / len2 is the table (b * N1, len1[b], b * N2, len2[b]) over des1.flatten(0, 1) and
+    des2.flatten(0, 1), with max_len1 = N1 and max_len2 = N2."""
+    max_len1, max_len2 = _max_lens(pairs, des1.size(0), des2.size(0), max_len1, max_len2)
+    d, i = _ops.match_pairs_topk(des1, des2, pairs, k, max_len1, max_len2, des1_16, des2_16)
+    return d, i.long()
 
 
 # ---- match-score counters (FDLNet-master/utils/eval_utils.py:112-197) -----------------------------------------------

@@ -285,11 +285,38 @@ int hn_match_pairs_typed(const void* q, const void* q16, long long Nq_rows, cons
                          int32_t* i1, int32_t* i2, unsigned char* mutual, void* workspace, long long workspace_bytes,
                          void* stream);                                                                        /* hn_match_pairs */
 
-/* Measurement hooks (process-wide): bracket the three stages of every hn_match / hn_match_batched / hn_match_pairs call
- * (0 = operand packing, not part of hn_match_pairs; 1 = GEMM + shortlist, 2 = exact re-rank) with CUDA events; hn_match_profile_read waits for them, returns the summed milliseconds and
+/* ---- k nearest neighbours -------------------------------------------------------------------------------------------------
+ * The k <= 8 gallery rows nearest to every query row in the FDLNet distance sqrt(clamp(2 - 2ab, 1e-8, 4)), sorted ascending
+ * by (distance, gallery index): the first k columns of the reference's full row sort (FDLNet-master/utils/eval_utils.py:168-175,
+ * `D.sort(dim=-1)`) without the Nq x Ng matrix. dist / idx are [rows][k]; a row with fewer than k gallery rows gets +inf / -1
+ * in the missing slots. Distances are the re-rank's fp32 arithmetic, bit-identical to what hn_match reports for the same
+ * (row, column). The result is always exact: it equals a brute-force fp32 evaluation of every column with that arithmetic
+ * followed by a stable sort, whatever the ties (hn_match's five-chunk limit does not apply; dist.cu gives the argument).
+ * k outside [1, 8] is rejected with HN_ERR_INVALID before any device work. Rows, dtypes (HN_F32 / HN_F16 / HN_BF16 /
+ * HN_F8E4M3, bit for bit the fp32 call on the rows converted to fp32), packed operands and validation are those of
+ * hn_match_typed (single problem, no g_offset) and hn_match_pairs_typed (pair table: indices local to the pair's gallery range,
+ * rows past q_len and pairs with g_len == 0 get +inf / -1, CUDA-graph capturable). A padded batch q [B, Nq, 128], g [B, Ng, 128]
+ * with lengths q_len / g_len is the pair table (b*Nq, q_len[b], b*Ng, g_len[b]) over the flattened [B*Nq] / [B*Ng] rows.
+ * The workspace (256-byte aligned) is sized by the two *_topk_workspace_bytes functions. */
+long long hn_match_topk_workspace_bytes(long long Nq, long long Ng);
+int hn_match_topk_typed(const void* q, const void* g, int desc_dtype, const void* q16, const void* g16, long long Nq, long long Ng,
+                        int k, float* dist, int32_t* idx, void* workspace, long long workspace_bytes, void* stream);
+long long hn_match_pairs_topk_workspace_bytes(long long B, long long max_q, long long max_g);
+int hn_match_pairs_topk_typed(const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16, long long Ng_rows,
+                              int desc_dtype, const int32_t* pairs, long long B, long long max_q, long long max_g, int k,
+                              float* dist, int32_t* idx, void* workspace, long long workspace_bytes, void* stream);
+
+/* Measurement hooks (process-wide): bracket the three stages of every hn_match / hn_match_batched / hn_match_pairs /
+ * hn_match_topk_typed / hn_match_pairs_topk_typed call (0 = operand packing, not part of the pair-table calls; 1 = GEMM +
+ * shortlist, 2 = exact re-rank) with CUDA events; hn_match_profile_read waits for them, returns the summed milliseconds and
  * launch counts per stage and resets the counters. */
 int hn_match_profile_enable(int on);
 int hn_match_profile_read(double ms_out[3], long long launches_out[3]);
+/* Count of the top-k rows whose re-rank scanned a whole candidate list because the list's dropped maximum reached the
+ * threshold (process-wide, current device, off by default): enable(1) resets and starts it, enable(0) stops it; read waits for
+ * the device, returns the count and resets it. */
+int hn_match_topk_fallback_enable(int on);
+int hn_match_topk_fallback_read(long long* rows_out);
 
 /* ---- evaluation metrics of the test loop (hardnet/HardNet.py:443-477) -------------------------------------------------- */
 /* Row-wise descriptor distance torch.sqrt(torch.sum((out_a - out_p) ** 2, 1)) (HardNet.py:458). a, p: [n,128] fp32; out: [n]. */
