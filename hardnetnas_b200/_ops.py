@@ -152,6 +152,8 @@ def match_top2(q: torch.Tensor, g: torch.Tensor, g_offset: int = 0, q16: torch.T
         if t is not None:
             _packed("match", t, n, dt)
     dev = q.device
+    if block_max is not None:
+        _buffer("match", "block_max", block_max, torch.float32, dev, min_numel=block_max_elems(nq, ng))
     with torch.cuda.device(dev):
         ws = _workspace(dev, lib.hn_dist_workspace_bytes(nq, ng, 0))
         d1 = torch.empty(nq, dtype=torch.float32, device=dev)
@@ -336,21 +338,48 @@ def match_pairs_topk(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, k: i
     return dist, idx
 
 
+def _buffer(name: str, what: str, t, dtype: torch.dtype, device: torch.device, numel: int | None = None,
+            min_numel: int | None = None) -> torch.Tensor:
+    """Checks a tensor the C ABI reads or writes through a bare pointer at a length it derives from other arguments: a wrong
+    dtype, device, layout or size would be read or written out of bounds."""
+    if not (isinstance(t, torch.Tensor) and t.dtype == dtype and t.device == device and t.is_contiguous()):
+        raise ValueError(f"{name}: {what} must be a contiguous {dtype} tensor on {device}")
+    if (numel is not None and t.numel() != numel) or (min_numel is not None and t.numel() < min_numel):
+        size = f"{numel}" if numel is not None else f"at least {min_numel}"
+        raise ValueError(f"{name}: {what} must have {size} elements, got {t.numel()}")
+    return t
+
+
 def mutual_claims(i1: torch.Tensor, d1: torch.Tensor, d2: torch.Tensor, q_offset: int, claim: torch.Tensor) -> torch.Tensor:
     """atomicMin of (distance, global row) into claim[int64, Ng] (pre-filled with INT64_MAX = unclaimed); returns the per
     32-row-block minimum of d2 the verification needs."""
     lib = _lib.load()
-    rbmin = torch.empty((i1.numel() + 31) // 32, dtype=torch.float32, device=i1.device)
-    with torch.cuda.device(i1.device):
-        _lib.check(lib.hn_mutual_claims(_ptr(i1), _ptr(d1), _ptr(d2), i1.numel(), q_offset, _ptr(claim), claim.numel(), _ptr(rbmin),
+    if not (isinstance(i1, torch.Tensor) and i1.is_cuda):
+        raise ValueError("mutual_claims: i1 must be a CUDA tensor")
+    dev, nq = i1.device, i1.numel()
+    _buffer("mutual_claims", "i1", i1, torch.int32, dev)
+    _buffer("mutual_claims", "d1", d1, torch.float32, dev, numel=nq)
+    _buffer("mutual_claims", "d2", d2, torch.float32, dev, numel=nq)
+    _buffer("mutual_claims", "claim", claim, torch.int64, dev)
+    rbmin = torch.empty((nq + 31) // 32, dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.hn_mutual_claims(_ptr(i1), _ptr(d1), _ptr(d2), nq, q_offset, _ptr(claim), claim.numel(), _ptr(rbmin),
                                         _stream_ptr()), "hn_mutual_claims")
     return rbmin
 
 
 def mutual_verify(q: torch.Tensor, q_offset: int, g: torch.Tensor, claim: torch.Tensor, block_max: torch.Tensor,
                   rb_min_d2: torch.Tensor, beaten: torch.Tensor):
-    """beaten[uint8, Ng] |= some local query row is nearer to g_j than the claimant of column j."""
+    """beaten[uint8, Ng] |= some local query row is nearer to g_j than the claimant of column j. q / g: fp32 [n,128] rows."""
     lib = _lib.load()
-    with torch.cuda.device(q.device):
-        _lib.check(lib.hn_mutual_verify(_ptr(q), q.size(0), q_offset, _ptr(g), g.size(0), _ptr(claim), _ptr(block_max),
+    q, g = _require_cuda_desc("mutual_verify", q), _require_cuda_desc("mutual_verify", g)
+    dev, nq, ng = q.device, q.size(0), g.size(0)
+    _buffer("mutual_verify", "q", q, torch.float32, dev)
+    _buffer("mutual_verify", "g", g, torch.float32, dev)
+    _buffer("mutual_verify", "claim", claim, torch.int64, dev, numel=ng)
+    _buffer("mutual_verify", "block_max", block_max, torch.float32, dev, min_numel=block_max_elems(nq, ng))
+    _buffer("mutual_verify", "rb_min_d2", rb_min_d2, torch.float32, dev, min_numel=(nq + 31) // 32)
+    _buffer("mutual_verify", "beaten", beaten, torch.uint8, dev, numel=ng)
+    with torch.cuda.device(dev):
+        _lib.check(lib.hn_mutual_verify(_ptr(q), nq, q_offset, _ptr(g), ng, _ptr(claim), _ptr(block_max),
                                         _ptr(rb_min_d2), _ptr(beaten), _stream_ptr()), "hn_mutual_verify")

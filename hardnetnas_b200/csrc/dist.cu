@@ -1218,6 +1218,8 @@ static int check_match(const char* fn, int desc_dtype, const void* q, const void
                        const void* workspace) {
   HN_TRY(check_rows(fn, desc_dtype, q, g));
   HN_REQUIRE(Nq >= 1 && Ng >= 1, "%s: empty input (Nq=%lld, Ng=%lld)", fn, Nq, Ng);
+  // a negative offset would make indices that collide with the -1 "no neighbour" fill
+  HN_REQUIRE(g_offset >= 0, "%s: g_offset must be >= 0 (got %lld)", fn, g_offset);
   HN_REQUIRE(Nq < (1LL << 31) && Ng + g_offset < (1LL << 31), "%s: more than 2^31 rows", fn);
   HN_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "%s: workspace must be 256-byte aligned", fn);
   return HN_OK;
@@ -1265,6 +1267,8 @@ extern "C" long long hn_block_max_elems(long long Nq, long long Ng) {
 extern "C" int hn_mutual_claims(const int32_t* i1, const float* d1, const float* d2, long long Nq, long long q_offset,
                                 unsigned long long* claim, long long Ng, float* rb_min_d2, void* stream) {
   HN_REQUIRE(i1 && d1 && d2 && claim && rb_min_d2, "hn_mutual_claims: NULL argument");
+  // claims hold the global row as an unsigned 32-bit id: a negative offset would wrap to huge ids
+  HN_REQUIRE(q_offset >= 0, "hn_mutual_claims: q_offset must be >= 0 (got %lld)", q_offset);
   HN_REQUIRE(Nq >= 1 && Ng >= 1 && Nq + q_offset < (1LL << 32), "hn_mutual_claims: size out of range");
   mutual_claim_kernel<<<static_cast<unsigned>((Nq + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(i1, d1, d2, Nq, q_offset, claim, Ng, rb_min_d2);
   HN_CUDA(cudaGetLastError());
@@ -1290,6 +1294,7 @@ extern "C" int hn_mutual_verify(const float* q, long long Nq, long long q_offset
                                 const unsigned long long* claim, const float* block_max, const float* rb_min_d2,
                                 unsigned char* beaten, void* stream) {
   HN_REQUIRE(q && g && claim && block_max && rb_min_d2 && beaten, "hn_mutual_verify: NULL argument");
+  HN_REQUIRE(q_offset >= 0, "hn_mutual_verify: q_offset must be >= 0 (got %lld)", q_offset);
   HN_REQUIRE(Nq >= 1 && Ng >= 1 && Nq + q_offset < (1LL << 32), "hn_mutual_verify: size out of range");
   return launch_verify(q, Nq, q_offset, g, Ng, claim, block_max, rb_min_d2, beaten, static_cast<cudaStream_t>(stream));
 }

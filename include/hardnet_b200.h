@@ -159,6 +159,7 @@ int hn_loss_hardnet(const float* anchor, const float* positive, long long N, flo
 /* Brute-force matching in the FDLNet distance form: for every query row the nearest and second nearest
  * gallery rows (D.min(dim=-1) of eval_utils.py:113-114 and sorted[:,0:2] of :168-175).
  * q:[Nq,128], g:[Ng,128] fp32. Outputs: d1[Nq], d2[Nq] distances, i1[Nq] gallery index (+g_offset).
+ * Requires g_offset >= 0 and Ng + g_offset < 2^31. A missing second neighbour (Ng == 1) is i2 = -1 whatever the offset.
  * Precondition: L2-normalised rows (|x| <= 1 up to rounding), the only input the FDLNet distance form is defined for
  * (math_utils.py:15-18 clamps 2 - 2ab to [1e-8, 4]): the exactness guarantee of the shortlist + fp32 re-rank rests on the
  * 2^-10 error bound of the fp16-operand dot product of unit vectors, and |x| >= 256 would overflow the packed operands. */
@@ -205,7 +206,8 @@ int hn_match_mutual(const float* q, const float* g, const void* q16, const void*
 /* The column-side steps on their own, for the sharded form (each rank holds a block of query rows starting at global row
  * q_offset and the whole gallery): claims of the local rows into `claim` [Ng] (initialised to INT64_MAX = unclaimed;
  * all_reduce(MIN) as int64 across ranks afterwards), then verification of the GLOBAL claims against the local rows with the block maxima of the
- * local hn_match_ex call into `beaten` [Ng] (initialised to 0; all_reduce(MAX) afterwards). */
+ * local hn_match_ex call into `beaten` [Ng] (initialised to 0; all_reduce(MAX) afterwards). Both require q_offset >= 0 and
+ * Nq + q_offset < 2^32: the claims hold the global row as an unsigned 32-bit id, so the largest row id is 2^32 - 2. */
 long long hn_block_max_elems(long long Nq, long long Ng);
 int hn_mutual_claims(const int32_t* i1, const float* d1, const float* d2, long long Nq, long long q_offset,
                      unsigned long long* claim, long long Ng, float* rb_min_d2 /*[ceil(Nq/32)] out*/, void* stream);
