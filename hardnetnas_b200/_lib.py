@@ -69,6 +69,16 @@ SIGNATURES = {
     "hn_match_pairs_topk_workspace_bytes": (C.c_longlong, [C.c_longlong, C.c_longlong, C.c_longlong]),
     "hn_match_pairs_topk_typed": (C.c_int, [_P, _P, C.c_longlong, _P, _P, C.c_longlong, C.c_int, _P, C.c_longlong, C.c_longlong,
                                             C.c_longlong, C.c_int, _P, _P, _P, C.c_longlong, _P]),
+    "hn_match_radius_workspace_bytes": (C.c_longlong, [C.c_longlong, C.c_longlong]),
+    "hn_match_radius_count_typed": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_longlong, C.c_longlong, C.c_float, _P, _P, C.c_longlong,
+                                              _P]),
+    "hn_match_radius_fill_typed": (C.c_int, [_P, _P, C.c_int, C.c_longlong, C.c_longlong, C.c_float, _P, C.c_longlong, _P, _P, _P,
+                                             C.c_longlong, _P]),
+    "hn_match_pairs_radius_workspace_bytes": (C.c_longlong, [C.c_longlong, C.c_longlong, C.c_longlong]),
+    "hn_match_pairs_radius_count_typed": (C.c_int, [_P, _P, C.c_longlong, _P, _P, C.c_longlong, C.c_int, _P, C.c_longlong, C.c_longlong,
+                                                    C.c_longlong, C.c_float, _P, _P, C.c_longlong, _P]),
+    "hn_match_pairs_radius_fill_typed": (C.c_int, [_P, _P, C.c_longlong, _P, _P, C.c_longlong, C.c_int, _P, C.c_longlong, C.c_longlong,
+                                                   C.c_longlong, C.c_float, _P, C.c_longlong, _P, _P, _P, C.c_longlong, _P]),
     "hn_match_topk_fallback_enable": (C.c_int, [C.c_int]),
     "hn_match_topk_fallback_read": (C.c_int, [C.POINTER(C.c_longlong)]),
     "hn_match_profile_enable": (C.c_int, [C.c_int]),

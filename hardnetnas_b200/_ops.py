@@ -2,6 +2,7 @@
 from __future__ import annotations
 
 import ctypes as C
+import numbers
 
 import torch
 
@@ -336,6 +337,82 @@ def match_pairs_topk(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, k: i
                                                  _ptr(dist), _ptr(idx), _ptr(ws), ws.numel(), _stream_ptr()),
                    "hn_match_pairs_topk_typed")
     return dist, idx
+
+
+def _check_radius(name: str, radius, capacity) -> tuple[float, int | None]:
+    if isinstance(radius, bool) or not isinstance(radius, numbers.Real) or radius != radius:
+        raise ValueError(f"{name}: radius must be a real number, got {radius!r}")
+    if capacity is not None and (isinstance(capacity, bool) or not isinstance(capacity, int) or capacity < 0):
+        raise ValueError(f"{name}: capacity must be None or an integer >= 0, got {capacity!r}")
+    return float(radius), capacity
+
+
+def _radius_csr(dev: torch.device, rows: int, capacity: int | None, count, fill):
+    """Count into row_ptr [rows + 1], then fill col int32 / dist fp32 buffers of `capacity` entries, or, with capacity None, of the
+    counted size (one host read of row_ptr[rows]). count(row_ptr) and fill(row_ptr, capacity, col, dist) launch the two phases."""
+    with torch.cuda.device(dev):
+        row_ptr = torch.empty(rows + 1, dtype=torch.int64, device=dev)
+        count(row_ptr)
+        n = int(row_ptr[rows]) if capacity is None else capacity
+        col = torch.empty(n, dtype=torch.int32, device=dev)
+        dist = torch.empty(n, dtype=torch.float32, device=dev)
+        fill(row_ptr, n, col, dist)
+    return row_ptr, col, dist
+
+
+def match_radius(q: torch.Tensor, g: torch.Tensor, radius: float, capacity: int | None = None, q16: torch.Tensor | None = None,
+                 g16: torch.Tensor | None = None):
+    """(row_ptr int64 [Nq + 1], col int32, dist fp32): CSR of every (query, gallery) pair with d < radius, columns ascending per
+    row (hn_match_radius_count_typed + hn_match_radius_fill_typed). Rows and packed operands as in match_topk. capacity=None:
+    exact-size outputs after one host read of the total; capacity=n: buffers of n entries and no host synchronisation, entries at
+    CSR positions >= n are not written (row_ptr[-1] > n tells the output was truncated)."""
+    radius, capacity = _check_radius("match_radius", radius, capacity)
+    lib = _lib.load()
+    q, g, dt = _desc_rows(_require_cuda_desc("match_radius", q), _require_cuda_desc("match_radius", g))
+    nq, ng = q.size(0), g.size(0)
+    for t, n in ((q16, nq), (g16, ng)):
+        if t is not None:
+            _packed("match_radius", t, n, dt)
+    dev = q.device
+    with torch.cuda.device(dev):
+        ws = _workspace(dev, lib.hn_match_radius_workspace_bytes(nq, ng))
+    r = C.c_float(radius)
+
+    def count(row_ptr):
+        _lib.check(lib.hn_match_radius_count_typed(_ptr(q), _ptr(g), dt, _ptr(q16), _ptr(g16), nq, ng, r, _ptr(row_ptr), _ptr(ws),
+                                                   ws.numel(), _stream_ptr()), "hn_match_radius_count_typed")
+
+    def fill(row_ptr, n, col, dist):
+        _lib.check(lib.hn_match_radius_fill_typed(_ptr(q), _ptr(g), dt, nq, ng, r, _ptr(row_ptr), n, _ptr(col), _ptr(dist), _ptr(ws),
+                                                  ws.numel(), _stream_ptr()), "hn_match_radius_fill_typed")
+
+    return _radius_csr(dev, nq, capacity, count, fill)
+
+
+def match_pairs_radius(q: torch.Tensor, g: torch.Tensor, pairs: torch.Tensor, radius: float, max_q: int, max_g: int,
+                       capacity: int | None = None, q16: torch.Tensor | None = None, g16: torch.Tensor | None = None):
+    """(row_ptr int64 [P * max_q + 1], col int32, dist fp32): match_radius over the [P * max_q] padded rows of the pair table
+    (hn_match_pairs_radius_*_typed; arguments as in match_pairs), columns local to the pair's gallery range."""
+    radius, capacity = _check_radius("match_pairs_radius", radius, capacity)
+    lib = _lib.load()
+    q, g, dt, table, q16, g16 = _pair_operands("match_pairs_radius", q, g, pairs, q16, g16)
+    nq, ng, b = q.size(0), g.size(0), table.size(0)
+    dev = q.device
+    with torch.cuda.device(dev):
+        ws = _workspace(dev, max(lib.hn_match_pairs_radius_workspace_bytes(b, max_q, max_g), 1))
+    r = C.c_float(radius)
+
+    def count(row_ptr):
+        _lib.check(lib.hn_match_pairs_radius_count_typed(_ptr(q), _ptr(q16), nq, _ptr(g), _ptr(g16), ng, dt, _ptr(table), b, max_q, max_g,
+                                                         r, _ptr(row_ptr), _ptr(ws), ws.numel(), _stream_ptr()),
+                   "hn_match_pairs_radius_count_typed")
+
+    def fill(row_ptr, n, col, dist):
+        _lib.check(lib.hn_match_pairs_radius_fill_typed(_ptr(q), _ptr(q16), nq, _ptr(g), _ptr(g16), ng, dt, _ptr(table), b, max_q, max_g,
+                                                        r, _ptr(row_ptr), n, _ptr(col), _ptr(dist), _ptr(ws), ws.numel(), _stream_ptr()),
+                   "hn_match_pairs_radius_fill_typed")
+
+    return _radius_csr(dev, b * max_q, capacity, count, fill)
 
 
 def _buffer(name: str, what: str, t, dtype: torch.dtype, device: torch.device, numel: int | None = None,

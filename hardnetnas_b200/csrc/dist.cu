@@ -1,6 +1,7 @@
 // C ABI for the distance / hardest-in-batch / matching path: operand packing, the fused tcgen05
 // distance kernels (tc_dist.cuh), fp32 re-ranking of shortlisted candidates and the small finalisers.
 #include <algorithm>
+#include <cmath>
 #include <type_traits>
 #include <vector>
 
@@ -529,6 +530,218 @@ __global__ void __launch_bounds__(128, kRerankTopkCtasPerSm) rerank_topk_pairs_k
                                       cand_val + row * segments * kTopKC, cand_drop + row * segments, segments, k, margin, lane,
                                       scanned);
   store_topk_row(e, row, k, scanned, dist, idx, fallback_rows, lane);
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// radius matching (hn_match_radius_*, hn_match_pairs_radius_*): every column j with d(i, j) < r, as CSR
+// ------------------------------------------------------------------------------------------------------------
+// The GEMM is the top-k one (kTopKC chunks per list and each list's dropped maximum); the re-rank is rerank_topk_row's
+// selection with a threshold fixed by the radius instead of derived from M_k:
+//   - thr = P(r) / kDotScale - kRerankMargin, with P(r) = 1 - r^2 (1 + 2^-20) / 2 (radius_threshold, on the host);
+//   - every kept chunk whose maximum is >= thr is evaluated, and every list whose dropped maximum is >= thr is evaluated over its
+//     whole column range instead of its kept chunks.
+// Why this is exact. d = sqrtf(min(max(fl(2 - 2p), 1e-8), 4)) with p the re-rank's fp32 dot. sqrtf is correctly rounded and r is
+// an fp32 value, so d < r implies sqrt(x) < r for the clamped x, hence fl(2 - 2p) <= x < r^2; fl(y) >= y (1 - 2^-24) for y > 0
+// gives 2 - 2p < r^2 / (1 - 2^-24), i.e. p > P(r) (the factor 1 + 2^-20 covers 1 / (1 - 2^-24)). The exact dot is within the
+// fp32 summation error (some 1e-6) of p and the approximate dot within eps = 2^-10 of the exact one (the bound of the margins
+// above), so the chunk holding j has an approximate maximum >= P(r) - 2 eps; kRerankMargin is 4 eps, and rounding thr to fp32
+// moves it by less than 2^-7 of the 2^16 scaled units. So a column with d < r lies in a kept chunk at or above thr, or in the
+// dropped part of a list whose dropped maximum reaches thr: it is evaluated, and the result is a brute-force evaluation of every
+// column with this arithmetic, whatever the ties. Each column is evaluated at most once (the chunks of a list are distinct, lists
+// cover disjoint column ranges, a scanned list's kept chunks are skipped), so no entry repeats.
+// Ascending columns without a sort: the lists are walked in segment order (segment ranges ascend), a scanned list over its
+// range, a kept list's taken chunks in ascending id order (one __reduce_min_sync each); inside a chunk the hits are placed with
+// one ballot. The count and the fill run the same selection on the same lists, so the fill writes exactly the counted entries.
+// Kept apart from rerank_topk_row rather than sharing its selection: the top-k kernels keep their instructions.
+template <bool FILL, typename T>
+__device__ __forceinline__ int rerank_radius_row(const float* sqw, const T* g, long long ng, const int* crow, const float* cvrow,
+                                                 const float* drow, int segments, float thr, float radius, int lane, bool& scanned,
+                                                 long long base, long long capacity, int* col, float* dist) {
+  const float inf = __int_as_float(0x7f800000);
+  const int slots = segments * kTopKC;
+  // slot c = lane + 32 j (list c / kTopKC) is held by this lane; bit j of tk: a kept chunk at or above the threshold
+  int cid[4];
+  unsigned tk = 0;
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const int c = lane + 32 * j;
+    cid[j] = c < slots ? crow[c] : -1;
+    if (cid[j] >= 0 && cvrow[c] >= thr) tk |= 1u << j;
+  }
+  const float dl = lane < segments ? drow[lane] : -inf;
+  const unsigned scan = __ballot_sync(0xffffffffu, dl > -inf && dl >= thr);
+  scanned = scan != 0;
+
+  int n = 0;   // entries of the row so far
+  const float4 qv = reinterpret_cast<const float4*>(sqw)[lane];
+  auto eval_chunk = [&](long long chunk) {
+    const long long col0 = chunk * kChunk, left = ng - col0;   // column col0 + r exists iff r < left
+    const float mine = chunk_distance(qv, g, col0, left, lane);   // lane r < kChunk: column col0 + r
+    const bool hit = lane < kChunk && lane < left && mine < radius;
+    const unsigned hits = __ballot_sync(0xffffffffu, hit);
+    if (FILL && hit) {
+      const long long pos = base + n + __popc(hits & ((1u << lane) - 1u));
+      if (pos < capacity) {
+        col[pos] = static_cast<int>(col0) + lane;   // ng < 2^31
+        if (dist) dist[pos] = mine;
+      }
+    }
+    n += __popc(hits);
+  };
+  // One walk, so that eval_chunk has one call site: list l = 0, 1, ... either as its range [c, c1) or as its taken chunks, which
+  // the lanes of slots l * kTopKC ... (lanes 8 (l % 4) ... of j = l / 4) offer in `offer` and the warp takes smallest first.
+  const long long tiles = (ng + kDistTile - 1) / kDistTile, chunks = (ng + kChunk - 1) / kChunk;
+  constexpr int kNone = 0x7fffffff;
+  int l = 0, offer = kNone;
+  long long c = 0, c1 = 0;
+  for (;;) {
+    long long chunk;
+    if (c < c1) {
+      chunk = c++;
+    } else {
+      const int m = __reduce_min_sync(0xffffffffu, offer);
+      if (m != kNone) {
+        chunk = m;
+        if (offer == m) offer = kNone;
+      } else if (l < segments) {
+        if ((scan >> l) & 1u) {
+          c = tiles * l / segments * (kDistTile / kChunk);
+          c1 = std::min(tiles * (l + 1) / segments * (kDistTile / kChunk), chunks);
+        } else {
+          const int j = l >> 2;
+          const int held = j == 0 ? cid[0] : j == 1 ? cid[1] : j == 2 ? cid[2] : cid[3];
+          offer = (lane >> 3) == (l & 3) && ((tk >> j) & 1u) ? held : kNone;
+        }
+        ++l;
+        continue;
+      } else {
+        break;
+      }
+    }
+    eval_chunk(chunk);
+  }
+  return n;
+}
+
+// Count (FILL = false) or fill of hn_match_radius_* (TABLE = false: `rows` query rows of q against ng_pad gallery rows of g_all)
+// and hn_match_pairs_radius_* (TABLE: pair b = row / nq_pad, ranges from the table as rerank_topk_pairs_kernel). Lists
+// [rows][segments][kTopKC], dropped maxima [rows][segments]. The count writes row i's number of entries to row_ptr[i + 1] (rows
+// past q_len: 0); the fill writes row i's entries from position row_ptr[i] on, those below `capacity`.
+template <bool TABLE, bool FILL, typename T>
+__global__ void __launch_bounds__(128, kRerankTopkCtasPerSm) rerank_radius_kernel(
+    const T* __restrict__ q, const T* __restrict__ g_all, const int* __restrict__ cand, const float* __restrict__ cand_val,
+    const float* __restrict__ cand_drop, float thr, float radius, long long rows, long long nq_pad, long long ng_pad,
+    const int* __restrict__ pairs, long long q_rows, long long g_rows, int segments, long long* __restrict__ row_ptr,
+    long long capacity, int* __restrict__ col, float* __restrict__ dist, unsigned long long* fallback_rows) {
+  __shared__ __align__(16) float sq[4][128];
+  const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long row = static_cast<long long>(blockIdx.x) * 4 + w;
+  if (row >= rows) return;
+  long long base = 0;
+  if constexpr (FILL) {
+    base = row_ptr[row];
+    if (row_ptr[row + 1] == base || base >= capacity) return;   // nothing of this row to write
+  } else {
+    if (row == 0 && lane == 0) row_ptr[0] = 0;
+  }
+  const T* qrow = q + row * 128;
+  const T* g = g_all;
+  long long ng = ng_pad;
+  if constexpr (TABLE) {
+    const int b = static_cast<int>(row) / static_cast<int>(nq_pad);   // B * nq_pad < 2^31
+    const Span qs = table_span(pairs, b, 0, nq_pad, q_rows), gs = table_span(pairs, b, 1, ng_pad, g_rows);
+    if (row - b * nq_pad >= qs.len || gs.len == 0) {
+      if (!FILL && lane == 0) row_ptr[row + 1] = 0;
+      return;
+    }
+    qrow = q + (qs.start + (row - b * nq_pad)) * 128;
+    g = g_all + gs.start * 128;
+    ng = gs.len;
+  }
+  reinterpret_cast<float4*>(sq[w])[lane] = ld_row4(qrow, lane);
+  __syncwarp();
+  bool scanned = false;
+  const int n = rerank_radius_row<FILL>(sq[w], g, ng, cand + row * segments * kTopKC, cand_val + row * segments * kTopKC,
+                                        cand_drop + row * segments, segments, thr, radius, lane, scanned, base, capacity, col, dist);
+  if (!FILL && lane == 0) {
+    row_ptr[row + 1] = n;
+    if (fallback_rows && scanned) atomicAdd(fallback_rows, 1ull);
+  }
+}
+
+// Exclusive scan of the radius counts into row offsets, in place over x = row_ptr + 1 ([n] counts -> [n] inclusive sums): tile
+// sums, an exclusive scan of the tile sums in one block, then each tile's inclusive scan plus its offset. A thread owns kScanItems
+// consecutive elements of a kScanTile-element tile.
+constexpr int kScanThreads = 1024, kScanItems = 8, kScanTile = kScanThreads * kScanItems;
+
+// Inclusive scan of v over the block (kScanThreads threads); *total receives the block's sum. s: 32 words of shared memory.
+__device__ __forceinline__ long long block_inclusive_scan(long long v, long long* s, long long* total) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const long long t = __shfl_up_sync(0xffffffffu, v, o);
+    if (lane >= o) v += t;
+  }
+  if (lane == 31) s[w] = v;
+  __syncthreads();
+  if (w == 0) {
+    long long x = s[lane];
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const long long t = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= o) x += t;
+    }
+    s[lane] = x;
+  }
+  __syncthreads();
+  if (w > 0) v += s[w - 1];
+  *total = s[31];
+  __syncthreads();   // s is reused by the caller's next scan
+  return v;
+}
+
+__global__ void __launch_bounds__(kScanThreads) scan_tile_sum_kernel(const long long* __restrict__ x, long long n,
+                                                                     long long* __restrict__ tile_sum) {
+  __shared__ long long s[32];
+  const long long i0 = static_cast<long long>(blockIdx.x) * kScanTile + threadIdx.x * kScanItems;
+  long long v = 0;
+#pragma unroll
+  for (int k = 0; k < kScanItems; ++k) v += i0 + k < n ? x[i0 + k] : 0;
+  long long total;
+  block_inclusive_scan(v, s, &total);
+  if (threadIdx.x == 0) tile_sum[blockIdx.x] = total;
+}
+
+__global__ void __launch_bounds__(kScanThreads) scan_tile_offsets_kernel(long long* __restrict__ tile_sum, long long tiles) {
+  __shared__ long long s[32];
+  long long carry = 0;
+  for (long long t0 = 0; t0 < tiles; t0 += kScanThreads) {
+    const long long t = t0 + threadIdx.x;
+    const long long v = t < tiles ? tile_sum[t] : 0;
+    long long total;
+    const long long incl = block_inclusive_scan(v, s, &total);
+    if (t < tiles) tile_sum[t] = carry + incl - v;
+    carry += total;
+  }
+}
+
+__global__ void __launch_bounds__(kScanThreads) scan_tile_apply_kernel(long long* __restrict__ x, long long n,
+                                                                       const long long* __restrict__ tile_off) {
+  __shared__ long long s[32];
+  const long long i0 = static_cast<long long>(blockIdx.x) * kScanTile + threadIdx.x * kScanItems;
+  long long v[kScanItems], sum = 0;
+#pragma unroll
+  for (int k = 0; k < kScanItems; ++k) {
+    v[k] = i0 + k < n ? x[i0 + k] : 0;
+    sum += v[k];
+  }
+  long long total;
+  long long run = block_inclusive_scan(sum, s, &total) - sum + tile_off[blockIdx.x];
+#pragma unroll
+  for (int k = 0; k < kScanItems; ++k) {
+    run += v[k];
+    if (i0 + k < n) x[i0 + k] = run;
+  }
 }
 
 // Process-wide count of top-k rows that scanned a list (hn_match_topk_fallback_*): off by default (nullptr), else a device word
@@ -1560,11 +1773,12 @@ extern "C" long long hn_match_pairs_topk_workspace_bytes(long long B, long long 
   return static_cast<long long>(carve_batched(nullptr, B, max_q, max_g, false, false, kTopKC).bytes);
 }
 
-// The launch sequence of hn_match_topk_typed on validated arguments: the single-CTA GEMM with top-kTopKC lists over (up to)
-// kMaxBatchedSegments segments, so that a list spans at most 1/16 of the gallery (the bound on a fallback scan), then the re-rank.
+// Stages 0 and 1 of hn_match_topk_typed and hn_match_radius_count_typed on validated arguments: packing, then the single-CTA
+// GEMM with top-kTopKC lists over batched_max_segments(Ng) (up to kMaxBatchedSegments) segments, so that a list spans at most
+// 1/16 of the gallery (the bound on a fallback scan).
 template <typename T>
-static int run_match_topk(const T* q, const T* g, const void* q16_in, const void* g16_in, long long Nq, long long Ng, int k, float* dist,
-                          int32_t* idx, const MatchWs& w, cudaStream_t s) {
+static int run_topk_lists(const T* q, const T* g, const void* q16_in, const void* g16_in, long long Nq, long long Ng, const MatchWs& w,
+                          cudaStream_t s) {
   int sm = 0;
   HN_TRY(device_sm_count(&sm));
   constexpr bool F8 = kF8Rows<T>;
@@ -1574,17 +1788,23 @@ static int run_match_topk(const T* q, const T* g, const void* q16_in, const void
   HN_TRY(make_operand_map(&dp.side[0].tmA, q16_in ? q16_in : w.q16, F8, 128, Nq, 0, kDistTile));
   HN_TRY(make_operand_map(&dp.side[0].tmB, g16_in ? g16_in : w.g16, F8, 128, Ng, 0, kDistTile));
   dp.segments = static_cast<int>(batched_max_segments(Ng));
-  {
-    MatchTimer timer(1, s);
-    const long long items = ((Nq + 2 * kDistTile - 1) / (2 * kDistTile)) * dp.segments;
-    HN_TRY((launch_dist<2, EPI_SHORTLIST, F8, kTopKC>(dp, static_cast<int>(std::min<long long>(items, sm)), 1, s)));
-  }
+  MatchTimer timer(1, s);
+  const long long items = ((Nq + 2 * kDistTile - 1) / (2 * kDistTile)) * dp.segments;
+  return launch_dist<2, EPI_SHORTLIST, F8, kTopKC>(dp, static_cast<int>(std::min<long long>(items, sm)), 1, s);
+}
+
+// The launch sequence of hn_match_topk_typed on validated arguments: the top-k lists, then the re-rank.
+template <typename T>
+static int run_match_topk(const T* q, const T* g, const void* q16_in, const void* g16_in, long long Nq, long long Ng, int k, float* dist,
+                          int32_t* idx, const MatchWs& w, cudaStream_t s) {
+  HN_TRY(run_topk_lists(q, g, q16_in, g16_in, Nq, Ng, w, s));
+  const int segments = static_cast<int>(batched_max_segments(Ng));
   unsigned long long* fallback_rows = nullptr;
   HN_TRY(topk_fallback_counter(&fallback_rows));
   {
     MatchTimer timer(2, s);
     rerank_topk_kernel<T><<<static_cast<unsigned>((Nq + 3) / 4), 128, 0, s>>>(q, g, w.cand, w.cand_val, w.cand_drop, kRerankMargin, Nq,
-                                                                                Ng, dp.segments, k, dist, idx, fallback_rows);
+                                                                                Ng, segments, k, dist, idx, fallback_rows);
     HN_CUDA(cudaGetLastError());
     count_launch();
   }
@@ -1608,29 +1828,33 @@ extern "C" int hn_match_topk_typed(const void* q, const void* g, int desc_dtype,
   });
 }
 
-// The launch sequence of hn_match_pairs_topk_typed on validated arguments: the pair-table GEMM with top-kTopKC lists over
-// (up to) kMaxBatchedSegments segments of each pair's gallery, then the re-rank.
-template <typename T>
-static int run_pairs_topk(const T* q, const void* q16, const T* g, const void* g16, const PairLayout& L, int k, float* dist, int32_t* idx,
-                          const MatchWs& w, cudaStream_t s) {
-  constexpr bool F8 = kF8Rows<T>;
+// Stage 1 of hn_match_pairs_topk_typed and hn_match_pairs_radius_count_typed on validated arguments: the pair-table GEMM with
+// top-kTopKC lists over batched_max_segments(max_g) (up to kMaxBatchedSegments) segments of each pair's gallery.
+template <bool F8>
+static int run_pairs_topk_lists(const void* q16, const void* g16, const PairLayout& L, const MatchWs& w, cudaStream_t s) {
   int sm = 0;
   HN_TRY(device_sm_count(&sm));
   DistParams dp;
   HN_TRY(pairs_params(F8, true, q16, g16, L, w, &dp));
   dp.segments = static_cast<int>(batched_max_segments(L.max_g));
-  {
-    MatchTimer timer(1, s);
-    const long long m_blocks = (L.max_q + 2 * kDistTile - 1) / (2 * kDistTile);
-    const int grid = static_cast<int>(std::min<long long>(L.B * m_blocks * dp.segments, sm));
-    HN_TRY((launch_dist<2, EPI_SHORTLIST_PAIRS, F8, kTopKC>(dp, grid, 1, s)));
-  }
+  MatchTimer timer(1, s);
+  const long long m_blocks = (L.max_q + 2 * kDistTile - 1) / (2 * kDistTile);
+  const int grid = static_cast<int>(std::min<long long>(L.B * m_blocks * dp.segments, sm));
+  return launch_dist<2, EPI_SHORTLIST_PAIRS, F8, kTopKC>(dp, grid, 1, s);
+}
+
+// The launch sequence of hn_match_pairs_topk_typed on validated arguments: the top-k lists, then the re-rank.
+template <typename T>
+static int run_pairs_topk(const T* q, const void* q16, const T* g, const void* g16, const PairLayout& L, int k, float* dist, int32_t* idx,
+                          const MatchWs& w, cudaStream_t s) {
+  HN_TRY(run_pairs_topk_lists<kF8Rows<T>>(q16, g16, L, w, s));
+  const int segments = static_cast<int>(batched_max_segments(L.max_g));
   unsigned long long* fallback_rows = nullptr;
   HN_TRY(topk_fallback_counter(&fallback_rows));
   {
     MatchTimer timer(2, s);
     rerank_topk_pairs_kernel<T><<<static_cast<unsigned>((L.B * L.max_q + 3) / 4), 128, 0, s>>>(
-        q, g, w.cand, w.cand_val, w.cand_drop, kRerankMargin, L.B, L.max_q, L.max_g, L.pairs, L.q_rows, L.g_rows, dp.segments, k, dist,
+        q, g, w.cand, w.cand_val, w.cand_drop, kRerankMargin, L.B, L.max_q, L.max_g, L.pairs, L.q_rows, L.g_rows, segments, k, dist,
         idx, fallback_rows);
     HN_CUDA(cudaGetLastError());
     count_launch();
@@ -1655,6 +1879,149 @@ extern "C" int hn_match_pairs_topk_typed(const void* q, const void* q16, long lo
     return run_pairs_topk(static_cast<const T*>(q), q16, static_cast<const T*>(g), g16, L, k, dist, idx, w,
                           static_cast<cudaStream_t>(stream));
   });
+}
+
+// ---- radius matching -----------------------------------------------------------------------------------------------------
+
+// The re-rank threshold of radius r in the GEMM's scaled dot units (see rerank_radius_row): -inf when every column is an entry
+// (d <= sqrtf(4) = 2 < r), +inf when none is (d >= sqrtf(1e-8f) >= r; r <= 0 included), else P(r) / kDotScale - kRerankMargin.
+static float radius_threshold(float r) {
+  if (r > 2.0f) return -INFINITY;
+  if (!(r > sqrtf(1e-8f))) return INFINITY;
+  const double p = 1.0 - 0.5 * static_cast<double>(r) * static_cast<double>(r) * (1.0 + 0x1p-20);
+  return static_cast<float>(p / kDotScale) - kRerankMargin;
+}
+
+// Workspace of a radius call: the top-k layout m (carve_match / carve_batched with kTopKC), then the scan's tile sums.
+struct RadiusWs {
+  MatchWs m;
+  long long* tile_sum;
+  size_t bytes;
+};
+static RadiusWs carve_radius(void* ws, const MatchWs& m, long long rows) {
+  RadiusWs w{m, ws ? reinterpret_cast<long long*>(static_cast<char*>(ws) + m.bytes) : nullptr, 0};
+  w.bytes = m.bytes + align256(static_cast<size_t>((rows + kScanTile - 1) / kScanTile) * 8);
+  return w;
+}
+
+extern "C" long long hn_match_radius_workspace_bytes(long long Nq, long long Ng) {
+  if (Nq < 0 || Ng < 0) return 0;
+  return static_cast<long long>(carve_radius(nullptr, carve_match(nullptr, Nq, Ng, false, kTopKC), Nq).bytes);
+}
+
+extern "C" long long hn_match_pairs_radius_workspace_bytes(long long B, long long max_q, long long max_g) {
+  if (B < 0 || max_q < 0 || max_g < 0) return 0;
+  return static_cast<long long>(carve_radius(nullptr, carve_batched(nullptr, B, max_q, max_g, false, false, kTopKC), B * max_q).bytes);
+}
+
+// Argument checks shared by the four radius entry points (the count passes capacity 0 and no col / dist).
+static int check_radius(const char* fn, float radius, const long long* row_ptr, long long capacity, const int32_t* col, const float* dist) {
+  HN_REQUIRE(!std::isnan(radius), "%s: radius is NaN", fn);
+  HN_REQUIRE(capacity >= 0, "%s: capacity must be >= 0 (got %lld)", fn, capacity);
+  HN_REQUIRE(col || capacity == 0, "%s: col is NULL with capacity %lld > 0", fn, capacity);
+  HN_REQUIRE((reinterpret_cast<uintptr_t>(row_ptr) & 7) == 0, "%s: row_ptr must be 8-byte aligned", fn);
+  HN_REQUIRE(((reinterpret_cast<uintptr_t>(col) | reinterpret_cast<uintptr_t>(dist)) & 3) == 0, "%s: col and dist must be 4-byte aligned",
+             fn);
+  return HN_OK;
+}
+
+// The count or fill re-rank of a radius call (stage 2) over `rows` rows; the count also turns the counts into row offsets.
+template <bool TABLE, bool FILL, typename T>
+static int launch_radius(const T* q, const T* g, const RadiusWs& w, float radius, long long rows, long long nq_pad, long long ng_pad,
+                         const PairLayout* L, int segments, long long* row_ptr, long long capacity, int32_t* col, float* dist,
+                         cudaStream_t s) {
+  unsigned long long* fallback_rows = nullptr;
+  if (!FILL) HN_TRY(topk_fallback_counter(&fallback_rows));
+  MatchTimer timer(2, s);
+  rerank_radius_kernel<TABLE, FILL, T><<<static_cast<unsigned>((rows + 3) / 4), 128, 0, s>>>(
+      q, g, w.m.cand, w.m.cand_val, w.m.cand_drop, radius_threshold(radius), radius, rows, nq_pad, ng_pad, L ? L->pairs : nullptr,
+      L ? L->q_rows : 0, L ? L->g_rows : 0, segments, row_ptr, capacity, col, dist, fallback_rows);
+  HN_CUDA(cudaGetLastError());
+  count_launch();
+  if (!FILL) {
+    const unsigned tiles = static_cast<unsigned>((rows + kScanTile - 1) / kScanTile);
+    scan_tile_sum_kernel<<<tiles, kScanThreads, 0, s>>>(row_ptr + 1, rows, w.tile_sum);
+    scan_tile_offsets_kernel<<<1, kScanThreads, 0, s>>>(w.tile_sum, tiles);
+    scan_tile_apply_kernel<<<tiles, kScanThreads, 0, s>>>(row_ptr + 1, rows, w.tile_sum);
+    HN_CUDA(cudaGetLastError());
+    count_launch(3);
+  }
+  return HN_OK;
+}
+
+// hn_match_radius_count_typed (FILL = false: q16 / g16 may be given) and hn_match_radius_fill_typed.
+template <bool FILL>
+static int radius_entry(const char* fn, const void* q, const void* g, int desc_dtype, const void* q16, const void* g16, long long Nq,
+                        long long Ng, float radius, long long* row_ptr, long long capacity, int32_t* col, float* dist, void* workspace,
+                        long long workspace_bytes, void* stream) {
+  HN_REQUIRE(q && g && row_ptr && workspace, "%s: NULL argument (q, g, row_ptr and workspace are required)", fn);
+  HN_TRY(check_radius(fn, radius, row_ptr, capacity, col, dist));
+  HN_TRY(check_match(fn, desc_dtype, q, g, Nq, Ng, 0, workspace));
+  HN_REQUIRE(workspace_bytes >= hn_match_radius_workspace_bytes(Nq, Ng), "%s: workspace too small", fn);
+  HN_REQUIRE((reinterpret_cast<uintptr_t>(q16) & 15) == 0 && (reinterpret_cast<uintptr_t>(g16) & 15) == 0,
+             "%s: packed operands must be 16-byte aligned", fn);
+  const RadiusWs w = carve_radius(workspace, carve_match(workspace, Nq, Ng, false, kTopKC), Nq);
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int segments = static_cast<int>(batched_max_segments(Ng));
+  return with_rows(desc_dtype, [&](auto t) -> int {
+    using T = decltype(t);
+    const T *qt = static_cast<const T*>(q), *gt = static_cast<const T*>(g);
+    if (!FILL) HN_TRY(run_topk_lists(qt, gt, q16, g16, Nq, Ng, w.m, s));
+    return launch_radius<false, FILL>(qt, gt, w, radius, Nq, Nq, Ng, nullptr, segments, row_ptr, capacity, col, dist, s);
+  });
+}
+
+extern "C" int hn_match_radius_count_typed(const void* q, const void* g, int desc_dtype, const void* q16, const void* g16, long long Nq,
+                                           long long Ng, float radius, long long* row_ptr, void* workspace, long long workspace_bytes,
+                                           void* stream) {
+  return radius_entry<false>("hn_match_radius_count_typed", q, g, desc_dtype, q16, g16, Nq, Ng, radius, row_ptr, 0, nullptr, nullptr,
+                             workspace, workspace_bytes, stream);
+}
+
+extern "C" int hn_match_radius_fill_typed(const void* q, const void* g, int desc_dtype, long long Nq, long long Ng, float radius,
+                                          const long long* row_ptr, long long capacity, int32_t* col, float* dist, void* workspace,
+                                          long long workspace_bytes, void* stream) {
+  return radius_entry<true>("hn_match_radius_fill_typed", q, g, desc_dtype, nullptr, nullptr, Nq, Ng, radius,
+                            const_cast<long long*>(row_ptr), capacity, col, dist, workspace, workspace_bytes, stream);
+}
+
+// hn_match_pairs_radius_count_typed and hn_match_pairs_radius_fill_typed.
+template <bool FILL>
+static int pairs_radius_entry(const char* fn, const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16,
+                              long long Ng_rows, int desc_dtype, const int32_t* pairs, long long B, long long max_q, long long max_g,
+                              float radius, long long* row_ptr, long long capacity, int32_t* col, float* dist, void* workspace,
+                              long long workspace_bytes, void* stream) {
+  HN_REQUIRE(q && q16 && g && g16 && pairs && row_ptr && workspace,
+             "%s: NULL argument (q, q16, g, g16, pairs, row_ptr and workspace are required)", fn);
+  HN_TRY(check_radius(fn, radius, row_ptr, capacity, col, dist));
+  HN_TRY(check_pairs(fn, desc_dtype, q, q16, Nq_rows, g, g16, Ng_rows, B, max_q, max_g, workspace));
+  HN_REQUIRE(workspace_bytes >= hn_match_pairs_radius_workspace_bytes(B, max_q, max_g), "%s: workspace too small", fn);
+  const RadiusWs w = carve_radius(workspace, carve_batched(workspace, B, max_q, max_g, false, false, kTopKC), B * max_q);
+  const PairLayout L = {pairs, nullptr, nullptr, B, max_q, max_g, Nq_rows, Ng_rows};
+  const cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int segments = static_cast<int>(batched_max_segments(max_g));
+  return with_rows(desc_dtype, [&](auto t) -> int {
+    using T = decltype(t);
+    if (!FILL) HN_TRY(run_pairs_topk_lists<kF8Rows<T>>(q16, g16, L, w.m, s));
+    return launch_radius<true, FILL>(static_cast<const T*>(q), static_cast<const T*>(g), w, radius, B * max_q, max_q, max_g, &L, segments,
+                                     row_ptr, capacity, col, dist, s);
+  });
+}
+
+extern "C" int hn_match_pairs_radius_count_typed(const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16,
+                                                 long long Ng_rows, int desc_dtype, const int32_t* pairs, long long B, long long max_q,
+                                                 long long max_g, float radius, long long* row_ptr, void* workspace,
+                                                 long long workspace_bytes, void* stream) {
+  return pairs_radius_entry<false>("hn_match_pairs_radius_count_typed", q, q16, Nq_rows, g, g16, Ng_rows, desc_dtype, pairs, B, max_q,
+                                   max_g, radius, row_ptr, 0, nullptr, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int hn_match_pairs_radius_fill_typed(const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16,
+                                                long long Ng_rows, int desc_dtype, const int32_t* pairs, long long B, long long max_q,
+                                                long long max_g, float radius, const long long* row_ptr, long long capacity,
+                                                int32_t* col, float* dist, void* workspace, long long workspace_bytes, void* stream) {
+  return pairs_radius_entry<true>("hn_match_pairs_radius_fill_typed", q, q16, Nq_rows, g, g16, Ng_rows, desc_dtype, pairs, B, max_q,
+                                  max_g, radius, const_cast<long long*>(row_ptr), capacity, col, dist, workspace, workspace_bytes, stream);
 }
 
 extern "C" int hn_match_force_kernel(int mode) {

@@ -80,6 +80,25 @@ def match_topk(des1, des2, k):
     return d, i.long()
 
 
+def match_radius(des1, des2, radius, capacity=None):
+    """(row_ptr int64 [Nq + 1], col int64, dist fp32): every pair with d < radius as CSR, exact (hn_match_radius_*_typed) - the
+    entries of `distance_matrix_vector(des1, des2).lt(radius).nonzero()` (math_utils.py:8-19) without the Nq x Ng matrix,
+    columns ascending within a row; (row_ptr, col) feed torch.sparse_csr_tensor as they are. capacity=None: one host read of the
+    total, outputs of exactly that size; capacity=n: no host synchronisation, outputs of n entries, of which the first
+    min(n, row_ptr[-1]) are written. radius is used as an fp32 value."""
+    row_ptr, col, dist = _ops.match_radius(des1, des2, radius, capacity)
+    return row_ptr, col.long(), dist
+
+
+def threshold_matches(des1, des2, des_thrsh):
+    """(pairs [M, 2] int64, dist [M] fp32) with pairs = D.lt(des_thrsh).nonzero() of the reference composition
+    (D = distance_matrix_vector(des1, des2); DES_THRSH, config.py:47), in its row-major order: the threshold strategy of
+    descriptor evaluation, one host synchronisation."""
+    row_ptr, col, dist = match_radius(des1, des2, des_thrsh)
+    rows = torch.repeat_interleave(torch.arange(row_ptr.numel() - 1, device=col.device), row_ptr.diff(), output_size=col.numel())
+    return torch.stack([rows, col], dim=1), dist
+
+
 def mutual_nn_ratio(des1, des2, threshold=0.7, return_pairs=True):
     """Mutual nearest neighbours AND the ratio test of BASELINE config 4 in one call:
     (pairs [M,2] int64 or None, mutual bool[Nq], ratio_label bool[Nq], Ia int64[Nq], Da, Db).
@@ -201,6 +220,16 @@ def match_topk_pairs(des1, des2, pairs, k, max_len1=None, max_len2=None, des1_16
     max_len1, max_len2 = _max_lens(pairs, des1.size(0), des2.size(0), max_len1, max_len2)
     d, i = _ops.match_pairs_topk(des1, des2, pairs, k, max_len1, max_len2, des1_16, des2_16)
     return d, i.long()
+
+
+def match_radius_pairs(des1, des2, pairs, radius, max_len1=None, max_len2=None, capacity=None, des1_16=None, des2_16=None):
+    """match_radius for every row-range pair of the table -> (row_ptr int64 [P * max_len1 + 1], col int64, dist fp32) over the
+    padded rows (row r of pair p at p * max_len1 + r); columns local to the pair's gallery range; rows past len1 and pairs
+    without gallery rows have no entries. With max_len1, max_len2 and capacity given (and the table on the device) the call is
+    free of host synchronisation and CUDA-graph capturable."""
+    max_len1, max_len2 = _max_lens(pairs, des1.size(0), des2.size(0), max_len1, max_len2)
+    row_ptr, col, dist = _ops.match_pairs_radius(des1, des2, pairs, radius, max_len1, max_len2, capacity, des1_16, des2_16)
+    return row_ptr, col.long(), dist
 
 
 # ---- match-score counters (FDLNet-master/utils/eval_utils.py:112-197) -----------------------------------------------

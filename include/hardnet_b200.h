@@ -308,15 +308,55 @@ int hn_match_pairs_topk_typed(const void* q, const void* q16, long long Nq_rows,
                               int desc_dtype, const int32_t* pairs, long long B, long long max_q, long long max_g, int k,
                               float* dist, int32_t* idx, void* workspace, long long workspace_bytes, void* stream);
 
+/* ---- radius matching ------------------------------------------------------------------------------------------------------
+ * Every gallery row closer than `radius` to each query row: the entries of row i are the columns j with d(i, j) < radius
+ * (strict, like D.lt(radius)), d the FDLNet distance in the re-rank's fp32 arithmetic, bit-identical to what hn_match /
+ * hn_match_topk_typed report for the same (row, column). The result is exact: it equals a brute-force fp32 evaluation of every
+ * column with that arithmetic (dist.cu gives the argument). Output is CSR: row_ptr int64 [rows + 1] (row_ptr[0] = 0,
+ * row_ptr[rows] = nnz, up to rows * Ng), col int32 [capacity] and optional dist fp32 [capacity]; within a row the columns
+ * ascend, so the flattened entries are in the row-major order of D.lt(radius).nonzero() and feed torch.sparse_csr_tensor as
+ * they are. radius <= sqrtf(1e-8f) (about 1e-4; the clamp keeps every d at or above it) gives no entries, radius > 2 every
+ * column; all-zero rows are at d = sqrt(2) from every column.
+ * Two phases, as the output size is unknown in advance:
+ *   1. count: packing, the top-k GEMM, a counting re-rank and an exclusive scan into row_ptr;
+ *   2. fill: writes every entry whose CSR position is below `capacity` (nothing at or past it; row_ptr[rows] > capacity means
+ *      the output was truncated). dist may be NULL; col may be NULL when capacity is 0.
+ * The fill reads the candidate lists the count left in the workspace: call it with the same rows, table and radius, on the same
+ * stream, with nothing run on the workspace in between. Neither phase reads anything on the host or allocates, so count + fill
+ * with a known capacity is CUDA-graph capturable (and a captured pair-table graph follows edits of the table).
+ * Rows, dtypes (HN_F32 / HN_F16 / HN_BF16 / HN_F8E4M3, bit for bit the fp32 call on the rows converted to fp32), packed operands
+ * and validation are those of hn_match_topk_typed and hn_match_pairs_topk_typed. Pair tables: rows are the [B * max_q] padded
+ * rows (row r of pair b at b * max_q + r), col is local to the pair's gallery range, rows past q_len and pairs with g_len == 0
+ * have no entries. Also rejected with HN_ERR_INVALID before any device work: a NaN radius, capacity < 0, col == NULL with
+ * capacity > 0, a row_ptr that is not 8-byte aligned, col / dist that are not 4-byte aligned, a workspace (256-byte aligned)
+ * smaller than the *_radius_workspace_bytes function gives. */
+long long hn_match_radius_workspace_bytes(long long Nq, long long Ng);
+int hn_match_radius_count_typed(const void* q, const void* g, int desc_dtype, const void* q16, const void* g16, long long Nq,
+                                long long Ng, float radius, long long* row_ptr, void* workspace, long long workspace_bytes,
+                                void* stream);
+int hn_match_radius_fill_typed(const void* q, const void* g, int desc_dtype, long long Nq, long long Ng, float radius,
+                               const long long* row_ptr, long long capacity, int32_t* col, float* dist, void* workspace,
+                               long long workspace_bytes, void* stream);
+long long hn_match_pairs_radius_workspace_bytes(long long B, long long max_q, long long max_g);
+int hn_match_pairs_radius_count_typed(const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16,
+                                      long long Ng_rows, int desc_dtype, const int32_t* pairs, long long B, long long max_q,
+                                      long long max_g, float radius, long long* row_ptr, void* workspace, long long workspace_bytes,
+                                      void* stream);
+int hn_match_pairs_radius_fill_typed(const void* q, const void* q16, long long Nq_rows, const void* g, const void* g16,
+                                     long long Ng_rows, int desc_dtype, const int32_t* pairs, long long B, long long max_q,
+                                     long long max_g, float radius, const long long* row_ptr, long long capacity, int32_t* col,
+                                     float* dist, void* workspace, long long workspace_bytes, void* stream);
+
 /* Measurement hooks (process-wide): bracket the three stages of every hn_match / hn_match_batched / hn_match_pairs /
- * hn_match_topk_typed / hn_match_pairs_topk_typed call (0 = operand packing, not part of the pair-table calls; 1 = GEMM +
- * shortlist, 2 = exact re-rank) with CUDA events; hn_match_profile_read waits for them, returns the summed milliseconds and
- * launch counts per stage and resets the counters. */
+ * hn_match_topk_typed / hn_match_pairs_topk_typed call and of the radius calls (0 = operand packing, not part of the pair-table
+ * calls; 1 = GEMM + shortlist, the count phase only; 2 = exact re-rank: the count re-rank with its scan, and the fill re-rank)
+ * with CUDA events; hn_match_profile_read waits for them, returns the summed milliseconds and launch counts per stage and
+ * resets the counters. */
 int hn_match_profile_enable(int on);
 int hn_match_profile_read(double ms_out[3], long long launches_out[3]);
-/* Count of the top-k rows whose re-rank scanned a whole candidate list because the list's dropped maximum reached the
- * threshold (process-wide, current device, off by default): enable(1) resets and starts it, enable(0) stops it; read waits for
- * the device, returns the count and resets it. */
+/* Count of the top-k rows, and of the rows of radius count phases, whose re-rank scanned a whole candidate list because the
+ * list's dropped maximum reached the threshold (process-wide, current device, off by default): enable(1) resets and starts it,
+ * enable(0) stops it; read waits for the device, returns the count and resets it. */
 int hn_match_topk_fallback_enable(int on);
 int hn_match_topk_fallback_read(long long* rows_out);
 
